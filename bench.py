@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload reddit|wikipedia|enron|flights]
     python bench.py --impl reference ...        # the CPU oracle port of the reference path
+    python bench.py --dump-outputs DIR ...      # also write the last timed step's outputs to DIR/*.npy (see dump_outputs)
 
 A step is one pass of the module-boundary PE path over one batch of the synthetic edge stream
 (SURVEY §8(d)): DFT filter on the batch nodes (a3), C=4 neighbourhood aggregates (a6: pos src,
@@ -138,22 +139,16 @@ def workload_config(workload, g, B, K, world=1):
             "l2_policy": f"inputs larger than L2: PE history {(g.num_nodes + 1) * T_HIST * D * 4 / 1e6:.0f} MB, a different node set is read each step"}
 
 
-def run_ours(args, rank, world, own_pg=True):
-    """The headline workload on every rank (N > 1: independent replicas, weak scaling — the path does not shard at
-    this size). Returns the result line on rank 0; emits it when it owns the process group."""
+def headline_setup(workload, seed, dev):
+    """The state the headline workload starts from: the seeded synthetic stream of `workload`, the device sampler over it,
+    the drop-in with seeded weights, a PEStream over the evaluation split (the last 30 % of the stream, like val+test; nb
+    full batches, wrapped around when more steps are asked for) and the negatives. `queries(b)`: the four query sets of
+    batch b (the eval loop's calls: positive source, positive destination, negative source, negative destination)."""
+    import types
     import torch
-    import torch.distributed as dist
-    from lstep_b200 import NeighborSampler, PEStream, _lib
-
-    local = int(os.environ.get("LOCAL_RANK", 0))
-    torch.cuda.set_device(local)
-    dev = torch.device("cuda", local)
-    if world > 1 and own_pg:
-        dist.init_process_group("nccl", device_id=dev)
-    lib = _lib.load()
-    assert lib.lstep_device_ok() == 1
-    B, K = WORKLOADS[args.workload]
-    g = synth.make_graph(args.workload, seed=0 + rank, zipf_s=ZIPF_S)  # replicas: each rank its own stream of the same shape
+    from lstep_b200 import NeighborSampler, PEStream
+    B, K = WORKLOADS[workload]
+    g = synth.make_graph(workload, seed=seed, zipf_s=ZIPF_S)
     V1 = g.num_nodes + 1
     t0 = time.time()
     sampler = NeighborSampler.from_edges(g.src_node_ids, g.dst_node_ids, g.edge_ids, g.node_interact_times, "recent", num_rows=V1)
@@ -161,7 +156,6 @@ def run_ours(args, rank, world, own_pg=True):
     t_csr = time.time() - t0
     model = make_params_model(g, sampler, dev)
     init = torch.from_numpy(synth.make_initial_pe(g.num_nodes, D, seed=1)).to(dev)
-    # evaluate on the tail of the stream (last 30 %, like val+test), wrapping around if more steps are asked for
     e0 = int(g.num_edges * 0.7) // B * B
     stream = PEStream(model, g.src_node_ids, g.dst_node_ids, g.node_interact_times, B, K, initial_pe=init, start=e0)
     nb = stream.num_batches
@@ -175,16 +169,42 @@ def run_ours(args, rank, world, own_pg=True):
         lo, hi, _, _ = stream.batch_arrays(b)
         return [stream.src[lo:hi], stream.dst[lo:hi], stream.src[lo:hi], neg_dev[lo - e0:hi - e0]]
 
+    return types.SimpleNamespace(g=g, sampler=sampler, model=model, stream=stream, nb=nb, e0=e0, neg_all=neg_all, neg_dev=neg_dev,
+                                 queries=queries, t_csr=t_csr)
+
+
+def run_ours(args, rank, world, own_pg=True):
+    """The headline workload on every rank (N > 1: independent replicas, weak scaling — the path does not shard at
+    this size). Returns the result line on rank 0; emits it when it owns the process group."""
+    import torch
+    import torch.distributed as dist
+    from lstep_b200 import _lib
+
+    local = int(os.environ.get("LOCAL_RANK", 0))
+    torch.cuda.set_device(local)
+    dev = torch.device("cuda", local)
+    if world > 1 and own_pg:
+        dist.init_process_group("nccl", device_id=dev)
+    lib = _lib.load()
+    assert lib.lstep_device_ok() == 1
+    B, K = WORKLOADS[args.workload]
+    h = headline_setup(args.workload, rank, dev)  # replicas: each rank its own stream of the same shape
+    g, sampler, model, stream, nb, e0, neg_all, neg_dev, queries = (h.g, h.sampler, h.model, h.stream, h.nb, h.e0, h.neg_all,
+                                                                    h.neg_dev, h.queries)
+    V1 = g.num_nodes + 1
+
     def run_steps(first, n):
         """n consecutive steps starting at step number `first` (wrapping over the evaluation split): one native call per
-        contiguous run of batches."""
-        done = 0
+        contiguous run of batches. Returns the neighbourhood PEs of the last step [C, B, d]."""
+        done, last = 0, None
         while done < n:
             b0 = (first + done) % nb
             cnt = min(n - done, nb - b0)
             lo0 = stream.batch_lo[b0]
-            stream.run(b0, cnt, [stream.src[lo0:], stream.dst[lo0:], stream.src[lo0:], neg_dev[lo0 - e0:]])
+            del last  # free the previous call's output before the next call allocates its own
+            last = stream.run(b0, cnt, [stream.src[lo0:], stream.dst[lo0:], stream.src[lo0:], neg_dev[lo0 - e0:]])
             done += cnt
+        return last
 
     outs = torch.empty((C_CALLS, B, D), dtype=torch.float32, device=dev)
     W, Ksteps = args.warmup, args.steps
@@ -217,12 +237,14 @@ def run_ours(args, rank, world, own_pg=True):
     # launches already queued behind it, so the timed region is the device's own chain of kernels at any K
     torch.cuda._sleep(int(1.0e6))
     ev0.record()
-    run_steps(step_no, Ksteps)
+    last_out = run_steps(step_no, Ksteps)
     ev1.record()
     torch.cuda.synchronize()
     step_no += Ksteps
     ms_total = ev0.elapsed_time(ev1)
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, stream, last_out)
     t_max = torch.tensor([ms_total], device=dev)
     edges_t = torch.tensor([float(edges)], device=dev)
     if world > 1:
@@ -267,7 +289,7 @@ def run_ours(args, rank, world, own_pg=True):
     if rank == 0:
         cfg = workload_config(args.workload, g, B, K, world)
         info = {"timed_region": "K steps in one native call (PEStream.run -> lstep_pe_steps) queued behind a spin kernel; CUDA events on the launch stream",
-                "N_mean": N_mean, "M_mean": M_mean, "csr_build_s": t_csr, "history_fill_steps_before_warmup": fill}
+                "N_mean": N_mean, "M_mean": M_mean, "csr_build_s": h.t_csr, "history_fill_steps_before_warmup": fill}
         out = {
             "metric": "temporal edges/sec through PE update+aggregation; % HBM roofline", "value": value, "unit": "edges/s",
             "n_gpus": world, "steps": Ksteps, "warmup": W, "ms_per_step": ms_total_max / Ksteps, "higher_is_better": True,
@@ -297,6 +319,29 @@ def run_ours(args, rank, world, own_pg=True):
     del stream, model, sampler
     torch.cuda.empty_cache()
     return out
+
+
+DUMP_HISTORY_ROWS = 256  # node rows of the PE history in the dump: all T steps of each (the whole history is 756 MB at Reddit size)
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_outputs(path, stream, nbr_pe):
+    """Writes what the timed path computed in its last step, as a caller of PEStream.run receives it, to path/<name>.npy
+    (float32): the step's neighbourhood PEs [C, B, d] (run's return value), the updated PE table [V1, d], and the PE history
+    [rows, T, d] (oldest step first) of a fixed sample of node rows (seed 0). The inputs are seeded, so two builds run with
+    the same arguments can be compared output for output."""
+    import torch
+    rows = np.sort(np.random.default_rng(0).choice(stream.V1, size=min(DUMP_HISTORY_ROWS, stream.V1), replace=False))
+    arrays = {"neighborhood_pe": nbr_pe, "pe_table": stream.cur,
+              "pe_history_sample": stream.export_history()[torch.from_numpy(rows).to(stream.dev)]}
+    arrays = {k: v.float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES} byte budget")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+    log(f"dumped {', '.join(f'{k} {list(a.shape)}' for k, a in arrays.items())} ({total / 1e6:.1f} MB) -> {path}")
 
 
 def run_sharded(args, rank, world, own_pg=True):
@@ -651,8 +696,9 @@ def e2e_pass(stream, g, e0, neg_all, step_no, nb, n, B, world, dev):
 
 # ------------------------------------------------------------------------------------------------
 def oracle_setup(workload, B, K, n_batches, seed=0):
-    """(fallback when oracle/_ref is absent) bounded sample of the workload for the numpy port: the first 15 % of the
-    stream builds the adjacency (python loops dominate beyond that), batches are taken from its tail."""
+    """(fallback when oracle/_ref is absent) bounded sample of the workload for the numpy port: the first
+    max(40 000, 4 x the edges of n_batches + 4 batches) edges of the stream, the whole stream at most, build the adjacency
+    (its python loops dominate the set-up); the timed batches come from the sample's tail (oracle_batch_starts)."""
     from oracle import lstep_oracle as orc
     full = synth.SHAPES[workload]["num_edges"]
     n_edges = min(full, max(40_000, (n_batches + 4) * B * 4))
@@ -663,6 +709,13 @@ def oracle_setup(workload, B, K, n_batches, seed=0):
     rng = np.random.default_rng(1)
     hist = (rng.standard_normal((V1, T_HIST, D)) * 0.1).astype(np.float32)
     return orc, g, adj, p, hist, n_edges
+
+
+def oracle_batch_starts(n_edges, B, n):
+    """Start offsets of the n batches the port times: consecutive full batches that end at the end of the sample, wrapping
+    over its last 30 % when more batches are asked for than that holds."""
+    k = min(n, (n_edges - int(n_edges * 0.7)) // B)
+    return [n_edges - k * B + (i % k) * B for i in range(n)]
 
 
 def oracle_batch(orc, g, adj, p, hist, lo, B, K, neg):
@@ -767,9 +820,7 @@ def cpu_baseline(workload, B, K, n_batches):
                           f"reference sampler build {arm.t_sampler:.1f} s (untimed)"}
     orc, g, adj, p, hist, n_edges = oracle_setup(workload, B, K, n_batches)
     rng = np.random.default_rng(3)
-    start = n_edges - (n_batches + 3) * B
-    for i in range(n_batches + 3):
-        lo = start + i * B
+    for i, lo in enumerate(oracle_batch_starts(n_edges, B, n_batches + 3)):
         neg = rng.choice(g.dst_node_ids, B)
         dt = oracle_batch(orc, g, adj, p, hist, lo, B, K, neg)
         if i >= 3:
@@ -792,7 +843,6 @@ def run_reference(args, rank, world):
         workload, T_HIST = "flights", (args.scaleout_T or T_HIST)
     B, K = WORKLOADS[workload]
     steps, warm = args.steps, max(args.warmup, 1)
-    steps = min(steps, 100)  # each step is one batch of CPU work (~0.1 s at B=200); bounded
     warm = min(warm, 5)
     kind = "reference"
     try:
@@ -802,27 +852,20 @@ def run_reference(args, rank, world):
         arm, kind = None, "port"
     tot, edges = 0.0, 0
     if arm is not None:
-        budget = time.time() + 150.0
-        done = 0
         for i in range(steps + warm):
             dt, ne = arm.batch(i)
             if i >= warm:
                 tot += dt
                 edges += ne
-                done += 1
-            if time.time() > budget and done >= 3:
-                break
-        steps = done
         g = arm.g
         sample = (f"{steps} batches of {B} edges: the unmodified reference (oracle/_ref) on torch CPU, {os.cpu_count()} threads, full "
                   f"{workload}-shaped graph, same weights as the CUDA arm, T={T_HIST}; module-boundary functions only")
     else:
         orc, g, adj, p, hist, n_edges = oracle_setup(workload, B, K, steps + warm)
         rng = np.random.default_rng(3)
-        start = n_edges - (steps + warm) * B
-        for i in range(steps + warm):
+        for i, lo in enumerate(oracle_batch_starts(n_edges, B, steps + warm)):
             neg = rng.choice(g.dst_node_ids, B)
-            dt = oracle_batch(orc, g, adj, p, hist, start + i * B, B, K, neg)
+            dt = oracle_batch(orc, g, adj, p, hist, lo, B, K, neg)
             if i >= warm:
                 tot += dt
                 edges += B
@@ -880,13 +923,19 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--zipf", type=float, default=0.8, help="endpoint skew of the synthetic stream (0.8: the headline workload; 1.2: hub-heavy)")
     ap.add_argument("--cpu-batches", type=int, default=40)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed steps computed in the last one to DIR/<name>.npy (headline workload, rank 0)")
     args = ap.parse_args()
     global ZIPF_S
     ZIPF_S = float(args.zipf)
-    if args.steps is None:
-        args.steps = 1000 if args.workload != "scaleout" else 100
+    if args.steps is None:  # (the reference arm runs its steps on the host CPU: a shorter default)
+        args.steps = 1000 if args.workload != "scaleout" and args.impl != "reference" else 100
     if args.warmup is None:
         args.warmup = 120 if args.workload != "scaleout" else 30
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "scaleout"):
+        ap.error("--dump-outputs writes the outputs of the CUDA path's headline workload (not --impl reference, not --workload scaleout)")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     quiet_stdout()

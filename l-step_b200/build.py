@@ -29,6 +29,19 @@ def _nvcc() -> str:
     raise RuntimeError("nvcc not found; the lstep_b200 CUDA library cannot be built")
 
 
+def cuobjdump() -> str:
+    """The cuobjdump of the toolkit whose nvcc builds the library (CUDA's bin directory need not be on PATH), else the one
+    on PATH."""
+    nvcc = _nvcc()
+    for cand in (os.path.join(os.path.dirname(d), "cuobjdump") for d in (nvcc, os.path.realpath(nvcc))):
+        if os.path.exists(cand):
+            return cand
+    found = shutil.which("cuobjdump")
+    if found is None:
+        raise RuntimeError(f"cuobjdump not found next to {nvcc} or on PATH")
+    return found
+
+
 def _digest() -> str:
     """Content hash of the sources and flags. File NAMES enter relative to the repo (the snapshot on the GPU box lives
     under another path; an absolute path here would force a rebuild there, by every rank at once)."""

@@ -41,6 +41,6 @@ def test_status_strings_and_sizes():
 def test_sass_is_sm100a_only():
     """The library carries sm_100a code and nothing else (no multi-arch fatbin)."""
     import subprocess
-    out = subprocess.run(["cuobjdump", "-lelf", build.LIB], capture_output=True, text=True).stdout
+    out = subprocess.run([build.cuobjdump(), "-lelf", build.LIB], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs

@@ -136,6 +136,35 @@ def test_header_cites_the_reference_interface_it_replaces():
     assert len(re.findall(r"(?:LSTEP|utils|modules|evaluate_model_utils)\.py:\d+", text)) >= 10
 
 
+@pytest.mark.parametrize("args", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"],
+                                  ["--workload", "scaleout", "--dump-outputs", "out"]])
+def test_bench_rejects_arguments_it_cannot_honour(args, tmp_path):
+    """bench.py refuses, before any work, a run with no timed step and an output dump of a path it does not dump."""
+    import subprocess
+    import sys
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args, capture_output=True, text=True, timeout=120,
+                         cwd=tmp_path)
+    assert out.returncode == 2 and "error:" in out.stderr, out.stderr[-2000:]
+    assert out.stdout == "" and not os.listdir(tmp_path)
+
+
+def test_reference_arm_runs_more_steps_than_the_stream_has_batches():
+    """--steps is honoured exactly even when it exceeds the batches of the (sampled) stream: the port's batches wrap over the
+    tail of its sample, every one a full batch (tiny_bip: 40 batches of 50 edges)."""
+    import json
+    import subprocess
+    import sys
+    import bench
+    starts = bench.oracle_batch_starts(2000, 50, 60)
+    assert len(starts) == 60 and min(starts) >= 1400 and max(starts) + 50 <= 2000 and starts[:3] == [1400, 1450, 1500]
+    assert bench.oracle_batch_starts(40_000, 200, 10) == list(range(38_000, 40_000, 200))  # fits: the last n batches
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "tiny_bip", "--steps", "50",
+                          "--warmup", "1"], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads(out.stdout)
+    assert d["steps"] == 50 and d["value"] > 0 and np.isfinite(d["ms_per_step"])
+
+
 def test_reference_arm_under_torchrun_prints_one_line_from_rank_0():
     """bench.py --impl reference launched like the driver launches it for N > 1 (torchrun, one process per rank): rank 0 alone
     runs the reference's CPU path and prints ONE JSON line, the other ranks exit 0 without work. CPU only (gloo is not even
