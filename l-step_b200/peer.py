@@ -21,8 +21,10 @@ import numpy as np
 import torch
 
 from . import _lib
+from . import checkpoint as ckpt
 from .model import LSTEP
 from .sampler import NeighborSampler
+from .stream import _changelog_load, _changelog_save
 
 
 class _DevMem:
@@ -85,12 +87,20 @@ def peer_batch_plan(src: np.ndarray, dst: np.ndarray, batch_size: int, world: in
 class PeerRank:
     """Rank `rank` of `world` (see the module docstring). src / dst / t: the whole edge stream (replicated, device or host
     arrays); the per-batch plan (sorted unique batch nodes, the owned ones and their positions) of the resident stream
-    [start, stop) is computed once, like PEStream's."""
+    [start, stop) is computed once, like PEStream's.
+
+    The PE state comes from exactly one of `initial_pe` (the table [V1, d]), `history` (a dense history [V1, Th, d],
+    oldest first, as ChangeLogStream.import_history takes it) and `checkpoint` (a directory that save_checkpoint wrote at
+    any world size, or ChangeLogStream.save_checkpoint; or the checkpoint.History that checkpoint.read returned: head, len,
+    batch_idx and steps_done continue from it). `batch_idx` overrides the batch index the next step masks the filter with
+    while the history is shorter than T (the reference's evaluate loop restarts it at 0: Q5)."""
 
     def __init__(self, model: LSTEP, rank: int, world: int, src, dst, t, num_nodes: int, batch_size: int, num_neighbors: int,
-                 initial_pe: torch.Tensor, start: int = 0, stop: int = None, device=None, sampler: NeighborSampler = None,
-                 event_capacity: int = None, timeout_ms: int = 4000):
+                 initial_pe: torch.Tensor = None, start: int = 0, stop: int = None, device=None, sampler: NeighborSampler = None,
+                 event_capacity: int = None, timeout_ms: int = 4000, history: torch.Tensor = None, checkpoint=None, batch_idx: int = None):
         assert 1 <= world <= 16 and 0 <= rank < world
+        if (initial_pe is None) + (history is None) + (checkpoint is None) != 2:
+            raise ValueError("PeerRank: give exactly one of initial_pe, history and checkpoint")
         self.m, self.rank, self.G = model, int(rank), int(world)
         self.dev = dev = torch.device(device) if device is not None else model._dev()
         self.B, self.K, self.T = int(batch_size), int(num_neighbors), model.num_fft_batches
@@ -99,6 +109,14 @@ class PeerRank:
         self.timeout_ms = int(timeout_ms)
         if self.T > 128:
             raise _lib.LstepError("the change-log history supports T <= 128 window steps")
+        hist = None
+        if checkpoint is not None:
+            hist = checkpoint if isinstance(checkpoint, ckpt.History) else ckpt.read(checkpoint)
+        elif history is not None:
+            with torch.cuda.device(dev):
+                hist = ckpt.from_dense(history.to(dev, torch.float32), self.T)
+        if hist is not None:
+            hist.check(V1=self.V1, d=self.d, T=self.T)
         lib = self.lib = _lib.load()
         as_dev = lambda a, dt: (a.to(dev, dt) if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a)).to(dev, dt))
         T, d, G, B = self.T, self.d, self.G, self.B
@@ -126,10 +144,11 @@ class PeerRank:
             self._mem_inbox = _DevMem(lib, max(int(lib.lstep_peer_inbox_bytes(G, cap, d)), 256))
             self._mem_flags = _DevMem(lib, 16 * 4)
             self.cur = torch.empty((self.V1, d), dtype=torch.float32, device=dev)
-            self.cur.copy_(initial_pe.to(dev, torch.float32))
+            if hist is None:
+                self.cur.copy_(initial_pe.to(dev, torch.float32))
             self.new_rows = self._mem_rows.tensor((2 * B, d), torch.float32, dev)
             # ---- change log of the owned nodes
-            self.base = self.cur[self.rank::G].contiguous().clone()
+            self.base = self.cur[self.rank::G].contiguous().clone()  # (overwritten by _changelog_load from a history)
             self.ev_node = torch.zeros((T, cap), dtype=torch.int32, device=dev)
             self.ev_row = torch.empty((T, cap, d), dtype=torch.float32, device=dev)
             self.ev_cnt = torch.zeros(T, dtype=torch.int32, device=dev)
@@ -161,9 +180,16 @@ class PeerRank:
             self.ws = torch.empty(need + 4096, dtype=torch.uint8, device=dev)
             _lib.check(lib.lstep_update_pe_workspace_init(_lib.ptr(self.ws), self.ws.numel(), self.V1, _lib.stream_ptr()), "ws init")
         self.head, self.len, self.batch_idx = 0, 1, 0
-        self.epoch = ctypes.c_uint32(0)
+        self.steps_done, self.edges_done = 0, self.start
+        self.epoch = ctypes.c_uint32(0)  # (a fresh rank: the flag blocks are zeroed by lstep_ipc_alloc)
         self.grp = None
         self._opened = []
+        if hist is not None:
+            _changelog_load(self, hist, G, self.rank)
+            if checkpoint is not None:
+                self.batch_idx, self.steps_done, self.edges_done = (int(hist.meta[k]) for k in ("batch_idx", "steps_done", "edges_done"))
+        if batch_idx is not None:
+            self.batch_idx = int(batch_idx)
 
     # ---- group wiring ---------------------------------------------------------------------------------------------------
     _SHARED = ("_mem_rows", "_mem_filt", "_mem_inbox", "_mem_flags")
@@ -246,6 +272,7 @@ class PeerRank:
                        "lstep_pe_step_peer")
         if phases & 4:
             self._advance(1)
+            self.edges_done = hi
         return out
 
     def _advance(self, n: int):
@@ -255,6 +282,7 @@ class PeerRank:
             else:
                 self.head = (self.head + 1) % self.T
         self.batch_idx += n
+        self.steps_done += n
         self.epoch = ctypes.c_uint32((self.epoch.value + 2 * n) & 0xffffffff)
 
     def run(self, b0: int, n_steps: int, query_arrays, out: torch.Tensor = None, out_step_stride: int = 0):
@@ -281,7 +309,9 @@ class PeerRank:
                                          self.m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(), _lib.ptr(self.sampler._err),
                                          ctypes.byref(epoch), self.timeout_ms, _lib.stream_ptr())
         done = ((epoch.value - self.epoch.value) & 0xffffffff) // 2
-        self.head, self.batch_idx = head.value, self.batch_idx + done
+        self.head, self.batch_idx, self.steps_done = head.value, self.batch_idx + done, self.steps_done + done
+        if done:
+            self.edges_done = int(self.lo[b0 + done - 1] + self.n_edges[b0 + done - 1])
         self.epoch = epoch
         _lib.check(rc, "lstep_pe_steps_peer")
         return out
@@ -304,6 +334,13 @@ class PeerRank:
             self.sampler._err.zero_()
             raise _lib.LstepError(f"a step changed more owned rows than the change-log history's event capacity ({self.cap})")
         self.sampler.check_errors()
+
+    def save_checkpoint(self, path: str):
+        """Write this rank's shard of a checkpoint into directory `path` (l-step_b200/checkpoint.py): the base rows and the
+        events of the nodes it owns. Every rank of the group calls it after the same step; no barrier is needed (an owner's
+        history is always current on its own rank). The checkpoint loads into a group of any world size, or a
+        ChangeLogStream, and the resumed run computes the bits of the uninterrupted one."""
+        _changelog_save(self, path, self.G, self.rank)
 
     def history_bytes(self) -> int:
         return sum(t.numel() * t.element_size() for t in (self.base, self.ev_node, self.ev_row, self.ev_cnt, self.ev_hash, self.ev_mask))

@@ -26,11 +26,79 @@ import numpy as np
 import torch
 
 from . import _lib
+from . import checkpoint as ckpt
 from .model import LSTEP
 
 C_void_p = ctypes.c_void_p
 C_byref = ctypes.byref
 _I64, _F64 = np.dtype(np.int64), np.dtype(np.float64)
+
+
+def _to_dev(a, dev, dtype):
+    """A tensor, or a host numpy array (memory-mapped ones included: copied first), on `dev`."""
+    if isinstance(a, torch.Tensor):
+        return a.to(dev, dtype)
+    return torch.from_numpy(np.array(a, dtype={torch.float32: np.float32, torch.int64: np.int64}[dtype])).to(dev)
+
+
+def _changelog_load(obj, hist: "ckpt.History", world: int, rank: int):
+    """Load a logical history (checkpoint.History, any world size) into the change log of `obj` (a
+    ChangeLogStream: world 1, rank 0; a PeerRank: its group) and into its table replica obj.cur. cur = every node's base
+    row; then, for every window position f in order, cur[nodes of f] = their rows and lstep_changelog_append records the
+    rows of the nodes this rank owns as the events of slot f, exactly as a live step records them. After the last position
+    cur is the current table. The event count of every position is checked against the capacity before any device write."""
+    cnt = hist.counts(world)[:, rank]
+    if len(cnt) and int(cnt.max()) > obj.cap:
+        f = int(cnt.argmax())
+        raise _lib.LstepError(f"window position {f} of the history holds {int(cnt[f])} events of rank {rank} of {world} but "
+                              f"event_capacity is {obj.cap}: pass a larger event_capacity")
+    lib = _lib.load()
+    dev = obj.dev
+    chunk = max(1, (256 << 20) // (4 * hist.d))
+    with torch.cuda.device(dev), torch.no_grad():
+        for g, sh in enumerate(hist.shards):
+            dst = obj.cur[g::hist.world]
+            for a in range(0, dst.shape[0], chunk):
+                dst[a:a + chunk].copy_(_to_dev(sh["base"][a:a + chunk], dev, torch.float32))
+        obj.base.copy_(obj.cur[rank::world])
+        obj.ev_cnt.zero_()
+        obj.ev_hash.fill_(-1)
+        obj.ev_mask.zero_()
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+        for f in range(hist.len):
+            nodes, rows = hist.events(f)
+            ids = _to_dev(nodes, dev, torch.int64) if len(nodes) else None
+            if ids is not None:
+                obj.cur[ids] = _to_dev(rows, dev, torch.float32)
+            _lib.check(lib.lstep_changelog_append(C_byref(obj.cl), f, 0, _lib.ptr(obj.cur), None, None, 0, _lib.ptr(ids), len(nodes), None, 0, 0,
+                                                  _lib.ptr(err), _lib.stream_ptr()), "lstep_changelog_append")
+        if int(err.item()):
+            raise _lib.LstepError(f"loading the history overflowed the change log (flag {int(err.item())})")
+    obj.head, obj.len = 0, hist.len
+
+
+def _changelog_save(obj, path: str, world: int, rank: int):
+    """Write the change log of `obj` (rank `rank` of a world-`world` group) as shard `rank` of a checkpoint in directory
+    `path`: its base rows and the events of every window position in logical order (from the ring's head; sorted by node
+    within a position, so that one state always gives the same files)."""
+    obj.check_errors()
+    torch.cuda.synchronize(obj.dev)
+    cnt = obj.ev_cnt.cpu().numpy()
+    slots = [(obj.head + f) % obj.T for f in range(obj.len)]
+    off = np.cumsum([0] + [int(cnt[s]) for s in slots]).astype(np.int64)
+    ev_node = np.empty(int(off[-1]), np.int64)
+    ev_row = np.empty((int(off[-1]), obj.d), np.float32)
+    for f, s in enumerate(slots):
+        n = int(cnt[s])
+        if n:
+            nodes = obj.ev_node[s, :n].cpu().numpy()
+            order = np.argsort(nodes, kind="stable")
+            ev_node[off[f]:off[f + 1]] = nodes[order]
+            ev_row[off[f]:off[f + 1]] = obj.ev_row[s, :n].cpu().numpy()[order]
+    base = obj.base[:ckpt.rows_of(obj.V1, world, rank)].cpu().numpy()
+    meta = dict(world=world, rank=rank, V1=obj.V1, d=obj.d, T=obj.T, len=obj.len, batch_idx=obj.batch_idx, steps_done=obj.steps_done,
+                edges_done=obj.edges_done)
+    ckpt.write_shard(path, meta, base, off, ev_node, ev_row)
 
 
 class PEStream:
@@ -434,19 +502,47 @@ class ChangeLogStream(PEStream):
     Same API (step, cur, export_history / import_history); the DFT filter sums (events in window + 1) rows per node with
     span sums of G as weights. `event_capacity`: events one step may record (default: every row a batch can touch,
     2B + 2BK + 2, capped at V1); importing a dense history needs capacity for the rows that differ between consecutive
-    snapshots. `row_mul` / `row_add`: node-id sharded groups keep only the nodes v % row_mul == row_add."""
+    snapshots. `row_mul` / `row_add`: node-id sharded groups keep only the nodes v % row_mul == row_add.
 
-    def __init__(self, *args, event_capacity: int = None, **kw):
+    `checkpoint`: resume from a checkpoint directory that save_checkpoint or a PeerRank group of any world size wrote (or
+    the checkpoint.History that checkpoint.read returned), instead of initial_pe / history; head, len, batch_idx and
+    steps_done continue from it. `batch_idx` overrides the batch index the next step masks the filter with while the
+    history is shorter than T (the reference's evaluate loop restarts it at 0: Q5)."""
+
+    def __init__(self, *args, event_capacity: int = None, checkpoint=None, batch_idx: int = None, **kw):
         self._cap_arg = event_capacity
+        hist = None
+        if checkpoint is not None:
+            if any(a is not None for a in args[6:8]) or kw.get("initial_pe") is not None or kw.get("history") is not None:
+                raise ValueError("ChangeLogStream: give one of initial_pe, history and checkpoint")
+            hist = checkpoint if isinstance(checkpoint, ckpt.History) else ckpt.read(checkpoint)
+            model = args[0] if args else kw["model"]
+            hist.check(d=model.pe_dim, T=model.num_fft_batches)
+        self.edges_done = 0
         super().__init__(*args, **kw)
+        if hist is not None:
+            self._load(hist)
+            self.batch_idx, self.steps_done, self.edges_done = (int(hist.meta[k]) for k in ("batch_idx", "steps_done", "edges_done"))
+        if batch_idx is not None:
+            self.batch_idx = int(batch_idx)
 
     def import_history(self, history: torch.Tensor):
         history = history.to(self.dev, torch.float32)
-        V1, Th, d = history.shape
-        assert d == self.d
-        if Th > self.T:
-            history = history[:, -self.T:, :]
-            Th = self.T
+        assert history.shape[2] == self.d
+        self._load(ckpt.from_dense(history, self.T))
+        self.steps_done = 0
+        self.edges_done = self.start
+
+    def save_checkpoint(self, path: str):
+        """Write the history into directory `path` as a world-1 checkpoint (l-step_b200/checkpoint.py: base rows and the
+        events of every window position, about V1 + T * (rows changed per step) rows; not the table, the CSR or the model
+        parameters). ChangeLogStream(..., checkpoint=path) and PeerRank(..., checkpoint=path) at any world size resume
+        from it with the bits of the uninterrupted run."""
+        _changelog_save(self, path, 1, 0)
+
+    def _load(self, hist: "ckpt.History"):
+        """Allocate the change log for hist.V1 rows and load `hist` into it (_changelog_load)."""
+        V1, d = hist.V1, self.d
         if len(self.ids_np):
             lo_id, hi_id = int(self.ids_np.min()), int(self.ids_np.max())
             if lo_id < 0 or hi_id >= V1:
@@ -464,7 +560,7 @@ class ChangeLogStream(PEStream):
         while H < 2 * cap:
             H *= 2
         dev = self.dev
-        self.base = history[:, 0, :].contiguous().clone()
+        self.base = torch.empty((V1, d), dtype=torch.float32, device=dev)
         self.ev_node = torch.zeros((T, cap), dtype=torch.int32, device=dev)
         self.ev_row = torch.empty((T, cap, d), dtype=torch.float32, device=dev)
         self.ev_cnt = torch.zeros(T, dtype=torch.int32, device=dev)
@@ -473,25 +569,11 @@ class ChangeLogStream(PEStream):
         self.cl = _lib.ChangeLog(self.base.data_ptr(), self.ev_node.data_ptr(), self.ev_row.data_ptr(), self.ev_cnt.data_ptr(),
                                  self.ev_hash.data_ptr(), self.ev_mask.data_ptr(), V1, T, cap, H, d, 1, 0)
         self.ring = None
-        self.head, self.len = 0, 1
-        self.cur = self.base.clone()
-        lib = _lib.load()
-        err = torch.zeros(1, dtype=torch.int32, device=dev)
-        with torch.cuda.device(dev):
-            for s in range(1, Th):  # every later snapshot: the rows that differ from the previous one are that step's events
-                snap = history[:, s, :].contiguous()
-                changed = torch.nonzero((snap != self.cur).any(dim=1)).flatten()
-                if changed.numel() > cap:
-                    raise _lib.LstepError(f"snapshot {s} differs from the previous one in {changed.numel()} rows but event_capacity is {cap}")
-                _lib.check(lib.lstep_changelog_append(ctypes.byref(self.cl), s, 0, _lib.ptr(snap), None, None, 0, _lib.ptr(changed), changed.numel(),
-                                                      None, 0, 0, _lib.ptr(err), _lib.stream_ptr()), "lstep_changelog_append")
-                self.cur = snap
-                self.len = s + 1
-            self.cur = self.cur.clone()
+        self.cur = torch.empty((V1, d), dtype=torch.float32, device=dev)
+        _changelog_load(self, hist, 1, 0)
         self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.t.data_ptr(), None, self.cur.data_ptr(), V1, T, d)
         self._ws = None
         self._ws_cap = (0, 0, 0)
-        self.steps_done = 0
 
     def history_bytes(self) -> int:
         """Bytes the history occupies (base + event rows + index structures) — against V1 * T * d * 4 for the dense ring."""
@@ -540,6 +622,7 @@ class ChangeLogStream(PEStream):
                 self.head = (self.head + 1) % T
         self.batch_idx = bi + 1
         self.steps_done += 1
+        self.edges_done = lo + n_edges
 
     def run(self, b0: int, n_steps: int, queries, out: torch.Tensor = None, check: bool = False):
         lo0 = self.batch_lo[b0]
