@@ -43,6 +43,7 @@ typedef enum lstep_status {
 #define LSTEP_FLAG_UNSORTED_STREAM 2u
 #define LSTEP_FLAG_CHANGELOG_FULL 4u /* a step changed more rows than the change-log history has event capacity for */
 #define LSTEP_FLAG_PEER_TIMEOUT 8u   /* a peer GPU did not reach a step barrier within the time limit (peer group step) */
+#define LSTEP_FLAG_CSR_FULL 16u      /* an append to a growable CSR found no room in a row; nothing was written to that row */
 
 const char* lstep_strerror(int status);
 const char* lstep_last_cuda_error(void);
@@ -81,6 +82,27 @@ int lstep_csr_build_from_entries(const int64_t* owner, const int64_t* nbr, const
                                  int64_t n_entries, int64_t num_rows, int64_t* out_indptr, int32_t* out_nbr,
                                  int32_t* out_eid, double* out_t, void* workspace, size_t workspace_bytes,
                                  uint32_t* err_flag, void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Growable CSR (csrc/csr_grow.cu): an lstep_csr whose rows end in padding, plus int32 fill[num_rows]. Row v holds its
+ * real entries at [indptr[v], indptr[v] + fill[v]); the rest of [indptr[v], indptr[v+1]) is padding (t = +inf, nbr = 0,
+ * eid = 0), which no lookup selects (every reader counts entries with t < tq, strict, and none reads nnz). Every entry
+ * point that takes an lstep_csr reads a growable one unchanged and returns what it returns on the exact CSR of the
+ * same edges.
+ * lstep_csr_relayout copies each row's real entries (src_fill NULL: src is exact, every entry is real) to
+ * [new_indptr[v], ...) of the output arrays, pads the rest of each new row and writes out_fill. Output arrays must not
+ * alias src's. A row whose new capacity is below its fill keeps its first entries and raises LSTEP_FLAG_CSR_FULL.
+ * lstep_csr_ingest appends a batch of edges in the reference's order (utils/utils.py:292-299): for edge i, (dst, eid, t)
+ * to row src, then (src, eid, t) to row dst (a self-loop gives two entries); eid NULL: eid_base + i. Times must be
+ * non-decreasing across the batch and not earlier than any real entry of a row they go to (else
+ * LSTEP_FLAG_UNSORTED_STREAM); a row without room for its entries of a chunk of 2048 edges gets none of them
+ * (LSTEP_FLAG_CSR_FULL); an edge with an id outside the rows or an eid outside int32 is dropped
+ * (LSTEP_FLAG_NODE_OUT_OF_RANGE).
+ * ------------------------------------------------------------------------------------------ */
+int lstep_csr_relayout(const lstep_csr* src, const int32_t* src_fill, const int64_t* new_indptr, int32_t* out_nbr,
+                       int32_t* out_eid, double* out_t, int32_t* out_fill, uint32_t* err_flag, void* stream);
+int lstep_csr_ingest(const lstep_csr* csr, int32_t* fill, const int64_t* src, const int64_t* dst, const int64_t* eid,
+                     int64_t eid_base, const double* t, int64_t n_edges, uint32_t* err_flag, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * a2 — most-recent-K temporal neighbour lookup (kernel K1).
@@ -447,6 +469,16 @@ int lstep_pe_step_host(lstep_host_stepper* h, const lstep_pe_stream* s, const ls
                        const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes,
                        uint32_t* err_flag, void* stream, int64_t* ticket);
 int lstep_host_step_result(lstep_host_stepper* h, int64_t ticket, const float** result_host, int64_t* n_floats);
+/* Arms the stepper to grow a growable CSR (see lstep_csr_ingest; `fill` its fill array, the csr being the one each call
+ * passes): every later lstep_pe_step_host / lstep_pe_steps_host call first appends its batch, with edge ids next_eid + i,
+ * then runs its step on the grown CSR. Before anything is enqueued a call rejects a batch whose times are not finite, decrease,
+ * or start before last_t (LSTEP_ERR_INVALID_ARG), or whose ids or edge ids fall outside the CSR's rows or int32
+ * (LSTEP_ERR_ID_RANGE). The append runs on the copy-in path, between the batch's copy-in and its hand-over to the
+ * compute stream, on a stream of the highest priority (created by the first arming). The first append after arming, or after the CSR's arrays change, also waits for the work enqueued on
+ * the compute stream so far (a relayout, or appends made there). The append of batch b+1 is not ordered after work the caller
+ * enqueues on the compute stream after step b: a lookup there is exact at times <= the times of batch b only. fill = NULL
+ * disarms. */
+int lstep_host_stepper_set_ingest(lstep_host_stepper* h, int32_t* fill, int64_t next_eid, double last_t);
 void lstep_host_stepper_bytes(const lstep_host_stepper* h, uint64_t* h2d_bytes, uint64_t* d2h_bytes);
 /* A run of consecutive batches in one call (an evaluation split, evaluate_model_utils.py:38-142): the loop over
  * lstep_pe_step_host / lstep_host_step_result is done natively, results read one step behind. Full history ring only

@@ -58,6 +58,8 @@ _SIGS = {
     "lstep_csr_build_workspace_bytes": (sz, [i64, i64]),
     "lstep_csr_build_from_edges": (i32, [vp, vp, vp, vp, i64, i64, vp, vp, vp, vp, vp, sz, vp, vp]),
     "lstep_csr_build_from_entries": (i32, [vp, vp, vp, vp, i64, i64, vp, vp, vp, vp, vp, sz, vp, vp]),
+    "lstep_csr_relayout": (i32, [C.POINTER(CSR), vp, vp, vp, vp, vp, vp, vp, vp]),
+    "lstep_csr_ingest": (i32, [C.POINTER(CSR), vp, vp, vp, vp, i64, vp, i64, vp, vp]),
     "lstep_sample_recent": (i32, [C.POINTER(CSR), vp, vp, i64, i64, i32, vp, vp, vp, vp, vp]),
     "lstep_sample_recent_compact": (i32, [C.POINTER(CSR), vp, vp, i64, i64, i32, vp, vp, vp, vp]),
     "lstep_dft_collapse": (i32, [vp, vp, i32, i32, i32, vp, vp]),
@@ -127,6 +129,7 @@ _SIGS = {
     "lstep_pe_steps_host": (i32, [vp, C.POINTER(PEStreamDesc), C.POINTER(CSR), i64, i64, vp, vp, vp, C.POINTER(C.c_void_p), i32,
                                   C.POINTER(i32), C.POINTER(i32), vp, i32, C.POINTER(PEMLP), C.POINTER(PEMLP), vp, sz, vp, vp, vp,
                                   C.POINTER(i64)]),
+    "lstep_host_stepper_set_ingest": (i32, [vp, vp, i64, C.c_double]),
     "lstep_host_step_result": (i32, [vp, i64, C.POINTER(C.POINTER(C.c_float)), C.POINTER(i64)]),
     "lstep_host_stepper_bytes": (None, [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
 }
@@ -194,5 +197,7 @@ def stream_ptr():
 
 
 FLAG_NODE_OUT_OF_RANGE = 1
+FLAG_UNSORTED_STREAM = 2
 FLAG_CHANGELOG_FULL = 4
 FLAG_PEER_TIMEOUT = 8
+FLAG_CSR_FULL = 16

@@ -17,7 +17,7 @@ ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "liblstep_b200.so")
 STAMP = os.path.join(PKG, ".liblstep_b200.stamp")
-SOURCES = ["api.cu", "sampler.cu", "dft_filter.cu", "mlp.cu", "mlp_cluster.cu", "mlp_umma.cu", "aggregate.cu", "update.cu", "update_push.cu", "csr_build.cu", "step.cu", "host_step.cu", "changelog.cu", "peer.cu"]
+SOURCES = ["api.cu", "sampler.cu", "dft_filter.cu", "mlp.cu", "mlp_cluster.cu", "mlp_umma.cu", "aggregate.cu", "update.cu", "update_push.cu", "csr_build.cu", "csr_grow.cu", "step.cu", "host_step.cu", "changelog.cu", "peer.cu"]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-Xcompiler", "-fPIC",
               "--shared", "-Xptxas", "-v", "-Wno-deprecated-gpu-targets"]
 

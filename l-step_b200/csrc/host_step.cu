@@ -9,6 +9,7 @@
 // synchronising. lstep_host_step_result waits for a ticket's event and hands out the pinned result, so a
 // loop can keep `slots - 1` steps in flight (results read one step behind hide the host's own time).
 #include <algorithm>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <new>
@@ -76,6 +77,15 @@ struct lstep_host_stepper {
   float* d_nbr_out;              // [max_queries][max_edges][d] when the caller keeps no copy of its own
   int64_t next_ticket;
   uint64_t h2d_bytes, d2h_bytes;
+  // lstep_host_stepper_set_ingest: append each batch to a growable CSR before its step (ing_fill NULL: disarmed)
+  int32_t* ing_fill;
+  int64_t ing_next_eid;
+  double ing_last_t;
+  bool ing_wait;              // the next append waits for the compute stream (just armed, or the CSR's arrays changed)
+  const void* ing_arrays[4];  // indptr, nbr, eid, t of the CSR the last append wrote
+  cudaEvent_t ing_ev;         // compute stream -> append (ing_wait)
+  cudaEvent_t ing_staged;     // copy-in -> append
+  cudaStream_t ing_stream;    // the appends: highest priority, so that the append CTA gets the first free SM slot
 };
 
 // sorted unique ids of src[0..n) U dst[0..n) -> out[<= 2n]. Small id spaces: a bitmap over [0, V1) scanned in
@@ -134,6 +144,9 @@ extern "C" void lstep_host_stepper_destroy(lstep_host_stepper* h) {
     if (h->d_res[i]) cudaFree(h->d_res[i]);
   }
   if (h->d_nbr_out) cudaFree(h->d_nbr_out);
+  if (h->ing_ev) cudaEventDestroy(h->ing_ev);
+  if (h->ing_staged) cudaEventDestroy(h->ing_staged);
+  if (h->ing_stream) cudaStreamDestroy(h->ing_stream);
   if (h->in_stream) cudaStreamDestroy(h->in_stream);
   if (h->out_stream) cudaStreamDestroy(h->out_stream);
   delete h;
@@ -155,6 +168,13 @@ extern "C" int lstep_host_stepper_create(int slots, int64_t max_edges, int max_q
   h->h2d_bytes = h->d2h_bytes = 0;
   h->d_nbr_out = nullptr;
   h->in_stream = h->out_stream = nullptr;
+  h->ing_fill = nullptr;
+  h->ing_next_eid = 0;
+  h->ing_last_t = 0.0;
+  h->ing_wait = false;
+  for (int k = 0; k < 4; ++k) h->ing_arrays[k] = nullptr;
+  h->ing_ev = h->ing_staged = nullptr;
+  h->ing_stream = nullptr;
   for (int i = 0; i < kMaxSlots; ++i) {
     h->h_in[i] = h->d_in[i] = nullptr;
     h->h_res[i] = h->d_res[i] = nullptr;
@@ -232,6 +252,18 @@ extern "C" int lstep_pe_step_host(lstep_host_stepper* h, const lstep_pe_stream* 
     for (size_t i = 0; i < (size_t)n_queries * n && ok; ++i) ok = h_q[i] >= 0 && h_q[i] < V1;
     if (!ok) return LSTEP_ERR_ID_RANGE;
   }
+  const bool ingest = h->ing_fill != nullptr;
+  if (ingest) {  // the batch goes into the growable CSR: the same conditions lstep_csr_ingest's guards check, on the host
+    if (!csr) return LSTEP_ERR_INVALID_ARG;
+    double prev = h->ing_last_t;
+    for (size_t i = 0; i < n; ++i) {
+      if (!std::isfinite(t_host[i]) || t_host[i] < prev) return LSTEP_ERR_INVALID_ARG;
+      prev = t_host[i];
+    }
+    for (size_t i = 0; i < n; ++i)
+      if (src_host[i] >= csr->num_rows || dst_host[i] >= csr->num_rows) return LSTEP_ERR_ID_RANGE;  // (>= 0: checked above)
+    if (h->ing_next_eid < 0 || h->ing_next_eid + n_edges - 1 > 0x7fffffffLL) return LSTEP_ERR_ID_RANGE;
+  }
   const size_t bytes = 8 * n * (size_t)(5 + n_queries);
   const bool use_memcpy = tuning().host_memcpy != 0;
   // copy-in on its own stream: it only has to wait for the slot's previous use (synchronised above), so it runs
@@ -245,7 +277,36 @@ extern "C" int lstep_pe_step_host(lstep_host_stepper* h, const lstep_pe_stream* 
     int rc0 = check_launch("stage_in");
     if (rc0 != LSTEP_OK) return rc0;
   }
-  if ((e = cudaEventRecord(h->in_ready[slot], h->in_stream)) != cudaSuccess) return cuda_fail(e, "pe_step_host event");
+  if (ingest) {
+    // The batch is appended to the CSR from the staged slot, on the copy-in path: on a high-priority stream that waits for
+    // the copy-in and records in_ready, so the compute stream sees the grown CSR and the step's launch chain is unchanged.
+    // (The step's kernels, launched ahead with programmatic dependent launch, keep the SMs occupied; at default priority the
+    // append CTA only found room between two steps.) The append of batch b+1 may run while step b still reads the
+    // CSR. That is safe: step b queries at times <= tmax_b (a6 at its edge times, phase B at its edge times), every time
+    // being written is >= the last time ingested >= tmax_b, and every slot being written held padding (t = +inf). Each
+    // reader counts the entries of a row with t < tq (strict) and reads nothing at or after that count, so the written
+    // slots count as "not earlier" both before and after the write (an aligned 8-byte store is seen whole or not at all),
+    // and step b selects the same entries whichever it sees. fill[] is read by the appends only.
+    const void* arrays[4] = {csr->indptr, csr->nbr, csr->eid, csr->t};
+    bool changed = false;
+    for (int k = 0; k < 4; ++k) changed |= arrays[k] != h->ing_arrays[k];
+    if ((e = cudaEventRecord(h->ing_staged, h->in_stream)) != cudaSuccess) return cuda_fail(e, "pe_step_host ingest event");
+    if ((e = cudaStreamWaitEvent(h->ing_stream, h->ing_staged, 0)) != cudaSuccess) return cuda_fail(e, "pe_step_host ingest wait");
+    if (h->ing_wait || changed) {  // a relayout or an append enqueued on the compute stream must land first
+      if ((e = cudaEventRecord(h->ing_ev, st)) != cudaSuccess) return cuda_fail(e, "pe_step_host ingest event");
+      if ((e = cudaStreamWaitEvent(h->ing_stream, h->ing_ev, 0)) != cudaSuccess) return cuda_fail(e, "pe_step_host ingest wait");
+    }
+    const int64_t* dp_in = reinterpret_cast<const int64_t*>(h->d_in[slot]);
+    const int rc1 = lstep_csr_ingest(csr, h->ing_fill, dp_in, dp_in + n, nullptr, h->ing_next_eid,
+                                     reinterpret_cast<const double*>(dp_in + 2 * n), n_edges, err_flag, h->ing_stream);
+    if (rc1 != LSTEP_OK) return rc1;
+    h->ing_wait = false;
+    for (int k = 0; k < 4; ++k) h->ing_arrays[k] = arrays[k];
+    h->ing_next_eid += n_edges;
+    h->ing_last_t = t_host[n - 1];
+  }
+  if ((e = cudaEventRecord(h->in_ready[slot], ingest ? h->ing_stream : h->in_stream)) != cudaSuccess)
+    return cuda_fail(e, "pe_step_host event");
   if ((e = cudaStreamWaitEvent(st, h->in_ready[slot], 0)) != cudaSuccess) return cuda_fail(e, "pe_step_host wait");
   h->h2d_bytes += bytes;
   const int64_t* dp = reinterpret_cast<const int64_t*>(h->d_in[slot]);
@@ -294,6 +355,24 @@ extern "C" int lstep_host_step_result(lstep_host_stepper* h, int64_t ticket, con
   if (e != cudaSuccess) return cuda_fail(e, "host_step_result");
   if (result_host) *result_host = h->h_res[slot];
   if (n_floats) *n_floats = h->res_n[slot];
+  return LSTEP_OK;
+}
+
+extern "C" int lstep_host_stepper_set_ingest(lstep_host_stepper* h, int32_t* fill, int64_t next_eid, double last_t) {
+  if (!h) return LSTEP_ERR_INVALID_ARG;
+  if (fill && (next_eid < 0 || next_eid > 0x7fffffffLL || std::isnan(last_t))) return LSTEP_ERR_INVALID_ARG;
+  if (fill && !h->ing_stream) {
+    int least = 0, greatest = 0;
+    cudaError_t e = cudaDeviceGetStreamPriorityRange(&least, &greatest);
+    if (e == cudaSuccess && !h->ing_ev) e = cudaEventCreateWithFlags(&h->ing_ev, cudaEventDisableTiming);
+    if (e == cudaSuccess && !h->ing_staged) e = cudaEventCreateWithFlags(&h->ing_staged, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&h->ing_stream, cudaStreamNonBlocking, greatest);
+    if (e != cudaSuccess) return cuda_fail(e, "host_stepper_set_ingest");
+  }
+  h->ing_fill = fill;
+  h->ing_next_eid = next_eid;
+  h->ing_last_t = last_t;
+  h->ing_wait = fill != nullptr;
   return LSTEP_OK;
 }
 

@@ -14,6 +14,11 @@ Only the 'recent' strategy — the one LSTEP's defaults and best-configs use
 (utils/load_configs.py:22,81-96) — runs on the device; 'uniform' / 'time_interval_aware' draw from
 numpy's RandomState on the host in the reference and are outside the hot path (SURVEY §2 #1):
 asking for them raises NotImplementedError instead of silently computing on the CPU.
+
+A GROWABLE sampler (NeighborSampler.growable, csrc/csr_grow.cu) serves an edge stream that is still arriving: its
+rows end in padding, `ingest` appends a batch on the device, and every lookup returns what the exact sampler of the
+edges ingested so far returns. Capacity is planned on the host (check_edges, overflow_rows, plan_capacity below:
+numpy only), so deciding to regrow never synchronises.
 """
 from __future__ import annotations
 
@@ -25,6 +30,69 @@ import torch
 from . import _lib
 
 _STRATEGIES = ("uniform", "recent", "time_interval_aware")
+
+# Smallest spare room a regrow gives a row. Every row gets need + max(MIN_SLACK, need), so rows can double before the
+# next regrow; the floor keeps rows that are still small from forcing one regrow after another while a stream starts
+# from empty. The floor is also room on every row, untouched ones included. Measured on a B200 (profiles/r03_csr_grow.json):
+#   Reddit shape (11 k rows, 1.3 M entries, B=200): floor 1 / 4 / 16 / 64 -> 253 / 52 / 19 / 12 regrows, 38 / 9.5 / 3.7 /
+#   2.1 ms of regrows in all, CSR 39 / 39 / 43 / 34 MB at the end;
+#   2 M rows, 4 M entries (B=2000): floor 4 / 16 / 64 -> 56 / 19 / 11 regrows, 530 / 179 / 167 ms, CSR 0.25 / 0.62 / 2.1 GB.
+# 64 saves a few regrows on the small graph but makes a graph with many rows and few entries per row 3.4x larger than 16,
+# for 12 ms less regrowing; 4 regrows three times as often. Hence 16.
+MIN_SLACK = 16
+_EID_MAX = 0x7FFFFFFF
+
+
+def check_edges(src, dst, edge_ids, times, num_rows: int, last_time: float = -np.inf):
+    """Validate a batch for ingestion into a growable CSR and return it as contiguous (int64, int64, int64, float64)
+    arrays. Raises ValueError for unequal lengths, non-finite or decreasing times, a first time before `last_time` (the
+    last time ingested) and edge ids outside [0, 2^31); IndexError for a node id outside [0, num_rows), as the
+    reference's adjacency lookup does (SURVEY Q8). edge_ids may be an int: the first of n consecutive ids, returned as
+    the array of all n."""
+    src = np.ascontiguousarray(src, dtype=np.int64)
+    dst = np.ascontiguousarray(dst, dtype=np.int64)
+    t = np.ascontiguousarray(times, dtype=np.float64)
+    n = len(src)
+    if isinstance(edge_ids, (int, np.integer)):
+        eid = np.arange(int(edge_ids), int(edge_ids) + n, dtype=np.int64)
+        n_eid = n
+    else:
+        eid = np.ascontiguousarray(edge_ids, dtype=np.int64)
+        n_eid = len(eid)
+    if len(dst) != n or n_eid != n or len(t) != n:
+        raise ValueError(f"ingest: src, dst, edge_ids and times must have the same length ({n}, {len(dst)}, {n_eid}, {len(t)})")
+    if n == 0:
+        return src, dst, eid, t
+    lo, hi = min(int(src.min()), int(dst.min())), max(int(src.max()), int(dst.max()))
+    if lo < 0 or hi >= num_rows:
+        raise IndexError(f"list index out of range: node id {lo if lo < 0 else hi} is outside the sampler's {num_rows} rows")
+    if not np.isfinite(t).all():
+        raise ValueError("ingest: times must be finite")
+    if n > 1 and not (np.diff(t) >= 0).all():
+        raise ValueError("ingest: times must be non-decreasing within a batch")
+    if t[0] < last_time:
+        raise ValueError(f"ingest: the batch starts at time {t[0]!r}, before the last time ingested ({last_time!r})")
+    if int(eid.min()) < 0 or int(eid.max()) > _EID_MAX:
+        raise ValueError("ingest: edge ids must lie in [0, 2^31)")
+    return src, dst, eid, t
+
+
+def row_counts(src: np.ndarray, dst: np.ndarray):
+    """(rows, counts): the rows a batch appends to and how many entries each gets (one per endpoint: a self-loop
+    counts twice)."""
+    return np.unique(np.concatenate([src, dst]), return_counts=True)
+
+
+def overflow_rows(fill: np.ndarray, cap: np.ndarray, src: np.ndarray, dst: np.ndarray) -> np.ndarray:
+    """Rows the batch (src, dst) touches that have no room for its entries. O(batch): only touched rows are looked at."""
+    rows, cnt = row_counts(src, dst)
+    return rows[fill[rows] + cnt > cap[rows]]
+
+
+def plan_capacity(need: np.ndarray, min_slack: int = MIN_SLACK) -> np.ndarray:
+    """Row capacities of a regrow: need + max(min_slack, need) for every row."""
+    need = np.asarray(need, dtype=np.int64)
+    return need + np.maximum(int(min_slack), need)
 
 
 def _dev(device=None) -> torch.device:
@@ -46,6 +114,7 @@ class NeighborSampler:
         self._lib = _lib.load()
         self.device = _dev(device)
         self._err = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self.fill = None  # growable samplers only: device int32 [num_rows], see growable()
         if _csr_tensors is not None:
             self._set_csr(*_csr_tensors)
             return
@@ -73,6 +142,134 @@ class NeighborSampler:
         self._build("lstep_csr_build_from_edges", (src_node_ids, dst_node_ids, edge_ids, node_interact_times), E, 2 * E,
                     int(num_rows))
         return self
+
+    @classmethod
+    def growable(cls, num_rows: int, src=(), dst=(), edge_ids=(), times=(), sample_neighbor_strategy="recent",
+                 time_scaling_factor=0.0, seed=None, device=None, min_slack: int = MIN_SLACK):
+        """A sampler that grows batch by batch (`ingest`), for a stream whose edges are not known in advance. The optional
+        prefix (src, dst, edge_ids, times; times non-decreasing) is built with the exact builder and then laid out with
+        room to grow. Node ids must lie in [0, num_rows). Lookups equal those of from_edges on the edges ingested so far."""
+        num_rows = int(num_rows)
+        if num_rows <= 0:
+            raise ValueError("growable: num_rows must be positive")
+        src, dst, eid, t = check_edges(src, dst, edge_ids, times, num_rows)
+        self = cls.from_edges(src, dst, eid, t, sample_neighbor_strategy, time_scaling_factor, seed, device, num_rows=num_rows)
+        self.min_slack = int(min_slack)
+        self._version = 0
+        fill = np.bincount(src, minlength=num_rows) + np.bincount(dst, minlength=num_rows)
+        self._fill_h = fill.astype(np.int64)
+        self._n_entries = int(2 * len(src))
+        self._last_t = float(t[-1]) if len(t) else -np.inf
+        self._next_eid = int(eid[-1]) + 1 if len(eid) else 1
+        self.regrows = 0
+        self._regrow(self._fill_h)
+        self.regrows = 0  # regrows after construction
+        return self
+
+    @property
+    def is_growable(self) -> bool:
+        return self.fill is not None
+
+    @property
+    def num_entries(self) -> int:
+        """Real (ingested) adjacency entries; `nnz` is the length of the arrays, padding included."""
+        return self._n_entries if self.is_growable else self.nnz
+
+    @property
+    def last_time(self) -> float:
+        """Time of the last edge ingested (-inf before the first); the next batch may not start earlier."""
+        return self._last_t
+
+    @property
+    def next_edge_id(self) -> int:
+        """Edge id after the last one ingested (1 before the first: the reference's edge ids start at 1, 0 is padding)."""
+        return self._next_eid
+
+    def _require_growable(self):
+        if not self.is_growable:
+            raise ValueError("this NeighborSampler holds an exact CSR; build one with NeighborSampler.growable(...) to ingest edges")
+
+    def _regrow(self, need: np.ndarray):
+        """Lay the CSR out again with capacity plan_capacity(need) per row. Synchronises the device once (appends may
+        still be in flight on other streams, and the old arrays are released afterwards)."""
+        cap = plan_capacity(need, self.min_slack)
+        indptr_h = np.zeros(self.num_rows + 1, dtype=np.int64)
+        np.cumsum(cap, out=indptr_h[1:])
+        total = int(indptr_h[-1])
+        if total > _EID_MAX:  # the kernels index entries with int64 but the builder's limit is kept for the whole CSR
+            raise _lib.LstepError(f"growable CSR: {total} entries of capacity exceed 2^31")
+        dev = self.device
+        torch.cuda.synchronize(dev)
+        indptr = torch.from_numpy(indptr_h).to(dev)
+        nbr = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
+        eid = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
+        t = torch.empty(max(total, 1), dtype=torch.float64, device=dev)
+        fill = torch.empty(self.num_rows, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            rc = self._lib.lstep_csr_relayout(self.csr_ref, _lib.ptr(self.fill), _lib.ptr(indptr), _lib.ptr(nbr), _lib.ptr(eid),
+                                              _lib.ptr(t), _lib.ptr(fill), _lib.ptr(self._err), _lib.stream_ptr())
+        _lib.check(rc, "lstep_csr_relayout")
+        self._set_csr(indptr, nbr[:total], eid[:total], t[:total])
+        self.fill = fill
+        self._cap_h = cap
+        self.regrows += 1
+        self._version += 1
+
+    def reserve(self, src, dst):
+        """Make room for the entries the edges (src, dst) will add (known future endpoints, e.g. a whole split). Regrows
+        (one device synchronisation) only when a touched row lacks room; every row then gets need + max(min_slack, need)."""
+        self._require_growable()
+        src = np.ascontiguousarray(src, dtype=np.int64)
+        dst = np.ascontiguousarray(dst, dtype=np.int64)
+        if len(src) == 0:
+            return
+        rows, cnt = row_counts(src, dst)
+        if int(rows[0]) < 0 or int(rows[-1]) >= self.num_rows:
+            raise IndexError(f"list index out of range: node id outside the sampler's {self.num_rows} rows")
+        if (self._fill_h[rows] + cnt > self._cap_h[rows]).any():
+            need = self._fill_h.copy()
+            need[rows] += cnt
+            self._regrow(need)
+
+    def _note_ingested(self, src, dst, last_eid: int, last_t: float):
+        """Host mirror of an append enqueued on the device (here or by a host-fed stream step)."""
+        rows, cnt = row_counts(src, dst)
+        self._fill_h[rows] += cnt
+        self._n_entries += 2 * len(src)
+        self._next_eid = int(last_eid) + 1
+        self._last_t = float(last_t)
+
+    def _resync(self, src, dst, eid0: int, times):
+        """After a failed call that may have enqueued the appends of a prefix of the edges (src[i], dst[i], eid0 + i,
+        times[i]) before failing: synchronise, take fill from the device, and count the edges that landed (appends are
+        whole batches, in order). The version bump makes a host-fed stream re-arm its stepper from this state."""
+        torch.cuda.synchronize(self.device)
+        fill = self.fill.cpu().numpy().astype(np.int64)
+        landed = int(fill.sum() - self._n_entries) // 2
+        if landed > 0:
+            self._note_ingested(src[:landed], dst[:landed], eid0 + landed - 1, times[landed - 1])
+        self._fill_h = fill
+        self._version += 1
+
+    def ingest(self, src, dst, edge_ids, times):
+        """Append a batch of edges (the reference's get_neighbor_sampler order: source side, then destination side, in
+        edge order). edge_ids may be an int: the first of len(src) consecutive ids. The batch is validated on the host
+        before any device write (check_edges), copied to the device (a synchronous copy from pageable memory), and the
+        append is enqueued on the current stream."""
+        self._require_growable()
+        src, dst, eid, t = check_edges(src, dst, edge_ids, times, self.num_rows, self._last_t)
+        n = len(src)
+        if n == 0:
+            return
+        self.reserve(src, dst)
+        dev = self.device
+        a = [torch.from_numpy(x).to(dev, non_blocking=False) for x in (src, dst, eid, t)]
+        with torch.cuda.device(dev):
+            rc = self._lib.lstep_csr_ingest(self.csr_ref, _lib.ptr(self.fill), _lib.ptr(a[0]), _lib.ptr(a[1]), _lib.ptr(a[2]), 0,
+                                            _lib.ptr(a[3]), n, _lib.ptr(self._err), _lib.stream_ptr())
+        _lib.check(rc, "lstep_csr_ingest")
+        self._note_ingested(src, dst, int(eid[-1]), float(t[-1]))
+        self._version += 1
 
     @classmethod
     def from_reference(cls, ref_sampler, device=None):
@@ -148,6 +345,10 @@ class NeighborSampler:
             self._err.zero_()
         if flag & _lib.FLAG_NODE_OUT_OF_RANGE:
             raise IndexError("list index out of range")  # utils/utils.py:140 on an unknown node id (SURVEY Q8)
+        if flag & _lib.FLAG_CSR_FULL:
+            raise _lib.LstepError("an append to the growable CSR found a row without room (reserve before appending)")
+        if flag & _lib.FLAG_UNSORTED_STREAM:
+            raise ValueError("an append to the growable CSR was earlier than the row's last entry")
 
     def get_historical_neighbors(self, node_ids: np.ndarray, node_interact_times: np.ndarray, num_neighbors: int = 20):
         assert num_neighbors > 0, 'Number of sampled neighbors for each node should be greater than 0!'
@@ -180,6 +381,8 @@ class NeighborSampler:
             raise IndexError("list index out of range")
         node_id %= self.num_rows
         lo, hi = (int(x) for x in self.indptr[node_id:node_id + 2].tolist())
+        if self.is_growable:
+            hi = lo + int(self._fill_h[node_id])  # the rest of the row is padding
         t = self.t[lo:hi].cpu().numpy()
         i = int(np.searchsorted(t, interact_time))
         return (self.nbr[lo:lo + i].cpu().numpy().astype(np.int64), self.eid[lo:lo + i].cpu().numpy().astype(np.int64), t[:i], None)

@@ -28,6 +28,7 @@ import torch
 from . import _lib
 from . import checkpoint as ckpt
 from .model import LSTEP
+from .sampler import check_edges
 
 C_void_p = ctypes.c_void_p
 C_byref = ctypes.byref
@@ -137,6 +138,7 @@ class PEStream:
         self.num_batches = len(self.batch_lo)
         self.batch_tmax = [float(self.t_np[lo:min(lo + self.B, self.stop)].max()) for lo in self.batch_lo]
         self._host_stepper = None
+        self._armed = None  # (stepper, sampler, sampler version) the stepper was armed to ingest into, see _arm_ingest
         self._ticket_shape = {}
         self._drained = {}  # public ticket -> result read out before its stepper was replaced
         self._epoch = 0
@@ -337,6 +339,7 @@ class PEStream:
                 self._ticket_shape.clear()
                 lib.lstep_host_stepper_destroy(st[0])
                 self._epoch += 1
+                self._armed = None
             h = C_void_p()
             cap_e, cap_c = max(self.B, n_edges), max(C, 4)
             with torch.cuda.device(self.dev):
@@ -355,8 +358,39 @@ class PEStream:
                 pass
             self._host_stepper = None
 
+    def _growable_sampler(self):
+        samp = self.model.neighbor_sampler
+        if samp is None or not samp.is_growable:
+            raise ValueError("ingest=True needs a growable neighbor sampler: model.set_neighbor_sampler(NeighborSampler.growable(...))")
+        return samp
+
+    def _check_ingest(self, src, dst, times, edge_id_start):
+        """Validate a host batch for ingestion and make room for it; returns its first edge id. Nothing is written to
+        the device unless a regrow is needed."""
+        samp = self._growable_sampler()
+        eid0 = samp.next_edge_id if edge_id_start is None else int(edge_id_start)
+        check_edges(src, dst, eid0, times, samp.num_rows, samp.last_time)
+        samp.reserve(src, dst)
+        return eid0
+
+    def _arm_ingest(self, h, eid0: int):
+        """Arm the stepper to append each batch to the sampler's CSR before its step (lstep_host_stepper_set_ingest). Re-armed
+        only when the stepper, the sampler or its arrays changed, or edge ids do not continue: arming makes the next append
+        wait for the compute stream, which costs the copy-in its overlap with the previous step."""
+        samp = self.model.neighbor_sampler
+        key = (h.value, id(samp), samp._version)
+        if self._armed != key or eid0 != samp.next_edge_id:
+            _lib.check(self._libc.lstep_host_stepper_set_ingest(h, _lib.ptr(samp.fill), eid0, samp.last_time),
+                       "lstep_host_stepper_set_ingest")
+            self._armed = key
+
+    def _disarm_ingest(self, h):
+        if self._armed is not None:
+            _lib.check(self._libc.lstep_host_stepper_set_ingest(h, None, 0, 0.0), "lstep_host_stepper_set_ingest")
+            self._armed = None
+
     def step_host_async(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None,
-                        ids: np.ndarray = None, out: torch.Tensor = None) -> int:
+                        ids: np.ndarray = None, out: torch.Tensor = None, ingest: bool = False, edge_id_start: int = None) -> int:
         """One step fed from HOST arrays (what a loop holding numpy batches calls): the batch's endpoints,
         times and the query id sets are packed into a pinned slot and uploaded by one async copy inside the
         native call, the step's kernels are enqueued behind it, and the per-query row sums [C, n] of the
@@ -364,7 +398,10 @@ class PEStream:
         synchronises); `result(ticket)` waits for that step only, so a loop can read results one step behind.
         `ids` (sorted unique batch nodes) is computed natively when omitted; `out` [C, n, d] keeps the full
         neighbourhood PEs on the device. This is the per-batch host path: it avoids every avoidable Python
-        call (≈ 25 µs of interpreter time per step)."""
+        call (≈ 25 µs of interpreter time per step).
+        ingest=True: the batch's edges are not in the sampler yet. The model's sampler must be growable
+        (NeighborSampler.growable); the batch is validated, room is reserved, and the native call appends it to the CSR
+        (edge ids edge_id_start + i, default: the sampler's next_edge_id) before the step's lookups run."""
         lib = self._libc
         m = self.model
         n = len(src)
@@ -380,6 +417,8 @@ class PEStream:
             raise ValueError("step_host: src, dst, times and every query set must have the same length")
         if ids is not None:
             ids = np.ascontiguousarray(ids, dtype=_I64)
+        if ingest:
+            eid0 = self._check_ingest(src, dst, times, edge_id_start)
         T = self.T
         bi = self.batch_idx if batch_idx is None else batch_idx
         bmask = min(max(bi, 0), T) if self.len < T else T
@@ -390,6 +429,10 @@ class PEStream:
             h = self._stepper(n, C)
         else:
             h = st[0]
+        if ingest:
+            self._arm_ingest(h, eid0)
+        elif self._armed is not None:
+            self._disarm_ingest(h)
         G = m._collapsed_filter(bmask, False)
         ws = self._ws
         if ws is None or n > self._ws_cap[1] or C > self._ws_cap[2] or 2 * n > self._ws_cap[0]:
@@ -407,7 +450,11 @@ class PEStream:
                                     m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(), samp._err.data_ptr(),
                                     torch.cuda.current_stream().cuda_stream, C_byref(ticket))
         if rc != 0:
+            if ingest:  # the append may have been enqueued before the step failed
+                samp._resync(src, dst, eid0, times)
             _lib.check(rc, "lstep_pe_step_host")
+        if ingest:
+            samp._note_ingested(src, dst, eid0 + n - 1, times[-1])
         self.head, self.len = new_head, new_len
         self.batch_idx = bi + 1
         self.steps_done += 1
@@ -418,12 +465,14 @@ class PEStream:
         m.h2d_bytes += 8 * n * (5 + C)  # what lstep_pe_step_host copies: src, dst, t, <= 2n ids, C query sets
         return tk
 
-    def run_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids) -> np.ndarray:
+    def run_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, ingest: bool = False,
+                 edge_id_start: int = None) -> np.ndarray:
         """A run of consecutive batches fed from HOST arrays in ONE native call (an evaluation split): batch b is edges
         [b*B, (b+1)*B) of the given arrays; every step copies its own inputs in and its own per-query row sums out
         (read one step behind inside the call). Returns [n_batches, C, B] float32 (tail of a ragged last batch zero).
         While the history ring is still filling (the filter changes with every step) the batches go through
-        step_host_async one by one."""
+        step_host_async one by one. ingest=True: as in step_host_async; room for the whole run is reserved first, so the
+        native loop never needs a regrow."""
         n_total, B, C = len(src), self.B, len(query_ids)
         src = np.ascontiguousarray(src, dtype=_I64)
         dst = np.ascontiguousarray(dst, dtype=_I64)
@@ -431,13 +480,15 @@ class PEStream:
         qs = [np.ascontiguousarray(q, dtype=_I64) for q in query_ids]
         if len(dst) != n_total or len(times) != n_total or any(len(q) != n_total for q in qs):
             raise ValueError("run_host: src, dst, times and every query set must have the same length")
+        eid0 = self._check_ingest(src, dst, times, edge_id_start) if ingest else None
         nb = (n_total + B - 1) // B
         res = np.zeros((nb, C, B), dtype=np.float32)
         lo = 0
         pend = []
         while lo < n_total and self.len < self.T:  # masked regime: per-step calls
             hi = min(lo + B, n_total)
-            pend.append((lo // B, hi - lo, self.step_host_async(src[lo:hi], dst[lo:hi], times[lo:hi], [q[lo:hi] for q in qs])))
+            pend.append((lo // B, hi - lo, self.step_host_async(src[lo:hi], dst[lo:hi], times[lo:hi], [q[lo:hi] for q in qs], ingest=ingest,
+                                                                 edge_id_start=None if eid0 is None else eid0 + lo)))
             if len(pend) > 1:
                 b, n, tk = pend.pop(0)
                 res[b, :, :n] = self.result(tk)
@@ -450,6 +501,10 @@ class PEStream:
         if torch.cuda.current_device() != self.dev.index:
             torch.cuda.set_device(self.dev)
         h = self._stepper(B, C)
+        if ingest:
+            self._arm_ingest(h, eid0 + lo)
+        elif self._armed is not None:
+            self._disarm_ingest(h)
         G = m._collapsed_filter(self.T, False)
         ws = self._workspace(2 * B, B, C)
         qptrs = (C_void_p * max(C, 1))(*[q[lo:].ctypes.data for q in qs])
@@ -465,7 +520,12 @@ class PEStream:
         self.head = head.value
         self.batch_idx += steps
         self.steps_done += steps
-        m.h2d_bytes += 8 * min(steps * B, n_total - lo) * (5 + C)
+        n_app = min(steps * B, n_total - lo)
+        m.h2d_bytes += 8 * n_app * (5 + C)
+        if ingest and rc != 0:  # the failed batch's append may have been enqueued although its step was not applied
+            samp._resync(src[lo:], dst[lo:], eid0 + lo, times[lo:])
+        elif ingest and n_app > 0:
+            samp._note_ingested(src[lo:lo + n_app], dst[lo:lo + n_app], eid0 + lo + n_app - 1, times[lo + n_app - 1])
         if rc != 0:
             _lib.check(rc, "lstep_pe_steps_host")
         return res
@@ -490,9 +550,10 @@ class PEStream:
             return np.zeros((C, n), np.float32)
         return np.ctypeslib.as_array(p, shape=(C, n)).copy()
 
-    def step_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None, ids: np.ndarray = None):
+    def step_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None, ids: np.ndarray = None,
+                  ingest: bool = False, edge_id_start: int = None):
         """Synchronous form: run the step and return its per-query row sums [len(query_ids), n]."""
-        return self.result(self.step_host_async(src, dst, times, query_ids, batch_idx, ids))
+        return self.result(self.step_host_async(src, dst, times, query_ids, batch_idx, ids, ingest=ingest, edge_id_start=edge_id_start))
 
 
 class ChangeLogStream(PEStream):
