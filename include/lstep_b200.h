@@ -480,6 +480,16 @@ int lstep_host_step_result(lstep_host_stepper* h, int64_t ticket, const float** 
  * disarms. */
 int lstep_host_stepper_set_ingest(lstep_host_stepper* h, int32_t* fill, int64_t next_eid, double last_t);
 void lstep_host_stepper_bytes(const lstep_host_stepper* h, uint64_t* h2d_bytes, uint64_t* d2h_bytes);
+/* lstep_pe_step_host on a change-log history (lstep_pe_step_changelog; cl->row_mul == 1): the same staging, host checks,
+ * optional append (lstep_host_stepper_set_ingest) and result path, around the change-log step: filter of the batch nodes into
+ * the table, the step's kernels, retire + append. Its events go to slot (head + len) % T while the log fills, to `head` (after
+ * retiring it) once len == T. s->src / s->dst / s->t are never read, so a descriptor over an empty edge stream serves it. */
+int lstep_pe_step_changelog_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr,
+                                 int64_t n_edges, const int64_t* src_host, const int64_t* dst_host, const double* t_host,
+                                 const int64_t* ids_host, int64_t n_ids, int head, int len, const float* G,
+                                 const int64_t* const* query_ids_host_arrays, int n_queries, float* nbr_out, int K,
+                                 const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes,
+                                 uint32_t* err_flag, void* stream, int64_t* ticket);
 /* A run of consecutive batches in one call (an evaluation split, evaluate_model_utils.py:38-142): the loop over
  * lstep_pe_step_host / lstep_host_step_result is done natively, results read one step behind. Full history ring only
  * (*len_io == T, one collapsed filter G); batch b = edges [b*batch_size, min((b+1)*batch_size, n_total)) of the host
@@ -491,6 +501,15 @@ int lstep_pe_steps_host(lstep_host_stepper* h, const lstep_pe_stream* s, const l
                         const int64_t* const* query_ids_host_arrays, int n_queries, int* head_io, int* len_io,
                         const float* G, int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace,
                         size_t workspace_bytes, uint32_t* err_flag, void* stream, float* results_host, int64_t* n_done_out);
+/* lstep_pe_steps_host on a change-log history: every batch through lstep_pe_step_changelog_host. Full log only (*len_io == T,
+ * else LSTEP_ERR_UNSUPPORTED); results one step behind; on an error in batch k batches [0, k) stay applied and *head_io /
+ * *n_done_out report the position reached. */
+int lstep_pe_steps_changelog_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr,
+                                  int64_t n_total, int64_t batch_size, const int64_t* src_host, const int64_t* dst_host,
+                                  const double* t_host, const int64_t* const* query_ids_host_arrays, int n_queries, int* head_io,
+                                  int* len_io, const float* G, int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd,
+                                  void* workspace, size_t workspace_bytes, uint32_t* err_flag, void* stream, float* results_host,
+                                  int64_t* n_done_out);
 
 /* ------------------------------------------------------------------------------------------
  * Measurement / A-B plumbing (no reference counterpart).

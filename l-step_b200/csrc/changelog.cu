@@ -428,22 +428,27 @@ extern "C" int lstep_changelog_append(const lstep_changelog* cl, int slot, int r
   return check_launch("changelog_append");
 }
 
-/* lstep_pe_step on a change-log history: filter of the batch nodes into the table, the step's kernels, retire + append.
- * head / len: the window (slot of its oldest step, number of valid steps <= T); the step's events go to slot
- * (head + len) % T while the history is filling, to `head` (after retiring it) once len == T. q_off / q_rows as in
- * lstep_pe_step_sharded (q_rows < 0: all edges). filter_ids / n_filter: the batch nodes whose history THIS rank holds
- * (= ids for a single GPU); their filtered rows are written to filter_out (row i, pitch d) when filter_out != NULL — the
- * caller all-gathers and scatters them — and straight into the table otherwise. */
-extern "C" int lstep_pe_step_changelog(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, int64_t lo, int64_t n_edges,
-                                       const int64_t* ids, int64_t n_ids, double current_time, int head, int len, const float* G,
-                                       const int64_t* const* query_ids_host, int n_queries, int64_t q_off, int64_t q_rows, float* nbr_out,
-                                       int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace,
-                                       size_t workspace_bytes, uint32_t* err_flag, void* stream, int phase) {
-  // phase 0: everything; 1: filter only (into filter destination = table); 2: everything after the filter
-  if (!s || !s->src || !s->dst || !s->t || !s->cur || !valid(cl) || lo < 0 || n_edges < 0 || n_ids < 0 || !mlp_upd) return LSTEP_ERR_INVALID_ARG;
+namespace lstep {
+// The argument checks of the change-log step that do not concern the batch pointers (every caller makes them before it
+// enqueues anything, so a host-fed call rejects bad arguments before its copy-in and append).
+int changelog_step_check(const lstep_pe_stream* s, const lstep_changelog* cl, int head, int len, const lstep_pe_mlp* mlp_upd) {
+  if (!s || !s->cur || !valid(cl) || !mlp_upd) return LSTEP_ERR_INVALID_ARG;
   if (cl->d != s->d || head < 0 || head >= cl->T || len < 0 || len > cl->T) return LSTEP_ERR_INVALID_ARG;
   if (!update_push_available(mlp_upd)) return LSTEP_ERR_UNSUPPORTED;  // the append needs the push kernel's U list and stamp map
-  int rc;
+  return LSTEP_OK;
+}
+
+// The change-log step on explicit batch pointers (src/dst/tq = the batch's n_edges endpoints and times on the device): the
+// resident lstep_pe_step_changelog passes the stream's edges, the host-fed calls (csrc/host_step.cu) their staged slot.
+// Never reads s->src / s->dst / s->t.
+int changelog_step_core(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const int64_t* src, const int64_t* dst,
+                        const double* tq, int64_t n_edges, const int64_t* ids, int64_t n_ids, double current_time, int head, int len,
+                        const float* G, const int64_t* const* query_ids_host, int n_queries, int64_t q_off, int64_t q_rows, float* nbr_out,
+                        int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes,
+                        uint32_t* err_flag, void* stream, int phase) {
+  if (n_edges < 0 || n_ids < 0) return LSTEP_ERR_INVALID_ARG;
+  int rc = changelog_step_check(s, cl, head, len, mlp_upd);
+  if (rc != LSTEP_OK) return rc;
   if (phase != 2 && n_ids > 0) {
     if (cl->row_mul != 1) return LSTEP_ERR_INVALID_ARG;  // sharded groups filter through lstep_changelog_filter themselves
     if ((rc = lstep_changelog_filter(cl, head, len, ids, n_ids, G, s->cur, s->d, ids, stream)) != LSTEP_OK) return rc;
@@ -458,8 +463,8 @@ extern "C" int lstep_pe_step_changelog(const lstep_pe_stream* s, const lstep_cha
   lstep_pe_stream s2 = *s;
   if (!s2.ring) s2.ring = s2.cur;  // (never touched: the core neither filters nor appends)
   const int64_t qr = q_rows < 0 ? n_edges : q_rows;
-  rc = pe_step_core_ex(&s2, csr, s->src + lo, s->dst + lo, s->t + lo, n_edges, ids, n_ids, current_time, 0, 0, 0, nullptr, query_ids_host,
-                       qr > 0 ? n_queries : 0, nbr_out, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, stream, opt);
+  rc = pe_step_core_ex(&s2, csr, src, dst, tq, n_edges, ids, n_ids, current_time, 0, 0, 0, nullptr, query_ids_host, qr > 0 ? n_queries : 0,
+                       nbr_out, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, stream, opt);
   if (rc != LSTEP_OK) return rc;
   const int64_t* U = nullptr;
   const int32_t *n_dest = nullptr, *stamp_map = nullptr;
@@ -473,4 +478,22 @@ extern "C" int lstep_pe_step_changelog(const lstep_pe_stream* s, const lstep_cha
   const int slot = full ? head : (head + len) % cl->T;
   return lstep_changelog_append(cl, slot, full ? 1 : 0, s->cur, U, n_dest, n_u_max, ids, n_ids, stamp_map, stamp, n_ids > 0 ? 1 : 0, err_flag,
                                 stream);
+}
+}  // namespace lstep
+
+/* lstep_pe_step on a change-log history: filter of the batch nodes into the table, the step's kernels, retire + append.
+ * head / len: the window (slot of its oldest step, number of valid steps <= T); the step's events go to slot
+ * (head + len) % T while the history is filling, to `head` (after retiring it) once len == T. q_off / q_rows as in
+ * lstep_pe_step_sharded (q_rows < 0: all edges). filter_ids / n_filter: the batch nodes whose history THIS rank holds
+ * (= ids for a single GPU); their filtered rows are written to filter_out (row i, pitch d) when filter_out != NULL — the
+ * caller all-gathers and scatters them — and straight into the table otherwise. */
+extern "C" int lstep_pe_step_changelog(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, int64_t lo, int64_t n_edges,
+                                       const int64_t* ids, int64_t n_ids, double current_time, int head, int len, const float* G,
+                                       const int64_t* const* query_ids_host, int n_queries, int64_t q_off, int64_t q_rows, float* nbr_out,
+                                       int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace,
+                                       size_t workspace_bytes, uint32_t* err_flag, void* stream, int phase) {
+  // phase 0: everything; 1: filter only (into filter destination = table); 2: everything after the filter
+  if (!s || !s->src || !s->dst || !s->t || !s->cur || !valid(cl) || lo < 0 || n_edges < 0 || n_ids < 0 || !mlp_upd) return LSTEP_ERR_INVALID_ARG;
+  return changelog_step_core(s, cl, csr, s->src + lo, s->dst + lo, s->t + lo, n_edges, ids, n_ids, current_time, head, len, G, query_ids_host,
+                             n_queries, q_off, q_rows, nbr_out, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, stream, phase);
 }

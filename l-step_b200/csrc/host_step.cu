@@ -8,6 +8,8 @@
 // sums a caller reads back, and copies those to a pinned result slot, all on the caller's stream, without
 // synchronising. lstep_host_step_result waits for a ticket's event and hands out the pinned result, so a
 // loop can keep `slots - 1` steps in flight (results read one step behind hide the host's own time).
+// lstep_pe_step_changelog_host is the same hand-over around the change-log step (changelog_step_core, csrc/changelog.cu):
+// host_stage and host_finish below are the two halves both share, the step between them is the only difference.
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
@@ -16,14 +18,9 @@
 #include <vector>
 
 #include "common.cuh"
+#include "step_core.cuh"
 
 namespace lstep {
-
-int pe_step_core(const lstep_pe_stream* s, const lstep_csr* csr, const int64_t* src, const int64_t* dst, const double* tq,
-                 int64_t n_edges, const int64_t* ids, int64_t n_ids, double current_time, int head, int len, int append_slot,
-                 const float* G, const int64_t* const* query_ids_host, int n_queries, float* nbr_out, int K,
-                 const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes,
-                 uint32_t* err_flag, void* stream);
 
 // The batch moves in and the result moves out through KERNELS that read / write the pinned slots directly
 // (pinned host memory is device-addressable under unified virtual addressing): a copy-engine transfer between
@@ -204,20 +201,27 @@ extern "C" int lstep_host_stepper_create(int slots, int64_t max_edges, int max_q
   return LSTEP_OK;
 }
 
-extern "C" int lstep_pe_step_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_csr* csr, int64_t n_edges,
-                                  const int64_t* src_host, const int64_t* dst_host, const double* t_host,
-                                  const int64_t* ids_host, int64_t n_ids, int head, int len, int append_slot, const float* G,
-                                  const int64_t* const* query_ids_host_arrays, int n_queries, float* nbr_out, int K,
-                                  const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace,
-                                  size_t workspace_bytes, uint32_t* err_flag, void* stream, int64_t* ticket) {
-  if (!h || !s || !ticket || n_edges <= 0 || n_edges > h->max_edges || n_queries < 0 || n_queries > h->max_queries)
-    return LSTEP_ERR_INVALID_ARG;
+// A batch staged by host_stage: its slot and, in the slot's device copy, src | dst | t | ids | query sets.
+struct HostBatch {
+  int slot;
+  int64_t n_ids;
+  double tmax;
+  const int64_t* dp;
+  const int64_t* qdev[8];
+  bool use_memcpy;
+};
+
+// The first half of a host-fed step: slot wait, pack, the host id-range and ingest checks, copy-in, the optional append on
+// ing_stream, and the hand-over to the compute stream (in_ready). A call rejected by a check has enqueued nothing.
+static int host_stage(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_csr* csr, int64_t n_edges, const int64_t* src_host,
+                      const int64_t* dst_host, const double* t_host, const int64_t* ids_host, int64_t n_ids,
+                      const int64_t* const* query_ids_host_arrays, int n_queries, uint32_t* err_flag, cudaStream_t st, HostBatch* hb) {
+  if (!h || !s || n_edges <= 0 || n_edges > h->max_edges || n_queries < 0 || n_queries > h->max_queries) return LSTEP_ERR_INVALID_ARG;
   if (!src_host || !dst_host || !t_host || (n_queries > 0 && !query_ids_host_arrays)) return LSTEP_ERR_INVALID_ARG;
   if (ids_host && (n_ids < 0 || n_ids > 2 * n_edges)) return LSTEP_ERR_INVALID_ARG;
   for (int c = 0; c < n_queries; ++c)
     if (!query_ids_host_arrays[c]) return LSTEP_ERR_INVALID_ARG;
   if (s->d != h->d) return LSTEP_ERR_INVALID_ARG;
-  cudaStream_t st = as_stream(stream);
   const int slot = (int)(h->next_ticket % h->slots);
   cudaError_t e;
   if (h->ticket_of[slot] >= 0) {  // the slot's previous step (copy in, kernels, copy out) must have drained
@@ -287,6 +291,9 @@ extern "C" int lstep_pe_step_host(lstep_host_stepper* h, const lstep_pe_stream* 
     // reader counts the entries of a row with t < tq (strict) and reads nothing at or after that count, so the written
     // slots count as "not earlier" both before and after the write (an aligned 8-byte store is seen whole or not at all),
     // and step b selects the same entries whichever it sees. fill[] is read by the appends only.
+    // The change-log step (lstep_pe_step_changelog_host) reads the CSR in the same two places only, the a6 gather and
+    // phase B's push, through the same strict-< counts; its filter, retire and append kernels read the change log and the
+    // table, never the CSR. So the same argument covers it and its appends overlap the same way.
     const void* arrays[4] = {csr->indptr, csr->nbr, csr->eid, csr->t};
     bool changed = false;
     for (int k = 0; k < 4; ++k) changed |= arrays[k] != h->ing_arrays[k];
@@ -310,19 +317,27 @@ extern "C" int lstep_pe_step_host(lstep_host_stepper* h, const lstep_pe_stream* 
   if ((e = cudaStreamWaitEvent(st, h->in_ready[slot], 0)) != cudaSuccess) return cuda_fail(e, "pe_step_host wait");
   h->h2d_bytes += bytes;
   const int64_t* dp = reinterpret_cast<const int64_t*>(h->d_in[slot]);
-  const int64_t* qdev[8];
   for (int c = 0; c < n_queries; ++c) {
     // the same host array passed twice (negative sources == sources under random negative sampling) becomes the same
     // device pointer, which is what pe_step_core recognises as an identical query set
     int u = 0;
     while (u < c && query_ids_host_arrays[u] != query_ids_host_arrays[c]) ++u;
-    qdev[c] = dp + 5 * n + (size_t)u * n;
+    hb->qdev[c] = dp + 5 * n + (size_t)u * n;
   }
-  float* outp = nbr_out ? nbr_out : h->d_nbr[slot];
-  int rc = pe_step_core(s, csr, dp, dp + n, reinterpret_cast<const double*>(dp + 2 * n), n_edges, dp + 3 * n, n_ids, tmax, head,
-                        len, append_slot, G, qdev, n_queries, outp, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag,
-                        stream);
-  if (rc != LSTEP_OK) return rc;
+  hb->slot = slot;
+  hb->n_ids = n_ids;
+  hb->tmax = tmax;
+  hb->dp = dp;
+  hb->use_memcpy = use_memcpy;
+  return LSTEP_OK;
+}
+
+// The second half: the per-query row sums of outp into the slot's pinned result, the slot's done event and the ticket.
+static int host_finish(lstep_host_stepper* h, const HostBatch& hb, int64_t n_edges, int n_queries, float* nbr_out, const float* outp,
+                       cudaStream_t st, int64_t* ticket) {
+  const int slot = hb.slot;
+  cudaError_t e;
+  int rc;
   const int64_t rows = (int64_t)n_queries * n_edges;
   // result path on its own stream, behind the step: the next step does not queue behind it. (A caller-owned
   // nbr_out is reused by the caller's next step, so in that case the result kernel stays on the compute stream.)
@@ -333,9 +348,9 @@ extern "C" int lstep_pe_step_host(lstep_host_stepper* h, const lstep_pe_stream* 
   }
   if (rows > 0) {
     // the row sums go straight into the pinned result slot (visible to the host once the event below has fired)
-    row_sum_kernel<<<(unsigned)ceil_div(rows * 32, 256), 256, 0, rs>>>(outp, rows, h->d, use_memcpy ? h->d_res[slot] : h->h_res[slot]);
+    row_sum_kernel<<<(unsigned)ceil_div(rows * 32, 256), 256, 0, rs>>>(outp, rows, h->d, hb.use_memcpy ? h->d_res[slot] : h->h_res[slot]);
     if ((rc = check_launch("row_sum")) != LSTEP_OK) return rc;
-    if (use_memcpy &&
+    if (hb.use_memcpy &&
         (e = cudaMemcpyAsync(h->h_res[slot], h->d_res[slot], sizeof(float) * (size_t)rows, cudaMemcpyDeviceToHost, rs)) != cudaSuccess)
       return cuda_fail(e, "pe_step_host d2h");
     h->d2h_bytes += sizeof(float) * (size_t)rows;
@@ -345,6 +360,48 @@ extern "C" int lstep_pe_step_host(lstep_host_stepper* h, const lstep_pe_stream* 
   h->ticket_of[slot] = h->next_ticket;
   *ticket = h->next_ticket++;
   return LSTEP_OK;
+}
+
+extern "C" int lstep_pe_step_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_csr* csr, int64_t n_edges,
+                                  const int64_t* src_host, const int64_t* dst_host, const double* t_host,
+                                  const int64_t* ids_host, int64_t n_ids, int head, int len, int append_slot, const float* G,
+                                  const int64_t* const* query_ids_host_arrays, int n_queries, float* nbr_out, int K,
+                                  const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace,
+                                  size_t workspace_bytes, uint32_t* err_flag, void* stream, int64_t* ticket) {
+  if (!ticket) return LSTEP_ERR_INVALID_ARG;
+  const cudaStream_t st = as_stream(stream);
+  HostBatch hb;
+  int rc = host_stage(h, s, csr, n_edges, src_host, dst_host, t_host, ids_host, n_ids, query_ids_host_arrays, n_queries, err_flag, st, &hb);
+  if (rc != LSTEP_OK) return rc;
+  const int64_t* dp = hb.dp;
+  float* outp = nbr_out ? nbr_out : h->d_nbr[hb.slot];
+  rc = pe_step_core(s, csr, dp, dp + n_edges, reinterpret_cast<const double*>(dp + 2 * n_edges), n_edges, dp + 3 * n_edges, hb.n_ids, hb.tmax,
+                    head, len, append_slot, G, hb.qdev, n_queries, outp, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, stream);
+  if (rc != LSTEP_OK) return rc;
+  return host_finish(h, hb, n_edges, n_queries, nbr_out, outp, st, ticket);
+}
+
+extern "C" int lstep_pe_step_changelog_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr,
+                                            int64_t n_edges, const int64_t* src_host, const int64_t* dst_host, const double* t_host,
+                                            const int64_t* ids_host, int64_t n_ids, int head, int len, const float* G,
+                                            const int64_t* const* query_ids_host_arrays, int n_queries, float* nbr_out, int K,
+                                            const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace,
+                                            size_t workspace_bytes, uint32_t* err_flag, void* stream, int64_t* ticket) {
+  if (!h || !s || !cl || !csr || !G || !mlp_nbr || K <= 0 || !ticket) return LSTEP_ERR_INVALID_ARG;
+  int rc = changelog_step_check(s, cl, head, len, mlp_upd);
+  if (rc != LSTEP_OK) return rc;
+  if (cl->row_mul != 1) return LSTEP_ERR_INVALID_ARG;  // one GPU's whole history (a peer group steps through lstep_pe_step_peer)
+  const cudaStream_t st = as_stream(stream);
+  HostBatch hb;
+  rc = host_stage(h, s, csr, n_edges, src_host, dst_host, t_host, ids_host, n_ids, query_ids_host_arrays, n_queries, err_flag, st, &hb);
+  if (rc != LSTEP_OK) return rc;
+  const int64_t* dp = hb.dp;
+  float* outp = nbr_out ? nbr_out : h->d_nbr[hb.slot];
+  rc = changelog_step_core(s, cl, csr, dp, dp + n_edges, reinterpret_cast<const double*>(dp + 2 * n_edges), n_edges, dp + 3 * n_edges, hb.n_ids,
+                           hb.tmax, head, len, G, hb.qdev, n_queries, 0, -1, outp, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag,
+                           stream, 0);
+  if (rc != LSTEP_OK) return rc;
+  return host_finish(h, hb, n_edges, n_queries, nbr_out, outp, st, ticket);
 }
 
 extern "C" int lstep_host_step_result(lstep_host_stepper* h, int64_t ticket, const float** result_host, int64_t* n_floats) {
@@ -382,23 +439,12 @@ extern "C" void lstep_host_stepper_bytes(const lstep_host_stepper* h, uint64_t* 
   if (d2h_bytes) *d2h_bytes = h->d2h_bytes;
 }
 
-// A whole run of consecutive batches in one call (an evaluation split: evaluate_model_utils.py:38-142 loops over
-// batches of the split): the loop of lstep_pe_step_host + lstep_host_step_result lives here, results read one step
-// behind, so the host cost per batch is the CUDA launches alone. Steady-state regime only (the history ring is full:
-// *len_io == T, one collapsed filter G for every step); batch b is edges [b*batch_size, min((b+1)*batch_size, n_total)).
-// results_host: [n_batches][n_queries][batch_size] floats (the tail of a ragged last batch is left untouched).
-// Synchronous: every result has been read when the call returns.
-extern "C" int lstep_pe_steps_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_csr* csr, int64_t n_total,
-                                   int64_t batch_size, const int64_t* src_host, const int64_t* dst_host, const double* t_host,
-                                   const int64_t* const* query_ids_host_arrays, int n_queries, int* head_io, int* len_io,
-                                   const float* G, int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd,
-                                   void* workspace, size_t workspace_bytes, uint32_t* err_flag, void* stream,
-                                   float* results_host, int64_t* n_done_out) {
-  if (n_done_out) *n_done_out = 0;
-  if (!h || !s || !head_io || !len_io || !results_host || n_total < 0 || batch_size <= 0 || batch_size > h->max_edges)
-    return LSTEP_ERR_INVALID_ARG;
-  if (n_queries < 0 || n_queries > 8 || (n_queries > 0 && !query_ids_host_arrays)) return LSTEP_ERR_INVALID_ARG;
-  if (*len_io != s->T) return LSTEP_ERR_UNSUPPORTED;  // masked regime: the filter changes every step, use the per-step call
+// The loop of a multi-batch host-fed call: batch b = edges [b*batch_size, min((b+1)*batch_size, n_total)), stepped by
+// step(lo, n, query sets, head, &ticket) with the full window (the oldest slot, head, is overwritten and becomes the newest),
+// its result read one step behind into results_host [n_batches][n_queries][batch_size].
+template <class Step>
+static int steps_host_loop(lstep_host_stepper* h, int T, int64_t n_total, int64_t batch_size, const int64_t* const* query_ids_host_arrays,
+                           int n_queries, int* head_io, float* results_host, int64_t* n_done_out, Step&& step) {
   int head = *head_io;
   int64_t pending = -1, pending_b = -1, pending_n = 0;
   auto collect = [&](int64_t ticket, int64_t b, int64_t n) -> int {
@@ -416,18 +462,16 @@ extern "C" int lstep_pe_steps_host(lstep_host_stepper* h, const lstep_pe_stream*
     const int64_t* q[8];
     for (int c = 0; c < n_queries; ++c) q[c] = query_ids_host_arrays[c] + lo;
     int64_t ticket = -1;
-    // full ring: the oldest slot (head) is overwritten, then becomes the newest
-    int rc = lstep_pe_step_host(h, s, csr, n, src_host + lo, dst_host + lo, t_host + lo, nullptr, 0, head, s->T, head, G, q, n_queries,
-                                nullptr, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, stream, &ticket);
+    int rc = step(lo, n, q, head, &ticket);
     if (rc != LSTEP_OK) {
-      // batches [0, b) HAVE been applied to the ring: report the position reached (head, and the count in *len_io's place is
+      // batches [0, b) HAVE been applied to the history: report the position reached (head, and the count in *len_io's place is
       // not possible — len stays T — so the caller derives it from the returned head and n_done below) and drain the pending result
       if (pending >= 0) (void)collect(pending, pending_b, pending_n);
       *head_io = head;
       if (n_done_out) *n_done_out = b;
       return rc;
     }
-    head = (head + 1) % s->T;
+    head = (head + 1) % T;
     if (pending >= 0 && (rc = collect(pending, pending_b, pending_n)) != LSTEP_OK) {
       *head_io = head;
       if (n_done_out) *n_done_out = b + 1;
@@ -444,4 +488,53 @@ extern "C" int lstep_pe_steps_host(lstep_host_stepper* h, const lstep_pe_stream*
     if (rc != LSTEP_OK) return rc;
   }
   return LSTEP_OK;
+}
+
+// A whole run of consecutive batches in one call (an evaluation split: evaluate_model_utils.py:38-142 loops over
+// batches of the split): the loop of lstep_pe_step_host + lstep_host_step_result lives here, results read one step
+// behind, so the host cost per batch is the CUDA launches alone. Steady-state regime only (the history ring is full:
+// *len_io == T, one collapsed filter G for every step); batch b is edges [b*batch_size, min((b+1)*batch_size, n_total)).
+// results_host: [n_batches][n_queries][batch_size] floats (the tail of a ragged last batch is left untouched).
+// Synchronous: every result has been read when the call returns.
+extern "C" int lstep_pe_steps_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_csr* csr, int64_t n_total,
+                                   int64_t batch_size, const int64_t* src_host, const int64_t* dst_host, const double* t_host,
+                                   const int64_t* const* query_ids_host_arrays, int n_queries, int* head_io, int* len_io,
+                                   const float* G, int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd,
+                                   void* workspace, size_t workspace_bytes, uint32_t* err_flag, void* stream,
+                                   float* results_host, int64_t* n_done_out) {
+  if (n_done_out) *n_done_out = 0;
+  if (!h || !s || !head_io || !len_io || !results_host || n_total < 0 || batch_size <= 0 || batch_size > h->max_edges)
+    return LSTEP_ERR_INVALID_ARG;
+  if (n_queries < 0 || n_queries > 8 || (n_queries > 0 && !query_ids_host_arrays)) return LSTEP_ERR_INVALID_ARG;
+  if (*len_io != s->T) return LSTEP_ERR_UNSUPPORTED;  // masked regime: the filter changes every step, use the per-step call
+  return steps_host_loop(h, s->T, n_total, batch_size, query_ids_host_arrays, n_queries, head_io, results_host, n_done_out,
+                         [&](int64_t lo, int64_t n, const int64_t* const* q, int head, int64_t* ticket) {
+                           return lstep_pe_step_host(h, s, csr, n, src_host + lo, dst_host + lo, t_host + lo, nullptr, 0, head, s->T, head, G,
+                                                     q, n_queries, nullptr, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag,
+                                                     stream, ticket);
+                         });
+}
+
+// lstep_pe_steps_host on a change-log history: every batch through lstep_pe_step_changelog_host with the full window (its
+// events retire slot head and take its place). Same contract: steady state only, results one step behind, and on an error in
+// batch k batches [0, k) stay applied, with *head_io / *n_done_out reporting the position reached.
+extern "C" int lstep_pe_steps_changelog_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr,
+                                             int64_t n_total, int64_t batch_size, const int64_t* src_host, const int64_t* dst_host,
+                                             const double* t_host, const int64_t* const* query_ids_host_arrays, int n_queries, int* head_io,
+                                             int* len_io, const float* G, int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd,
+                                             void* workspace, size_t workspace_bytes, uint32_t* err_flag, void* stream, float* results_host,
+                                             int64_t* n_done_out) {
+  if (n_done_out) *n_done_out = 0;
+  if (!h || !s || !cl || !head_io || !len_io || !results_host || n_total < 0 || batch_size <= 0 || batch_size > h->max_edges)
+    return LSTEP_ERR_INVALID_ARG;
+  if (n_queries < 0 || n_queries > 8 || (n_queries > 0 && !query_ids_host_arrays)) return LSTEP_ERR_INVALID_ARG;
+  const int rc = changelog_step_check(s, cl, *head_io, *len_io, mlp_upd);
+  if (rc != LSTEP_OK) return rc;
+  if (*len_io != cl->T) return LSTEP_ERR_UNSUPPORTED;  // the log is still filling: the filter changes every step, use the per-step call
+  return steps_host_loop(h, cl->T, n_total, batch_size, query_ids_host_arrays, n_queries, head_io, results_host, n_done_out,
+                         [&](int64_t lo, int64_t n, const int64_t* const* q, int head, int64_t* ticket) {
+                           return lstep_pe_step_changelog_host(h, s, cl, csr, n, src_host + lo, dst_host + lo, t_host + lo, nullptr, 0, head,
+                                                               cl->T, G, q, n_queries, nullptr, K, mlp_nbr, mlp_upd, workspace,
+                                                               workspace_bytes, err_flag, stream, ticket);
+                         });
 }

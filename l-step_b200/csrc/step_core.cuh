@@ -45,5 +45,13 @@ int pe_step_core(const lstep_pe_stream* s, const lstep_csr* csr, const int64_t* 
 void update_ws_phase_b_lists(void* workspace, int64_t n_ids, int64_t n_edges, int K, int d, int t, int64_t pe_rows, const int64_t** U,
                              const int32_t** n_dest_dev, const int32_t** stamp_map);
 bool update_push_available(const lstep_pe_mlp* mlp);
+// csrc/changelog.cu: the change-log step on explicit batch pointers (never reads s->src / s->dst / s->t), and its checks of
+// everything but the batch, which callers make before they enqueue anything
+int changelog_step_check(const lstep_pe_stream* s, const lstep_changelog* cl, int head, int len, const lstep_pe_mlp* mlp_upd);
+int changelog_step_core(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const int64_t* src, const int64_t* dst,
+                        const double* tq, int64_t n_edges, const int64_t* ids, int64_t n_ids, double current_time, int head, int len,
+                        const float* G, const int64_t* const* query_ids_host, int n_queries, int64_t q_off, int64_t q_rows, float* nbr_out,
+                        int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes,
+                        uint32_t* err_flag, void* stream, int phase);
 
 }  // namespace lstep

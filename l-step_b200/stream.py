@@ -402,7 +402,6 @@ class PEStream:
         ingest=True: the batch's edges are not in the sampler yet. The model's sampler must be growable
         (NeighborSampler.growable); the batch is validated, room is reserved, and the native call appends it to the CSR
         (edge ids edge_id_start + i, default: the sampler's next_edge_id) before the step's lookups run."""
-        lib = self._libc
         m = self.model
         n = len(src)
         C = len(query_ids)
@@ -444,15 +443,11 @@ class PEStream:
         qptrs = (C_void_p * max(C, 1))(*[q.ctypes.data for q in qs])
         ticket = ctypes.c_int64(-1)
         samp = m.neighbor_sampler
-        rc = lib.lstep_pe_step_host(h, self._desc_ref, samp.csr_ref, n, src.ctypes.data, dst.ctypes.data, times.ctypes.data,
-                                    ids.ctypes.data if ids is not None else None, len(ids) if ids is not None else 0, self.head,
-                                    self.len, slot, G.data_ptr(), qptrs, C, out.data_ptr() if out is not None else None, self.K,
-                                    m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(), samp._err.data_ptr(),
-                                    torch.cuda.current_stream().cuda_stream, C_byref(ticket))
+        rc = self._step_host_native(h, samp, n, src, dst, times, ids, slot, G, qptrs, C, out, ws, ticket)
         if rc != 0:
             if ingest:  # the append may have been enqueued before the step failed
                 samp._resync(src, dst, eid0, times)
-            _lib.check(rc, "lstep_pe_step_host")
+            _lib.check(rc, self._HOST_CALLS[0])
         if ingest:
             samp._note_ingested(src, dst, eid0 + n - 1, times[-1])
         self.head, self.len = new_head, new_len
@@ -497,7 +492,7 @@ class PEStream:
             res[b, :, :n] = self.result(tk)
         if lo >= n_total:
             return res
-        m, lib = self.model, self._libc
+        m = self.model
         if torch.cuda.current_device() != self.dev.index:
             torch.cuda.set_device(self.dev)
         h = self._stepper(B, C)
@@ -511,10 +506,7 @@ class PEStream:
         head, ln, done = ctypes.c_int(self.head), ctypes.c_int(self.len), ctypes.c_int64(0)
         sub = res[lo // B:]
         samp = m.neighbor_sampler
-        rc = lib.lstep_pe_steps_host(h, self._desc_ref, samp.csr_ref, n_total - lo, B, src[lo:].ctypes.data, dst[lo:].ctypes.data,
-                                     times[lo:].ctypes.data, qptrs, C, C_byref(head), C_byref(ln), G.data_ptr(), self.K,
-                                     m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(), samp._err.data_ptr(),
-                                     torch.cuda.current_stream().cuda_stream, sub.ctypes.data, C_byref(done))
+        rc = self._steps_host_native(h, samp, n_total - lo, src[lo:], dst[lo:], times[lo:], qptrs, C, head, ln, G, ws, sub, done)
         # batches applied before an error stay applied: the host-side ring position follows the device ring either way
         steps = done.value
         self.head = head.value
@@ -527,8 +519,27 @@ class PEStream:
         elif ingest and n_app > 0:
             samp._note_ingested(src[lo:lo + n_app], dst[lo:lo + n_app], eid0 + lo + n_app - 1, times[lo + n_app - 1])
         if rc != 0:
-            _lib.check(rc, "lstep_pe_steps_host")
+            _lib.check(rc, self._HOST_CALLS[1])
         return res
+
+    # The native calls of the host-fed steps, the only part ChangeLogStream replaces: the staging, validation, ingest arming,
+    # workspace and ticket bookkeeping above are shared. Each returns the native status.
+    _HOST_CALLS = ("lstep_pe_step_host", "lstep_pe_steps_host")
+
+    def _step_host_native(self, h, samp, n, src, dst, times, ids, slot, G, qptrs, C, out, ws, ticket):
+        m = self.model
+        return self._libc.lstep_pe_step_host(h, self._desc_ref, samp.csr_ref, n, src.ctypes.data, dst.ctypes.data, times.ctypes.data,
+                                             ids.ctypes.data if ids is not None else None, len(ids) if ids is not None else 0, self.head,
+                                             self.len, slot, G.data_ptr(), qptrs, C, out.data_ptr() if out is not None else None, self.K,
+                                             m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(), samp._err.data_ptr(),
+                                             torch.cuda.current_stream().cuda_stream, C_byref(ticket))
+
+    def _steps_host_native(self, h, samp, n_total, src, dst, times, qptrs, C, head, ln, G, ws, sub, done):
+        m = self.model
+        return self._libc.lstep_pe_steps_host(h, self._desc_ref, samp.csr_ref, n_total, self.B, src.ctypes.data, dst.ctypes.data,
+                                              times.ctypes.data, qptrs, C, C_byref(head), C_byref(ln), G.data_ptr(), self.K,
+                                              m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(), samp._err.data_ptr(),
+                                              torch.cuda.current_stream().cuda_stream, sub.ctypes.data, C_byref(done))
 
     def result(self, ticket: int) -> np.ndarray:
         """Per-query row sums [C, n] of step `ticket` (waits for that step's device-to-host copy)."""
@@ -560,7 +571,7 @@ class ChangeLogStream(PEStream):
     """PEStream on a CHANGE-LOG history (csrc/changelog.cu) instead of the dense ring: base rows + the rows every step
     changed, V1 + T * (rows changed per step) rows instead of V1 * T — 7.8 GB instead of 688 GB for the 10 M-node graph at
     T = 100, and ~9 MB written per step instead of 13.8 GB (the dense ring's append copies one row per node per step).
-    Same API (step, cur, export_history / import_history); the DFT filter sums (events in window + 1) rows per node with
+    Same API (step, the host-fed step_host_async / step_host / run_host with ingest=, cur, export_history / import_history); the DFT filter sums (events in window + 1) rows per node with
     span sums of G as weights. `event_capacity`: events one step may record (default: every row a batch can touch,
     2B + 2BK + 2, capped at V1); importing a dense history needs capacity for the rows that differ between consecutive
     snapshots. `row_mul` / `row_add`: node-id sharded groups keep only the nodes v % row_mul == row_add.
@@ -695,7 +706,36 @@ class ChangeLogStream(PEStream):
             self.check_errors()
         return out if out is not None else last
 
-    def step_host_async(self, *a, **k):
-        raise NotImplementedError("host-fed steps run on the dense-ring PEStream")
+    # ---- host-fed steps: PEStream's, with the change-log step as the native call --------------------------------------
+    def step_host_async(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, *args, **kw) -> int:
+        """PEStream.step_host_async on the change-log history (lstep_pe_step_changelog_host), ingest=True included. A step
+        records its events in the log: event_capacity, sized from batch_size by default, bounds them, so a batch longer than
+        batch_size is rejected before anything is enqueued. edges_done advances by the edges stepped."""
+        if len(src) > self.B:
+            raise ValueError(f"ChangeLogStream: a host batch of {len(src)} edges is longer than batch_size ({self.B}), which sizes the "
+                             f"change log's event_capacity ({self.cap}); split the batch or build the stream with a larger batch_size")
+        return super().step_host_async(src, dst, times, query_ids, *args, **kw)
 
-    run_host = step_host = step_host_async
+    _HOST_CALLS = ("lstep_pe_step_changelog_host", "lstep_pe_steps_changelog_host")
+
+    def _step_host_native(self, h, samp, n, src, dst, times, ids, slot, G, qptrs, C, out, ws, ticket):
+        m = self.model
+        rc = self._libc.lstep_pe_step_changelog_host(h, self._desc_ref, C_byref(self.cl), samp.csr_ref, n, src.ctypes.data, dst.ctypes.data,
+                                                     times.ctypes.data, ids.ctypes.data if ids is not None else None,
+                                                     len(ids) if ids is not None else 0, self.head, self.len, G.data_ptr(), qptrs, C,
+                                                     out.data_ptr() if out is not None else None, self.K, m._mlp_ref("nbr"),
+                                                     m._mlp_ref("update"), ws.data_ptr(), ws.numel(), samp._err.data_ptr(),
+                                                     torch.cuda.current_stream().cuda_stream, C_byref(ticket))
+        if rc == 0:
+            self.edges_done += n
+        return rc
+
+    def _steps_host_native(self, h, samp, n_total, src, dst, times, qptrs, C, head, ln, G, ws, sub, done):
+        m = self.model
+        rc = self._libc.lstep_pe_steps_changelog_host(h, self._desc_ref, C_byref(self.cl), samp.csr_ref, n_total, self.B, src.ctypes.data,
+                                                      dst.ctypes.data, times.ctypes.data, qptrs, C, C_byref(head), C_byref(ln), G.data_ptr(),
+                                                      self.K, m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(),
+                                                      samp._err.data_ptr(), torch.cuda.current_stream().cuda_stream, sub.ctypes.data,
+                                                      C_byref(done))
+        self.edges_done += min(done.value * self.B, n_total)
+        return rc
