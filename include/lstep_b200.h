@@ -44,6 +44,12 @@ typedef enum lstep_status {
 #define LSTEP_FLAG_CHANGELOG_FULL 4u /* a step changed more rows than the change-log history has event capacity for */
 #define LSTEP_FLAG_PEER_TIMEOUT 8u   /* a peer GPU did not reach a step barrier within the time limit (peer group step) */
 #define LSTEP_FLAG_CSR_FULL 16u      /* an append to a growable CSR found no room in a row; nothing was written to that row */
+/* Phase B of update_pe adds its contributions in 32.32 fixed point (int64). A call with n rows of K slots raises this flag
+ * when a contribution it adds that way is non-finite or has |x| >= 2^31 / (n*K + 1) (fp32, rounded toward zero): below that
+ * bound every column sum provably fits in int64, at or above it the sum may wrap and the updated rows are not the
+ * reference's. The push form checks every batch row's phase-A values and time features; the pull form checks the
+ * contributions to lists longer than 4 slots (shorter lists and the padding row are fp32 sums there). */
+#define LSTEP_FLAG_FIXED_POINT_RANGE 32u
 
 const char* lstep_strerror(int status);
 const char* lstep_last_cuda_error(void);

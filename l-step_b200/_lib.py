@@ -207,3 +207,15 @@ FLAG_UNSORTED_STREAM = 2
 FLAG_CHANGELOG_FULL = 4
 FLAG_PEER_TIMEOUT = 8
 FLAG_CSR_FULL = 16
+FLAG_FIXED_POINT_RANGE = 32
+
+
+def fixed_point_bound(n_ids: int, K: int) -> float:
+    """The magnitude phase B's 32.32 fixed-point sums take: 2^31 / (n_ids*K + 1), rounded toward zero to fp32
+    (fixed_point_bound() in csrc/common.cuh). A contribution x is in range when |x| < bound."""
+    import numpy as np
+    b = 2.0 ** 31 / (float(n_ids) * int(K) + 1.0)
+    f = np.float32(b)
+    if float(f) > b:
+        f = np.nextafter(f, np.float32(0))
+    return float(f)

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <cmath>
 #include <utility>
 
 #include "lstep_b200.h"
@@ -165,6 +166,16 @@ struct RowIds {
 constexpr int kPushRow0Parts = 32;
 constexpr int kPushRow0Cols = 256;  // >= d
 constexpr size_t kPushRow0Bytes = sizeof(unsigned long long) * kPushRow0Parts * kPushRow0Cols;
+// Range of phase B's 32.32 fixed-point sums (both forms): a call adds at most n_ids*K contributions to one column, each
+// converted as round(x * 2^32). With |x| < 2^31 / (n_ids*K + 1) every converted value is below 2^63 / (n_ids*K + 1) + 1/2,
+// so every column sum (and z * fx of the padding row) stays inside int64 for any n_ids*K < 2^31 (check_update_args). The
+// kernels raise LSTEP_FLAG_FIXED_POINT_RANGE for a contribution that fails `|x| < bound` (NaN included); they only compare,
+// the values they add are unchanged. Rounded toward zero to fp32 (l-step_b200/_lib.py::fixed_point_bound computes the same).
+inline float fixed_point_bound(int64_t n_ids, int K) {
+  const double b = 2147483648.0 / ((double)n_ids * K + 1.0);
+  const float f = (float)b;
+  return (double)f > b ? std::nextafter(f, 0.f) : f;
+}
 // update_pe inside a peer group (csrc/peer.cu): this rank accumulates / rewrites only the phase-B destinations u with
 // u % mul == add and applies only the phase-A rows of the batch nodes it owns; new_rows holds phase A's rows of ALL batch
 // nodes (row i = ids[i], written by their owners through peer memory).

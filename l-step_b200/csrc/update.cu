@@ -20,7 +20,7 @@
 //     ranks, and when the cluster MLP does not cover the shape; LSTEP_PHASEB_PULL=1): an inverse index
 //     (destination -> slots) is built with integer atomics on a per-node counter map (count / scan / fill), one
 //     warp per destination sorts its slot list (ascending flat index = the reference's add order) and reduces it;
-//     longer lists (hubs) are summed in 32.32 fixed point. The padding row 0 collects every empty slot —
+//     longer lists (hubs) are summed in 32.32 fixed point (range: fixed_point_bound, csrc/common.cuh). The padding row 0 collects every empty slot —
 //     thousands of contributions at B=200 — and is reduced by a two-level tree.
 // All gathers of a phase finish (kernel boundary) before its rows are written, which is what
 // makes the in-place write-back safe for nodes that are both source and destination (Q6).
@@ -293,7 +293,8 @@ __global__ void __launch_bounds__(256, DVPL <= 2 ? 2 : 1) phaseB_gather_kernel(
     const int32_t* __restrict__ off, const int32_t* __restrict__ list, const int32_t* __restrict__ hubs,
     int32_t* __restrict__ hub_remaining, const int32_t* __restrict__ task_hub, const int32_t* __restrict__ task_chunk,
     unsigned long long* __restrict__ hub_acc, const int32_t* __restrict__ counters, float tc, const float* __restrict__ tw, int d,
-    int t, const float* __restrict__ row0_part, float* __restrict__ A, int64_t lda, int warp_blocks, int hub_blocks) {
+    int t, const float* __restrict__ row0_part, float* __restrict__ A, int64_t lda, int warp_blocks, int hub_blocks, float fx_bound,
+    uint32_t* err_flag) {
   pdl_launch_dependents();
   pdl_wait();
   const int in1 = d + t;
@@ -362,9 +363,10 @@ __global__ void __launch_bounds__(256, DVPL <= 2 ? 2 : 1) phaseB_gather_kernel(
     return;
   }
 
-  // ---- hub chunk tasks
+  // ---- hub chunk tasks (fixed point: a contribution outside fixed_point_bound, csrc/common.cuh, raises the range flag)
   constexpr float kScale = 4294967296.f;           // 2^32
   constexpr float kInv = 2.3283064365386963e-10f;  // 2^-32
+  bool bad = false;
   for (int task = ((int)blockIdx.x - warp_blocks) * nw + wid; task < n_tasks; task += hub_blocks * nw) {
     const int h = ld_dep(task_hub + task), c0 = ld_dep(task_chunk + task) << kChunkLog2;
     const int s = ld_dep(hubs + h);
@@ -403,6 +405,8 @@ __global__ void __launch_bounds__(256, DVPL <= 2 ? 2 : 1) phaseB_gather_kernel(
 #pragma unroll
           for (int q = 0; q < DVPL; ++q)
             if (lane + 32 * q < dvec) {
+              bad |= !(fabsf(v[u][q].x) < fx_bound) || !(fabsf(v[u][q].y) < fx_bound) || !(fabsf(v[u][q].z) < fx_bound) ||
+                     !(fabsf(v[u][q].w) < fx_bound);
               facc[q][0] += __float2ll_rn(v[u][q].x * kScale);
               facc[q][1] += __float2ll_rn(v[u][q].y * kScale);
               facc[q][2] += __float2ll_rn(v[u][q].z * kScale);
@@ -410,7 +414,11 @@ __global__ void __launch_bounds__(256, DVPL <= 2 ? 2 : 1) phaseB_gather_kernel(
             }
 #pragma unroll
           for (int q = 0; q < TFPL; ++q)
-            if (lane + 32 * q < t) ftf[q] += __float2ll_rn(time_feature(dt[u], w[q]) * kScale);
+            if (lane + 32 * q < t) {
+              const float f = time_feature(dt[u], w[q]);
+              bad |= !(fabsf(f) <= 1.f);
+              ftf[q] += __float2ll_rn(f * kScale);
+            }
         }
       }
     }
@@ -436,6 +444,7 @@ __global__ void __launch_bounds__(256, DVPL <= 2 ? 2 : 1) phaseB_gather_kernel(
       for (int c = lane; c < in1; c += 32) arow[c] = (float)(long long)__ldcg(hrow + c) * kInv;
     }
   }
+  if (__any_sync(kFull, bad) && lane == 0 && err_flag) atomicOr(err_flag, LSTEP_FLAG_FIXED_POINT_RANGE);
 }
 
 }  // namespace lstep
@@ -564,14 +573,15 @@ static int phase_b_partial(float* pe, int64_t pe_rows, const UpdateWs& w, const 
   int hub_blocks = (int)(((total >> kChunkLog2) + total / (kHubLen + 1)) / 8) + 1;  // enough warps for every possible chunk task
   if (hub_blocks > 4 * num_sms()) hub_blocks = 4 * num_sms();
   const unsigned blocks = (unsigned)(warp_blocks + hub_blocks + 1);
+  const float bound = fixed_point_bound(n_ids, K);
   if (dvec <= 64 && t <= 128)
     launch_k(phaseB_gather_kernel<2, 4>, dim3(blocks), dim3(256), 0, st, pe, row_ids, K, w.ntB, w.off, w.list, w.hubs, w.hub_remaining, w.task_hub,
                                                        w.task_chunk, w.hub_acc, w.counters, tc, mlp->tw, d, t, w.row0_part, w.A, w.lda,
-                                                       warp_blocks, hub_blocks);
+                                                       warp_blocks, hub_blocks, bound, err_flag);
   else
     launch_k(phaseB_gather_kernel<8, 8>, dim3(blocks), dim3(256), 0, st, pe, row_ids, K, w.ntB, w.off, w.list, w.hubs, w.hub_remaining, w.task_hub,
                                                        w.task_chunk, w.hub_acc, w.counters, tc, mlp->tw, d, t, w.row0_part, w.A, w.lda,
-                                                       warp_blocks, hub_blocks);
+                                                       warp_blocks, hub_blocks, bound, err_flag);
   return check_launch("phaseB_gather");
 }
 

@@ -18,6 +18,8 @@
 //     run to run, and one rounding (at the final conversion) instead of one per addition of the
 //     reference's sequential fp32 sum. The padding destination 0 receives z_i * pe[ids[i]] (z_i = number of
 //     padded slots of row i) as one contribution per row.
+//     Exact only while every column sum fits in int64: the kernel raises LSTEP_FLAG_FIXED_POINT_RANGE when a batch row's
+//     value is non-finite or reaches fixed_point_bound(n_ids, K) (csrc/common.cuh), or a time feature is non-finite.
 // The claim map is returned to all-zero by the MLP kernel once a row has been consumed; U (row -> node id)
 // and the row count (counters[2]) are what the MLP launch reads. Accumulator rows need no invariant: a row
 // is zeroed by whoever claims it.
@@ -42,7 +44,7 @@ __global__ void __launch_bounds__(kPushThreads) phaseB_push_kernel(const int64_t
                                                           int64_t* __restrict__ U, int32_t* counters,
                                                           unsigned long long* acc, int32_t* dirty, int stamp, const float* new_rows, uint32_t* err_flag,
                                                           unsigned long long* row0_part, int own_mul, int own_add, int kPushSplit,
-                                                          int use_parts) {
+                                                          int use_parts, float fx_bound) {
   // own_mul > 1 (peer group, csrc/peer.cu): this rank accumulates only the destinations u with u % own_mul == own_add and
   // applies only the phase-A rows of the batch nodes it owns; the lookup of every batch node is replicated.
   // Dependency structure (programmatic dependent launch): the kernel in front is the phase-A MLP, launched with
@@ -225,6 +227,7 @@ __global__ void __launch_bounds__(kPushThreads) phaseB_push_kernel(const int64_t
   float w[TQ];
 #pragma unroll
   for (int q = 0; q < TQ; ++q) w[q] = (lane + 32 * q < t) ? tw[lane + 32 * q] : 0.f;
+  bool bad = false;  // a contribution outside the fixed-point range (fixed_point_bound, csrc/common.cuh); a cosine fails only when non-finite
   for (int k = warp; k < k_hi - k_lo; k += nwarps) {
     const int j = s_slot[k];
     if (j < 0) continue;
@@ -233,7 +236,11 @@ __global__ void __launch_bounds__(kPushThreads) phaseB_push_kernel(const int64_t
 #pragma unroll
     for (int q = 0; q < TQ; ++q) {
       const int jf = lane + 32 * q;
-      if (jf < t) atomicAdd(rowp + jf, (unsigned long long)__float2ll_rn(time_feature(dt, w[q]) * kFixScale));
+      if (jf < t) {
+        const float f = time_feature(dt, w[q]);
+        bad |= !(fabsf(f) <= 1.f);
+        atomicAdd(rowp + jf, (unsigned long long)__float2ll_rn(f * kFixScale));
+      }
     }
   }
 
@@ -251,8 +258,12 @@ __global__ void __launch_bounds__(kPushThreads) phaseB_push_kernel(const int64_t
 #pragma unroll
   for (int q = 0; q < DQ; ++q) {
     const int c = lane + 32 * q;
-    fx[q] = (c < d && node > 0) ? __float2ll_rn(ld_dep(src_row + c) * kFixScale) : 0ll;
+    const float x = (c < d && node > 0) ? ld_dep(src_row + c) : 0.f;
+    bad |= !(fabsf(x) < fx_bound);
+    fx[q] = __float2ll_rn(x * kFixScale);
   }
+  // (every slot of a batch row adds the row somewhere: to its destination or, padded, to row 0 — on the rank that owns it)
+  if (__any_sync(kFull, bad) && lane == 0 && err_flag) atomicOr(err_flag, LSTEP_FLAG_FIXED_POINT_RANGE);
   if (new_rows && part == 0 && node > 0 && (own_mul == 1 || node % own_mul == own_add))  // row 0 is zeroed above (LSTEP.py:317 follows the phase-A write)
     for (int c = threadIdx.x; c < d; c += blockDim.x) pe[node * (int64_t)d + c] = ld_dep(src_row + c);
   for (int k = warp; k < k_hi - k_lo; k += nwarps) {
@@ -267,11 +278,11 @@ __global__ void __launch_bounds__(kPushThreads) phaseB_push_kernel(const int64_t
   }
   if (s_z > 0 && warp == nwarps - 1) {
     unsigned long long* rowp = use_parts ? row0_part + (size_t)(row % kPushRow0Parts) * kPushRow0Cols : acc + (size_t)s_j0 * in1;
-    const long long zz = s_z;
+    const unsigned long long zz = (unsigned long long)s_z;
 #pragma unroll
     for (int q = 0; q < DQ; ++q) {
       const int c = lane + 32 * q;
-      if (c < d) atomicAdd(rowp + c, (unsigned long long)(zz * fx[q]));
+      if (c < d) atomicAdd(rowp + c, zz * (unsigned long long)fx[q]);  // (two's complement: the signed product's bits; no overflow in range)
     }
   }
   finish();
@@ -292,12 +303,13 @@ int launch_phaseB_push(const lstep_csr* csr, const int64_t* ids, const double* q
   const int threads = (split == 4 || own_mul >= 4) ? 64 : kPushThreads;
   const size_t smem = (size_t)((K + split - 1) / split) * 12;
   const int use_parts = split < 4 ? 1 : 0;  // padding-row partial sums + fold: only where thousands of CTAs would hit one row
+  const float bound = fixed_point_bound(n_ids, K);
   if (d <= 6 * 32 && t <= 4 * 32)
     launch_k(phaseB_push_kernel<6, 4>, dim3((unsigned)(n_ids * split)), dim3(threads), smem, st, csr->indptr, csr->nbr, csr->t, csr->num_rows, ids,
-             q_time, n_ids, n_valid, K, pe, d, t, tw, tc, claim_of, U, counters, acc, dirty, stamp, new_rows, err_flag, row0_part, own_mul, own_add, split, use_parts);
+             q_time, n_ids, n_valid, K, pe, d, t, tw, tc, claim_of, U, counters, acc, dirty, stamp, new_rows, err_flag, row0_part, own_mul, own_add, split, use_parts, bound);
   else if (d <= 8 * 32 && t <= 8 * 32)
     launch_k(phaseB_push_kernel<8, 8>, dim3((unsigned)(n_ids * split)), dim3(threads), smem, st, csr->indptr, csr->nbr, csr->t, csr->num_rows, ids,
-             q_time, n_ids, n_valid, K, pe, d, t, tw, tc, claim_of, U, counters, acc, dirty, stamp, new_rows, err_flag, row0_part, own_mul, own_add, split, use_parts);
+             q_time, n_ids, n_valid, K, pe, d, t, tw, tc, claim_of, U, counters, acc, dirty, stamp, new_rows, err_flag, row0_part, own_mul, own_add, split, use_parts, bound);
   else
     return LSTEP_ERR_UNSUPPORTED;
   return check_launch("phaseB_push");

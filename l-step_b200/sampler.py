@@ -349,6 +349,9 @@ class NeighborSampler:
             raise _lib.LstepError("an append to the growable CSR found a row without room (reserve before appending)")
         if flag & _lib.FLAG_UNSORTED_STREAM:
             raise ValueError("an append to the growable CSR was earlier than the row's last entry")
+        if flag & _lib.FLAG_FIXED_POINT_RANGE:
+            raise FloatingPointError("update_pe phase B met a PE value that is non-finite or at least 2^31 / (n_ids*K + 1) in "
+                                     "magnitude (the limit of its 32.32 fixed-point sums); the updated rows are not valid")
 
     def get_historical_neighbors(self, node_ids: np.ndarray, node_interact_times: np.ndarray, num_neighbors: int = 20):
         assert num_neighbors > 0, 'Number of sampled neighbors for each node should be greater than 0!'

@@ -216,13 +216,13 @@ def scatter_sum_rows(src: np.ndarray, index: np.ndarray, out: np.ndarray):
 # --------------------------------------------------------------------------------------------
 # a7 + a8 — LSTEP.update_pe (models/LSTEP.py:268-341); mutates and returns `pe`
 # --------------------------------------------------------------------------------------------
-def update_pe(p: dict, adj: Adjacency, pe: np.ndarray, node_ids, batch_src_node_ids, batch_dst_node_ids,
-              node_interact_times, current_time, num_neighbors: int = 30):
+def update_pe_phase_a(p: dict, pe: np.ndarray, node_ids, batch_src_node_ids, batch_dst_node_ids, node_interact_times,
+                      current_time):
+    """Phase A of update_pe (models/LSTEP.py:273-303) on its own; mutates and returns `pe`. Phase B adds these rows."""
     w = p["time_encoder.w.weight"].reshape(-1)
     d = pe.shape[1]
     tc = np.float32(current_time)  # torch.Tensor([current_time]) is fp32 (Q4)
     node_pe = pe[node_ids].copy()  # :273
-    # ---- phase A (:277-303)
     dt = (np.float64(tc) - np.asarray(node_interact_times, dtype=np.float64)).astype(F32)  # f32 - f64 -> f64 -> float
     tf = time_encode(dt, w)  # [E,t]
     agg = np.zeros((pe.shape[0], d + tf.shape[1]), ACC)  # :282
@@ -232,6 +232,16 @@ def update_pe(p: dict, adj: Adjacency, pe: np.ndarray, node_ids, batch_src_node_
     h = _linear(np.maximum(_linear(a, p, "pe_mlp_1"), 0), p, "pe_mlp_2")  # :294-297
     upd = node_pe + np.tanh(_linear(node_pe, p, "self_update_pe") + h, dtype=ACC)  # :299-301
     pe[node_ids] = upd  # :303
+    return pe
+
+
+def update_pe(p: dict, adj: Adjacency, pe: np.ndarray, node_ids, batch_src_node_ids, batch_dst_node_ids,
+              node_interact_times, current_time, num_neighbors: int = 30):
+    w = p["time_encoder.w.weight"].reshape(-1)
+    d = pe.shape[1]
+    tc = np.float32(current_time)  # torch.Tensor([current_time]) is fp32 (Q4)
+    # ---- phase A (:277-303)
+    update_pe_phase_a(p, pe, node_ids, batch_src_node_ids, batch_dst_node_ids, node_interact_times, current_time)
     # ---- phase B (:306-339)
     nbr, _, nt = sample_recent(adj, node_ids, node_interact_times, num_neighbors)  # N ids zipped with B times (Q1/Q1b)
     src_flat = np.broadcast_to(np.asarray(node_ids)[:, None], nbr.shape).reshape(-1)  # :310
