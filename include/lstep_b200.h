@@ -519,10 +519,10 @@ int lstep_pe_steps_changelog_host(lstep_host_stepper* h, const lstep_pe_stream* 
 
 /* ------------------------------------------------------------------------------------------
  * Measurement / A-B plumbing (no reference counterpart).
- * lstep_set_option: structural switches of the launch paths ("pdl", "gather_fuse", "mlp_pair", "phaseb_push",
- * "early_append", "dft_prefetch", "dft_early_trigger", "dft_ctas_per_sm", "dft_generic", "gather_narrow", "mlp_ring",
- * "host_memcpy", "mlp_umma", "mlp_umma_min_rows"); defaults are the measured winners, the LSTEP_* environment
- * variables of DESIGN.md set them once at first use. None changes results beyond fp32 summation order.
+ * lstep_set_option: switches of the launch paths ("pdl", "phaseb_push", "gather_pipe", "mlp_umma", "mlp_umma_min_rows",
+ * "profile"), each selecting a shipped path or its reference on the same inputs; defaults are the shipped paths, the LSTEP_*
+ * environment variables of DESIGN.md set them once at first use. None changes results beyond fp32 summation order.
+ * An unknown name returns LSTEP_ERR_INVALID_ARG.
  * lstep_step_profile(1): every streaming step records CUDA events around its kernels; lstep_step_profile_read returns
  * the six durations (ms) of the last step: DFT filter, fused gather, paired MLP, phase-B push, phase-B MLP, ring append.
  * ------------------------------------------------------------------------------------------ */

@@ -20,7 +20,7 @@ __global__ void __launch_bounds__(512) nbr_aggregate_kernel(const float* __restr
                                                             float* __restrict__ S, int64_t ldS, int64_t period, LookupArgs lk) {
   pdl_launch_dependents();
   pdl_wait();
-  nbr_aggregate_rows<VEC, kLookup>(blockIdx.x, gridDim.x, false, pe, q_time, nbr, nbr_t, n_rows, K, tw, d, t, t_pad, S, ldS, period, lk, t);
+  nbr_aggregate_rows<VEC, kLookup>(blockIdx.x, gridDim.x, false, pe, q_time, nbr, nbr_t, n_rows, K, tw, d, t, t_pad, S, ldS, period, lk);
 }
 
 __global__ void __launch_bounds__(256) nbr_aggregate_bwd_kernel(const float* __restrict__ dS,

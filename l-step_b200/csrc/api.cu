@@ -34,20 +34,8 @@ struct OptName {
 };
 const OptName kOpts[] = {
     {"pdl", &Tuning::pdl, "LSTEP_NO_PDL", 0},
-    {"gather_fuse", &Tuning::gather_fuse, "LSTEP_NO_GATHER_FUSE", 0},
-    {"mlp_pair", &Tuning::mlp_pair, "LSTEP_NO_MLP_PAIR", 0},
     {"phaseb_push", &Tuning::phaseb_push, "LSTEP_PHASEB_PULL", 0},
-    {"early_append", &Tuning::early_append, "LSTEP_NO_EARLY_APPEND", 0},
-    {"dft_prefetch", &Tuning::dft_prefetch, "LSTEP_NO_DFT_PREFETCH", 0},
-    {"dft_early_trigger", &Tuning::dft_early_trigger, "LSTEP_DFT_EARLY_TRIGGER", 1},
-    {"dft_ctas_per_sm", &Tuning::dft_ctas_per_sm, "LSTEP_DFT_CTAS_PER_SM", -1},
-    {"dft_generic", &Tuning::dft_generic, "LSTEP_DFT_GENERIC", 1},
-    {"gather_narrow", &Tuning::gather_narrow, "LSTEP_GATHER_NARROW", 1},
-    {"mlp_ring", &Tuning::mlp_ring, "LSTEP_MLP_RING", 1},
-    {"host_memcpy", &Tuning::host_memcpy, "LSTEP_HOST_MEMCPY", 1},
-    {"query_dedup", &Tuning::query_dedup, "LSTEP_NO_QUERY_DEDUP", 0},
     {"gather_pipe", &Tuning::gather_pipe, "LSTEP_NO_GATHER_PIPE", 0},
-    {"cos_spread", &Tuning::cos_spread, "LSTEP_COS_SPREAD", 1},
     {"mlp_umma", &Tuning::mlp_umma, "LSTEP_NO_MLP_UMMA", 0},
     {"mlp_umma_min_rows", &Tuning::mlp_umma_min_rows, "LSTEP_MLP_UMMA_MIN_ROWS", -1},
     {"profile", &Tuning::profile, nullptr, 0},

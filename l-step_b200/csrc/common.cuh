@@ -15,25 +15,13 @@ constexpr unsigned kFull = 0xffffffffu;
 // SM count of the current device (B200: 148 = 2 dies x 74), queried once per process; grids are sized in multiples of it
 int num_sms();
 
-// Structural A/B switches. Initialised ONCE (first use) from the LSTEP_* environment variables DESIGN.md lists and changed
-// with lstep_set_option(); the launch paths read plain ints. Every default is the measured winner.
+// Runtime switches, each the way a test reaches a shipped path or its reference on the same inputs. Initialised ONCE
+// (first use) from the LSTEP_* environment variables DESIGN.md lists and changed with lstep_set_option(); the launch paths
+// read plain ints. Every default is the shipped path.
 struct Tuning {
   int pdl = 1;                // programmatic dependent launch along the step's kernel chain      (LSTEP_NO_PDL=1 -> 0)
-  int gather_fuse = 1;        // a6 lookup+aggregate and a7 edge aggregate in one launch           (LSTEP_NO_GATHER_FUSE)
-  int mlp_pair = 1;           // neighbourhood MLP and phase-A MLP in one launch                   (LSTEP_NO_MLP_PAIR)
   int phaseb_push = 1;        // push form of phase B (0: count / scan / fill / gather pull form)  (LSTEP_PHASEB_PULL)
-  int early_append = 1;       // ring append copies unchanged rows before its dependency wait      (LSTEP_NO_EARLY_APPEND)
-  int dft_prefetch = 1;       // DFT filter requests the older history rows before its wait        (LSTEP_NO_DFT_PREFETCH)
-  int dft_early_trigger = 0;  //                                                                   (LSTEP_DFT_EARLY_TRIGGER)
-  int dft_ctas_per_sm = 3;    //                                                                   (LSTEP_DFT_CTAS_PER_SM)
-  int dft_generic = 0;        // strided generic filter kernel instead of the bulk-copy one        (LSTEP_DFT_GENERIC)
-  int gather_narrow = 0;      // 128-thread gather CTAs                                            (LSTEP_GATHER_NARROW)
-  int mlp_ring = 0;           // all-columns ring MLP kernel instead of the cluster kernel         (LSTEP_MLP_RING)
-  int host_memcpy = 0;        // cudaMemcpyAsync instead of the copy-in kernel in the host-fed step (LSTEP_HOST_MEMCPY)
-  int query_dedup = 1;        // identical query sets of a step are computed once                  (LSTEP_NO_QUERY_DEDUP)
   int gather_pipe = 1;        // multi-row gather CTAs with a look-ahead lookup warp (B = 2000)     (LSTEP_NO_GATHER_PIPE)
-  int cos_spread = 0;         // a query row's K * t cosines spread over all threads of its CTA     (LSTEP_COS_SPREAD; measured SLOWER:
-                              // gather 16.4 -> 18.6 us at B=200, 68.6 -> 88.1 us at B=2000 — the cosine phase is issue bound, not chain bound)
   int mlp_umma = 1;           // tcgen05 tensor-core MLP for launches with >= mlp_umma_min_rows rows (LSTEP_NO_MLP_UMMA)
   int mlp_umma_min_rows = 1536;  //                                                                (LSTEP_MLP_UMMA_MIN_ROWS)
   int profile = 0;            // lstep_step_profile(): CUDA events around every kernel of the streaming step

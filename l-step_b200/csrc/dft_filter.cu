@@ -182,7 +182,7 @@ __global__ void __launch_bounds__(kDftThreads, 5) dft_filter_bulk_kernel(const f
                                                                       int ring, int Th, int d, const int64_t* __restrict__ ids,
                                                                       int64_t n_ids, const float* __restrict__ G,
                                                                       float* __restrict__ out, int64_t out_stride,
-                                                                      const int64_t* __restrict__ out_ids, int prefetch, int early_trigger) {
+                                                                      const int64_t* __restrict__ out_ids, int prefetch) {
   extern __shared__ __align__(16) unsigned char smem_raw[];  // (bulk-copy destinations need 16-byte alignment)
   __shared__ __align__(8) uint64_t bar[kDftChunks];
   float4* xs = reinterpret_cast<float4*>(smem_raw);  // [Th][dvec] logical time order
@@ -194,11 +194,6 @@ __global__ void __launch_bounds__(kDftThreads, 5) dft_filter_bulk_kernel(const f
   // chunks 0 .. kDftChunks-2: the Th-1 older rows; last chunk: the newest row alone (the same partition with and
   // without prefetch, so both forms add in the same order and agree bit for bit)
   TL_ENTRY(0);
-  // early_trigger (streaming step, push form): the previous step ended with "phase-B MLP (late trigger) -> ring append",
-  // so this kernel being resident already means everything before that MLP has completed and the MLP has read its row
-  // counter — nothing the next kernel (the fused gather) writes before ITS wait is still in use. Triggering at once
-  // lets the gather start its lookups ~3 us earlier. Otherwise the trigger follows this kernel's own wait.
-  if (early_trigger) pdl_launch_dependents();
   const int rc = (Th - 1 + kDftChunks - 2) / (kDftChunks - 1);  // rows per chunk
   auto bounds = [&](int c, int& a, int& b) {
     if (c == kDftChunks - 1) {
@@ -242,7 +237,7 @@ __global__ void __launch_bounds__(kDftThreads, 5) dft_filter_bulk_kernel(const f
   TL_WAITED(0);
   // late trigger: the next kernel of the step (the fused gather) does its lookups and cosines before its own wait;
   // it may only become resident once everything before this filter has completed
-  if (!early_trigger) pdl_launch_dependents();
+  pdl_launch_dependents();
   const float4* Gv = reinterpret_cast<const float4*>(G);
   uint32_t it = 0;
   // Streaming across the nodes of a CTA (launches with more nodes than resident CTAs: B = 2000): chunk c of the NEXT node
@@ -359,7 +354,7 @@ extern "C" int lstep_dft_collapse(const float* W_c64, const float* a, int T, int
 namespace lstep {
 int launch_dft_filter(const float* hist, int64_t node_stride, int64_t time_stride, int s0, int ring, int Th, int d,
                       const int64_t* ids, int64_t n_ids, const float* G, float* out, int64_t out_stride,
-                      const int64_t* out_ids, void* stream, bool prefetch_old_rows, bool early_trigger) {
+                      const int64_t* out_ids, void* stream, bool prefetch_old_rows) {
   if (n_ids < 0 || Th < 0 || d <= 0 || ring < Th || s0 < 0 || (ring > 0 && s0 >= ring)) return LSTEP_ERR_INVALID_ARG;
   if (n_ids == 0) return LSTEP_OK;
   if (!ids || !out || !G || (Th > 0 && !hist)) return LSTEP_ERR_INVALID_ARG;
@@ -372,9 +367,9 @@ int launch_dft_filter(const float* hist, int64_t node_stride, int64_t time_strid
   cudaStream_t st = as_stream(stream);
   {
     // node-major history: bulk-async kernel (one CTA stages a node's whole block in shared memory)
-    const bool no_bulk = tuning().dft_generic != 0;
+    constexpr int kBulkCtasPerSm = 3;  // what <= 74 KB of shared memory per CTA leaves room for
     const size_t bulk_smem = ((size_t)Th * dvec + (size_t)groups * dvec) * 16;
-    if (v4 && !no_bulk && time_stride == d && Th > 0 && bulk_smem <= 74 * 1024) {  // <= 74 KB: 3 CTAs per SM
+    if (v4 && time_stride == d && Th > 0 && bulk_smem <= 74 * 1024) {
       static bool attr_set = false;
       if (!attr_set) {
         cudaError_t e = cudaFuncSetAttribute(dft_filter_bulk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 74 * 1024);
@@ -384,10 +379,9 @@ int launch_dft_filter(const float* hist, int64_t node_stride, int64_t time_strid
         }
         attr_set = true;
       }
-      const int per_sm = tuning().dft_ctas_per_sm > 0 ? tuning().dft_ctas_per_sm : 3;
-      const int64_t bgrid = n_ids < (int64_t)num_sms() * per_sm ? n_ids : (int64_t)num_sms() * per_sm;
+      const int64_t bgrid = n_ids < (int64_t)num_sms() * kBulkCtasPerSm ? n_ids : (int64_t)num_sms() * kBulkCtasPerSm;
       launch_k(dft_filter_bulk_kernel, dim3((unsigned)bgrid), dim3(kDftThreads), bulk_smem, st, hist, node_stride, s0, ring, Th, d, ids,
-               n_ids, G, out, out_stride, out_ids, prefetch_old_rows ? 1 : 0, early_trigger ? 1 : 0);
+               n_ids, G, out, out_stride, out_ids, prefetch_old_rows ? 1 : 0);
       return check_launch("dft_filter_bulk");
     }
   }
@@ -404,7 +398,7 @@ int launch_dft_filter(const float* hist, int64_t node_stride, int64_t time_strid
 extern "C" int lstep_dft_filter(const float* hist, int64_t node_stride, int64_t time_stride, int s0, int ring, int Th,
                                 int d, const int64_t* ids, int64_t n_ids, const float* G, float* out,
                                 int64_t out_stride, void* stream) {
-  return lstep::launch_dft_filter(hist, node_stride, time_stride, s0, ring, Th, d, ids, n_ids, G, out, out_stride, nullptr, stream, false, false);
+  return lstep::launch_dft_filter(hist, node_stride, time_stride, s0, ring, Th, d, ids, n_ids, G, out, out_stride, nullptr, stream, false);
 }
 
 /* Same filter with the result row n written to out + out_ids[n]*out_stride (history rows and table rows
@@ -413,7 +407,7 @@ extern "C" int lstep_dft_filter_scatter(const float* hist, int64_t node_stride, 
                                         int d, const int64_t* ids, const int64_t* out_ids, int64_t n_ids, const float* G,
                                         float* out, int64_t out_stride, void* stream) {
   if (!out_ids && n_ids > 0) return LSTEP_ERR_INVALID_ARG;
-  return lstep::launch_dft_filter(hist, node_stride, time_stride, s0, ring, Th, d, ids, n_ids, G, out, out_stride, out_ids, stream, false, false);
+  return lstep::launch_dft_filter(hist, node_stride, time_stride, s0, ring, Th, d, ids, n_ids, G, out, out_stride, out_ids, stream, false);
 }
 
 extern "C" int lstep_dft_filter_bwd(const float* hist, int64_t node_stride, int64_t time_stride, int s0, int ring,

@@ -24,19 +24,11 @@ __device__ __forceinline__ void nbr_aggregate_rows(int64_t first_row, int64_t ro
                                                             const int32_t* __restrict__ nbr,
                                                             const float* __restrict__ nbr_t, int64_t n_rows, int K,
                                                             const float* __restrict__ tw, int d, int t, int t_pad,
-                                                            float* __restrict__ S, int64_t ldS, int64_t period, LookupArgs lk,
-                                                            int tf_threads, int spread = 0) {
-  // tf_threads: how many threads (tid < tf_threads) share the t time frequencies; thread i takes i, i + tf_threads, ...
-  // spread (dynamic shared memory holds K * t more floats): the K * t cosines of a row are spread over ALL threads of the CTA
-  // and parked in shared memory; the frequency threads then add them in the same order k = 0 .. K-1 (bit-identical sums).
-  // An experiment (option cos_spread, off by default): the idea was that the warp holding the low frequencies (large arguments,
-  // both cosine paths in one warp, K cosines one after the other) is a serial chain that bounds the gather; spreading the
-  // cosines measured SLOWER (16.4 -> 18.6 us at B = 200, 68.6 -> 88.1 us at B = 2000): the phase is bound by instruction issue
-  // and the extra index arithmetic, shared-memory round trip and barrier cost more than the shorter chains save.
+                                                            float* __restrict__ S, int64_t ldS, int64_t period, LookupArgs lk) {
+  // thread f < t owns time frequency f and adds its K cosines in order k = 0 .. K-1
   extern __shared__ __align__(16) unsigned char smem_raw[];
   int32_t* s_nbr = reinterpret_cast<int32_t*>(smem_raw);
   float* s_dt = reinterpret_cast<float*>(s_nbr + K);
-  float* s_val = s_dt + K;  // [K][t] when spread
   const int tid = threadIdx.x;
   const int dvec = d / VEC;
   for (int64_t row = first_row; row < n_rows; row += row_stride) {
@@ -75,32 +67,16 @@ __device__ __forceinline__ void nbr_aggregate_rows(int64_t first_row, int64_t ro
 #ifdef LSTEP_TIMELINE
     if (late_wait && tid == 0) atomicMax(&g_timeline[6 * 4 + 2], gtimer());  // last lookup done
 #endif
-    if (spread) {
-      for (int i = tid; i < K * t; i += blockDim.x) {
-        const int k = i / t, f = i - k * t;
-        s_val[i] = s_nbr[k] != 0 ? time_feature(s_dt[k], tw[f]) : 0.f;
-      }
-      __syncthreads();
-    }
-    if (tid < tf_threads) {
-      for (int f = tid; f < t; f += tf_threads) {
-        float acc = 0.f;
-        if (spread) {
-          for (int k = 0; k < K; ++k)
-            if (s_nbr[k] != 0) acc += s_val[k * t + f];
-        } else {
-          const float w = tw[f];
-          for (int k = 0; k < K; ++k)
-            if (s_nbr[k] != 0) acc += time_feature(s_dt[k], w);
-        }
-        S[row * ldS + d + f] = acc;
-      }
+    if (tid < t) {
+      float acc = 0.f;
+      const float w = tw[tid];
+      for (int k = 0; k < K; ++k)
+        if (s_nbr[k] != 0) acc += time_feature(s_dt[k], w);
+      S[row * ldS + d + tid] = acc;
 #ifdef LSTEP_TIMELINE
       if (late_wait && tid == 0) atomicMax(&g_timeline[7 * 4 + 2], gtimer());  // last cosine block done
 #endif
     }
-    // (two independent tests: with t_pad = 0 — the streaming step's 128-thread CTAs — the same threads first do a time
-    // frequency and then a table column group; with t_pad >= t the two roles are disjoint threads working side by side)
     if (tid >= t_pad && tid - t_pad < dvec) {
       // late_wait (fused launch of the streaming step): lookups and cosines depend on nothing the kernel in front
       // writes, so only the threads that read the table wait for it
@@ -169,12 +145,10 @@ __device__ __forceinline__ void nbr_aggregate_rows(int64_t first_row, int64_t ro
 __device__ __forceinline__ void nbr_aggregate_rows_piped(int64_t first_row, int64_t row_stride, bool late_wait, const float* __restrict__ pe,
                                                          const double* __restrict__ q_time, int64_t n_rows, int K,
                                                          const float* __restrict__ tw, int d, int t, int t_pad, float* __restrict__ S,
-                                                         int64_t ldS, int64_t period, LookupArgs lk, int tf_threads, int lk_base,
-                                                         int spread) {
+                                                         int64_t ldS, int64_t period, LookupArgs lk, int lk_base) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   int32_t* s_nbr_all = reinterpret_cast<int32_t*>(smem_raw);       // [2][K]
   float* s_dt_all = reinterpret_cast<float*>(s_nbr_all + 2 * K);   // [2][K]
-  float* s_val = s_dt_all + 2 * K;                                 // [K][t] when spread (see nbr_aggregate_rows)
   const int tid = threadIdx.x;
   const int dvec = d / 4;
   const bool is_lk = tid >= lk_base && tid < lk_base + 32;
@@ -213,26 +187,12 @@ __device__ __forceinline__ void nbr_aggregate_rows_piped(int64_t first_row, int6
     if (is_lk) {
       if (row + row_stride < n_rows) lookup(row + row_stride, buf ^ 1);
     } else {
-      if (spread) {  // threads [0, lk_base) share the K * t cosines, then meet (named barrier 1: the lookup warp is elsewhere)
-        for (int i = tid; i < K * t; i += lk_base) {
-          const int k = i / t, f = i - k * t;
-          s_val[i] = s_nbr[k] != 0 ? time_feature(s_dt[k], tw[f]) : 0.f;
-        }
-        asm volatile("bar.sync 1, %0;" ::"r"(lk_base) : "memory");
-      }
-      if (tid < tf_threads) {
-        for (int f = tid; f < t; f += tf_threads) {
-          float acc = 0.f;
-          if (spread) {
-            for (int k = 0; k < K; ++k)
-              if (s_nbr[k] != 0) acc += s_val[k * t + f];
-          } else {
-            const float w = tw[f];
-            for (int k = 0; k < K; ++k)
-              if (s_nbr[k] != 0) acc += time_feature(s_dt[k], w);
-          }
-          S[row * ldS + d + f] = acc;
-        }
+      if (tid < t) {
+        float acc = 0.f;
+        const float w = tw[tid];
+        for (int k = 0; k < K; ++k)
+          if (s_nbr[k] != 0) acc += time_feature(s_dt[k], w);
+        S[row * ldS + d + tid] = acc;
       }
       if (tid >= t_pad && tid - t_pad < dvec) {
         if (late_wait) pdl_wait();

@@ -27,7 +27,6 @@ namespace lstep {
 // two kernels costs a stream hand-over in each direction (~6-8 us each for these 14 KB / 3 KB payloads) and
 // is slower than a 4-CTA copy kernel. The copy-in runs on a side stream (it overlaps the previous step; the
 // compute stream waits on its event), the result kernel on another (the next step does not queue behind it).
-// LSTEP_HOST_MEMCPY=1 selects cudaMemcpyAsync instead (A/B).
 __global__ void __launch_bounds__(256) stage_in_kernel(const uint4* __restrict__ host_slot, uint4* __restrict__ dev_slot, int64_t n16) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n16; i += (int64_t)gridDim.x * blockDim.x)
     dev_slot[i] = __ldcv(host_slot + i);  // the host rewrites the pinned slot between launches: never cached
@@ -63,7 +62,6 @@ struct lstep_host_stepper {
   char* h_in[kMaxSlots];
   char* d_in[kMaxSlots];
   float* h_res[kMaxSlots];
-  float* d_res[kMaxSlots];
   cudaEvent_t done[kMaxSlots];       // result of the slot's step is in the pinned result slot
   cudaEvent_t in_ready[kMaxSlots];   // the slot's batch is on the device
   cudaEvent_t step_done[kMaxSlots];  // the slot's step has written nbr_out
@@ -138,7 +136,6 @@ extern "C" void lstep_host_stepper_destroy(lstep_host_stepper* h) {
     if (h->h_in[i]) cudaFreeHost(h->h_in[i]);
     if (h->h_res[i]) cudaFreeHost(h->h_res[i]);
     if (h->d_in[i]) cudaFree(h->d_in[i]);
-    if (h->d_res[i]) cudaFree(h->d_res[i]);
   }
   if (h->d_nbr_out) cudaFree(h->d_nbr_out);
   if (h->ing_ev) cudaEventDestroy(h->ing_ev);
@@ -174,7 +171,7 @@ extern "C" int lstep_host_stepper_create(int slots, int64_t max_edges, int max_q
   h->ing_stream = nullptr;
   for (int i = 0; i < kMaxSlots; ++i) {
     h->h_in[i] = h->d_in[i] = nullptr;
-    h->h_res[i] = h->d_res[i] = nullptr;
+    h->h_res[i] = nullptr;
     h->done[i] = h->in_ready[i] = h->step_done[i] = nullptr;
     h->d_nbr[i] = nullptr;
     h->ticket_of[i] = -1;
@@ -185,7 +182,6 @@ extern "C" int lstep_host_stepper_create(int slots, int64_t max_edges, int max_q
     if ((e = cudaHostAlloc((void**)&h->h_in[i], h->in_bytes, cudaHostAllocDefault)) != cudaSuccess) break;
     if ((e = cudaHostAlloc((void**)&h->h_res[i], sizeof(float) * h->res_floats, cudaHostAllocDefault)) != cudaSuccess) break;
     if ((e = cudaMalloc((void**)&h->d_in[i], h->in_bytes)) != cudaSuccess) break;
-    if ((e = cudaMalloc((void**)&h->d_res[i], sizeof(float) * h->res_floats)) != cudaSuccess) break;
     if ((e = cudaEventCreateWithFlags(&h->done[i], cudaEventDisableTiming)) != cudaSuccess) break;
     if ((e = cudaEventCreateWithFlags(&h->in_ready[i], cudaEventDisableTiming)) != cudaSuccess) break;
     if ((e = cudaEventCreateWithFlags(&h->step_done[i], cudaEventDisableTiming)) != cudaSuccess) break;
@@ -208,7 +204,6 @@ struct HostBatch {
   double tmax;
   const int64_t* dp;
   const int64_t* qdev[8];
-  bool use_memcpy;
 };
 
 // The first half of a host-fed step: slot wait, pack, the host id-range and ingest checks, copy-in, the optional append on
@@ -269,18 +264,12 @@ static int host_stage(lstep_host_stepper* h, const lstep_pe_stream* s, const lst
     if (h->ing_next_eid < 0 || h->ing_next_eid + n_edges - 1 > 0x7fffffffLL) return LSTEP_ERR_ID_RANGE;
   }
   const size_t bytes = 8 * n * (size_t)(5 + n_queries);
-  const bool use_memcpy = tuning().host_memcpy != 0;
   // copy-in on its own stream: it only has to wait for the slot's previous use (synchronised above), so it runs
   // while the previous step is still computing; the compute stream picks it up through an event
-  if (use_memcpy) {
-    if ((e = cudaMemcpyAsync(h->d_in[slot], h->h_in[slot], bytes, cudaMemcpyHostToDevice, h->in_stream)) != cudaSuccess)
-      return cuda_fail(e, "pe_step_host h2d");
-  } else {
-    stage_in_kernel<<<4, 256, 0, h->in_stream>>>(reinterpret_cast<const uint4*>(h->h_in[slot]), reinterpret_cast<uint4*>(h->d_in[slot]),
-                                                 (int64_t)((bytes + 15) / 16));
-    int rc0 = check_launch("stage_in");
-    if (rc0 != LSTEP_OK) return rc0;
-  }
+  stage_in_kernel<<<4, 256, 0, h->in_stream>>>(reinterpret_cast<const uint4*>(h->h_in[slot]), reinterpret_cast<uint4*>(h->d_in[slot]),
+                                               (int64_t)((bytes + 15) / 16));
+  int rc0 = check_launch("stage_in");
+  if (rc0 != LSTEP_OK) return rc0;
   if (ingest) {
     // The batch is appended to the CSR from the staged slot, on the copy-in path: on a high-priority stream that waits for
     // the copy-in and records in_ready, so the compute stream sees the grown CSR and the step's launch chain is unchanged.
@@ -328,7 +317,6 @@ static int host_stage(lstep_host_stepper* h, const lstep_pe_stream* s, const lst
   hb->n_ids = n_ids;
   hb->tmax = tmax;
   hb->dp = dp;
-  hb->use_memcpy = use_memcpy;
   return LSTEP_OK;
 }
 
@@ -348,11 +336,8 @@ static int host_finish(lstep_host_stepper* h, const HostBatch& hb, int64_t n_edg
   }
   if (rows > 0) {
     // the row sums go straight into the pinned result slot (visible to the host once the event below has fired)
-    row_sum_kernel<<<(unsigned)ceil_div(rows * 32, 256), 256, 0, rs>>>(outp, rows, h->d, hb.use_memcpy ? h->d_res[slot] : h->h_res[slot]);
+    row_sum_kernel<<<(unsigned)ceil_div(rows * 32, 256), 256, 0, rs>>>(outp, rows, h->d, h->h_res[slot]);
     if ((rc = check_launch("row_sum")) != LSTEP_OK) return rc;
-    if (hb.use_memcpy &&
-        (e = cudaMemcpyAsync(h->h_res[slot], h->d_res[slot], sizeof(float) * (size_t)rows, cudaMemcpyDeviceToHost, rs)) != cudaSuccess)
-      return cuda_fail(e, "pe_step_host d2h");
     h->d2h_bytes += sizeof(float) * (size_t)rows;
   }
   if ((e = cudaEventRecord(h->done[slot], rs)) != cudaSuccess) return cuda_fail(e, "pe_step_host event");

@@ -4,7 +4,7 @@
 //
 // launch_pe_mlp() dispatches to the cluster split-K kernel (csrc/mlp_cluster.cu, the default). This file holds the
 // weight packing and the ALL-COLUMNS ring kernel it replaced, kept as the fallback for shapes the cluster kernel does
-// not cover (LSTEP_MLP_RING=1 forces it):
+// not cover:
 //
 // fp32 FMA throughout: the parity bar (1e-5) rules out single-pass TF32/BF16 tensor-core math.
 //   * weights are pre-packed (lstep_pack_linear) as [in_pad][ldo] row-major, in_pad = in rounded up
@@ -310,15 +310,9 @@ int launch_pe_mlp(const float* A, int64_t lda, const float* pe, RowIds base_ids,
                   cudaStream_t st, bool late_trigger) {
   if (n_rows <= 0) return LSTEP_OK;
   if (!A || !pe || !base_ids.p[0] || !m || (!out && !pe_inplace)) return LSTEP_ERR_INVALID_ARG;
-  {
-    // default: the cluster split-K kernel (csrc/mlp_cluster.cu); LSTEP_MLP_RING=1 selects the all-columns
-    // weight-ring kernel below, which also serves shapes the cluster kernel does not cover
-    const bool use_ring = tuning().mlp_ring != 0;
-    if (!use_ring) {
-      const int rc = launch_pe_mlp_cluster(A, lda, pe, base_ids, n_rows, expected_rows, n_rows_dev, m, out, out_stride, pe_inplace, nullptr, nullptr, st, late_trigger);
-      if (rc != LSTEP_ERR_UNSUPPORTED) return rc;
-    }
-  }
+  // the cluster split-K kernel (csrc/mlp_cluster.cu); the all-columns weight-ring kernel below serves the shapes it does not cover
+  const int rc = launch_pe_mlp_cluster(A, lda, pe, base_ids, n_rows, expected_rows, n_rows_dev, m, out, out_stride, pe_inplace, nullptr, nullptr, st, late_trigger);
+  if (rc != LSTEP_ERR_UNSUPPORTED) return rc;
   const int ldo = lstep_packed_ld(m->d);
   // rows per CTA: the largest tile that still gives about one CTA per SM; k-split while the CTA stays <= 1024 threads
   if (ldo <= 192) {  // 4 k-split groups of <= 192 threads + the producer warp = 800 threads

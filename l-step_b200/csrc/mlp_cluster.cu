@@ -563,8 +563,7 @@ int launch_pe_mlp_cluster_pair(const float* pe, const float* A0, int64_t lda0, R
 
 // true when the cluster kernel covers this MLP shape (the push form of update_pe phase B depends on it)
 bool pe_mlp_cluster_supports(const lstep_pe_mlp* m) {
-  const bool off = tuning().mlp_ring != 0;
-  if (off || !m) return false;
+  if (!m) return false;
   const ClShape sh = cl_shape(m->d, m->t, m->ws != nullptr, 32);
   return sh.smem_floats * sizeof(float) <= 226 * 1024 && sh.nthreads <= 512 && sh.ncg % kCl == 0;
 }

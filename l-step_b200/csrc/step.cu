@@ -41,13 +41,13 @@ int launch_phase_a_to_new_rows(const float* pe, void* workspace, int64_t ws_ids,
 // read the current table and neither depends on the other, so the short edge kernel (and its hub chain) hides
 // behind the cosine-bound neighbourhood rows instead of being a link of the step's dependency chain.
 __global__ void __launch_bounds__(512) gather_ab_kernel(const float* __restrict__ pe, const double* __restrict__ q_time, int64_t n_rows,
-                                                        int K, const float* __restrict__ tw_q, int d, int t, int t_pad, int t_pad_e,
+                                                        int K, const float* __restrict__ tw_q, int d, int t, int t_pad,
                                                         float* __restrict__ S, int64_t ldS, int64_t period, LookupArgs lk, int grid_q,
                                                         const int64_t* __restrict__ ids, int64_t n_ids,
                                                         const int64_t* __restrict__ src, const int64_t* __restrict__ dst,
                                                         const double* __restrict__ times, int64_t n_edges, float tc,
                                                         const float* __restrict__ tw_u, float* __restrict__ A, int64_t lda,
-                                                        int32_t* __restrict__ counters, int lk_base, int spread) {
+                                                        int32_t* __restrict__ counters, int lk_base) {
   // The kernel in front (the DFT filter, launched with a late trigger: this kernel is resident only after
   // everything before the filter has completed) writes the table and nothing else this kernel touches. Lookups,
   // edge scans and all cosines therefore run BEFORE the dependency wait, next to the HBM-bound filter; only the
@@ -60,14 +60,12 @@ __global__ void __launch_bounds__(512) gather_ab_kernel(const float* __restrict_
   // lk_base > 0: the CTAs walk several query rows each; the warp at threads [lk_base, lk_base + 32) looks one row ahead
   if ((int)blockIdx.x < grid_q) {
     if (lk_base > 0)
-      nbr_aggregate_rows_piped(blockIdx.x, grid_q, true, pe, q_time, n_rows, K, tw_q, d, t, t_pad, S, ldS, period, lk, t_pad < t ? t_pad : t, lk_base,
-                               spread);
+      nbr_aggregate_rows_piped(blockIdx.x, grid_q, true, pe, q_time, n_rows, K, tw_q, d, t, t_pad, S, ldS, period, lk, lk_base);
     else
-      nbr_aggregate_rows<4, true>(blockIdx.x, grid_q, true, pe, q_time, nullptr, nullptr, n_rows, K, tw_q, d, t, t_pad, S, ldS, period, lk,
-                                  t_pad < t ? t_pad : t, spread);
+      nbr_aggregate_rows<4, true>(blockIdx.x, grid_q, true, pe, q_time, nullptr, nullptr, n_rows, K, tw_q, d, t, t_pad, S, ldS, period, lk);
   } else
     edge_aggregate_rows((int64_t)blockIdx.x - grid_q, (int64_t)gridDim.x - grid_q, (int)blockIdx.x == grid_q, true, pe, ids, n_ids, src, dst,
-                        times, n_edges, tc, tw_u, d, t, t_pad_e, A, lda, counters);
+                        times, n_edges, tc, tw_u, d, t, t_pad, A, lda, counters);
 #ifdef LSTEP_TIMELINE
   if (threadIdx.x == 0) atomicMax(&g_timeline[((int)blockIdx.x < grid_q ? 11 : 12) * 4 + 2], gtimer());  // last CTA EXIT (nbr / edge)
 #endif
@@ -78,7 +76,7 @@ int launch_pe_mlp(const float* A, int64_t lda, const float* pe, RowIds base_ids,
                   cudaStream_t st, bool late_trigger = false);
 int launch_dft_filter(const float* hist, int64_t node_stride, int64_t time_stride, int s0, int ring, int Th, int d,
                       const int64_t* ids, int64_t n_ids, const float* G, float* out, int64_t out_stride,
-                      const int64_t* out_ids, void* stream, bool prefetch_old_rows, bool early_trigger);
+                      const int64_t* out_ids, void* stream, bool prefetch_old_rows);
 
 // ring[v][slot][:] = cur[v][:]  (node-major ring: 688-byte rows at a 68.8 KB pitch)
 // table row of ring row v is v*row_mul + row_add (1, 0 for a single GPU; G, rank for a node-id sharded ring)
@@ -234,14 +232,7 @@ int pe_step_core_ex(const lstep_pe_stream* s, const lstep_csr* csr, const int64_
   if (!opt.peer) prof_mark(st, kProfStart);
   // a3: filtered history of the batch nodes straight into the current table
   if (n_ids > 0 && !opt.skip_dft) {
-    const bool no_prefetch = tuning().dft_prefetch == 0;
-    // every step of this stream ends with "phase-B MLP (late trigger) -> ring append" when the push form and the early
-    // append are in use: only then may the filter let the gather in at once (see dft_filter_bulk_kernel)
-    // (LSTEP_DFT_EARLY_TRIGGER=1; measured within noise of the late trigger — 65.9 vs 64.9 us resident, 70.4 vs 72.3 us end
-    // to end — so it stays opt-in)
-    const bool want_early = tuning().dft_early_trigger != 0 && tuning().early_append != 0;
-    const bool early_trigger = want_early && n_queries > 0 && n_edges > 0 && update_push_available(mlp_upd);
-    rc = launch_dft_filter(s->ring, (int64_t)T * d, d, head, T, len, d, ids, n_ids, G, s->cur, d, ids, stream, !no_prefetch, early_trigger);
+    rc = launch_dft_filter(s->ring, (int64_t)T * d, d, head, T, len, d, ids, n_ids, G, s->cur, d, ids, stream, true);
     if (rc != LSTEP_OK) return rc;
     prof_mark(st, kProfDft);
   }
@@ -259,9 +250,9 @@ int pe_step_core_ex(const lstep_pe_stream* s, const lstep_csr* csr, const int64_
     if (u == n_uniq) q.p[n_uniq++] = query_ids_host[c];
     fan.src_of[c] = (signed char)u;
   }
-  const bool can_pair = tuning().mlp_pair != 0 && tuning().gather_fuse != 0 && mlp_nbr->ws && mlp_upd->ws && update_push_available(mlp_upd) &&
-                        pe_mlp_cluster_supports(mlp_nbr) && (opt.peer ? opt.peer->n_mine : n_ids) > 0 && n_edges > 0;
-  const bool dedup = tuning().query_dedup != 0 && can_pair && n_uniq < n_queries && q_rows > 0;
+  const bool can_pair = mlp_nbr->ws && mlp_upd->ws && update_push_available(mlp_upd) && pe_mlp_cluster_supports(mlp_nbr) &&
+                        (opt.peer ? opt.peer->n_mine : n_ids) > 0 && n_edges > 0;
+  const bool dedup = can_pair && n_uniq < n_queries && q_rows > 0;
   if (!dedup) {
     for (int c = 0; c < n_queries; ++c) q.p[c] = query_ids_host[c];
     n_uniq = n_queries;
@@ -284,37 +275,26 @@ int pe_step_core_ex(const lstep_pe_stream* s, const lstep_csr* csr, const int64_
   float* new_rows = nullptr;
   int64_t ldA = 0;
   int32_t* counters = nullptr;
-  const bool no_fuse = tuning().gather_fuse == 0;
   // CTA shape of the fused gather: the stand-alone kernels' 192 threads (t time-frequency threads + d/4 table threads).
-  // LSTEP_GATHER_NARROW=1: 128 threads — in a neighbourhood row 64 threads share the t time frequencies (two each) and
-  // d/4 threads gather table rows; in an edge row the same threads are first time-frequency and then table threads
-  // (t_pad_e = 0). It makes every CTA resident beside the DFT filter at once, but the instrumented timeline shows
-  // the gather is not bound by residency: all its CTAs start within 4 us, lookups end 5 us later and the 1.6 M
-  // cosines take ~9 us of issue-bound work either way.
-  const bool wide = tuning().gather_narrow == 0;  // measured: no gain from the narrow shape (the cosine phase is issue bound)
-  const int t_al = (int)align_up((size_t)t, 32);
-  const int t_half = (int)align_up((size_t)(t + 1) / 2, 32);
-  const bool narrow = !wide && t_half + d / 4 <= 128 && t <= 128 && d / 4 <= 128;
-  const int t_pad = narrow ? t_half : t_al;
-  const int t_pad_e = narrow ? 0 : t_al;
-  const int threads = narrow ? 128 : (int)align_up((size_t)t_al + d / 4, 32);
+  // Narrower CTAs (all resident beside the DFT filter at once) gave no gain: the gather is not bound by residency, its
+  // cosines are ~9 us of issue-bound work either way.
+  const int t_pad = (int)align_up((size_t)t, 32);
+  const int threads = (int)align_up((size_t)t_pad + d / 4, 32);
   const bool vec_ok = d % 4 == 0 && w.lda % 4 == 0 && reinterpret_cast<uintptr_t>(s->cur) % 16 == 0 && threads <= 512;
-  if (first_half && !no_fuse && rows > 0 && n_a > 0 && n_edges > 0 && vec_ok && t == mlp_upd->t && d == mlp_upd->d) {
+  if (first_half && rows > 0 && n_a > 0 && n_edges > 0 && vec_ok && t == mlp_upd->t && d == mlp_upd->d) {
     update_ws_phase_a(w.update, n_ids, n_edges, K, d, t, s->V1, &A, &ldA, &counters, &new_rows);
     const int64_t cap = (int64_t)num_sms() * 16;
     // more query rows than one launch has CTAs for (B = 2000): one wave of CTAs with a look-ahead lookup warp each (gather_pipe)
-    const bool piped = tuning().gather_pipe != 0 && !narrow && rows > cap && threads + 32 <= 512;
+    const bool piped = tuning().gather_pipe != 0 && rows > cap && threads + 32 <= 512;
     const int threads_l = piped ? threads + 32 : threads;
     const int64_t cap_q = piped ? (int64_t)num_sms() * (2048 / threads_l) : cap;
     const int grid_q = (int)(rows < cap_q ? rows : cap_q), grid_e = (int)(n_a < cap ? n_a : cap);
-    // the K * t cosines of a query row spread over all threads of its CTA (cos_spread; needs K * t floats of shared memory)
-    const bool spread = tuning().cos_spread != 0 && !narrow && (size_t)K * t * 4 <= 16 * 1024;
-    const size_t smem = std::max((size_t)K * 8 * (piped ? 2 : 1) + (spread ? (size_t)K * t * 4 : 0), (size_t)threads_l * kSegPerThread * 8 + 32 * 4);
+    const size_t smem = std::max((size_t)K * 8 * (piped ? 2 : 1), (size_t)threads_l * kSegPerThread * 8 + 32 * 4);
     if (smem <= 48 * 1024) {
       LookupArgs lk{csr->indptr, csr->nbr, csr->t, csr->num_rows, q, err_flag};
       launch_k(gather_ab_kernel, dim3((unsigned)(grid_q + grid_e)), dim3(threads_l), smem, st, s->cur, tq_q, rows, K, mlp_nbr->tw, d, t, t_pad,
-               t_pad_e, w.S, w.lda, q_rows, lk, grid_q, ids_a, n_a, src, dst, tq, n_edges, (float)current_time, mlp_upd->tw, A, ldA, counters,
-               piped ? threads : 0, spread ? 1 : 0);
+               w.S, w.lda, q_rows, lk, grid_q, ids_a, n_a, src, dst, tq, n_edges, (float)current_time, mlp_upd->tw, A, ldA, counters,
+               piped ? threads : 0);
       if ((rc = check_launch("gather_ab")) != LSTEP_OK) return rc;
       prof_mark(st, kProfGather);
       edges_done = true;
@@ -327,8 +307,7 @@ int pe_step_core_ex(const lstep_pe_stream* s, const lstep_csr* csr, const int64_
     }
     // the neighbourhood MLP and phase A's MLP in ONE launch when they fit one round of clusters: neither writes the
     // table then (phase A's rows go to new_rows and are applied by the push kernel), so they need no order
-    const bool no_pair = tuning().mlp_pair == 0;
-    if (edges_done && !no_pair && mlp_nbr->ws && mlp_upd->ws && update_push_available(mlp_upd)) {
+    if (edges_done && mlp_nbr->ws && mlp_upd->ws && update_push_available(mlp_upd)) {
       RowIds ida{};
       ida.p[0] = ids_a;
       ida.period = 0;
@@ -381,9 +360,8 @@ int pe_step_core_ex(const lstep_pe_stream* s, const lstep_csr* csr, const int64_
   }
   if (opt.stamp_out) *opt.stamp_out = stamp;
   int32_t* dirty = nullptr;
-  const bool no_early_append = tuning().early_append == 0;
   rc = update_pe_impl(s->cur, s->V1, csr, ids, n_ids, src, dst, tq, n_edges, current_time, K, mlp_upd, w.update, w.update_bytes,
-                      err_flag, stream, edges_done, (no_early_append || opt.skip_append) ? nullptr : &dirty, stamp, phase_a_done,
+                      err_flag, stream, edges_done, opt.skip_append ? nullptr : &dirty, stamp, phase_a_done,
                       s->ring + (int64_t)append_slot * d, (int64_t)T * d, peer ? &own : nullptr);
   if (rc != LSTEP_OK) return rc;
   // 2 CTAs per SM: the append is resident (copying, then waiting for the phase-B MLP) while the NEXT step's DFT filter

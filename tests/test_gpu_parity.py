@@ -884,6 +884,11 @@ def test_native_multi_step_run_and_profile_are_bit_identical_to_single_steps(tor
     v = ctypes.c_int(-1)
     assert lib.lstep_get_option(b"pdl", ctypes.byref(v)) == 0 and v.value == 1
     assert lib.lstep_set_option(b"no_such_option", 1) != 0
+    # switches that were removed must be rejected, not silently ignored
+    for name in (b"cos_spread", b"gather_narrow", b"dft_early_trigger", b"host_memcpy", b"dft_ctas_per_sm", b"dft_generic",
+                 b"mlp_ring", b"gather_fuse", b"mlp_pair", b"early_append", b"dft_prefetch", b"query_dedup"):
+        assert lib.lstep_set_option(name, 1) != 0, name
+        assert lib.lstep_get_option(name, ctypes.byref(v)) != 0, name
 
 
 @pytest.mark.parametrize("tag", ["small", "full"])
@@ -973,15 +978,15 @@ def test_stress_2000_steps_pdl_vs_plain_launches_bit_identical(torch_cuda, zipf_
     assert torch.isfinite(res[0][0]).all()
 
 
-def test_identical_query_sets_are_computed_once_with_identical_results(torch_cuda):
+def test_identical_query_sets_computed_once_match_equal_copies(torch_cuda):
     """The eval loop passes the batch's sources twice (positive source, negative source under random negative sampling:
     evaluate_model_utils.py:51-52). The step recognises identical sets (same device pointer / same host array), computes
     them once and fans the rows out in the MLP epilogue: outputs, tables and histories must be bit-identical to the step
-    with the optimisation off, for the device-resident and the host-fed step, B = 200 (SIMT MLP) and B = 2000 (tcgen05 MLP)."""
+    given an equal copy of the set instead (a distinct pointer / array: computed separately), for the device-resident and the
+    host-fed step, B = 200 (SIMT MLP) and B = 2000 (tcgen05 MLP)."""
     torch = torch_cuda
     from harness import build_dropin
-    from lstep_b200 import NeighborSampler, PEStream, _lib
-    lib = _lib.load()
+    from lstep_b200 import NeighborSampler, PEStream
     for B in (200, 2000):
         g = synth.make_graph("reddit", seed=1, num_edges=40_000)
         V, d, T, K = g.num_nodes, 172, 100, 20
@@ -993,24 +998,21 @@ def test_identical_query_sets_are_computed_once_with_identical_results(torch_cud
         neg_np = np.random.default_rng(0).integers(1, V + 1, g.num_edges - e0).astype(np.int64)
         neg = torch.from_numpy(neg_np).cuda()
         res = []
-        try:
-            for dedup in (1, 0):
-                _lib.check(lib.lstep_set_option(b"query_dedup", dedup), "opt")
-                st = PEStream(lstep, g.src_node_ids, g.dst_node_ids, g.node_interact_times, B, K, history=hist, start=e0)
-                outs = []
-                for b in range(2):
-                    lo, hi, _, _ = st.batch_arrays(b)
-                    src_view = st.src[lo:hi]
-                    outs.append(st.step(b, [src_view, st.dst[lo:hi], src_view, neg[lo - e0:hi - e0]]).clone())
-                for b in range(2, 4):  # host-fed: the same numpy array object twice
-                    lo, hi, _, _ = st.batch_arrays(b)
-                    src_np = g.src_node_ids[lo:hi]
-                    outs.append(torch.from_numpy(st.step_host(src_np, g.dst_node_ids[lo:hi], g.node_interact_times[lo:hi],
-                                                              [src_np, g.dst_node_ids[lo:hi], src_np, neg_np[lo - e0:hi - e0]])))
-                st.check_errors()
-                res.append((outs, st.cur.clone(), st.export_history()))
-        finally:
-            lib.lstep_set_option(b"query_dedup", 1)
+        for dedup in (1, 0):
+            st = PEStream(lstep, g.src_node_ids, g.dst_node_ids, g.node_interact_times, B, K, history=hist, start=e0)
+            outs = []
+            for b in range(2):
+                lo, hi, _, _ = st.batch_arrays(b)
+                src_view = st.src[lo:hi]
+                outs.append(st.step(b, [src_view, st.dst[lo:hi], src_view if dedup else src_view.clone(), neg[lo - e0:hi - e0]]).clone())
+            for b in range(2, 4):  # host-fed: the same numpy array object twice
+                lo, hi, _, _ = st.batch_arrays(b)
+                src_np = g.src_node_ids[lo:hi]
+                outs.append(torch.from_numpy(st.step_host(src_np, g.dst_node_ids[lo:hi], g.node_interact_times[lo:hi],
+                                                          [src_np, g.dst_node_ids[lo:hi], src_np if dedup else src_np.copy(),
+                                                           neg_np[lo - e0:hi - e0]])))
+            st.check_errors()
+            res.append((outs, st.cur.clone(), st.export_history()))
         for a, b_ in zip(res[0][0], res[1][0]):
             assert torch.equal(a, b_)
         assert torch.equal(res[0][0][0][0], res[0][0][0][2])  # the two source sets' outputs are the same rows
@@ -1018,12 +1020,11 @@ def test_identical_query_sets_are_computed_once_with_identical_results(torch_cud
 
 
 @pytest.mark.parametrize("B", [200, 2000])
-def test_gather_variants_are_bit_identical(torch_cuda, B):
-    """Two structural variants of the step's fused gather must not change a bit of the outputs, tables and histories:
-    cos_spread (an experiment, off by default: measured slower) — a query row's K x t cosines are spread over all threads of its
-    CTA and parked in shared memory, the frequency threads add them in the original order k = 0 .. K-1; gather_pipe — at B = 2000 (more query rows than the launch has CTAs)
-    the CTAs walk several rows each with an extra warp looking one row ahead (nbr_aggregate_rows_piped). With and without
-    query dedup, ragged last batch."""
+def test_gather_pipe_and_query_dedup_variants_are_bit_identical(torch_cuda, B):
+    """The variants of the step's fused gather must not change a bit of the outputs, tables and histories: gather_pipe — at
+    B = 2000 (more query rows than the launch has CTAs) the CTAs walk several rows each with an extra warp looking one row ahead
+    (nbr_aggregate_rows_piped) — on and off, each with the identical source query sets passed as one pointer (computed once)
+    and as an equal copy (computed separately). Ragged last batch."""
     torch = torch_cuda
     from harness import build_dropin
     from lstep_b200 import NeighborSampler, PEStream, _lib
@@ -1038,23 +1039,19 @@ def test_gather_variants_are_bit_identical(torch_cuda, B):
     neg = torch.from_numpy(np.random.default_rng(1).integers(1, V + 1, g.num_edges - e0).astype(np.int64)).cuda()
     res = {}
     try:
-        for dedup, pipe, spread in ((1, 0, 0), (1, 1, 0), (1, 0, 1), (1, 1, 1), (0, 1, 1), (0, 0, 0)):
-            _lib.check(lib.lstep_set_option(b"query_dedup", dedup), "opt")
+        for dedup, pipe in ((1, 0), (1, 1), (0, 1), (0, 0)):
             _lib.check(lib.lstep_set_option(b"gather_pipe", pipe), "opt")
-            _lib.check(lib.lstep_set_option(b"cos_spread", spread), "opt")
             st = PEStream(lstep, g.src_node_ids, g.dst_node_ids, g.node_interact_times, B, K, history=hist, start=e0)
             outs = []
             for b in range(st.num_batches):
                 lo, hi, _, _ = st.batch_arrays(b)
                 sv = st.src[lo:hi]
-                outs.append(st.step(b, [sv, st.dst[lo:hi], sv, neg[lo - e0:hi - e0]]).clone())
+                outs.append(st.step(b, [sv, st.dst[lo:hi], sv if dedup else sv.clone(), neg[lo - e0:hi - e0]]).clone())
             st.check_errors()
-            res[(dedup, pipe, spread)] = (outs, st.cur.clone(), st.export_history())
+            res[(dedup, pipe)] = (outs, st.cur.clone(), st.export_history())
     finally:
-        lib.lstep_set_option(b"query_dedup", 1)
         lib.lstep_set_option(b"gather_pipe", 1)
-        lib.lstep_set_option(b"cos_spread", 0)
-    ref = res[(1, 0, 0)]
+    ref = res[(1, 0)]
     for key, got in res.items():
         for a, b_ in zip(ref[0], got[0]):
             assert torch.equal(a, b_), key
