@@ -1,0 +1,144 @@
+"""The change-log PE history on the host side (csrc/changelog.cu on the device; layout in include/lstep_b200.h,
+`struct lstep_changelog`): one rank's log, the descriptor the kernels take, loading a logical history (checkpoint.History)
+into it, saving it as a checkpoint shard and replaying it into dense rows. ChangeLogStream (world 1),
+ReplicatedTableRank(history="changelog") and PeerRank each own one; they keep the window position (head, len) and move it
+with `advance`, the rule the native multi-step calls follow too. `filter_len` is the window the DFT filter is masked to."""
+from __future__ import annotations
+
+import ctypes
+
+import numpy as np
+import torch
+
+from . import _lib
+from . import checkpoint as ckpt
+
+
+def filter_len(batch_idx: int, length: int, T: int) -> int:
+    """Window length the next step's DFT filter is masked to: keyed on batch_idx while the history is shorter than T (Q5)."""
+    return min(max(batch_idx, 0), T) if length < T else T
+
+
+def advance(head: int, length: int, T: int):
+    """(slot, head, len) of a step on a window of T slots: the slot it writes, and the window after it. The window fills,
+    then each step overwrites its oldest slot."""
+    if length < T:
+        return (head + length) % T, head, length + 1
+    return head, (head + 1) % T, T
+
+
+def _to_dev(a, dev, dtype):
+    """A tensor, or a host numpy array (memory-mapped ones included: copied first), on `dev`."""
+    if isinstance(a, torch.Tensor):
+        return a.to(dev, dtype)
+    return torch.from_numpy(np.array(a, dtype={torch.float32: np.float32, torch.int64: np.int64}[dtype])).to(dev)
+
+
+class ChangeLogHistory:
+    """The change log of rank `rank` of a world-`world` group over V1 nodes: the nodes v with v % world == rank, node v at
+    row (v - rank) / world, `rows` of them (checkpoint.rows_of). `cap` events per window slot (at least 1). `ref` is the
+    lstep_changelog descriptor to pass to the native calls. The base rows of a new log are unset: `reset` or `load` fills
+    them."""
+
+    def __init__(self, V1: int, T: int, d: int, cap: int, world: int, rank: int, device):
+        if T > 128:
+            raise _lib.LstepError("the change-log history supports T <= 128 window steps")
+        self.V1, self.T, self.d, self.world, self.rank, self.dev = int(V1), int(T), int(d), int(world), int(rank), device
+        self.rows = ckpt.rows_of(self.V1, self.world, self.rank)
+        self.cap = cap = int(max(cap, 1))
+        H = 1
+        while H < 2 * cap:
+            H *= 2
+        self.base = torch.empty((self.rows, d), dtype=torch.float32, device=device)
+        self.ev_node = torch.zeros((T, cap), dtype=torch.int32, device=device)
+        self.ev_row = torch.empty((T, cap, d), dtype=torch.float32, device=device)
+        self.ev_cnt = torch.zeros(T, dtype=torch.int32, device=device)
+        self.ev_hash = torch.full((T, H), -1, dtype=torch.int64, device=device)
+        self.ev_mask = torch.zeros((max(self.rows, 1), 4), dtype=torch.int32, device=device)
+        self.desc = _lib.ChangeLog(self.base.data_ptr(), self.ev_node.data_ptr(), self.ev_row.data_ptr(), self.ev_cnt.data_ptr(),
+                                   self.ev_hash.data_ptr(), self.ev_mask.data_ptr(), max(self.rows, 1), T, cap, H, d, self.world,
+                                   self.rank)
+        self.ref = ctypes.byref(self.desc)
+
+    def reset(self, cur: torch.Tensor):
+        """A one-step history: base = the owned rows of the table `cur` [V1, d], no events. Returns the window (head, len)."""
+        self.base.copy_(cur[self.rank::self.world])
+        self.ev_cnt.zero_()
+        self.ev_hash.fill_(-1)
+        self.ev_mask.zero_()
+        return 0, 1
+
+    def load(self, hist: "ckpt.History", cur: torch.Tensor):
+        """Load a logical history (any world size) into this log and the table `cur` [V1, d]. cur = every node's base row;
+        then, for every window position f in order, cur[nodes of f] = their rows and lstep_changelog_append records the rows
+        of the owned nodes as the events of slot f, exactly as a live step records them. After the last position cur is the
+        current table. The event count of every position is checked against the capacity before any device write. Returns
+        the window (head, len)."""
+        world, rank, dev = self.world, self.rank, self.dev
+        cnt = hist.counts(world)[:, rank]
+        if len(cnt) and int(cnt.max()) > self.cap:
+            f = int(cnt.argmax())
+            raise _lib.LstepError(f"window position {f} of the history holds {int(cnt[f])} events of rank {rank} of {world} but "
+                                  f"event_capacity is {self.cap}: pass a larger event_capacity")
+        lib = _lib.load()
+        chunk = max(1, (256 << 20) // (4 * hist.d))
+        with torch.cuda.device(dev), torch.no_grad():
+            for g, sh in enumerate(hist.shards):
+                dst = cur[g::hist.world]
+                for a in range(0, dst.shape[0], chunk):
+                    dst[a:a + chunk].copy_(_to_dev(sh["base"][a:a + chunk], dev, torch.float32))
+            self.reset(cur)
+            err = torch.zeros(1, dtype=torch.int32, device=dev)
+            for f in range(hist.len):
+                nodes, rows = hist.events(f)
+                ids = _to_dev(nodes, dev, torch.int64) if len(nodes) else None
+                if ids is not None:
+                    cur[ids] = _to_dev(rows, dev, torch.float32)
+                _lib.check(lib.lstep_changelog_append(self.ref, f, 0, _lib.ptr(cur), None, None, 0, _lib.ptr(ids), len(nodes), None, 0, 0,
+                                                      _lib.ptr(err), _lib.stream_ptr()), "lstep_changelog_append")
+            if int(err.item()):
+                raise _lib.LstepError(f"loading the history overflowed the change log (flag {int(err.item())})")
+        return 0, hist.len
+
+    def save(self, path: str, head: int, length: int, meta: dict):
+        """Write the window (head, length) of this log as shard `rank` of a checkpoint in directory `path`: the base rows and
+        the events of every window position in logical order (sorted by node within a position, so that one state always
+        gives the same files). `meta`: batch_idx, steps_done and edges_done. Call the owner's check_errors() first."""
+        torch.cuda.synchronize(self.dev)
+        cnt = self.ev_cnt.cpu().numpy()
+        slots = [(head + f) % self.T for f in range(length)]
+        off = np.cumsum([0] + [int(cnt[s]) for s in slots]).astype(np.int64)
+        ev_node = np.empty(int(off[-1]), np.int64)
+        ev_row = np.empty((int(off[-1]), self.d), np.float32)
+        for f, s in enumerate(slots):
+            n = int(cnt[s])
+            if n:
+                nodes = self.ev_node[s, :n].cpu().numpy()
+                order = np.argsort(nodes, kind="stable")
+                ev_node[off[f]:off[f + 1]] = nodes[order]
+                ev_row[off[f]:off[f + 1]] = self.ev_row[s, :n].cpu().numpy()[order]
+        meta = dict(meta, world=self.world, rank=self.rank, V1=self.V1, d=self.d, T=self.T, len=length)
+        ckpt.write_shard(path, meta, self.base.cpu().numpy(), off, ev_node, ev_row)
+
+    def replay(self, head: int, length: int) -> torch.Tensor:
+        """The window (head, length) as dense rows [rows, length, d], oldest first (needs rows * length * d * 4 bytes)."""
+        snap = self.base.clone()
+        out = torch.empty((self.rows, length, self.d), dtype=torch.float32, device=self.dev)
+        cnt = self.ev_cnt.cpu().tolist()
+        for f in range(length):
+            s = (head + f) % self.T
+            if cnt[s]:
+                snap[(self.ev_node[s, :cnt[s]].long() - self.rank) // self.world] = self.ev_row[s, :cnt[s]]
+            out[:, f, :] = snap
+        return out
+
+    def nbytes(self) -> int:
+        """Bytes the log occupies (base + event rows + index structures)."""
+        return sum(t.numel() * t.element_size() for t in (self.base, self.ev_node, self.ev_row, self.ev_cnt, self.ev_hash, self.ev_mask))
+
+    def check_full(self, err: torch.Tensor, flag: int):
+        """LstepError if `flag`, the value read from the device error flag `err`, says a step recorded more events than the
+        capacity (FLAG_CHANGELOG_FULL); the flag is cleared first."""
+        if flag & _lib.FLAG_CHANGELOG_FULL:
+            err.zero_()
+            raise _lib.LstepError(f"a step changed more rows than the change-log history's event capacity ({self.cap})")

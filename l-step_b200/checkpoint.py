@@ -13,7 +13,7 @@ Shard g consists of
 
 History value x[v, f] = the row of v's latest event at a window position <= f, else base[v]; the current table is
 x[:, len - 1]. The ring slots of the change log are normalised away and ownership is a function of the node id, so a
-checkpoint loads into a change log of any world size (stream._changelog_load). The table, the CSR and the model
+checkpoint loads into a change log of any world size (changelog.ChangeLogHistory.load). The table, the CSR and the model
 parameters are not stored: the table is the newest window position, the CSR is rebuilt from the edge stream and the
 parameters are the caller's state_dict.
 

@@ -22,9 +22,9 @@ import torch
 
 from . import _lib
 from . import checkpoint as ckpt
+from .changelog import ChangeLogHistory, advance, filter_len
 from .model import LSTEP
 from .sampler import NeighborSampler
-from .stream import _changelog_load, _changelog_save
 
 
 class _DevMem:
@@ -107,8 +107,11 @@ class PeerRank:
         self.d, self.t_dim = model.pe_dim, model.time_feat_dim
         self.V1 = int(num_nodes) + 1
         self.timeout_ms = int(timeout_ms)
-        if self.T > 128:
-            raise _lib.LstepError("the change-log history supports T <= 128 window steps")
+        # change log of the owned nodes; its capacity is the same on every rank: the inbox blocks are laid out by it
+        G, B = self.G, self.B
+        cap = event_capacity if event_capacity is not None else min((self.V1 + G - 1) // G, 2 * (2 * B * (self.K + 1) + 2) // G + 1024)
+        self.changelog = ChangeLogHistory(self.V1, self.T, self.d, cap, G, self.rank, dev)
+        self.rows_local, self.cap = self.changelog.rows, self.changelog.cap
         hist = None
         if checkpoint is not None:
             hist = checkpoint if isinstance(checkpoint, ckpt.History) else ckpt.read(checkpoint)
@@ -119,7 +122,7 @@ class PeerRank:
             hist.check(V1=self.V1, d=self.d, T=self.T)
         lib = self.lib = _lib.load()
         as_dev = lambda a, dt: (a.to(dev, dt) if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a)).to(dev, dt))
-        T, d, G, B = self.T, self.d, self.G, self.B
+        T, d = self.T, self.d
         with torch.cuda.device(dev):
             self.src, self.dst, self.tt = as_dev(src, torch.int64), as_dev(dst, torch.int64), as_dev(t, torch.float64)
             E = int(self.src.shape[0])
@@ -132,30 +135,15 @@ class PeerRank:
             self.sampler = model.neighbor_sampler = sampler
             # ---- memory the other ranks WRITE (cudaMalloc + CUDA IPC; small fixed regions): phase-A row buffer, filtered-row buffer,
             # inbox (one block per source rank for the rows it changed in a step), barrier flags
-            self.rows_local = (self.V1 - self.rank + G - 1) // G
-            # (the same on every rank: the inbox blocks are laid out by it)
-            cap = event_capacity if event_capacity is not None else min((self.V1 + G - 1) // G, 2 * (2 * B * (self.K + 1) + 2) // G + 1024)
-            self.cap = cap = int(max(cap, 1))
-            H = 1
-            while H < 2 * cap:
-                H *= 2
             self._mem_rows = _DevMem(lib, 2 * B * d * 4)
             self._mem_filt = _DevMem(lib, 2 * B * d * 4)
-            self._mem_inbox = _DevMem(lib, max(int(lib.lstep_peer_inbox_bytes(G, cap, d)), 256))
+            self._mem_inbox = _DevMem(lib, max(int(lib.lstep_peer_inbox_bytes(G, self.cap, d)), 256))
             self._mem_flags = _DevMem(lib, 16 * 4)
             self.cur = torch.empty((self.V1, d), dtype=torch.float32, device=dev)
             if hist is None:
                 self.cur.copy_(initial_pe.to(dev, torch.float32))
+                self.head, self.len = self.changelog.reset(self.cur)
             self.new_rows = self._mem_rows.tensor((2 * B, d), torch.float32, dev)
-            # ---- change log of the owned nodes
-            self.base = self.cur[self.rank::G].contiguous().clone()  # (overwritten by _changelog_load from a history)
-            self.ev_node = torch.zeros((T, cap), dtype=torch.int32, device=dev)
-            self.ev_row = torch.empty((T, cap, d), dtype=torch.float32, device=dev)
-            self.ev_cnt = torch.zeros(T, dtype=torch.int32, device=dev)
-            self.ev_hash = torch.full((T, H), -1, dtype=torch.int64, device=dev)
-            self.ev_mask = torch.zeros((max(self.rows_local, 1), 4), dtype=torch.int32, device=dev)
-            self.cl = _lib.ChangeLog(self.base.data_ptr(), self.ev_node.data_ptr(), self.ev_row.data_ptr(), self.ev_cnt.data_ptr(),
-                                     self.ev_hash.data_ptr(), self.ev_mask.data_ptr(), max(self.rows_local, 1), T, cap, H, d, G, self.rank)
             self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.tt.data_ptr(), None, self.cur.data_ptr(), self.V1, T, d)
             # ---- per-batch plan of the resident stream: one pass on the host, uploaded once
             src_h = self.src[self.start:stop].cpu().numpy()
@@ -179,13 +167,12 @@ class PeerRank:
             need = lib.lstep_pe_step_workspace_bytes(2 * B, B, 8, self.K, d, self.t_dim, self.V1)
             self.ws = torch.empty(need + 4096, dtype=torch.uint8, device=dev)
             _lib.check(lib.lstep_update_pe_workspace_init(_lib.ptr(self.ws), self.ws.numel(), self.V1, _lib.stream_ptr()), "ws init")
-        self.head, self.len, self.batch_idx = 0, 1, 0
-        self.steps_done, self.edges_done = 0, self.start
+        self.batch_idx, self.steps_done, self.edges_done = 0, 0, self.start
         self.epoch = ctypes.c_uint32(0)  # (a fresh rank: the flag blocks are zeroed by lstep_ipc_alloc)
         self.grp = None
         self._opened = []
         if hist is not None:
-            _changelog_load(self, hist, G, self.rank)
+            self.head, self.len = self.changelog.load(hist, self.cur)
             if checkpoint is not None:
                 self.batch_idx, self.steps_done, self.edges_done = (int(hist.meta[k]) for k in ("batch_idx", "steps_done", "edges_done"))
         if batch_idx is not None:
@@ -257,14 +244,13 @@ class PeerRank:
         C = len(queries)
         i0, i1 = int(self.ids_off[b]), int(self.ids_off[b + 1])
         m0, m1 = int(self.mine_off[b]), int(self.mine_off[b + 1])
-        bmask = min(max(self.batch_idx, 0), T) if self.len < T else T
         with torch.cuda.device(self.dev), torch.no_grad():
-            Gt = self.m._collapsed_filter(bmask, False)
+            Gt = self.m._collapsed_filter(filter_len(self.batch_idx, self.len, T), False)
             if out is None:
                 out = torch.empty((max(C, 1), q_rows, d), dtype=torch.float32, device=self.dev)
             qptrs = (ctypes.c_void_p * max(C, 1))(*[q.data_ptr() + 8 * q_off for q in queries])
             i64p = lambda t_, o: ctypes.c_void_p(t_.data_ptr() + 8 * o)
-            _lib.check(lib.lstep_pe_step_peer(ctypes.byref(self.desc), ctypes.byref(self.cl), self.sampler.csr_ref, ctypes.byref(self.grp), lo, hi - lo,
+            _lib.check(lib.lstep_pe_step_peer(ctypes.byref(self.desc), self.changelog.ref, self.sampler.csr_ref, ctypes.byref(self.grp), lo, hi - lo,
                                               i64p(self.ids, i0), i1 - i0, i64p(self.ids_mine, m0), i64p(self.pos_mine, m0), m1 - m0,
                                               float(self.tmax[b]), self.head, self.len, _lib.ptr(Gt), qptrs, C, q_off, q_rows, _lib.ptr(out), self.K,
                                               self.m._mlp_ref("nbr"), self.m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(),
@@ -277,10 +263,7 @@ class PeerRank:
 
     def _advance(self, n: int):
         for _ in range(n):
-            if self.len < self.T:
-                self.len += 1
-            else:
-                self.head = (self.head + 1) % self.T
+            _, self.head, self.len = advance(self.head, self.len, self.T)
         self.batch_idx += n
         self.steps_done += n
         self.epoch = ctypes.c_uint32((self.epoch.value + 2 * n) & 0xffffffff)
@@ -302,7 +285,7 @@ class PeerRank:
         lo = np.ascontiguousarray(self.lo[b0:b0 + n_steps])
         with torch.cuda.device(self.dev), torch.no_grad():
             Gt = self.m._collapsed_filter(self.T, False)
-            rc = lib.lstep_pe_steps_peer(ctypes.byref(self.desc), ctypes.byref(self.cl), self.sampler.csr_ref, ctypes.byref(self.grp), n_steps,
+            rc = lib.lstep_pe_steps_peer(ctypes.byref(self.desc), self.changelog.ref, self.sampler.csr_ref, ctypes.byref(self.grp), n_steps,
                                          ap(lo, 0), ap(self.n_edges, b0), ap(self.tmax, b0), _lib.ptr(self.ids), ap(ids_off, 0),
                                          _lib.ptr(self.ids_mine), _lib.ptr(self.pos_mine), ap(mine_off, 0), ctypes.byref(head), _lib.ptr(Gt), qptrs,
                                          ap(lo, 0), C, _lib.ptr(out), int(out_step_stride), self.K, self.m._mlp_ref("nbr"),
@@ -330,9 +313,7 @@ class PeerRank:
         if flag & _lib.FLAG_PEER_TIMEOUT:
             self.sampler._err.zero_()
             raise _lib.LstepError("a peer GPU did not reach a step barrier in time (peer group step)")
-        if flag & _lib.FLAG_CHANGELOG_FULL:
-            self.sampler._err.zero_()
-            raise _lib.LstepError(f"a step changed more owned rows than the change-log history's event capacity ({self.cap})")
+        self.changelog.check_full(self.sampler._err, flag)
         self.sampler.check_errors()
 
     def save_checkpoint(self, path: str):
@@ -340,22 +321,15 @@ class PeerRank:
         events of the nodes it owns. Every rank of the group calls it after the same step; no barrier is needed (an owner's
         history is always current on its own rank). The checkpoint loads into a group of any world size, or a
         ChangeLogStream, and the resumed run computes the bits of the uninterrupted one."""
-        _changelog_save(self, path, self.G, self.rank)
+        self.check_errors()
+        self.changelog.save(path, self.head, self.len, dict(batch_idx=self.batch_idx, steps_done=self.steps_done, edges_done=self.edges_done))
 
     def history_bytes(self) -> int:
-        return sum(t.numel() * t.element_size() for t in (self.base, self.ev_node, self.ev_row, self.ev_cnt, self.ev_hash, self.ev_mask))
+        return self.changelog.nbytes()
 
     def export_history_rows(self) -> torch.Tensor:
         """[rows_local, len, d], oldest first: row l = node l * G + rank."""
-        snap = self.base.clone()
-        out = torch.empty((self.rows_local, self.len, self.d), dtype=torch.float32, device=self.dev)
-        cnt = self.ev_cnt.cpu().tolist()
-        for f in range(self.len):
-            slot = (self.head + f) % self.T
-            if cnt[slot]:
-                snap[(self.ev_node[slot, :cnt[slot]].long() - self.rank) // self.G] = self.ev_row[slot, :cnt[slot]]
-            out[:, f, :] = snap[:self.rows_local]
-        return out
+        return self.changelog.replay(self.head, self.len)
 
 
 class PeerLocalGroup:

@@ -29,6 +29,8 @@ import numpy as np
 import torch
 
 from . import _lib
+from . import checkpoint as ckpt
+from .changelog import ChangeLogHistory, advance, filter_len
 from .model import LSTEP
 from .sampler import NeighborSampler
 
@@ -413,7 +415,7 @@ class ReplicatedTableRank:
             self._cur_full[:self.V1] = initial_pe.to(dev, torch.float32)
             self._cur_full[self.V1].zero_()
             self.cur = self._cur_full[:self.V1]
-            self.rows_local = (self.V1 - self.rank + self.G - 1) // self.G  # owned node ids: rank, rank + G, ...
+            self.rows_local = ckpt.rows_of(self.V1, self.G, self.rank)  # owned node ids: rank, rank + G, ...
             self.head, self.len = 0, 1
             if history == "ring":
                 self.ring = torch.zeros((max(self.rows_local, 1), self.T, self.d), dtype=torch.float32, device=dev)
@@ -421,22 +423,10 @@ class ReplicatedTableRank:
                                                     _lib.stream_ptr()), "ring init")
                 ring_ptr = self.ring.data_ptr()
             else:
-                if self.T > 128:
-                    raise _lib.LstepError("the change-log history supports T <= 128 window steps")
-                T, d = self.T, self.d
                 cap = event_capacity if event_capacity is not None else min(self.rows_local, 2 * (2 * int(batch_size) * (self.K + 1) + 2) // self.G + 1024)
-                self.cap = cap = int(max(cap, 1))
-                H = 1
-                while H < 2 * cap:
-                    H *= 2
-                self.base = self.cur[self.rank::self.G].contiguous().clone()
-                self.ev_node = torch.zeros((T, cap), dtype=torch.int32, device=dev)
-                self.ev_row = torch.empty((T, cap, d), dtype=torch.float32, device=dev)
-                self.ev_cnt = torch.zeros(T, dtype=torch.int32, device=dev)
-                self.ev_hash = torch.full((T, H), -1, dtype=torch.int64, device=dev)
-                self.ev_mask = torch.zeros((max(self.rows_local, 1), 4), dtype=torch.int32, device=dev)
-                self.cl = _lib.ChangeLog(self.base.data_ptr(), self.ev_node.data_ptr(), self.ev_row.data_ptr(), self.ev_cnt.data_ptr(),
-                                         self.ev_hash.data_ptr(), self.ev_mask.data_ptr(), max(self.rows_local, 1), T, cap, H, d, self.G, self.rank)
+                self.changelog = ChangeLogHistory(self.V1, self.T, self.d, cap, self.G, self.rank, dev)
+                self.cap = self.changelog.cap
+                self.changelog.reset(self.cur)
                 self.ring = None
                 ring_ptr = None
             self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.tt.data_ptr(), ring_ptr, self.cur.data_ptr(),
@@ -494,16 +484,15 @@ class ReplicatedTableRank:
         n_mine = self.mine_off[b + 1] - self.mine_off[b]
         mx = self.max_n[b]
         send = self._mine[:mx]
-        bmask = min(max(self.batch_idx, 0), T) if self.len < T else T
         with torch.cuda.device(self.dev), torch.no_grad():
             if n_mine:
-                Gt = self.m._collapsed_filter(bmask, False)
+                Gt = self.m._collapsed_filter(filter_len(self.batch_idx, self.len, T), False)
                 loc = self.mine_local[self.mine_off[b]:self.mine_off[b + 1]]
                 if self.history == "ring":
                     _lib.check(lib.lstep_dft_filter(_lib.ptr(self.ring), T * d, d, self.head, T, self.len, d, _lib.ptr(loc), n_mine, _lib.ptr(Gt),
                                                     _lib.ptr(send), d, _lib.stream_ptr()), "dft_filter")
                 else:
-                    _lib.check(lib.lstep_changelog_filter(ctypes.byref(self.cl), self.head, self.len, _lib.ptr(loc), n_mine, _lib.ptr(Gt), _lib.ptr(send),
+                    _lib.check(lib.lstep_changelog_filter(self.changelog.ref, self.head, self.len, _lib.ptr(loc), n_mine, _lib.ptr(Gt), _lib.ptr(send),
                                                           d, None, _lib.stream_ptr()), "changelog_filter")
         return send
 
@@ -523,52 +512,37 @@ class ReplicatedTableRank:
             ids = self.ids[self.ids_off[b]:self.ids_off[b + 1]]
             qptrs = (ctypes.c_void_p * max(C, 1))(*[q.data_ptr() + 8 * q_off for q in queries])
             if self.history == "changelog":  # step + retire / append of the owned rows' events (phase 2: the filter is done)
-                _lib.check(lib.lstep_pe_step_changelog(ctypes.byref(self.desc), ctypes.byref(self.cl), self.sampler.csr_ref, lo, n, _lib.ptr(ids),
+                _lib.check(lib.lstep_pe_step_changelog(ctypes.byref(self.desc), self.changelog.ref, self.sampler.csr_ref, lo, n, _lib.ptr(ids),
                                                        ids.shape[0], self.tmax[b], self.head, self.len, None, qptrs, C, q_off, q_rows, _lib.ptr(out),
                                                        self.K, self.m._mlp_ref("nbr"), self.m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(),
                                                        _lib.ptr(self.sampler._err), _lib.stream_ptr(), 2), "lstep_pe_step_changelog")
-                if self.len < T:
-                    self.len += 1
-                else:
-                    self.head = (self.head + 1) % T
+                _, self.head, self.len = advance(self.head, self.len, T)
                 self.batch_idx += 1
                 return out
             _lib.check(lib.lstep_pe_step_sharded(ctypes.byref(self.desc), self.sampler.csr_ref, lo, n, _lib.ptr(ids), ids.shape[0], self.tmax[b],
                                                  qptrs, C, q_off, q_rows, _lib.ptr(out), self.K, self.m._mlp_ref("nbr"), self.m._mlp_ref("update"),
                                                  _lib.ptr(self.ws), self.ws.numel(), _lib.ptr(self.sampler._err), _lib.stream_ptr()),
                        "lstep_pe_step_sharded")
-            if self.len < T:
-                slot, self.len = (self.head + self.len) % T, self.len + 1
-            else:
-                slot, self.head = self.head, (self.head + 1) % T
+            slot, self.head, self.len = advance(self.head, self.len, T)
             _lib.check(lib.lstep_ring_copy_rows(_lib.ptr(self.ring), _lib.ptr(self.cur), self.rows_local, T, d, slot, G, self.rank, 1,
                                                 _lib.stream_ptr()), "ring append")
         self.batch_idx += 1
         return out
 
     def check_errors(self):
-        flag = int(self.sampler._err.item())
-        if flag & _lib.FLAG_CHANGELOG_FULL:
-            self.sampler._err.zero_()
-            raise _lib.LstepError(f"a step changed more owned rows than the change-log history's event capacity ({self.cap})")
+        if self.history == "changelog":
+            self.changelog.check_full(self.sampler._err, int(self.sampler._err.item()))
         self.sampler.check_errors()
 
     def history_bytes(self) -> int:
-        ts = (self.ring,) if self.history == "ring" else (self.base, self.ev_node, self.ev_row, self.ev_cnt, self.ev_hash, self.ev_mask)
-        return sum(t.numel() * t.element_size() for t in ts)
+        if self.history == "changelog":
+            return self.changelog.nbytes()
+        return self.ring.numel() * self.ring.element_size()
 
     def export_history_rows(self) -> torch.Tensor:
         """[rows_local, len, d], oldest first: row l = node l * G + rank."""
         if self.history == "changelog":
-            snap = self.base.clone()
-            out = torch.empty((self.rows_local, self.len, self.d), dtype=torch.float32, device=self.dev)
-            cnt = self.ev_cnt.cpu().tolist()
-            for f in range(self.len):
-                slot = (self.head + f) % self.T
-                if cnt[slot]:
-                    snap[(self.ev_node[slot, :cnt[slot]].long() - self.rank) // self.G] = self.ev_row[slot, :cnt[slot]]
-                out[:, f, :] = snap[:self.rows_local]
-            return out
+            return self.changelog.replay(self.head, self.len)
         idx = (self.head + torch.arange(self.len, device=self.dev)) % self.T
         return self.ring.index_select(1, idx)[:self.rows_local]
 

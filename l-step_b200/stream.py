@@ -27,79 +27,13 @@ import torch
 
 from . import _lib
 from . import checkpoint as ckpt
+from .changelog import ChangeLogHistory, advance, filter_len
 from .model import LSTEP
 from .sampler import check_edges
 
 C_void_p = ctypes.c_void_p
 C_byref = ctypes.byref
 _I64, _F64 = np.dtype(np.int64), np.dtype(np.float64)
-
-
-def _to_dev(a, dev, dtype):
-    """A tensor, or a host numpy array (memory-mapped ones included: copied first), on `dev`."""
-    if isinstance(a, torch.Tensor):
-        return a.to(dev, dtype)
-    return torch.from_numpy(np.array(a, dtype={torch.float32: np.float32, torch.int64: np.int64}[dtype])).to(dev)
-
-
-def _changelog_load(obj, hist: "ckpt.History", world: int, rank: int):
-    """Load a logical history (checkpoint.History, any world size) into the change log of `obj` (a
-    ChangeLogStream: world 1, rank 0; a PeerRank: its group) and into its table replica obj.cur. cur = every node's base
-    row; then, for every window position f in order, cur[nodes of f] = their rows and lstep_changelog_append records the
-    rows of the nodes this rank owns as the events of slot f, exactly as a live step records them. After the last position
-    cur is the current table. The event count of every position is checked against the capacity before any device write."""
-    cnt = hist.counts(world)[:, rank]
-    if len(cnt) and int(cnt.max()) > obj.cap:
-        f = int(cnt.argmax())
-        raise _lib.LstepError(f"window position {f} of the history holds {int(cnt[f])} events of rank {rank} of {world} but "
-                              f"event_capacity is {obj.cap}: pass a larger event_capacity")
-    lib = _lib.load()
-    dev = obj.dev
-    chunk = max(1, (256 << 20) // (4 * hist.d))
-    with torch.cuda.device(dev), torch.no_grad():
-        for g, sh in enumerate(hist.shards):
-            dst = obj.cur[g::hist.world]
-            for a in range(0, dst.shape[0], chunk):
-                dst[a:a + chunk].copy_(_to_dev(sh["base"][a:a + chunk], dev, torch.float32))
-        obj.base.copy_(obj.cur[rank::world])
-        obj.ev_cnt.zero_()
-        obj.ev_hash.fill_(-1)
-        obj.ev_mask.zero_()
-        err = torch.zeros(1, dtype=torch.int32, device=dev)
-        for f in range(hist.len):
-            nodes, rows = hist.events(f)
-            ids = _to_dev(nodes, dev, torch.int64) if len(nodes) else None
-            if ids is not None:
-                obj.cur[ids] = _to_dev(rows, dev, torch.float32)
-            _lib.check(lib.lstep_changelog_append(C_byref(obj.cl), f, 0, _lib.ptr(obj.cur), None, None, 0, _lib.ptr(ids), len(nodes), None, 0, 0,
-                                                  _lib.ptr(err), _lib.stream_ptr()), "lstep_changelog_append")
-        if int(err.item()):
-            raise _lib.LstepError(f"loading the history overflowed the change log (flag {int(err.item())})")
-    obj.head, obj.len = 0, hist.len
-
-
-def _changelog_save(obj, path: str, world: int, rank: int):
-    """Write the change log of `obj` (rank `rank` of a world-`world` group) as shard `rank` of a checkpoint in directory
-    `path`: its base rows and the events of every window position in logical order (from the ring's head; sorted by node
-    within a position, so that one state always gives the same files)."""
-    obj.check_errors()
-    torch.cuda.synchronize(obj.dev)
-    cnt = obj.ev_cnt.cpu().numpy()
-    slots = [(obj.head + f) % obj.T for f in range(obj.len)]
-    off = np.cumsum([0] + [int(cnt[s]) for s in slots]).astype(np.int64)
-    ev_node = np.empty(int(off[-1]), np.int64)
-    ev_row = np.empty((int(off[-1]), obj.d), np.float32)
-    for f, s in enumerate(slots):
-        n = int(cnt[s])
-        if n:
-            nodes = obj.ev_node[s, :n].cpu().numpy()
-            order = np.argsort(nodes, kind="stable")
-            ev_node[off[f]:off[f + 1]] = nodes[order]
-            ev_row[off[f]:off[f + 1]] = obj.ev_row[s, :n].cpu().numpy()[order]
-    base = obj.base[:ckpt.rows_of(obj.V1, world, rank)].cpu().numpy()
-    meta = dict(world=world, rank=rank, V1=obj.V1, d=obj.d, T=obj.T, len=obj.len, batch_idx=obj.batch_idx, steps_done=obj.steps_done,
-                edges_done=obj.edges_done)
-    ckpt.write_shard(path, meta, base, off, ev_node, ev_row)
 
 
 class PEStream:
@@ -226,17 +160,12 @@ class PEStream:
         """Device-resident core shared by step() and step_host()."""
         lib = _lib.load()
         m = self.model
-        T = self.T
         bi = self.batch_idx if batch_idx is None else batch_idx
-        bmask = min(max(bi, 0), T) if self.len < T else T  # mask keyed on batch_idx while the history is short (Q5)
         C = len(queries)
         with torch.cuda.device(self.dev), torch.no_grad():
-            G = m._collapsed_filter(bmask, False)
+            G = m._collapsed_filter(filter_len(bi, self.len, self.T), False)
             ws = self._workspace(ids.shape[0], n_edges, C)
-            if self.len < T:
-                slot, new_head, new_len = (self.head + self.len) % T, self.head, self.len + 1
-            else:
-                slot, new_head, new_len = self.head, (self.head + 1) % T, T
+            slot, new_head, new_len = advance(self.head, self.len, self.T)
             qptrs = (C_void_p * max(C, 1))(*[q.data_ptr() for q in queries])
             _lib.check(lib.lstep_pe_step(self._desc_ref, m.neighbor_sampler.csr_ref, lo, n_edges, _lib.ptr(ids), ids.shape[0],
                                          float(tmax), self.head, self.len, slot, _lib.ptr(G), qptrs, C, _lib.ptr(out), self.K,
@@ -418,9 +347,7 @@ class PEStream:
             ids = np.ascontiguousarray(ids, dtype=_I64)
         if ingest:
             eid0 = self._check_ingest(src, dst, times, edge_id_start)
-        T = self.T
         bi = self.batch_idx if batch_idx is None else batch_idx
-        bmask = min(max(bi, 0), T) if self.len < T else T
         if torch.cuda.current_device() != self.dev.index:
             torch.cuda.set_device(self.dev)
         st = self._host_stepper
@@ -432,14 +359,11 @@ class PEStream:
             self._arm_ingest(h, eid0)
         elif self._armed is not None:
             self._disarm_ingest(h)
-        G = m._collapsed_filter(bmask, False)
+        G = m._collapsed_filter(filter_len(bi, self.len, self.T), False)
         ws = self._ws
         if ws is None or n > self._ws_cap[1] or C > self._ws_cap[2] or 2 * n > self._ws_cap[0]:
             ws = self._workspace(len(ids) if ids is not None else 2 * n, n, C)
-        if self.len < T:
-            slot, new_head, new_len = (self.head + self.len) % T, self.head, self.len + 1
-        else:
-            slot, new_head, new_len = self.head, (self.head + 1) % T, T
+        slot, new_head, new_len = advance(self.head, self.len, self.T)
         qptrs = (C_void_p * max(C, 1))(*[q.ctypes.data for q in qs])
         ticket = ctypes.c_int64(-1)
         samp = m.neighbor_sampler
@@ -610,10 +534,11 @@ class ChangeLogStream(PEStream):
         events of every window position, about V1 + T * (rows changed per step) rows; not the table, the CSR or the model
         parameters). ChangeLogStream(..., checkpoint=path) and PeerRank(..., checkpoint=path) at any world size resume
         from it with the bits of the uninterrupted run."""
-        _changelog_save(self, path, 1, 0)
+        self.check_errors()
+        self.changelog.save(path, self.head, self.len, dict(batch_idx=self.batch_idx, steps_done=self.steps_done, edges_done=self.edges_done))
 
     def _load(self, hist: "ckpt.History"):
-        """Allocate the change log for hist.V1 rows and load `hist` into it (_changelog_load)."""
+        """Allocate the change log for hist.V1 rows and load `hist` into it."""
         V1, d = hist.V1, self.d
         if len(self.ids_np):
             lo_id, hi_id = int(self.ids_np.min()), int(self.ids_np.max())
@@ -622,76 +547,45 @@ class ChangeLogStream(PEStream):
             samp = self.model.neighbor_sampler
             if samp is not None and (hi_id >= samp.num_rows or samp.num_rows > V1):
                 raise IndexError("list index out of range: the neighbor sampler's rows do not cover the stream / exceed the table")
-        if self.T > 128:
-            raise _lib.LstepError("the change-log history supports T <= 128 window steps")
-        self.V1 = V1
-        T = self.T
         cap = self._cap_arg if self._cap_arg is not None else min(V1, 2 * self.B * (self.K + 1) + 2)
-        self.cap = cap = int(max(cap, 1))
-        H = 1
-        while H < 2 * cap:
-            H *= 2
-        dev = self.dev
-        self.base = torch.empty((V1, d), dtype=torch.float32, device=dev)
-        self.ev_node = torch.zeros((T, cap), dtype=torch.int32, device=dev)
-        self.ev_row = torch.empty((T, cap, d), dtype=torch.float32, device=dev)
-        self.ev_cnt = torch.zeros(T, dtype=torch.int32, device=dev)
-        self.ev_hash = torch.full((T, H), -1, dtype=torch.int64, device=dev)
-        self.ev_mask = torch.zeros((V1, 4), dtype=torch.int32, device=dev)
-        self.cl = _lib.ChangeLog(self.base.data_ptr(), self.ev_node.data_ptr(), self.ev_row.data_ptr(), self.ev_cnt.data_ptr(),
-                                 self.ev_hash.data_ptr(), self.ev_mask.data_ptr(), V1, T, cap, H, d, 1, 0)
+        self.changelog = ChangeLogHistory(V1, self.T, d, cap, 1, 0, self.dev)
+        self.cap = self.changelog.cap
+        self.V1 = V1
         self.ring = None
-        self.cur = torch.empty((V1, d), dtype=torch.float32, device=dev)
-        _changelog_load(self, hist, 1, 0)
-        self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.t.data_ptr(), None, self.cur.data_ptr(), V1, T, d)
+        self.cur = torch.empty((V1, d), dtype=torch.float32, device=self.dev)
+        self.head, self.len = self.changelog.load(hist, self.cur)
+        self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.t.data_ptr(), None, self.cur.data_ptr(), V1, self.T, d)
         self._ws = None
         self._ws_cap = (0, 0, 0)
 
     def history_bytes(self) -> int:
         """Bytes the history occupies (base + event rows + index structures) — against V1 * T * d * 4 for the dense ring."""
-        return sum(t.numel() * t.element_size() for t in (self.base, self.ev_node, self.ev_row, self.ev_cnt, self.ev_hash, self.ev_mask))
+        return self.changelog.nbytes()
 
     def export_history(self) -> torch.Tensor:
         """The dense layout [V1, len, d] (oldest first) replayed from the log (tests / save_pe; needs V1 * len * d * 4 bytes)."""
         self.check_errors()
-        snap = self.base.clone()
-        out = torch.empty((self.V1, self.len, self.d), dtype=torch.float32, device=self.dev)
-        cnt = self.ev_cnt.cpu().tolist()
-        for f in range(self.len):
-            slot = (self.head + f) % self.T
-            n = cnt[slot]
-            if n:
-                snap[self.ev_node[slot, :n].long()] = self.ev_row[slot, :n]
-            out[:, f, :] = snap
-        return out
+        return self.changelog.replay(self.head, self.len)
 
     def check_errors(self):
         samp = self.model.neighbor_sampler
-        flag = int(samp._err.item())
-        if flag & _lib.FLAG_CHANGELOG_FULL:
-            samp._err.zero_()
-            raise _lib.LstepError(f"a step changed more rows than the change-log history's event capacity ({self.cap})")
+        self.changelog.check_full(samp._err, int(samp._err.item()))
         samp.check_errors()
 
     def _run(self, lo, n_edges, ids, tmax, queries, out, batch_idx):
         lib = _lib.load()
         m = self.model
-        T = self.T
         bi = self.batch_idx if batch_idx is None else batch_idx
-        bmask = min(max(bi, 0), T) if self.len < T else T
         C = len(queries)
         with torch.cuda.device(self.dev), torch.no_grad():
-            G = m._collapsed_filter(bmask, False)
+            G = m._collapsed_filter(filter_len(bi, self.len, self.T), False)
             ws = self._workspace(ids.shape[0], n_edges, C)
             qptrs = (C_void_p * max(C, 1))(*[q.data_ptr() for q in queries])
-            _lib.check(lib.lstep_pe_step_changelog(self._desc_ref, ctypes.byref(self.cl), m.neighbor_sampler.csr_ref, lo, n_edges, _lib.ptr(ids),
+            _lib.check(lib.lstep_pe_step_changelog(self._desc_ref, self.changelog.ref, m.neighbor_sampler.csr_ref, lo, n_edges, _lib.ptr(ids),
                                                    ids.shape[0], float(tmax), self.head, self.len, _lib.ptr(G), qptrs, C, 0, -1, _lib.ptr(out),
                                                    self.K, m._mlp_ref("nbr"), m._mlp_ref("update"), _lib.ptr(ws), ws.numel(),
                                                    _lib.ptr(m.neighbor_sampler._err), _lib.stream_ptr(), 0), "lstep_pe_step_changelog")
-            if self.len < T:
-                self.len += 1
-            else:
-                self.head = (self.head + 1) % T
+            _, self.head, self.len = advance(self.head, self.len, self.T)
         self.batch_idx = bi + 1
         self.steps_done += 1
         self.edges_done = lo + n_edges
@@ -720,7 +614,7 @@ class ChangeLogStream(PEStream):
 
     def _step_host_native(self, h, samp, n, src, dst, times, ids, slot, G, qptrs, C, out, ws, ticket):
         m = self.model
-        rc = self._libc.lstep_pe_step_changelog_host(h, self._desc_ref, C_byref(self.cl), samp.csr_ref, n, src.ctypes.data, dst.ctypes.data,
+        rc = self._libc.lstep_pe_step_changelog_host(h, self._desc_ref, self.changelog.ref, samp.csr_ref, n, src.ctypes.data, dst.ctypes.data,
                                                      times.ctypes.data, ids.ctypes.data if ids is not None else None,
                                                      len(ids) if ids is not None else 0, self.head, self.len, G.data_ptr(), qptrs, C,
                                                      out.data_ptr() if out is not None else None, self.K, m._mlp_ref("nbr"),
@@ -732,7 +626,7 @@ class ChangeLogStream(PEStream):
 
     def _steps_host_native(self, h, samp, n_total, src, dst, times, qptrs, C, head, ln, G, ws, sub, done):
         m = self.model
-        rc = self._libc.lstep_pe_steps_changelog_host(h, self._desc_ref, C_byref(self.cl), samp.csr_ref, n_total, self.B, src.ctypes.data,
+        rc = self._libc.lstep_pe_steps_changelog_host(h, self._desc_ref, self.changelog.ref, samp.csr_ref, n_total, self.B, src.ctypes.data,
                                                       dst.ctypes.data, times.ctypes.data, qptrs, C, C_byref(head), C_byref(ln), G.data_ptr(),
                                                       self.K, m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(),
                                                       samp._err.data_ptr(), torch.cuda.current_stream().cuda_stream, sub.ctypes.data,

@@ -25,7 +25,6 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from lstep_b200 import LSTEP, PeerRank, _lib, checkpoint, synth  # noqa: E402
-from lstep_b200.stream import _changelog_load  # noqa: E402
 
 
 def card():
@@ -92,7 +91,7 @@ def main():
         t_mem = time.perf_counter() - t0
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        _changelog_load(rk2, hist, 1, 0)  # the same state again, from host memory: the device part alone
+        rk2.head, rk2.len = rk2.changelog.load(hist, rk2.cur)  # the same state again, from host memory: the device part alone
         torch.cuda.synchronize()
         t_dev = time.perf_counter() - t0
         n_ev = int(sum(int(sh["ev_off"][-1]) for sh in hist.shards))
