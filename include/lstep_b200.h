@@ -516,6 +516,36 @@ int lstep_pe_steps_changelog_host(lstep_host_stepper* h, const lstep_pe_stream* 
                                   int* len_io, const float* G, int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd,
                                   void* workspace, size_t workspace_bytes, uint32_t* err_flag, void* stream, float* results_host,
                                   int64_t* n_done_out);
+/* One rank's peer-group step (lstep_pe_step_peer) fed from HOST arrays: the same staging, host checks, optional append into the
+ * rank's own CSR replica (lstep_host_stepper_set_ingest) and result path as lstep_pe_step_host. The rank's owned ids of the batch
+ * and their positions are derived on the device from the staged ids, on the copy-in path. s->src / s->dst / s->t are never read.
+ * phases as in lstep_pe_step_peer; a single-process group issues each bit for every rank before the next:
+ *   - the call with bit 0 stages the batch and keeps it as the stepper's pending batch;
+ *   - later calls of the same step (bits 1, 2) use the pending batch: their n_edges, host arrays and n_queries are not read
+ *     (may be 0 / NULL), and nbr_out must be the one the staging call passed;
+ *   - the call with bit 2 finishes the step: row sums of this rank's share [n_queries][q_rows] (q_off = rank * n / world,
+ *     q_rows = (rank + 1) * n / world - q_off) into the pinned result, and *ticket.
+ * LSTEP_ERR_INVALID_ARG for a later phase with no pending batch and for staging while a batch is pending. Every check comes
+ * before anything is enqueued and depends only on the batch and the arguments, so the ranks of a group given the same batch
+ * all accept or all reject it. n_edges must not exceed the batch size the group's new_rows / filt buffers are sized for
+ * (2 * n_edges rows). */
+int lstep_pe_step_peer_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr,
+                            const lstep_peer_group* grp, int64_t n_edges, const int64_t* src_host, const int64_t* dst_host,
+                            const double* t_host, const int64_t* ids_host, int64_t n_ids, int head, int len, const float* G,
+                            const int64_t* const* query_ids_host_arrays, int n_queries, float* nbr_out, int K,
+                            const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes,
+                            uint32_t* err_flag, uint32_t epoch_base, int timeout_ms, int phases, void* stream, int64_t* ticket);
+/* lstep_pe_steps_host for one rank of a peer group: every batch through lstep_pe_step_peer_host (phases 7), full log only
+ * (*len_io == T, else LSTEP_ERR_UNSUPPORTED), results read one step behind into results_host [n_batches][n_queries][batch_size]
+ * (the first q_rows of each row: this rank's share), each step's publication on a side stream as in lstep_pe_steps_peer.
+ * *head_io and *epoch_io are advanced; on an error in batch k batches [0, k) stay applied and *head_io / *epoch_io /
+ * *n_done_out report the position reached. */
+int lstep_pe_steps_peer_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr,
+                             const lstep_peer_group* grp, int64_t n_total, int64_t batch_size, const int64_t* src_host,
+                             const int64_t* dst_host, const double* t_host, const int64_t* const* query_ids_host_arrays, int n_queries,
+                             int* head_io, int* len_io, const float* G, int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd,
+                             void* workspace, size_t workspace_bytes, uint32_t* err_flag, uint32_t* epoch_io, int timeout_ms,
+                             void* stream, float* results_host, int64_t* n_done_out);
 
 /* ------------------------------------------------------------------------------------------
  * Measurement / A-B plumbing (no reference counterpart).

@@ -135,6 +135,12 @@ _SIGS = {
     "lstep_pe_steps_changelog_host": (i32, [vp, C.POINTER(PEStreamDesc), C.POINTER(ChangeLog), C.POINTER(CSR), i64, i64, vp, vp, vp,
                                             C.POINTER(C.c_void_p), i32, C.POINTER(i32), C.POINTER(i32), vp, i32, C.POINTER(PEMLP),
                                             C.POINTER(PEMLP), vp, sz, vp, vp, vp, C.POINTER(i64)]),
+    "lstep_pe_step_peer_host": (i32, [vp, C.POINTER(PEStreamDesc), C.POINTER(ChangeLog), C.POINTER(CSR), C.POINTER(PeerGroup), i64, vp, vp, vp, vp,
+                                      i64, i32, i32, vp, C.POINTER(C.c_void_p), i32, vp, i32, C.POINTER(PEMLP), C.POINTER(PEMLP), vp, sz, vp,
+                                      C.c_uint32, i32, i32, vp, C.POINTER(i64)]),
+    "lstep_pe_steps_peer_host": (i32, [vp, C.POINTER(PEStreamDesc), C.POINTER(ChangeLog), C.POINTER(CSR), C.POINTER(PeerGroup), i64, i64, vp, vp,
+                                       vp, C.POINTER(C.c_void_p), i32, C.POINTER(i32), C.POINTER(i32), vp, i32, C.POINTER(PEMLP),
+                                       C.POINTER(PEMLP), vp, sz, vp, C.POINTER(C.c_uint32), i32, vp, vp, C.POINTER(i64)]),
     "lstep_host_stepper_set_ingest": (i32, [vp, vp, i64, C.c_double]),
     "lstep_host_step_result": (i32, [vp, i64, C.POINTER(C.POINTER(C.c_float)), C.POINTER(i64)]),
     "lstep_host_stepper_bytes": (None, [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),

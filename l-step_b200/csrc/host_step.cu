@@ -10,6 +10,8 @@
 // loop can keep `slots - 1` steps in flight (results read one step behind hide the host's own time).
 // lstep_pe_step_changelog_host is the same hand-over around the change-log step (changelog_step_core, csrc/changelog.cu):
 // host_stage and host_finish below are the two halves both share, the step between them is the only difference.
+// lstep_pe_step_peer_host puts one rank's peer-group step (peer_step_core, csrc/peer.cu) between them, with the rank's owned plan
+// of the batch derived on the device while the batch is staged.
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
@@ -52,6 +54,15 @@ constexpr int kMaxSlots = 8;
 
 using namespace lstep;
 
+// A batch staged by host_stage: its slot and, in the slot's device copy, src | dst | t | ids | query sets.
+struct HostBatch {
+  int slot;
+  int64_t n_ids;
+  double tmax;
+  const int64_t* dp;
+  const int64_t* qdev[8];
+};
+
 struct lstep_host_stepper {
   int slots;
   int64_t max_edges;
@@ -81,6 +92,14 @@ struct lstep_host_stepper {
   cudaEvent_t ing_ev;         // compute stream -> append (ing_wait)
   cudaEvent_t ing_staged;     // copy-in -> append
   cudaStream_t ing_stream;    // the appends: highest priority, so that the append CTA gets the first free SM slot
+  // lstep_pe_step_peer_host: per slot, the rank's owned ids of the staged batch and their positions (ids_mine | pos_mine,
+  // 2 x 2 * max_edges int64, allocated by the first peer call), and the batch a call with phase bit 0 staged for the later
+  // phases of the same step
+  int64_t* d_mine[kMaxSlots];
+  bool peer_pending;
+  HostBatch peer_hb;
+  int64_t peer_n_edges, peer_n_mine;
+  int peer_n_queries;
 };
 
 // sorted unique ids of src[0..n) U dst[0..n) -> out[<= 2n]. Small id spaces: a bitmap over [0, V1) scanned in
@@ -136,6 +155,7 @@ extern "C" void lstep_host_stepper_destroy(lstep_host_stepper* h) {
     if (h->h_in[i]) cudaFreeHost(h->h_in[i]);
     if (h->h_res[i]) cudaFreeHost(h->h_res[i]);
     if (h->d_in[i]) cudaFree(h->d_in[i]);
+    if (h->d_mine[i]) cudaFree(h->d_mine[i]);
   }
   if (h->d_nbr_out) cudaFree(h->d_nbr_out);
   if (h->ing_ev) cudaEventDestroy(h->ing_ev);
@@ -169,11 +189,16 @@ extern "C" int lstep_host_stepper_create(int slots, int64_t max_edges, int max_q
   for (int k = 0; k < 4; ++k) h->ing_arrays[k] = nullptr;
   h->ing_ev = h->ing_staged = nullptr;
   h->ing_stream = nullptr;
+  h->peer_pending = false;
+  h->peer_hb = HostBatch{};
+  h->peer_n_edges = h->peer_n_mine = 0;
+  h->peer_n_queries = 0;
   for (int i = 0; i < kMaxSlots; ++i) {
     h->h_in[i] = h->d_in[i] = nullptr;
     h->h_res[i] = nullptr;
     h->done[i] = h->in_ready[i] = h->step_done[i] = nullptr;
     h->d_nbr[i] = nullptr;
+    h->d_mine[i] = nullptr;
     h->ticket_of[i] = -1;
     h->res_n[i] = 0;
   }
@@ -197,20 +222,19 @@ extern "C" int lstep_host_stepper_create(int slots, int64_t max_edges, int max_q
   return LSTEP_OK;
 }
 
-// A batch staged by host_stage: its slot and, in the slot's device copy, src | dst | t | ids | query sets.
-struct HostBatch {
-  int slot;
-  int64_t n_ids;
-  double tmax;
-  const int64_t* dp;
-  const int64_t* qdev[8];
+// A peer rank's owned plan of the batch being staged (into the slot's d_mine): world and rank in, n_mine out.
+struct PeerStage {
+  int world, rank;
+  int64_t n_mine;
 };
 
-// The first half of a host-fed step: slot wait, pack, the host id-range and ingest checks, copy-in, the optional append on
-// ing_stream, and the hand-over to the compute stream (in_ready). A call rejected by a check has enqueued nothing.
+// The first half of a host-fed step: slot wait, pack, the host id-range and ingest checks, copy-in, the optional owned plan of a
+// peer rank and append, both on the copy-in path, and the hand-over to the compute stream (in_ready). A call rejected by a check
+// has enqueued nothing.
 static int host_stage(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_csr* csr, int64_t n_edges, const int64_t* src_host,
                       const int64_t* dst_host, const double* t_host, const int64_t* ids_host, int64_t n_ids,
-                      const int64_t* const* query_ids_host_arrays, int n_queries, uint32_t* err_flag, cudaStream_t st, HostBatch* hb) {
+                      const int64_t* const* query_ids_host_arrays, int n_queries, uint32_t* err_flag, cudaStream_t st, HostBatch* hb,
+                      PeerStage* peer = nullptr) {
   if (!h || !s || n_edges <= 0 || n_edges > h->max_edges || n_queries < 0 || n_queries > h->max_queries) return LSTEP_ERR_INVALID_ARG;
   if (!src_host || !dst_host || !t_host || (n_queries > 0 && !query_ids_host_arrays)) return LSTEP_ERR_INVALID_ARG;
   if (ids_host && (n_ids < 0 || n_ids > 2 * n_edges)) return LSTEP_ERR_INVALID_ARG;
@@ -270,6 +294,16 @@ static int host_stage(lstep_host_stepper* h, const lstep_pe_stream* s, const lst
                                                (int64_t)((bytes + 15) / 16));
   int rc0 = check_launch("stage_in");
   if (rc0 != LSTEP_OK) return rc0;
+  if (peer) {
+    // the rank's owned ids of the batch and their positions, from the staged ids, on the copy-in stream: off the compute stream's
+    // chain like the append. The filter launch is sized by n_mine, counted here from the same ids.
+    int64_t m = 0;
+    for (int64_t i = 0; i < n_ids; ++i) m += h_ids[i] % peer->world == peer->rank;
+    int64_t* mine = h->d_mine[slot];
+    const int64_t* ids_dev = reinterpret_cast<const int64_t*>(h->d_in[slot]) + 3 * n;
+    if ((rc0 = peer_plan_mine(ids_dev, n_ids, peer->world, peer->rank, mine, mine + 2 * h->max_edges, h->in_stream)) != LSTEP_OK) return rc0;
+    peer->n_mine = m;
+  }
   if (ingest) {
     // The batch is appended to the CSR from the staged slot, on the copy-in path: on a high-priority stream that waits for
     // the copy-in and records in_ready, so the compute stream sees the grown CSR and the step's launch chain is unchanged.
@@ -283,6 +317,10 @@ static int host_stage(lstep_host_stepper* h, const lstep_pe_stream* s, const lst
     // The change-log step (lstep_pe_step_changelog_host) reads the CSR in the same two places only, the a6 gather and
     // phase B's push, through the same strict-< counts; its filter, retire and append kernels read the change log and the
     // table, never the CSR. So the same argument covers it and its appends overlap the same way.
+    // A peer rank's step (lstep_pe_step_peer_host) appends to the rank's own CSR replica and reads it in the same two places:
+    // the a6 gather of its share of the query rows and the push kernel's lookups of all batch nodes, both through strict-<
+    // counts. Its owned-plan kernel, filter, barrier refresh, phase-A broadcast, change-log append and publication never read
+    // the CSR. So the append of batch b+1 overlaps step b there too.
     const void* arrays[4] = {csr->indptr, csr->nbr, csr->eid, csr->t};
     bool changed = false;
     for (int k = 0; k < 4; ++k) changed |= arrays[k] != h->ing_arrays[k];
@@ -321,12 +359,13 @@ static int host_stage(lstep_host_stepper* h, const lstep_pe_stream* s, const lst
 }
 
 // The second half: the per-query row sums of outp into the slot's pinned result, the slot's done event and the ticket.
-static int host_finish(lstep_host_stepper* h, const HostBatch& hb, int64_t n_edges, int n_queries, float* nbr_out, const float* outp,
+// rows_per_query: n_edges, or a peer rank's share q_rows of them.
+static int host_finish(lstep_host_stepper* h, const HostBatch& hb, int64_t rows_per_query, int n_queries, float* nbr_out, const float* outp,
                        cudaStream_t st, int64_t* ticket) {
   const int slot = hb.slot;
   cudaError_t e;
   int rc;
-  const int64_t rows = (int64_t)n_queries * n_edges;
+  const int64_t rows = (int64_t)n_queries * rows_per_query;
   // result path on its own stream, behind the step: the next step does not queue behind it. (A caller-owned
   // nbr_out is reused by the caller's next step, so in that case the result kernel stays on the compute stream.)
   cudaStream_t rs = nbr_out ? st : h->out_stream;
@@ -426,7 +465,8 @@ extern "C" void lstep_host_stepper_bytes(const lstep_host_stepper* h, uint64_t* 
 
 // The loop of a multi-batch host-fed call: batch b = edges [b*batch_size, min((b+1)*batch_size, n_total)), stepped by
 // step(lo, n, query sets, head, &ticket) with the full window (the oldest slot, head, is overwritten and becomes the newest),
-// its result read one step behind into results_host [n_batches][n_queries][batch_size].
+// its result read one step behind into results_host [n_batches][n_queries][batch_size] (the first rows of each query set's
+// row when a step's result covers only a share of the batch).
 template <class Step>
 static int steps_host_loop(lstep_host_stepper* h, int T, int64_t n_total, int64_t batch_size, const int64_t* const* query_ids_host_arrays,
                            int n_queries, int* head_io, float* results_host, int64_t* n_done_out, Step&& step) {
@@ -437,8 +477,10 @@ static int steps_host_loop(lstep_host_stepper* h, int T, int64_t n_total, int64_
     int64_t nf = 0;
     const int rc = lstep_host_step_result(h, ticket, &r, &nf);
     if (rc != LSTEP_OK) return rc;
+    // rows per query: n, or a peer rank's share of the batch (the row sums of query set c are at r + c * rows)
+    const int64_t rows = n_queries > 0 ? nf / n_queries : 0;
     float* dst = results_host + (size_t)b * n_queries * batch_size;
-    for (int c = 0; c < n_queries; ++c) memcpy(dst + (size_t)c * batch_size, r + (size_t)c * n, sizeof(float) * (size_t)n);
+    for (int c = 0; c < n_queries; ++c) memcpy(dst + (size_t)c * batch_size, r + (size_t)c * rows, sizeof(float) * (size_t)rows);
     return LSTEP_OK;
   };
   int64_t b = 0;
@@ -522,4 +564,101 @@ extern "C" int lstep_pe_steps_changelog_host(lstep_host_stepper* h, const lstep_
                                                                cl->T, G, q, n_queries, nullptr, K, mlp_nbr, mlp_upd, workspace,
                                                                workspace_bytes, err_flag, stream, ticket);
                          });
+}
+
+// One rank's peer step between host_stage and host_finish (see the header). The checks that depend on the batch (host_stage's)
+// and those that do not (peer_step_check) come before anything is enqueued, and every rank makes the same ones on the same
+// batch: either every rank enqueues the step, or none does, and no rank waits at a barrier for a peer that rejected it.
+static int step_peer_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const lstep_peer_group* grp,
+                          int64_t n_edges, const int64_t* src_host, const int64_t* dst_host, const double* t_host, const int64_t* ids_host,
+                          int64_t n_ids, int head, int len, const float* G, const int64_t* const* query_ids_host_arrays, int n_queries,
+                          float* nbr_out, int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace,
+                          size_t workspace_bytes, uint32_t* err_flag, uint32_t epoch_base, int timeout_ms, int phases, void* stream,
+                          int64_t* ticket, SideLane* side) {
+  if (!h || !s || !cl || !csr || !grp || !G || K <= 0 || phases <= 0 || (phases & ~7) || ((phases & 4) && !ticket)) return LSTEP_ERR_INVALID_ARG;
+  const bool stage = (phases & 1) != 0;
+  if (stage == h->peer_pending) return LSTEP_ERR_INVALID_ARG;  // staging over a pending batch, or a later phase with none
+  const int64_t n = stage ? n_edges : h->peer_n_edges;
+  const int C = stage ? n_queries : h->peer_n_queries;
+  if (grp->world < 1 || grp->world > LSTEP_MAX_PEERS || grp->rank < 0 || grp->rank >= grp->world) return LSTEP_ERR_INVALID_ARG;
+  const int64_t q_off = grp->rank * n / grp->world, q_rows = (grp->rank + 1) * n / grp->world - q_off;
+  int rc = peer_step_check(s, cl, csr, grp, n, head, len, mlp_nbr, mlp_upd, phases, q_rows);
+  if (rc != LSTEP_OK) return rc;
+  const cudaStream_t st = as_stream(stream);
+  if (stage) {
+    if (!h->d_mine[0]) {
+      for (int i = 0; i < h->slots; ++i) {
+        const cudaError_t e = cudaMalloc((void**)&h->d_mine[i], sizeof(int64_t) * 4 * (size_t)h->max_edges);
+        if (e != cudaSuccess) return cuda_fail(e, "pe_step_peer_host plan buffer");
+      }
+    }
+    PeerStage ps{grp->world, grp->rank, 0};
+    HostBatch hb;
+    rc = host_stage(h, s, csr, n_edges, src_host, dst_host, t_host, ids_host, n_ids, query_ids_host_arrays, n_queries, err_flag, st, &hb, &ps);
+    if (rc != LSTEP_OK) return rc;
+    h->peer_hb = hb;
+    h->peer_n_edges = n_edges;
+    h->peer_n_queries = n_queries;
+    h->peer_n_mine = ps.n_mine;
+    h->peer_pending = true;
+  }
+  const HostBatch& hb = h->peer_hb;
+  const int64_t* dp = hb.dp;
+  const int64_t* mine = h->d_mine[hb.slot];
+  float* outp = nbr_out ? nbr_out : h->d_nbr[hb.slot];
+  const int64_t* q[8] = {};
+  for (int c = 0; c < C; ++c) q[c] = hb.qdev[c] + q_off;
+  rc = peer_step_core(s, cl, csr, grp, dp, dp + n, reinterpret_cast<const double*>(dp + 2 * n), n, dp + 3 * n, hb.n_ids, mine,
+                      mine + 2 * h->max_edges, h->peer_n_mine, hb.tmax, head, len, G, q, C, q_off, q_rows, outp, K, mlp_nbr, mlp_upd, workspace,
+                      workspace_bytes, err_flag, epoch_base, timeout_ms, phases, stream, side);
+  if (rc != LSTEP_OK || (phases & 4)) h->peer_pending = false;
+  if (rc != LSTEP_OK || !(phases & 4)) return rc;
+  return host_finish(h, hb, q_rows, C, nbr_out, outp, st, ticket);
+}
+
+extern "C" int lstep_pe_step_peer_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr,
+                                       const lstep_peer_group* grp, int64_t n_edges, const int64_t* src_host, const int64_t* dst_host,
+                                       const double* t_host, const int64_t* ids_host, int64_t n_ids, int head, int len, const float* G,
+                                       const int64_t* const* query_ids_host_arrays, int n_queries, float* nbr_out, int K,
+                                       const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes,
+                                       uint32_t* err_flag, uint32_t epoch_base, int timeout_ms, int phases, void* stream, int64_t* ticket) {
+  return step_peer_host(h, s, cl, csr, grp, n_edges, src_host, dst_host, t_host, ids_host, n_ids, head, len, G, query_ids_host_arrays, n_queries,
+                        nbr_out, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, epoch_base, timeout_ms, phases, stream, ticket,
+                        nullptr);
+}
+
+// lstep_pe_steps_host for one rank of a peer group: every batch through the whole host-fed peer step (phases 7) with the full
+// window, results (this rank's share) read one step behind, the publication of each step on a side stream next to the next
+// step's filter, as in lstep_pe_steps_peer. On an error in batch k batches [0, k) stay applied: *head_io, *epoch_io and
+// *n_done_out report the position reached.
+extern "C" int lstep_pe_steps_peer_host(lstep_host_stepper* h, const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr,
+                                        const lstep_peer_group* grp, int64_t n_total, int64_t batch_size, const int64_t* src_host,
+                                        const int64_t* dst_host, const double* t_host, const int64_t* const* query_ids_host_arrays,
+                                        int n_queries, int* head_io, int* len_io, const float* G, int K, const lstep_pe_mlp* mlp_nbr,
+                                        const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes, uint32_t* err_flag,
+                                        uint32_t* epoch_io, int timeout_ms, void* stream, float* results_host, int64_t* n_done_out) {
+  if (n_done_out) *n_done_out = 0;
+  if (!h || !s || !cl || !csr || !grp || !head_io || !len_io || !epoch_io || !results_host || n_total < 0 || batch_size <= 0 ||
+      batch_size > h->max_edges)
+    return LSTEP_ERR_INVALID_ARG;
+  if (n_queries < 0 || n_queries > 8 || (n_queries > 0 && !query_ids_host_arrays)) return LSTEP_ERR_INVALID_ARG;
+  if (h->peer_pending) return LSTEP_ERR_INVALID_ARG;
+  int rc = peer_step_check(s, cl, csr, grp, batch_size, *head_io, *len_io, mlp_nbr, mlp_upd, 7, 0);
+  if (rc != LSTEP_OK) return rc;
+  if (*len_io != cl->T) return LSTEP_ERR_UNSUPPORTED;  // the log is still filling: the filter changes every step, use the per-step call
+  uint32_t epoch = *epoch_io;
+  SideLane lane;
+  const bool overlap = grp->world > 1 && n_total > batch_size;
+  if (overlap && (rc = side_lane_open(&lane)) != LSTEP_OK) return rc;
+  rc = steps_host_loop(h, cl->T, n_total, batch_size, query_ids_host_arrays, n_queries, head_io, results_host, n_done_out,
+                       [&](int64_t lo, int64_t n, const int64_t* const* q, int head, int64_t* ticket) {
+                         const int r = step_peer_host(h, s, cl, csr, grp, n, src_host + lo, dst_host + lo, t_host + lo, nullptr, 0, head, cl->T,
+                                                      G, q, n_queries, nullptr, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag,
+                                                      epoch, timeout_ms, 7, stream, ticket, overlap ? &lane : nullptr);
+                         if (r == LSTEP_OK) epoch += 2;
+                         return r;
+                       });
+  if (overlap) side_lane_close(&lane, as_stream(stream));
+  *epoch_io = epoch;
+  return rc;
 }

@@ -460,22 +460,97 @@ extern "C" int lstep_peer_wait(const lstep_peer_group* g, uint32_t epoch, int ti
   return peer_wait(g, epoch, timeout_ms, err_flag, as_stream(stream), false);
 }
 
-namespace {
-// side stream of the native multi-step call: the publication of a step's rows runs next to the NEXT step's filter (neither
-// touches what the other writes); the next barrier-1 launch waits for it
-struct SideLane {
-  cudaStream_t stream = nullptr;
-  cudaEvent_t appended = nullptr, published = nullptr;
-  bool pending = false;  // a publication has been enqueued and not yet waited for
-};
-}  // namespace
+int lstep::side_lane_open(SideLane* lane) {
+  if (cudaStreamCreateWithFlags(&lane->stream, cudaStreamNonBlocking) != cudaSuccess ||
+      cudaEventCreateWithFlags(&lane->appended, cudaEventDisableTiming) != cudaSuccess ||
+      cudaEventCreateWithFlags(&lane->published, cudaEventDisableTiming) != cudaSuccess) {
+    set_cuda_error(cudaGetLastError(), "peer side lane");
+    return LSTEP_ERR_CUDA;
+  }
+  return LSTEP_OK;
+}
 
+void lstep::side_lane_close(SideLane* lane, cudaStream_t st) {
+  // the caller's stream order must cover the last publication; the lane's objects are released once it has run
+  if (lane->pending) cudaStreamWaitEvent(st, lane->published, 0);
+  cudaEventDestroy(lane->appended);
+  cudaEventDestroy(lane->published);
+  cudaStreamDestroy(lane->stream);  // (asynchronous: the stream is released when its work has completed)
+}
+
+namespace lstep {
+namespace {
+// ids_mine / pos_mine of one batch (see peer_plan_mine): blocks of blockDim ids in order; in each, a warp ballot ranks a thread's
+// owned id within its warp and a scan of the warp counts ranks the warp within the block
+__global__ void __launch_bounds__(1024) peer_plan_kernel(const int64_t* __restrict__ ids, int64_t n_ids, int world, int rank,
+                                                         int64_t* __restrict__ ids_mine, int64_t* __restrict__ pos_mine) {
+  __shared__ int s_off[32];
+  __shared__ int s_total;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
+  int64_t base = 0;
+  for (int64_t i0 = 0; i0 < n_ids; i0 += blockDim.x) {
+    const int64_t i = i0 + threadIdx.x;
+    const int64_t v = i < n_ids ? ids[i] : -1;
+    const bool mine = v >= 0 && v % world == rank;
+    const unsigned bal = __ballot_sync(kFull, mine);
+    if (lane == 0) s_off[warp] = __popc(bal);
+    __syncthreads();
+    if (warp == 0) {
+      const int c = lane < n_warps ? s_off[lane] : 0;
+      int x = c;
+      for (int o = 1; o < 32; o <<= 1) {
+        const int y = __shfl_up_sync(kFull, x, o);
+        if (lane >= o) x += y;
+      }
+      s_off[lane] = x - c;  // exclusive
+      if (lane == 31) s_total = x;
+    }
+    __syncthreads();
+    if (mine) {
+      const int64_t p = base + s_off[warp] + __popc(bal & ((1u << lane) - 1u));
+      ids_mine[p] = v;
+      pos_mine[p] = i;
+    }
+    base += s_total;
+    __syncthreads();  // (s_off / s_total are rewritten by the next block of ids)
+  }
+}
+}  // namespace
+}  // namespace lstep
+
+int lstep::peer_plan_mine(const int64_t* ids, int64_t n_ids, int world, int rank, int64_t* ids_mine, int64_t* pos_mine, cudaStream_t st) {
+  if (n_ids < 0 || world < 1 || rank < 0 || rank >= world || (n_ids > 0 && (!ids || !ids_mine || !pos_mine))) return LSTEP_ERR_INVALID_ARG;
+  if (n_ids == 0) return LSTEP_OK;
+  const int threads = (int)std::min<int64_t>(1024, ceil_div(n_ids, 32) * 32);
+  peer_plan_kernel<<<1, threads, 0, st>>>(ids, n_ids, world, rank, ids_mine, pos_mine);
+  return check_launch("peer_plan");
+}
+
+int lstep::peer_step_check(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const lstep_peer_group* grp, int64_t n_edges,
+                           int head, int len, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, int phases, int64_t q_rows) {
+  if (!s || !s->cur || !cl || !csr || !valid_group(grp) || n_edges < 0 || !mlp_nbr || !mlp_upd || (phases & ~7) || q_rows < 0)
+    return LSTEP_ERR_INVALID_ARG;
+  if (grp->table[grp->rank] != s->cur || cl->row_mul != grp->world || cl->row_add != grp->rank || cl->d != s->d) return LSTEP_ERR_INVALID_ARG;
+  if (grp->world > 1 && grp->cap < cl->cap) return LSTEP_ERR_INVALID_ARG;
+  if (head < 0 || head >= cl->T || len < 0 || len > cl->T) return LSTEP_ERR_INVALID_ARG;
+  if (!update_push_available(mlp_upd)) return LSTEP_ERR_UNSUPPORTED;
+  return LSTEP_OK;
+}
+
+// the resident form: the batch is edges [lo, lo + n_edges) of the descriptor's stream
 static int step_peer_impl(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const lstep_peer_group* grp, int64_t lo,
                           int64_t n_edges, const int64_t* ids, int64_t n_ids, const int64_t* ids_mine, const int64_t* pos_mine, int64_t n_mine,
                           double current_time, int head, int len, const float* G, const int64_t* const* query_ids_host, int n_queries,
                           int64_t q_off, int64_t q_rows, float* nbr_out, int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd,
                           void* workspace, size_t workspace_bytes, uint32_t* err_flag, uint32_t epoch_base, int timeout_ms, int phases,
-                          void* stream, SideLane* side);
+                          void* stream, SideLane* side) {
+  if (!s || !s->src || !s->dst || !s->t || lo < 0 || n_ids < 0 || n_mine < 0 || n_mine > n_ids) return LSTEP_ERR_INVALID_ARG;
+  const int rc = peer_step_check(s, cl, csr, grp, n_edges, head, len, mlp_nbr, mlp_upd, phases, q_rows);
+  if (rc != LSTEP_OK) return rc;
+  return peer_step_core(s, cl, csr, grp, s->src + lo, s->dst + lo, s->t + lo, n_edges, ids, n_ids, ids_mine, pos_mine, n_mine, current_time, head,
+                        len, G, query_ids_host, n_queries, q_off, q_rows, nbr_out, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag,
+                        epoch_base, timeout_ms, phases, stream, side);
+}
 
 extern "C" int lstep_pe_step_peer(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const lstep_peer_group* grp,
                                   int64_t lo, int64_t n_edges, const int64_t* ids, int64_t n_ids, const int64_t* ids_mine,
@@ -489,19 +564,13 @@ extern "C" int lstep_pe_step_peer(const lstep_pe_stream* s, const lstep_changelo
                         nullptr);
 }
 
-static int step_peer_impl(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const lstep_peer_group* grp, int64_t lo,
-                          int64_t n_edges, const int64_t* ids, int64_t n_ids, const int64_t* ids_mine, const int64_t* pos_mine, int64_t n_mine,
-                          double current_time, int head, int len, const float* G, const int64_t* const* query_ids_host, int n_queries,
-                          int64_t q_off, int64_t q_rows, float* nbr_out, int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd,
-                          void* workspace, size_t workspace_bytes, uint32_t* err_flag, uint32_t epoch_base, int timeout_ms, int phases,
-                          void* stream, SideLane* side) {
-  if (!s || !s->src || !s->dst || !s->t || !s->cur || !cl || !csr || !valid_group(grp) || lo < 0 || n_edges < 0 || n_ids < 0 || n_mine < 0 ||
-      n_mine > n_ids || !mlp_nbr || !mlp_upd || (phases & ~7) || q_rows < 0)
-    return LSTEP_ERR_INVALID_ARG;
-  if (grp->table[grp->rank] != s->cur || cl->row_mul != grp->world || cl->row_add != grp->rank || cl->d != s->d) return LSTEP_ERR_INVALID_ARG;
-  if (grp->world > 1 && grp->cap < cl->cap) return LSTEP_ERR_INVALID_ARG;
-  if (head < 0 || head >= cl->T || len < 0 || len > cl->T) return LSTEP_ERR_INVALID_ARG;
-  if (!update_push_available(mlp_upd)) return LSTEP_ERR_UNSUPPORTED;
+// The step body on explicit batch pointers; the callers have made peer_step_check's checks.
+int lstep::peer_step_core(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const lstep_peer_group* grp, const int64_t* src,
+                          const int64_t* dst, const double* tq, int64_t n_edges, const int64_t* ids, int64_t n_ids, const int64_t* ids_mine,
+                          const int64_t* pos_mine, int64_t n_mine, double current_time, int head, int len, const float* G,
+                          const int64_t* const* query_ids_host, int n_queries, int64_t q_off, int64_t q_rows, float* nbr_out, int K,
+                          const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes, uint32_t* err_flag,
+                          uint32_t epoch_base, int timeout_ms, int phases, void* stream, SideLane* side) {
   cudaStream_t st = as_stream(stream);
   int rc;
   if (phases & 1) {
@@ -547,7 +616,7 @@ static int step_peer_impl(const lstep_pe_stream* s, const lstep_changelog* cl, c
   opt.stamp_out = &stamp;
   lstep_pe_stream s2 = *s;
   if (!s2.ring) s2.ring = s2.cur;  // (never touched: the core neither filters nor appends)
-  rc = pe_step_core_ex(&s2, csr, s->src + lo, s->dst + lo, s->t + lo, n_edges, ids, n_ids, current_time, 0, 0, 0, nullptr, query_ids_host,
+  rc = pe_step_core_ex(&s2, csr, src, dst, tq, n_edges, ids, n_ids, current_time, 0, 0, 0, nullptr, query_ids_host,
                        q_rows > 0 ? n_queries : 0, nbr_out, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, stream, opt);
   if (rc != LSTEP_OK || !(phases & 4)) return rc;
   const int64_t* U = nullptr;
@@ -592,12 +661,7 @@ extern "C" int lstep_pe_steps_peer(const lstep_pe_stream* s, const lstep_changel
   int rc = LSTEP_OK;
   SideLane lane;
   const bool overlap = grp->world > 1 && n_steps > 1;
-  if (overlap && (cudaStreamCreateWithFlags(&lane.stream, cudaStreamNonBlocking) != cudaSuccess ||
-                  cudaEventCreateWithFlags(&lane.appended, cudaEventDisableTiming) != cudaSuccess ||
-                  cudaEventCreateWithFlags(&lane.published, cudaEventDisableTiming) != cudaSuccess)) {
-    set_cuda_error(cudaGetLastError(), "peer side lane");
-    return LSTEP_ERR_CUDA;
-  }
+  if (overlap && (rc = side_lane_open(&lane)) != LSTEP_OK) return rc;
   for (int64_t i = 0; i < n_steps; ++i) {
     const int64_t n = n_edges_host[i];
     const int64_t q_off = grp->rank * n / grp->world, q_rows = (grp->rank + 1) * n / grp->world - q_off;
@@ -612,12 +676,7 @@ extern "C" int lstep_pe_steps_peer(const lstep_pe_stream* s, const lstep_changel
     epoch += 2;
     head = (head + 1) % T;
   }
-  if (overlap) {  // the caller's stream order must cover the last publication; the lane's objects are released once it has run
-    if (lane.pending) cudaStreamWaitEvent(as_stream(stream), lane.published, 0);
-    cudaEventDestroy(lane.appended);
-    cudaEventDestroy(lane.published);
-    cudaStreamDestroy(lane.stream);  // (asynchronous: the stream is released when its work has completed)
-  }
+  if (overlap) side_lane_close(&lane, as_stream(stream));
   *head_io = head;
   *epoch_io = epoch;
   return rc;

@@ -30,6 +30,30 @@ struct StepOpts {
 int peer_rows_bcast(const float* src, int64_t n_rows, int d, const int64_t* dst_rows, const lstep_peer_group* grp, int which, cudaStream_t st);
 int peer_signal(const lstep_peer_group* g, uint32_t epoch, cudaStream_t st);
 int peer_wait(const lstep_peer_group* g, uint32_t epoch, int timeout_ms, uint32_t* err_flag, cudaStream_t st, bool announce = false);
+// Side stream of a native multi-step peer call: the publication of a step's rows runs next to the NEXT step's filter (neither
+// touches what the other writes); the next barrier-1 launch waits for it. open creates the stream and events; close makes the
+// caller's stream wait for a pending publication and releases them.
+struct SideLane {
+  cudaStream_t stream = nullptr;
+  cudaEvent_t appended = nullptr, published = nullptr;
+  bool pending = false;  // a publication has been enqueued and not yet waited for
+};
+int side_lane_open(SideLane* lane);
+void side_lane_close(SideLane* lane, cudaStream_t st);
+// The peer step's checks of everything but the batch (callers make them before they enqueue anything), and the step itself on
+// explicit batch pointers (src / dst / tq: n_edges device entries; s->src / s->dst / s->t are never read). q_off / q_rows: this
+// rank's share of the batch's edges for the a6 queries, query_ids[c] pointing at the first of them.
+int peer_step_check(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const lstep_peer_group* grp, int64_t n_edges,
+                    int head, int len, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, int phases, int64_t q_rows);
+int peer_step_core(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const lstep_peer_group* grp, const int64_t* src,
+                   const int64_t* dst, const double* tq, int64_t n_edges, const int64_t* ids, int64_t n_ids, const int64_t* ids_mine,
+                   const int64_t* pos_mine, int64_t n_mine, double current_time, int head, int len, const float* G,
+                   const int64_t* const* query_ids, int n_queries, int64_t q_off, int64_t q_rows, float* nbr_out, int K,
+                   const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes, uint32_t* err_flag,
+                   uint32_t epoch_base, int timeout_ms, int phases, void* stream, SideLane* side);
+// A rank's owned plan of a batch on the device: ids_mine = the ids[0 .. n_ids) with v % world == rank, in order, and pos_mine =
+// their positions in ids (one CTA; an ordered compaction). The host-fed peer step runs it on its copy-in stream.
+int peer_plan_mine(const int64_t* ids, int64_t n_ids, int world, int rank, int64_t* ids_mine, int64_t* pos_mine, cudaStream_t st);
 
 int pe_step_core_ex(const lstep_pe_stream* s, const lstep_csr* csr, const int64_t* src, const int64_t* dst, const double* tq,
                     int64_t n_edges, const int64_t* ids, int64_t n_ids, double current_time, int head, int len, int append_slot,

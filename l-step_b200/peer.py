@@ -6,7 +6,8 @@ v % world == rank: their PE history (change log) and every piece of the step who
 contiguous blocks, into small fixed inbox regions of the other ranks through peer pointers (CUDA IPC over NVLink / NVSwitch);
 every rank scatters its inbox into its replica right after the first of the two flag barriers of a step (also in peer memory).
 No NCCL call, no host synchronisation and no data-dependent message size is on the step's path. The protocol and the argument why two barriers suffice are in csrc/peer.cu; the C entry points
-are lstep_pe_step_peer / lstep_pe_steps_peer (include/lstep_b200.h).
+are lstep_pe_step_peer / lstep_pe_steps_peer (include/lstep_b200.h), and lstep_pe_step_peer_host / lstep_pe_steps_peer_host for
+batches fed from host arrays (PeerRank.step_host / run_host, with ingest=True into every rank's own CSR replica).
 
     PeerRank         this rank's state: table replica, change log of the owned nodes, per-batch plan, peer-shared buffers
     PeerLocalGroup   all ranks of a group in ONE process on one device (tests): peer pointers are plain device pointers and the
@@ -23,8 +24,9 @@ import torch
 from . import _lib
 from . import checkpoint as ckpt
 from .changelog import ChangeLogHistory, advance, filter_len
+from .hostfeed import HostFed, host_arrays
 from .model import LSTEP
-from .sampler import NeighborSampler
+from .sampler import NeighborSampler, check_edges
 
 
 class _DevMem:
@@ -84,10 +86,48 @@ def peer_batch_plan(src: np.ndarray, dst: np.ndarray, batch_size: int, world: in
                 mine_off=np.asarray(mine_off, np.int64), share=share)
 
 
-class PeerRank:
+def share_of(n: int, world: int, rank: int):
+    """(q_off, q_rows): rank's share of a batch of n edges for the a6 queries; the shares of the ranks partition the batch."""
+    return rank * n // world, (rank + 1) * n // world - rank * n // world
+
+
+def check_host_batch(src, dst, times, query_ids, V1: int, batch_size: int, ids=None, ingest=None):
+    """Validation of a host batch for PeerRank.step_host_async, pure numpy (nothing is read from or written to a device). Every
+    rank of a group makes it on the same batch, so every rank accepts it or every rank rejects it, before any rank enqueues
+    anything. Raises ValueError for an empty batch, unequal lengths, more than 8 query sets, a batch longer than `batch_size`
+    (the change log's event capacity and the peer buffers are sized from it) and ids that are not sorted and unique; IndexError
+    for a node id outside [0, V1). ingest = (num_rows, last_time, first edge id): the conditions of sampler.check_edges (finite,
+    non-decreasing times from last_time on, ids inside the sampler's rows, edge ids inside [0, 2^31)). Returns the arrays as
+    host_arrays does, and ids."""
+    src, dst, times, qs = host_arrays(src, dst, times, query_ids, "step_host")
+    n = len(src)
+    if n == 0:
+        raise ValueError("step_host: empty batch")
+    if n > batch_size:
+        raise ValueError(f"PeerRank: a host batch of {n} edges is longer than batch_size ({batch_size}), which sizes the change log's "
+                         f"event_capacity and the peer buffers; split the batch or build the ranks with a larger batch_size")
+    if len(qs) > 8:
+        raise ValueError("step_host: at most 8 query sets")
+    for a in [src, dst] + qs:
+        lo, hi = int(a.min()), int(a.max())
+        if lo < 0 or hi >= V1:
+            raise IndexError(f"list index out of range: node id {lo if lo < 0 else hi} is outside the PE table's {V1} rows")
+    if ids is not None:
+        ids = np.ascontiguousarray(ids, dtype=np.int64)
+        if len(ids) > 2 * n or (len(ids) and (int(ids[0]) < 0 or int(ids[-1]) >= V1)) or (len(ids) > 1 and not (np.diff(ids) > 0).all()):
+            raise ValueError("step_host: ids must be the sorted unique batch nodes")
+    if ingest is not None:
+        num_rows, last_time, eid0 = ingest
+        check_edges(src, dst, int(eid0), times, num_rows, last_time)
+    return src, dst, times, qs, ids
+
+
+class PeerRank(HostFed):
     """Rank `rank` of `world` (see the module docstring). src / dst / t: the whole edge stream (replicated, device or host
     arrays); the per-batch plan (sorted unique batch nodes, the owned ones and their positions) of the resident stream
-    [start, stop) is computed once, like PEStream's.
+    [start, stop) is computed once, like PEStream's. src = dst = t = None: no resident stream; the rank then serves host-fed
+    steps (step_host_async / step_host / run_host), online with ingest=True into its own growable `sampler`
+    (NeighborSampler.growable; every rank holds its own CSR replica, so each rank needs a sampler of its own).
 
     The PE state comes from exactly one of `initial_pe` (the table [V1, d]), `history` (a dense history [V1, Th, d],
     oldest first, as ChangeLogStream.import_history takes it) and `checkpoint` (a directory that save_checkpoint wrote at
@@ -121,7 +161,8 @@ class PeerRank:
         if hist is not None:
             hist.check(V1=self.V1, d=self.d, T=self.T)
         lib = self.lib = _lib.load()
-        as_dev = lambda a, dt: (a.to(dev, dt) if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a)).to(dev, dt))
+        as_dev = lambda a, dt: (torch.zeros(0, dtype=dt, device=dev) if a is None else a.to(dev, dt) if isinstance(a, torch.Tensor) else
+                                torch.from_numpy(np.ascontiguousarray(a)).to(dev, dt))
         T, d = self.T, self.d
         with torch.cuda.device(dev):
             self.src, self.dst, self.tt = as_dev(src, torch.int64), as_dev(dst, torch.int64), as_dev(t, torch.float64)
@@ -171,6 +212,7 @@ class PeerRank:
         self.epoch = ctypes.c_uint32(0)  # (a fresh rank: the flag blocks are zeroed by lstep_ipc_alloc)
         self.grp = None
         self._opened = []
+        self._host_init()
         if hist is not None:
             self.head, self.len = self.changelog.load(hist, self.cur)
             if checkpoint is not None:
@@ -299,6 +341,143 @@ class PeerRank:
         _lib.check(rc, "lstep_pe_steps_peer")
         return out
 
+    # ---- host-fed steps (csrc/host_step.cu; stepper, ingest and tickets: hostfeed.HostFed) ---------------------------------
+    def _host_sampler(self):
+        return self.sampler  # (this rank's own CSR replica: in a single-process group the ranks share the model)
+
+    def share_of(self, n: int):
+        """(q_off, q_rows): this rank's share of a batch of n edges for the a6 queries (and of step_host's row sums)."""
+        return share_of(n, self.G, self.rank)
+
+    def _host_prepare(self, src, dst, times, query_ids, ids=None, ingest=False, edge_id_start=None) -> dict:
+        """Validate a host batch (check_host_batch) and, with ingest, make room for it in this rank's sampler. Nothing is
+        enqueued; a regrow synchronises."""
+        ing = None
+        if ingest:
+            samp = self._growable_sampler()
+            ing = (samp.num_rows, samp.last_time, samp.next_edge_id if edge_id_start is None else int(edge_id_start))
+        src, dst, times, qs, ids = check_host_batch(src, dst, times, query_ids, self.V1, self.B, ids, ing)
+        if ingest:
+            self.sampler.reserve(src, dst)
+        return dict(src=src, dst=dst, times=times, qs=qs, ids=ids, ingest=bool(ingest), eid0=None if ing is None else ing[2])
+
+    def _host_phase(self, hb: dict, phases: int, batch_idx: int = None, out: torch.Tensor = None):
+        """Issue `phases` of the step on the prepared batch hb (lstep_pe_step_peer_host): the call with bit 0 stages the batch,
+        the one with bit 2 finishes the step, advances the state and returns the ticket."""
+        assert self.grp is not None, "set_group / connect_ipc first"
+        src, dst, times, qs, ids, ingest = hb["src"], hb["dst"], hb["times"], hb["qs"], hb["ids"], hb["ingest"]
+        n, C = len(src), len(qs)
+        samp = self.sampler
+        if torch.cuda.current_device() != self.dev.index:
+            torch.cuda.set_device(self.dev)
+        if phases & 1:
+            hb["bi"] = self.batch_idx if batch_idx is None else int(batch_idx)
+            h = hb["h"] = self._host_stepper_for(n, C)
+            self._set_ingest(h, ingest, hb["eid0"])
+            hb["G"] = self.m._collapsed_filter(filter_len(hb["bi"], self.len, self.T), False)
+            hb["qptrs"] = (ctypes.c_void_p * max(C, 1))(*[q.ctypes.data for q in qs])
+            hb["out"] = out
+        ticket = ctypes.c_int64(-1)
+        rc = self._libc.lstep_pe_step_peer_host(
+            hb["h"], ctypes.byref(self.desc), self.changelog.ref, samp.csr_ref, ctypes.byref(self.grp), n, src.ctypes.data, dst.ctypes.data,
+            times.ctypes.data, ids.ctypes.data if ids is not None else None, len(ids) if ids is not None else 0, self.head, self.len,
+            _lib.ptr(hb["G"]), hb["qptrs"], C, _lib.ptr(hb["out"]), self.K, self.m._mlp_ref("nbr"), self.m._mlp_ref("update"),
+            _lib.ptr(self.ws), self.ws.numel(), _lib.ptr(samp._err), self.epoch.value, self.timeout_ms, phases, _lib.stream_ptr(),
+            ctypes.byref(ticket))
+        if rc != 0:  # (the append may have been enqueued before the step failed)
+            self._host_failed(rc, "lstep_pe_step_peer_host", ingest, samp, src, dst, hb["eid0"], times)
+        if ingest and (phases & 1):  # the append is enqueued with the staging
+            samp._note_ingested(src, dst, hb["eid0"] + n - 1, times[-1])
+        if not phases & 4:
+            return None
+        self.batch_idx = hb["bi"]
+        self._advance(1)
+        self.edges_done += n
+        self.m.h2d_bytes += 8 * n * (5 + C)  # (what the stepper copies: src, dst, t, <= 2n ids, C query sets)
+        return self._new_ticket(ticket.value, C, self.share_of(n)[1])
+
+    def step_host_async(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None,
+                        ids: np.ndarray = None, out: torch.Tensor = None, ingest: bool = False, edge_id_start: int = None) -> int:
+        """ChangeLogStream.step_host_async for this rank (lstep_pe_step_peer_host): the whole step on a batch of host arrays,
+        every rank of the group calling it with the same batch. result(ticket) is this rank's share [C, q_rows] of the per-query
+        row sums (share_of(n)); `out` [C, q_rows, d] keeps the share's neighbourhood PEs on the device. ingest=True appends the
+        batch to this rank's own growable sampler first. A batch longer than batch_size is rejected before anything is
+        enqueued. edges_done, steps_done, batch_idx and epoch advance as in step."""
+        return self._host_phase(self._host_prepare(src, dst, times, query_ids, ids, ingest, edge_id_start), 7, batch_idx, out)
+
+    def step_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None, ids: np.ndarray = None,
+                  ingest: bool = False, edge_id_start: int = None) -> np.ndarray:
+        """Synchronous form: this rank's share [len(query_ids), q_rows] of the per-query row sums."""
+        return self.result(self.step_host_async(src, dst, times, query_ids, batch_idx, ids, ingest=ingest, edge_id_start=edge_id_start))
+
+    def run_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, ingest: bool = False,
+                 edge_id_start: int = None) -> np.ndarray:
+        """ChangeLogStream.run_host for this rank: batch b = edges [b*B, (b+1)*B) of the host arrays, the steady-state batches
+        in ONE native call (lstep_pe_steps_peer_host), the ones while the log fills one by one. Returns [n_batches, C, B] float32:
+        row [b, c, :q_rows] is this rank's share of batch b (share_of), the rest zero. The whole run is validated first, and with
+        ingest=True room for all of it is reserved in this rank's sampler before the native call, so that no rank regrows (and
+        synchronises) while its peers wait at a barrier; the decision depends on the batches only, so every rank makes the
+        same one."""
+        assert self.grp is not None, "set_group / connect_ipc first"
+        n_total, B, C = len(src), self.B, len(query_ids)
+        src, dst, times, qs = host_arrays(src, dst, times, query_ids, "run_host")
+        nb = (n_total + B - 1) // B
+        res = np.zeros((nb, C, B), dtype=np.float32)
+        if n_total == 0:
+            return res
+        eid0, ing = None, None
+        if ingest:
+            samp = self._growable_sampler()
+            eid0 = samp.next_edge_id if edge_id_start is None else int(edge_id_start)
+            ing = (samp.num_rows, samp.last_time, eid0)
+        check_host_batch(src, dst, times, qs, self.V1, n_total, None, ing)  # (the whole run: batches of B follow from it)
+        if ingest:
+            self.sampler.reserve(src, dst)
+        lo = 0
+        pend = []
+        while lo < n_total and self.len < self.T:  # while the log fills: per-step calls
+            hi = min(lo + B, n_total)
+            pend.append((lo // B, self.step_host_async(src[lo:hi], dst[lo:hi], times[lo:hi], [q[lo:hi] for q in qs], ingest=ingest,
+                                                       edge_id_start=None if eid0 is None else eid0 + lo)))
+            if len(pend) > 1:
+                b, tk = pend.pop(0)
+                r = self.result(tk)
+                res[b, :, :r.shape[1]] = r
+            lo = hi
+        for b, tk in pend:
+            r = self.result(tk)
+            res[b, :, :r.shape[1]] = r
+        if lo >= n_total:
+            return res
+        if torch.cuda.current_device() != self.dev.index:
+            torch.cuda.set_device(self.dev)
+        h = self._stepper(B, C)
+        self._set_ingest(h, ingest, eid0 + lo if ingest else None)
+        G = self.m._collapsed_filter(self.T, False)
+        qptrs = (ctypes.c_void_p * max(C, 1))(*[q[lo:].ctypes.data for q in qs])
+        head, ln, done = ctypes.c_int(self.head), ctypes.c_int(self.len), ctypes.c_int64(0)
+        epoch = ctypes.c_uint32(self.epoch.value)
+        sub = res[lo // B:]
+        samp = self.sampler
+        rc = self._libc.lstep_pe_steps_peer_host(
+            h, ctypes.byref(self.desc), self.changelog.ref, samp.csr_ref, ctypes.byref(self.grp), n_total - lo, B, src[lo:].ctypes.data,
+            dst[lo:].ctypes.data, times[lo:].ctypes.data, qptrs, C, ctypes.byref(head), ctypes.byref(ln), _lib.ptr(G), self.K,
+            self.m._mlp_ref("nbr"), self.m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(), _lib.ptr(samp._err), ctypes.byref(epoch),
+            self.timeout_ms, _lib.stream_ptr(), sub.ctypes.data, ctypes.byref(done))
+        # batches applied before an error stay applied: the host state follows the device's
+        steps = done.value
+        self.head, self.epoch = head.value, epoch
+        self.batch_idx += steps
+        self.steps_done += steps
+        n_app = min(steps * B, n_total - lo)
+        self.edges_done += n_app
+        self.m.h2d_bytes += 8 * n_app * (5 + C)
+        if rc != 0:
+            self._host_failed(rc, "lstep_pe_steps_peer_host", ingest, samp, src[lo:], dst[lo:], eid0 + lo if ingest else None, times[lo:])
+        if ingest and n_app > 0:
+            samp._note_ingested(src[lo:lo + n_app], dst[lo:lo + n_app], eid0 + lo + n_app - 1, times[lo + n_app - 1])
+        return res
+
     def barrier(self):
         """Barrier + application of the inbox: once the kernels this enqueues have run, this replica holds the rows every rank changed
         in the last step."""
@@ -342,6 +521,16 @@ class PeerLocalGroup:
         ptrs = [[rk.local_ptrs()[k] for rk in ranks] for k in range(len(PeerRank._SHARED))]
         for rk in ranks:
             rk.set_group(*ptrs)
+
+    def step_host(self, src, dst, times, queries, ingest: bool = False, edge_id_start: int = None, batch_idx: int = None) -> np.ndarray:
+        """PeerRank.step_host for every rank on the same host batch: validated for all ranks before any rank stages anything,
+        then phases 1, 2 and 4 issued for every rank. Returns the shares concatenated, [C, n]: the single-GPU result."""
+        hbs = [rk._host_prepare(src, dst, times, queries, None, ingest, edge_id_start) for rk in self.ranks]
+        tks = [None] * self.G
+        for ph in (1, 2, 4):
+            for i, rk in enumerate(self.ranks):
+                tks[i] = rk._host_phase(hbs[i], ph, batch_idx)
+        return np.concatenate([rk.result(tk) for rk, tk in zip(self.ranks, tks)], axis=1)
 
     def step(self, b: int, queries):
         outs = [None] * self.G

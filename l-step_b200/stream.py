@@ -28,15 +28,15 @@ import torch
 from . import _lib
 from . import checkpoint as ckpt
 from .changelog import ChangeLogHistory, advance, filter_len
+from .hostfeed import HostFed, host_arrays
 from .model import LSTEP
-from .sampler import check_edges
 
 C_void_p = ctypes.c_void_p
 C_byref = ctypes.byref
-_I64, _F64 = np.dtype(np.int64), np.dtype(np.float64)
+_I64 = np.dtype(np.int64)
 
 
-class PEStream:
+class PEStream(HostFed):
     def __init__(self, model: LSTEP, src_node_ids: np.ndarray, dst_node_ids: np.ndarray, node_interact_times: np.ndarray,
                  batch_size: int, num_neighbors: int = 20, initial_pe: torch.Tensor = None, history: torch.Tensor = None,
                  start: int = 0, stop: int = None):
@@ -71,12 +71,7 @@ class PEStream:
         self.ids = torch.from_numpy(self.ids_np).to(dev)
         self.num_batches = len(self.batch_lo)
         self.batch_tmax = [float(self.t_np[lo:min(lo + self.B, self.stop)].max()) for lo in self.batch_lo]
-        self._host_stepper = None
-        self._armed = None  # (stepper, sampler, sampler version) the stepper was armed to ingest into, see _arm_ingest
-        self._ticket_shape = {}
-        self._drained = {}  # public ticket -> result read out before its stepper was replaced
-        self._epoch = 0
-        self._libc = _lib.load()
+        self._host_init()
         self.V1 = None
         self.batch_idx = 0
         if history is not None:
@@ -251,72 +246,9 @@ class PEStream:
         n_last = int(ne[-1])
         return buf.view(-1)[:max(C, 1) * n_last * d].view(max(C, 1), n_last, d)
 
-    # ---- host-fed steps (native stager: csrc/host_step.cu) -----------------------------------------
-    def _stepper(self, n_edges: int, C: int):
-        lib = _lib.load()
-        st = self._host_stepper
-        if st is None or st[1] < n_edges or st[2] < C:
-            if st is not None:
-                # a larger batch / more query sets than the stepper was sized for: results of tickets still outstanding
-                # are read out first (the native ticket numbering restarts with the new stepper; public tickets carry the
-                # stepper's epoch so an old one can never alias a new one)
-                for tk in sorted(self._ticket_shape):
-                    try:
-                        self._drained[tk] = self._result_now(tk)
-                    except ValueError:  # result slot already reused by later steps (e.g. a run_host call): nothing to keep
-                        pass
-                self._ticket_shape.clear()
-                lib.lstep_host_stepper_destroy(st[0])
-                self._epoch += 1
-                self._armed = None
-            h = C_void_p()
-            cap_e, cap_c = max(self.B, n_edges), max(C, 4)
-            with torch.cuda.device(self.dev):
-                _lib.check(lib.lstep_host_stepper_create(self.HOST_SLOTS, cap_e, cap_c, self.d, C_byref(h)), "lstep_host_stepper_create")
-            self._host_stepper = st = (h, cap_e, cap_c)
-        return st[0]
-
-    HOST_SLOTS = 4  # steps that may be in flight before step_host_async blocks on the oldest
-
-    def __del__(self):
-        st = getattr(self, "_host_stepper", None)
-        if st is not None:
-            try:
-                _lib.load(False).lstep_host_stepper_destroy(st[0])
-            except Exception:
-                pass
-            self._host_stepper = None
-
-    def _growable_sampler(self):
-        samp = self.model.neighbor_sampler
-        if samp is None or not samp.is_growable:
-            raise ValueError("ingest=True needs a growable neighbor sampler: model.set_neighbor_sampler(NeighborSampler.growable(...))")
-        return samp
-
-    def _check_ingest(self, src, dst, times, edge_id_start):
-        """Validate a host batch for ingestion and make room for it; returns its first edge id. Nothing is written to
-        the device unless a regrow is needed."""
-        samp = self._growable_sampler()
-        eid0 = samp.next_edge_id if edge_id_start is None else int(edge_id_start)
-        check_edges(src, dst, eid0, times, samp.num_rows, samp.last_time)
-        samp.reserve(src, dst)
-        return eid0
-
-    def _arm_ingest(self, h, eid0: int):
-        """Arm the stepper to append each batch to the sampler's CSR before its step (lstep_host_stepper_set_ingest). Re-armed
-        only when the stepper, the sampler or its arrays changed, or edge ids do not continue: arming makes the next append
-        wait for the compute stream, which costs the copy-in its overlap with the previous step."""
-        samp = self.model.neighbor_sampler
-        key = (h.value, id(samp), samp._version)
-        if self._armed != key or eid0 != samp.next_edge_id:
-            _lib.check(self._libc.lstep_host_stepper_set_ingest(h, _lib.ptr(samp.fill), eid0, samp.last_time),
-                       "lstep_host_stepper_set_ingest")
-            self._armed = key
-
-    def _disarm_ingest(self, h):
-        if self._armed is not None:
-            _lib.check(self._libc.lstep_host_stepper_set_ingest(h, None, 0, 0.0), "lstep_host_stepper_set_ingest")
-            self._armed = None
+    # ---- host-fed steps (native stager: csrc/host_step.cu; stepper, ingest and tickets: hostfeed.HostFed) -----------
+    def _host_sampler(self):
+        return self.model.neighbor_sampler
 
     def step_host_async(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None,
                         ids: np.ndarray = None, out: torch.Tensor = None, ingest: bool = False, edge_id_start: int = None) -> int:
@@ -334,15 +266,7 @@ class PEStream:
         m = self.model
         n = len(src)
         C = len(query_ids)
-        if src.dtype != _I64 or not src.flags.c_contiguous:
-            src = np.ascontiguousarray(src, dtype=_I64)
-        if dst.dtype != _I64 or not dst.flags.c_contiguous:
-            dst = np.ascontiguousarray(dst, dtype=_I64)
-        if times.dtype != _F64 or not times.flags.c_contiguous:
-            times = np.ascontiguousarray(times, dtype=_F64)
-        qs = [q if (q.dtype == _I64 and q.flags.c_contiguous) else np.ascontiguousarray(q, dtype=_I64) for q in query_ids]
-        if len(dst) != n or len(times) != n or any(len(q) != n for q in qs):
-            raise ValueError("step_host: src, dst, times and every query set must have the same length")
+        src, dst, times, qs = host_arrays(src, dst, times, query_ids, "step_host")
         if ids is not None:
             ids = np.ascontiguousarray(ids, dtype=_I64)
         if ingest:
@@ -350,15 +274,8 @@ class PEStream:
         bi = self.batch_idx if batch_idx is None else batch_idx
         if torch.cuda.current_device() != self.dev.index:
             torch.cuda.set_device(self.dev)
-        st = self._host_stepper
-        if st is None or st[1] < n or st[2] < C:
-            h = self._stepper(n, C)
-        else:
-            h = st[0]
-        if ingest:
-            self._arm_ingest(h, eid0)
-        elif self._armed is not None:
-            self._disarm_ingest(h)
+        h = self._host_stepper_for(n, C)
+        self._set_ingest(h, ingest, eid0 if ingest else None)
         G = m._collapsed_filter(filter_len(bi, self.len, self.T), False)
         ws = self._ws
         if ws is None or n > self._ws_cap[1] or C > self._ws_cap[2] or 2 * n > self._ws_cap[0]:
@@ -368,19 +285,14 @@ class PEStream:
         ticket = ctypes.c_int64(-1)
         samp = m.neighbor_sampler
         rc = self._step_host_native(h, samp, n, src, dst, times, ids, slot, G, qptrs, C, out, ws, ticket)
-        if rc != 0:
-            if ingest:  # the append may have been enqueued before the step failed
-                samp._resync(src, dst, eid0, times)
-            _lib.check(rc, self._HOST_CALLS[0])
+        if rc != 0:  # (the append may have been enqueued before the step failed)
+            self._host_failed(rc, self._HOST_CALLS[0], ingest, samp, src, dst, eid0 if ingest else None, times)
         if ingest:
             samp._note_ingested(src, dst, eid0 + n - 1, times[-1])
         self.head, self.len = new_head, new_len
         self.batch_idx = bi + 1
         self.steps_done += 1
-        tk = (self._epoch << 32) | ticket.value
-        self._ticket_shape[tk] = (C, n)
-        self._ticket_shape.pop(tk - self.HOST_SLOTS, None)
-        self._drained.pop(tk - 2 * self.HOST_SLOTS, None)
+        tk = self._new_ticket(ticket.value, C, n)
         m.h2d_bytes += 8 * n * (5 + C)  # what lstep_pe_step_host copies: src, dst, t, <= 2n ids, C query sets
         return tk
 
@@ -393,12 +305,7 @@ class PEStream:
         step_host_async one by one. ingest=True: as in step_host_async; room for the whole run is reserved first, so the
         native loop never needs a regrow."""
         n_total, B, C = len(src), self.B, len(query_ids)
-        src = np.ascontiguousarray(src, dtype=_I64)
-        dst = np.ascontiguousarray(dst, dtype=_I64)
-        times = np.ascontiguousarray(times, dtype=_F64)
-        qs = [np.ascontiguousarray(q, dtype=_I64) for q in query_ids]
-        if len(dst) != n_total or len(times) != n_total or any(len(q) != n_total for q in qs):
-            raise ValueError("run_host: src, dst, times and every query set must have the same length")
+        src, dst, times, qs = host_arrays(src, dst, times, query_ids, "run_host")
         eid0 = self._check_ingest(src, dst, times, edge_id_start) if ingest else None
         nb = (n_total + B - 1) // B
         res = np.zeros((nb, C, B), dtype=np.float32)
@@ -420,10 +327,7 @@ class PEStream:
         if torch.cuda.current_device() != self.dev.index:
             torch.cuda.set_device(self.dev)
         h = self._stepper(B, C)
-        if ingest:
-            self._arm_ingest(h, eid0 + lo)
-        elif self._armed is not None:
-            self._disarm_ingest(h)
+        self._set_ingest(h, ingest, eid0 + lo if ingest else None)
         G = m._collapsed_filter(self.T, False)
         ws = self._workspace(2 * B, B, C)
         qptrs = (C_void_p * max(C, 1))(*[q[lo:].ctypes.data for q in qs])
@@ -438,12 +342,10 @@ class PEStream:
         self.steps_done += steps
         n_app = min(steps * B, n_total - lo)
         m.h2d_bytes += 8 * n_app * (5 + C)
-        if ingest and rc != 0:  # the failed batch's append may have been enqueued although its step was not applied
-            samp._resync(src[lo:], dst[lo:], eid0 + lo, times[lo:])
-        elif ingest and n_app > 0:
+        if rc != 0:  # (the failed batch's append may have been enqueued although its step was not applied)
+            self._host_failed(rc, self._HOST_CALLS[1], ingest, samp, src[lo:], dst[lo:], eid0 + lo if ingest else None, times[lo:])
+        if ingest and n_app > 0:
             samp._note_ingested(src[lo:lo + n_app], dst[lo:lo + n_app], eid0 + lo + n_app - 1, times[lo + n_app - 1])
-        if rc != 0:
-            _lib.check(rc, self._HOST_CALLS[1])
         return res
 
     # The native calls of the host-fed steps, the only part ChangeLogStream replaces: the staging, validation, ingest arming,
@@ -464,26 +366,6 @@ class PEStream:
                                               times.ctypes.data, qptrs, C, C_byref(head), C_byref(ln), G.data_ptr(), self.K,
                                               m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(), samp._err.data_ptr(),
                                               torch.cuda.current_stream().cuda_stream, sub.ctypes.data, C_byref(done))
-
-    def result(self, ticket: int) -> np.ndarray:
-        """Per-query row sums [C, n] of step `ticket` (waits for that step's device-to-host copy)."""
-        r = self._drained.pop(ticket, None)
-        if r is not None:
-            return r
-        if ticket >> 32 != self._epoch or ticket not in self._ticket_shape:
-            raise KeyError(f"result: ticket {ticket} is not outstanding (already read, or overwritten: the last {self.HOST_SLOTS} are kept)")
-        return self._result_now(ticket)
-
-    def _result_now(self, ticket: int) -> np.ndarray:
-        p = ctypes.POINTER(ctypes.c_float)()
-        nf = ctypes.c_int64(0)
-        rc = self._libc.lstep_host_step_result(self._host_stepper[0], ticket & 0xFFFFFFFF, C_byref(p), C_byref(nf))
-        if rc != 0:
-            _lib.check(rc, "lstep_host_step_result")
-        C, n = self._ticket_shape[ticket]
-        if nf.value == 0:
-            return np.zeros((C, n), np.float32)
-        return np.ctypeslib.as_array(p, shape=(C, n)).copy()
 
     def step_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None, ids: np.ndarray = None,
                   ingest: bool = False, edge_id_start: int = None):
