@@ -109,6 +109,20 @@ int lstep_csr_relayout(const lstep_csr* src, const int32_t* src_fill, const int6
                        int32_t* out_eid, double* out_t, int32_t* out_fill, uint32_t* err_flag, void* stream);
 int lstep_csr_ingest(const lstep_csr* csr, int32_t* fill, const int64_t* src, const int64_t* dst, const int64_t* eid,
                      int64_t eid_base, const double* t, int64_t n_edges, uint32_t* err_flag, void* stream);
+/* Row capacity of a growable CSR: indptr has row_cap + 1 entries, csr->num_rows counts the LIVE rows (every lookup's
+ * bound), and the arrays end in a padded tail [indptr[num_rows], nnz) that new rows take their entries from.
+ * lstep_csr_relayout_rows is lstep_csr_relayout for a regrow that may add rows: rows [src->num_rows, new_rows) are new
+ * (all padding, fill 0), out_fill[new_rows .. row_cap) = 0, new_indptr holds new_rows + 1 entries (the caller may fill the
+ * rest), and the tail [new_indptr[new_rows], total) is padded (total < 0: no tail). lstep_csr_relayout(src, ...) is
+ * lstep_csr_relayout_rows(src, ..., src->num_rows, src->num_rows, ..., -1, ...).
+ * lstep_csr_add_rows makes n_rows more rows live without moving any entry: row csr->num_rows + i gets cap[i] (device
+ * int64 [n_rows]) entries of the tail, i.e. indptr[num_rows + 1 + i] = indptr[num_rows] + cap[0] + ... + cap[i], and fill 0;
+ * then csr->num_rows += n_rows (host side). The caller guarantees room: num_rows + n_rows <= row_cap and the caps fit the
+ * tail. One CTA; stream-ordered after lookups already enqueued, which never read rows at or above their num_rows. */
+int lstep_csr_relayout_rows(const lstep_csr* src, const int32_t* src_fill, int64_t new_rows, int64_t row_cap, const int64_t* new_indptr,
+                            int64_t total, int32_t* out_nbr, int32_t* out_eid, double* out_t, int32_t* out_fill, uint32_t* err_flag,
+                            void* stream);
+int lstep_csr_add_rows(lstep_csr* csr, int32_t* fill, int64_t n_rows, const int64_t* cap, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * a2 — most-recent-K temporal neighbour lookup (kernel K1).
@@ -295,13 +309,21 @@ typedef struct lstep_pe_stream {
   const double* t;
   float* ring;
   float* cur;
-  int64_t V1;
+  int64_t V1; /* live rows: every bound check and every full-table pass covers [0, V1) */
   int T;
   int d;
+  int64_t row_cap; /* rows allocated in ring / cur (>= V1) and covered by the update workspace's per-node maps; 0 = V1 */
 } lstep_pe_stream;
 
 size_t lstep_pe_step_workspace_bytes(int64_t max_ids, int64_t max_edges, int n_queries, int K, int d, int t, int64_t V1);
 int lstep_ring_load(const float* ring, float* cur, int64_t V1, int T, int d, int slot, void* stream);
+/* New nodes [r0, r1) of a stream that grows its node set: writes rows[(v - r0) * rows_stride .. + d) (rows_stride 0: one
+ * broadcast row [d]; device memory) to table row v (table != NULL), to all T slots of ring row v (ring != NULL; node-major,
+ * one contiguous T*d block per node) and, when v % world == rank, to change-log base row (v - rank) / world (base != NULL).
+ * d % 4 == 0 and 16-byte aligned pointers. Enqueued on `stream` behind the steps already there, which touch only rows
+ * below r0: a node no edge has touched holds its initial row in the table, in every ring slot and as its base row. */
+int lstep_pe_rows_init(float* table, float* ring, int T, int d, float* base, int64_t world, int64_t rank, int64_t r0, int64_t r1,
+                       const float* rows, int64_t rows_stride, void* stream);
 int lstep_pe_step(const lstep_pe_stream* s, const lstep_csr* csr, int64_t lo, int64_t n_edges, const int64_t* ids,
                   int64_t n_ids, double current_time, int head, int len, int append_slot, const float* G,
                   const int64_t* const* query_ids_host, int n_queries, float* nbr_out, int K,

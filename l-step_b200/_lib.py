@@ -29,7 +29,7 @@ class CSR(C.Structure):
 
 class PEStreamDesc(C.Structure):
     """struct lstep_pe_stream"""
-    _fields_ = [("src", vp), ("dst", vp), ("t", vp), ("ring", vp), ("cur", vp), ("V1", i64), ("T", i32), ("d", i32)]
+    _fields_ = [("src", vp), ("dst", vp), ("t", vp), ("ring", vp), ("cur", vp), ("V1", i64), ("T", i32), ("d", i32), ("row_cap", i64)]
 
 
 class ChangeLog(C.Structure):
@@ -60,6 +60,8 @@ _SIGS = {
     "lstep_csr_build_from_entries": (i32, [vp, vp, vp, vp, i64, i64, vp, vp, vp, vp, vp, sz, vp, vp]),
     "lstep_csr_relayout": (i32, [C.POINTER(CSR), vp, vp, vp, vp, vp, vp, vp, vp]),
     "lstep_csr_ingest": (i32, [C.POINTER(CSR), vp, vp, vp, vp, i64, vp, i64, vp, vp]),
+    "lstep_csr_relayout_rows": (i32, [C.POINTER(CSR), vp, i64, i64, vp, i64, vp, vp, vp, vp, vp, vp]),
+    "lstep_csr_add_rows": (i32, [C.POINTER(CSR), vp, i64, vp, vp]),
     "lstep_sample_recent": (i32, [C.POINTER(CSR), vp, vp, i64, i64, i32, vp, vp, vp, vp, vp]),
     "lstep_sample_recent_compact": (i32, [C.POINTER(CSR), vp, vp, i64, i64, i32, vp, vp, vp, vp]),
     "lstep_dft_collapse": (i32, [vp, vp, i32, i32, i32, vp, vp]),
@@ -90,6 +92,7 @@ _SIGS = {
     "lstep_ring_copy_rows": (i32, [vp, vp, i64, i32, i32, i32, i64, i64, i32, vp]),
     "lstep_pe_step_workspace_bytes": (sz, [i64, i64, i32, i32, i32, i32, i64]),
     "lstep_ring_load": (i32, [vp, vp, i64, i32, i32, i32, vp]),
+    "lstep_pe_rows_init": (i32, [vp, vp, i32, i32, vp, i64, i64, i64, i64, vp, i64, vp]),
     "lstep_pe_step": (i32, [C.POINTER(PEStreamDesc), C.POINTER(CSR), i64, i64, vp, i64, C.c_double, i32, i32, i32, vp,
                             C.POINTER(C.c_void_p), i32, vp, i32, C.POINTER(PEMLP), C.POINTER(PEMLP), vp, sz, vp, vp]),
     "lstep_pe_steps": (i32, [C.POINTER(PEStreamDesc), C.POINTER(CSR), i64, vp, vp, vp, vp, vp, C.POINTER(i32), C.POINTER(i32), vp,

@@ -38,31 +38,53 @@ class ChangeLogHistory:
     """The change log of rank `rank` of a world-`world` group over V1 nodes: the nodes v with v % world == rank, node v at
     row (v - rank) / world, `rows` of them (checkpoint.rows_of). `cap` events per window slot (at least 1). `ref` is the
     lstep_changelog descriptor to pass to the native calls. The base rows of a new log are unset: `reset` or `load` fills
-    them."""
+    them. `row_cap` (>= V1, default V1): nodes base / ev_mask are allocated for, so that `add_rows` can grow V1 in place;
+    the descriptor carries the live row count."""
 
-    def __init__(self, V1: int, T: int, d: int, cap: int, world: int, rank: int, device):
+    def __init__(self, V1: int, T: int, d: int, cap: int, world: int, rank: int, device, row_cap: int = None):
         if T > 128:
             raise _lib.LstepError("the change-log history supports T <= 128 window steps")
         self.V1, self.T, self.d, self.world, self.rank, self.dev = int(V1), int(T), int(d), int(world), int(rank), device
         self.rows = ckpt.rows_of(self.V1, self.world, self.rank)
+        self.row_cap = max(self.V1, int(row_cap or 0))
+        rows_cap = ckpt.rows_of(self.row_cap, self.world, self.rank)
         self.cap = cap = int(max(cap, 1))
         H = 1
         while H < 2 * cap:
             H *= 2
-        self.base = torch.empty((self.rows, d), dtype=torch.float32, device=device)
+        self.base = torch.empty((rows_cap, d), dtype=torch.float32, device=device)
         self.ev_node = torch.zeros((T, cap), dtype=torch.int32, device=device)
         self.ev_row = torch.empty((T, cap, d), dtype=torch.float32, device=device)
         self.ev_cnt = torch.zeros(T, dtype=torch.int32, device=device)
         self.ev_hash = torch.full((T, H), -1, dtype=torch.int64, device=device)
-        self.ev_mask = torch.zeros((max(self.rows, 1), 4), dtype=torch.int32, device=device)
+        self.ev_mask = torch.zeros((max(rows_cap, 1), 4), dtype=torch.int32, device=device)
         self.desc = _lib.ChangeLog(self.base.data_ptr(), self.ev_node.data_ptr(), self.ev_row.data_ptr(), self.ev_cnt.data_ptr(),
                                    self.ev_hash.data_ptr(), self.ev_mask.data_ptr(), max(self.rows, 1), T, cap, H, d, self.world,
                                    self.rank)
         self.ref = ctypes.byref(self.desc)
 
+    def grow_capacity(self, row_cap: int):
+        """Reallocate base and ev_mask for `row_cap` nodes and copy the live rows over (on the current stream, behind the steps
+        already enqueued). Both new tensors are allocated before either is swapped in."""
+        rows_cap = ckpt.rows_of(int(row_cap), self.world, self.rank)
+        base = torch.empty((rows_cap, self.d), dtype=torch.float32, device=self.dev)
+        mask = torch.zeros((max(rows_cap, 1), 4), dtype=torch.int32, device=self.dev)
+        base[:self.rows].copy_(self.base[:self.rows])
+        mask[:self.rows].copy_(self.ev_mask[:self.rows])
+        self.base, self.ev_mask, self.row_cap = base, mask, int(row_cap)
+        self.desc.base, self.desc.ev_mask = base.data_ptr(), mask.data_ptr()
+
+    def add_rows(self, V1: int):
+        """Make nodes [self.V1, V1) live (V1 <= row_cap). Their base rows must be written (lstep_pe_rows_init) before a step
+        reads them; their event masks are zero, as allocated."""
+        assert self.V1 <= V1 <= self.row_cap
+        self.V1 = int(V1)
+        self.rows = ckpt.rows_of(self.V1, self.world, self.rank)
+        self.desc.rows = max(self.rows, 1)
+
     def reset(self, cur: torch.Tensor):
         """A one-step history: base = the owned rows of the table `cur` [V1, d], no events. Returns the window (head, len)."""
-        self.base.copy_(cur[self.rank::self.world])
+        self.base[:self.rows].copy_(cur[:self.V1][self.rank::self.world])
         self.ev_cnt.zero_()
         self.ev_hash.fill_(-1)
         self.ev_mask.zero_()
@@ -84,7 +106,7 @@ class ChangeLogHistory:
         chunk = max(1, (256 << 20) // (4 * hist.d))
         with torch.cuda.device(dev), torch.no_grad():
             for g, sh in enumerate(hist.shards):
-                dst = cur[g::hist.world]
+                dst = cur[:self.V1][g::hist.world]
                 for a in range(0, dst.shape[0], chunk):
                     dst[a:a + chunk].copy_(_to_dev(sh["base"][a:a + chunk], dev, torch.float32))
             self.reset(cur)
@@ -118,11 +140,11 @@ class ChangeLogHistory:
                 ev_node[off[f]:off[f + 1]] = nodes[order]
                 ev_row[off[f]:off[f + 1]] = self.ev_row[s, :n].cpu().numpy()[order]
         meta = dict(meta, world=self.world, rank=self.rank, V1=self.V1, d=self.d, T=self.T, len=length)
-        ckpt.write_shard(path, meta, self.base.cpu().numpy(), off, ev_node, ev_row)
+        ckpt.write_shard(path, meta, self.base[:self.rows].cpu().numpy(), off, ev_node, ev_row)
 
     def replay(self, head: int, length: int) -> torch.Tensor:
         """The window (head, length) as dense rows [rows, length, d], oldest first (needs rows * length * d * 4 bytes)."""
-        snap = self.base.clone()
+        snap = self.base[:self.rows].clone()
         out = torch.empty((self.rows, length, self.d), dtype=torch.float32, device=self.dev)
         cnt = self.ev_cnt.cpu().tolist()
         for f in range(length):

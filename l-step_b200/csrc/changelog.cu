@@ -470,7 +470,7 @@ int changelog_step_core(const lstep_pe_stream* s, const lstep_changelog* cl, con
   const int32_t *n_dest = nullptr, *stamp_map = nullptr;
   int64_t n_u_max = 0;
   if (n_ids > 0) {
-    update_ws_phase_b_lists(workspace, n_ids, n_edges, K, s->d, mlp_upd->t, s->V1, &U, &n_dest, &stamp_map);
+    update_ws_phase_b_lists(workspace, n_ids, n_edges, K, s->d, mlp_upd->t, pe_ws_rows(s), &U, &n_dest, &stamp_map);
     const int64_t total = n_ids * (int64_t)K;
     n_u_max = (total < s->V1 - 1 ? total : s->V1 - 1) + 1;
   }

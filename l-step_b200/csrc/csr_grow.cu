@@ -20,18 +20,24 @@ namespace lstep {
 constexpr int kIngestChunkEdges = 2048;  // edges per chunk (<= 4096 entries = 32 KB of sort keys); chunks go in order
 constexpr int kIngestPosBits = 12;       // bits of an entry's position in its chunk: log2(2 * kIngestChunkEdges)
 
-// one warp per row: the row's real entries move to their new place, the rest of the new row becomes padding
+// one warp per row: the row's real entries move to their new place, the rest of the new row becomes padding. Rows
+// [src_rows, new_rows) are new (no entries: all padding); rows [new_rows, fill_rows) are allocated but not live: fill 0.
 __global__ void __launch_bounds__(256) csr_relayout_kernel(const int64_t* __restrict__ indptr, const int32_t* __restrict__ nbr,
                                                            const int32_t* __restrict__ eid, const double* __restrict__ t,
-                                                           const int32_t* __restrict__ fill, int64_t num_rows,
-                                                           const int64_t* __restrict__ new_indptr, int32_t* __restrict__ out_nbr,
-                                                           int32_t* __restrict__ out_eid, double* __restrict__ out_t,
-                                                           int32_t* __restrict__ out_fill, uint32_t* err_flag) {
+                                                           const int32_t* __restrict__ fill, int64_t src_rows, int64_t new_rows,
+                                                           int64_t fill_rows, const int64_t* __restrict__ new_indptr,
+                                                           int32_t* __restrict__ out_nbr, int32_t* __restrict__ out_eid,
+                                                           double* __restrict__ out_t, int32_t* __restrict__ out_fill,
+                                                           uint32_t* err_flag) {
   const int64_t v = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
-  if (v >= num_rows) return;
-  const int64_t lo = indptr[v];
-  const int64_t f = fill ? (int64_t)fill[v] : indptr[v + 1] - lo;
+  if (v >= fill_rows) return;
+  if (v >= new_rows) {
+    if (lane == 0) out_fill[v] = 0;
+    return;
+  }
+  const int64_t lo = v < src_rows ? indptr[v] : 0;
+  const int64_t f = v >= src_rows ? 0 : fill ? (int64_t)fill[v] : indptr[v + 1] - lo;
   const int64_t nlo = new_indptr[v], cap = new_indptr[v + 1] - nlo;
   const int64_t n = f < cap ? f : cap;
   for (int64_t k = lane; k < cap; k += 32) {
@@ -48,6 +54,47 @@ __global__ void __launch_bounds__(256) csr_relayout_kernel(const int64_t* __rest
   if (lane == 0) {
     out_fill[v] = (int32_t)n;
     if (n < f && err_flag) atomicOr(err_flag, LSTEP_FLAG_CSR_FULL);
+  }
+}
+
+// padding for the tail [new_indptr[new_rows], total) of a relaid CSR, which lstep_csr_add_rows hands out to new rows
+__global__ void __launch_bounds__(256) csr_pad_tail_kernel(const int64_t* __restrict__ new_indptr, int64_t new_rows, int64_t total,
+                                                           int32_t* __restrict__ out_nbr, int32_t* __restrict__ out_eid,
+                                                           double* __restrict__ out_t) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t k = new_indptr[new_rows] + blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < total; k += stride) {
+    out_nbr[k] = 0;
+    out_eid[k] = 0;
+    out_t[k] = CUDART_INF;
+  }
+}
+
+// rows [r0, r0 + n) become live: indptr[r0 + 1 + i] = indptr[r0] + cap[0] + ... + cap[i], fill = 0. One CTA, a block scan
+// per chunk of 1024 rows; the entries the rows take were padded when the tail was laid out, so nothing else is written.
+__global__ void __launch_bounds__(1024) csr_add_rows_kernel(int64_t* indptr, int32_t* fill, int64_t r0, int64_t n,
+                                                            const int64_t* __restrict__ cap) {
+  __shared__ int64_t s_sum[1024];
+  __shared__ int64_t s_base;
+  const int tid = threadIdx.x;
+  if (tid == 0) s_base = indptr[r0];
+  __syncthreads();
+  for (int64_t c0 = 0; c0 < n; c0 += 1024) {
+    const int64_t i = c0 + tid;
+    s_sum[tid] = i < n ? cap[i] : 0;
+    __syncthreads();
+    for (int o = 1; o < 1024; o <<= 1) {  // Hillis-Steele inclusive scan
+      const int64_t x = tid >= o ? s_sum[tid - o] : 0;
+      __syncthreads();
+      s_sum[tid] += x;
+      __syncthreads();
+    }
+    if (i < n) {
+      indptr[r0 + 1 + i] = s_base + s_sum[tid];
+      fill[r0 + i] = 0;
+    }
+    __syncthreads();
+    if (tid == 1023) s_base += s_sum[1023];
+    __syncthreads();
   }
 }
 
@@ -179,13 +226,37 @@ using namespace lstep;
 
 extern "C" int lstep_csr_relayout(const lstep_csr* src, const int32_t* src_fill, const int64_t* new_indptr, int32_t* out_nbr,
                                   int32_t* out_eid, double* out_t, int32_t* out_fill, uint32_t* err_flag, void* stream) {
+  if (!src || src->num_rows <= 0) return LSTEP_ERR_INVALID_ARG;
+  return lstep_csr_relayout_rows(src, src_fill, src->num_rows, src->num_rows, new_indptr, -1, out_nbr, out_eid, out_t, out_fill, err_flag,
+                                 stream);
+}
+
+extern "C" int lstep_csr_relayout_rows(const lstep_csr* src, const int32_t* src_fill, int64_t new_rows, int64_t row_cap,
+                                       const int64_t* new_indptr, int64_t total, int32_t* out_nbr, int32_t* out_eid, double* out_t,
+                                       int32_t* out_fill, uint32_t* err_flag, void* stream) {
   if (!src || !src->indptr || !new_indptr || !out_fill || src->num_rows <= 0) return LSTEP_ERR_INVALID_ARG;
-  if (src->num_rows > 0x7fffffffLL) return LSTEP_ERR_ID_RANGE;
+  if (new_rows < src->num_rows || row_cap < new_rows) return LSTEP_ERR_INVALID_ARG;
+  if (row_cap > 0x7fffffffLL) return LSTEP_ERR_ID_RANGE;
   if (!out_nbr || !out_eid || !out_t) return LSTEP_ERR_INVALID_ARG;
-  const int64_t rows = src->num_rows;
-  csr_relayout_kernel<<<(unsigned)ceil_div(rows * 32, 256), 256, 0, as_stream(stream)>>>(
-      src->indptr, src->nbr, src->eid, src->t, src_fill, rows, new_indptr, out_nbr, out_eid, out_t, out_fill, err_flag);
-  return check_launch("csr_relayout");
+  cudaStream_t st = as_stream(stream);
+  csr_relayout_kernel<<<(unsigned)ceil_div(row_cap * 32, 256), 256, 0, st>>>(src->indptr, src->nbr, src->eid, src->t, src_fill, src->num_rows,
+                                                                             new_rows, row_cap, new_indptr, out_nbr, out_eid, out_t, out_fill,
+                                                                             err_flag);
+  int rc = check_launch("csr_relayout");
+  if (rc != LSTEP_OK || total < 0) return rc;
+  csr_pad_tail_kernel<<<num_sms() * 4, 256, 0, st>>>(new_indptr, new_rows, total, out_nbr, out_eid, out_t);
+  return check_launch("csr_pad_tail");
+}
+
+extern "C" int lstep_csr_add_rows(lstep_csr* csr, int32_t* fill, int64_t n_rows, const int64_t* cap, void* stream) {
+  if (!csr || !csr->indptr || !fill || n_rows < 0 || (n_rows > 0 && !cap)) return LSTEP_ERR_INVALID_ARG;
+  if (csr->num_rows <= 0 || csr->num_rows + n_rows > 0x7fffffffLL) return LSTEP_ERR_ID_RANGE;
+  if (n_rows == 0) return LSTEP_OK;
+  // the CSR is caller-owned device memory; lstep_csr carries const pointers because the lookups only read it
+  csr_add_rows_kernel<<<1, 1024, 0, as_stream(stream)>>>(const_cast<int64_t*>(csr->indptr), fill, csr->num_rows, n_rows, cap);
+  const int rc = check_launch("csr_add_rows");
+  if (rc == LSTEP_OK) csr->num_rows += n_rows;
+  return rc;
 }
 
 extern "C" int lstep_csr_ingest(const lstep_csr* csr, int32_t* fill, const int64_t* src, const int64_t* dst, const int64_t* eid,

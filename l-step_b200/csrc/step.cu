@@ -184,6 +184,46 @@ extern "C" int lstep_ring_load(const float* ring, float* cur, int64_t V1, int T,
   return check_launch("ring_load");
 }
 
+namespace lstep {
+// Rows [r0, r1) of new nodes: table row, every ring slot (node-major, so one contiguous T*d block per node) and, for the owned
+// nodes (v % world == rank), the change-log base row at (v - rank) / world, from rows[(v - r0) * rows_stride] (stride 0: one
+// broadcast row). One float4 per thread-iteration, grid-stride over the nodes' blocks.
+__global__ void __launch_bounds__(256) pe_rows_init_kernel(float* __restrict__ table, float* __restrict__ ring, int T, int d,
+                                                           float* __restrict__ base, int64_t world, int64_t rank, int64_t r0,
+                                                           int64_t r1, const float* __restrict__ rows, int64_t rows_stride) {
+  const int dvec = d / 4;
+  const int64_t per_node = (int64_t)(1 + (ring ? T : 0)) * dvec;  // table row, then the T ring slots
+  const int64_t total = (r1 - r0) * per_node;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += stride) {
+    const int64_t k = i / per_node, j = i - k * per_node;
+    const int64_t v = r0 + k;
+    const int c = (int)(j % dvec);
+    const float4 x = reinterpret_cast<const float4*>(rows + k * rows_stride)[c];
+    if (j < dvec) {
+      if (table) reinterpret_cast<float4*>(table + v * d)[c] = x;
+      if (base && v % world == rank) reinterpret_cast<float4*>(base + ((v - rank) / world) * d)[c] = x;
+    } else {
+      reinterpret_cast<float4*>(ring + v * (int64_t)T * d)[j - dvec] = x;
+    }
+  }
+}
+}  // namespace lstep
+
+extern "C" int lstep_pe_rows_init(float* table, float* ring, int T, int d, float* base, int64_t world, int64_t rank, int64_t r0, int64_t r1,
+                                  const float* rows, int64_t rows_stride, void* stream) {
+  if (!rows || d <= 0 || d % 4 != 0 || r0 < 0 || r1 < r0 || rows_stride < 0 || rows_stride % 4 != 0) return LSTEP_ERR_INVALID_ARG;
+  if ((ring && T <= 0) || (base && (world <= 0 || rank < 0 || rank >= world))) return LSTEP_ERR_INVALID_ARG;
+  if (reinterpret_cast<uintptr_t>(rows) % 16 || reinterpret_cast<uintptr_t>(table) % 16 || reinterpret_cast<uintptr_t>(ring) % 16 ||
+      reinterpret_cast<uintptr_t>(base) % 16)
+    return LSTEP_ERR_INVALID_ARG;
+  if (r1 == r0 || (!table && !ring && !base)) return LSTEP_OK;
+  const int64_t work = (r1 - r0) * (int64_t)(1 + (ring ? T : 0)) * (d / 4);
+  const int64_t grid = std::min<int64_t>(ceil_div(work, 256), (int64_t)num_sms() * 8);
+  pe_rows_init_kernel<<<(unsigned)grid, 256, 0, as_stream(stream)>>>(table, ring, T, d, base, world, rank, r0, r1, rows, rows_stride);
+  return check_launch("pe_rows_init");
+}
+
 /* Sharded ring (rows v of the local ring <-> table rows v*row_mul + row_add): load / append one slot. */
 extern "C" int lstep_ring_copy_rows(float* ring, float* cur, int64_t ring_rows, int T, int d, int slot, int64_t row_mul,
                                     int64_t row_add, int to_ring, void* stream) {
@@ -224,9 +264,9 @@ int pe_step_core_ex(const lstep_pe_stream* s, const lstep_csr* csr, const int64_
   if (head < 0 || head >= s->T || len < 0 || len > s->T || append_slot < 0 || append_slot >= s->T) return LSTEP_ERR_INVALID_ARG;
   if (n_queries > 0 && (!query_ids_host || !nbr_out)) return LSTEP_ERR_INVALID_ARG;
   const int d = s->d, t = mlp_nbr->t, T = s->T;
-  const StepWs need = carve_step(nullptr, n_ids, n_edges, n_queries, K, d, t, s->V1);
+  const StepWs need = carve_step(nullptr, n_ids, n_edges, n_queries, K, d, t, pe_ws_rows(s));
   if (!workspace || workspace_bytes < need.bytes) return LSTEP_ERR_WORKSPACE;
-  StepWs w = carve_step(workspace, n_ids, n_edges, n_queries, K, d, t, s->V1);
+  StepWs w = carve_step(workspace, n_ids, n_edges, n_queries, K, d, t, pe_ws_rows(s));
   cudaStream_t st = as_stream(stream);
   int rc;
   if (!opt.peer) prof_mark(st, kProfStart);
@@ -282,7 +322,7 @@ int pe_step_core_ex(const lstep_pe_stream* s, const lstep_csr* csr, const int64_
   const int threads = (int)align_up((size_t)t_pad + d / 4, 32);
   const bool vec_ok = d % 4 == 0 && w.lda % 4 == 0 && reinterpret_cast<uintptr_t>(s->cur) % 16 == 0 && threads <= 512;
   if (first_half && rows > 0 && n_a > 0 && n_edges > 0 && vec_ok && t == mlp_upd->t && d == mlp_upd->d) {
-    update_ws_phase_a(w.update, n_ids, n_edges, K, d, t, s->V1, &A, &ldA, &counters, &new_rows);
+    update_ws_phase_a(w.update, n_ids, n_edges, K, d, t, pe_ws_rows(s), &A, &ldA, &counters, &new_rows);
     const int64_t cap = (int64_t)num_sms() * 16;
     // more query rows than one launch has CTAs for (B = 2000): one wave of CTAs with a look-ahead lookup warp each (gather_pipe)
     const bool piped = tuning().gather_pipe != 0 && rows > cap && threads + 32 <= 512;
@@ -334,11 +374,11 @@ int pe_step_core_ex(const lstep_pe_stream* s, const lstep_csr* csr, const int64_
       // phase A's rows of the owned batch nodes (stand-alone launches when the paired launch did not apply), then into every
       // rank's new_rows buffer at the node's position in the batch's id list, then barrier 2 is announced
       if (!phase_a_done) {
-        rc = launch_phase_a_to_new_rows(s->cur, w.update, n_ids, n_edges, K, s->V1, ids_a, n_a, src, dst, tq, n_edges, (float)current_time,
+        rc = launch_phase_a_to_new_rows(s->cur, w.update, n_ids, n_edges, K, pe_ws_rows(s), ids_a, n_a, src, dst, tq, n_edges, (float)current_time,
                                         mlp_upd, edges_done, st);
         if (rc != LSTEP_OK) return rc;
       }
-      update_ws_phase_a(w.update, n_ids, n_edges, K, d, t, s->V1, &A, &ldA, &counters, &new_rows);
+      update_ws_phase_a(w.update, n_ids, n_edges, K, d, t, pe_ws_rows(s), &A, &ldA, &counters, &new_rows);
       if (n_a > 0 && (rc = peer_rows_bcast(new_rows, n_a, d, peer->pos_mine, peer->grp, 1, st)) != LSTEP_OK) return rc;
       if (!second_half && (rc = peer_signal(peer->grp, peer->epoch2, st)) != LSTEP_OK) return rc;  // (else the wait launch announces)
       prof_mark(st, kProfBcast);
@@ -360,7 +400,7 @@ int pe_step_core_ex(const lstep_pe_stream* s, const lstep_csr* csr, const int64_
   }
   if (opt.stamp_out) *opt.stamp_out = stamp;
   int32_t* dirty = nullptr;
-  rc = update_pe_impl(s->cur, s->V1, csr, ids, n_ids, src, dst, tq, n_edges, current_time, K, mlp_upd, w.update, w.update_bytes,
+  rc = update_pe_impl(s->cur, pe_ws_rows(s), csr, ids, n_ids, src, dst, tq, n_edges, current_time, K, mlp_upd, w.update, w.update_bytes,
                       err_flag, stream, edges_done, opt.skip_append ? nullptr : &dirty, stamp, phase_a_done,
                       s->ring + (int64_t)append_slot * d, (int64_t)T * d, peer ? &own : nullptr);
   if (rc != LSTEP_OK) return rc;

@@ -4,6 +4,10 @@
 
 namespace lstep {
 
+// Rows the update workspace's per-node maps cover: the stream's row capacity, so that the workspace layout stays put while
+// the live row count V1 grows inside it (lstep_pe_stream.row_cap, 0 = V1).
+inline int64_t pe_ws_rows(const lstep_pe_stream* s) { return s->row_cap > s->V1 ? s->row_cap : s->V1; }
+
 // Owner-computes step of a peer group (csrc/peer.cu): phase A runs for the OWNED batch nodes only and its rows are stored
 // into every rank's new_rows buffer; phase B runs for the owned destinations only. `phases` bit 1: everything up to the
 // announcement of barrier 2; bit 2: from the wait on barrier 2 on (a single-process group runs bit 1 of every rank first).

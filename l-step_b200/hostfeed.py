@@ -5,7 +5,14 @@ slot, copies it in, runs the step and copies the per-query row sums back, and re
 what surrounds the native call: the normalisation of the host arrays, the validation and room-making of a batch that is ingested
 into a growable sampler (ingest=True), the arming of the stepper for it, the ticket bookkeeping and `result`, and the resync of
 the sampler after a failed call. A class that mixes it in provides `dev`, `B`, `d` and `_host_sampler()`, the sampler whose CSR
-its steps read."""
+its steps read.
+
+It also owns the growth of the node set (add_nodes, and grow=True on the host-fed steps): new node ids continue after the
+last live one, and a new node starts with its initial row r0 in the table, in every history slot and as its change-log base
+row, which is exactly the state a node no edge has touched has in a stream built with those rows from the start. So a grown
+stream computes the bits of the pre-sized one. The class provides `V1`, `row_cap`, `_grow_capacity(row_cap)`, which
+reallocates its tables for more rows (every new buffer allocated before any is swapped in), `_init_rows(v0, v1, rows,
+stride)`, which enqueues lstep_pe_rows_init, and `_set_live(V1)`."""
 from __future__ import annotations
 
 import ctypes
@@ -14,7 +21,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .sampler import check_edges
+from .sampler import NODE_ID_MAX, check_edges, new_row_need
 
 C_void_p = ctypes.c_void_p
 C_byref = ctypes.byref
@@ -90,6 +97,83 @@ class HostFed:
                 pass
             self._host_stepper = None
 
+    # ---- node growth --------------------------------------------------------------------------------------------------
+    def _growth_init(self, new_node_pe=None, max_nodes: int = None):
+        """new_node_pe: the row [d] a node added without explicit rows starts with (default zeros, what RandomWalkPE gives an
+        isolated node); max_nodes: optional limit on the node count (ids >= max_nodes raise IndexError)."""
+        r0 = np.zeros(self.d, np.float32) if new_node_pe is None else self._rows_array(new_node_pe, 1)
+        self._r0 = torch.from_numpy(r0).to(self.dev)
+        self.max_nodes = None if max_nodes is None else int(max_nodes)
+
+    def _rows_array(self, rows, ndim: int) -> np.ndarray:
+        """rows as a contiguous float32 host array of shape [d] (ndim 1) or [n, d] (ndim 2); ValueError otherwise."""
+        if isinstance(rows, torch.Tensor):
+            rows = rows.detach().cpu()
+        try:
+            a = np.ascontiguousarray(np.asarray(rows, dtype=np.float32))
+        except (TypeError, ValueError) as e:
+            raise ValueError(f"new node rows must convert to float32: {e}") from None
+        if a.ndim != ndim or a.shape[-1] != self.d:
+            raise ValueError(f"new node rows must have shape {'[d]' if ndim == 1 else '[n, d]'} with d = {self.d} (got {a.shape})")
+        if not np.isfinite(a).all():
+            raise ValueError("new node rows must be finite")
+        return a
+
+    def _check_new_ids(self, hi: int):
+        """IndexError when node id `hi` may not be added (int32 limit of the change log's node ids, max_nodes)."""
+        if hi > NODE_ID_MAX:
+            raise IndexError(f"node id {hi} exceeds the int32 node id limit ({NODE_ID_MAX})")
+        if self.max_nodes is not None and hi >= self.max_nodes:
+            raise IndexError(f"node id {hi} is outside max_nodes ({self.max_nodes})")
+
+    def _check_event_capacity(self, V1: int):
+        """Change-log histories: ValueError when a step on V1 nodes could change more rows than the log records per step."""
+
+    def _new_nodes_for(self, arrays) -> int:
+        """grow=True: validate the ids of a batch (or a run) and return how many nodes it adds (ids up to its maximum).
+        Nothing is written."""
+        lo = min(int(a.min()) for a in arrays if len(a))
+        hi = max(int(a.max()) for a in arrays if len(a))
+        if lo < 0:
+            raise IndexError(f"list index out of range: node id {lo}")
+        n_new = max(0, hi + 1 - self.V1)
+        if n_new:
+            self._check_new_ids(hi)
+            self._growable_sampler()
+        return n_new
+
+    def add_nodes(self, rows_or_count, _edges=None) -> int:
+        """Add nodes with the next ids and return the first of them. rows_or_count: a count n (each new node starts with
+        the stream's new_node_pe row) or per-node rows [n, d] (float32-convertible, finite). The table, the history and
+        the model's growable sampler grow together; everything is validated before any device write, and the rows are
+        written on the current stream, behind the steps already enqueued (which touch only rows below the old V1). When
+        the row capacity runs out it doubles: new buffers are allocated first, then the live rows are copied."""
+        if isinstance(rows_or_count, (int, np.integer)):
+            n, rows, stride = int(rows_or_count), self._r0, 0
+            if n < 0:
+                raise ValueError("add_nodes: the count must be >= 0")
+        else:
+            a = self._rows_array(rows_or_count, 2)
+            n, rows, stride = a.shape[0], a, self.d
+        v0 = self.V1
+        if n == 0:
+            return v0
+        self._check_new_ids(v0 + n - 1)
+        self._check_event_capacity(v0 + n)
+        samp = self._growable_sampler()
+        if isinstance(rows, np.ndarray):
+            rows = torch.from_numpy(rows).pin_memory().to(self.dev, non_blocking=True)
+        v1 = v0 + n
+        if v1 > self.row_cap:
+            self._grow_capacity(max(2 * self.row_cap, v1))
+        if v1 > samp.num_rows:
+            k = v1 - samp.num_rows
+            samp.add_rows(k, None if _edges is None else new_row_need(_edges[0], _edges[1], samp.num_rows, k))
+        with torch.cuda.device(self.dev):
+            self._init_rows(v0, v1, rows, stride)
+        self._set_live(v1)
+        return v0
+
     # ---- ingest -------------------------------------------------------------------------------------------------------
     def _growable_sampler(self):
         samp = self._host_sampler()
@@ -97,12 +181,15 @@ class HostFed:
             raise ValueError("ingest=True needs a growable neighbor sampler: model.set_neighbor_sampler(NeighborSampler.growable(...))")
         return samp
 
-    def _check_ingest(self, src, dst, times, edge_id_start):
-        """Validate a host batch for ingestion and make room for it; returns its first edge id. Nothing is written to
-        the device unless a regrow is needed."""
+    def _check_ingest(self, src, dst, times, edge_id_start, n_new: int = 0):
+        """Validate a host batch for ingestion (its ids against the rows it will have after n_new nodes are added), add
+        those nodes and make room for it; returns its first edge id. Nothing is written to the device before the batch is
+        validated."""
         samp = self._growable_sampler()
         eid0 = samp.next_edge_id if edge_id_start is None else int(edge_id_start)
-        check_edges(src, dst, eid0, times, samp.num_rows, samp.last_time)
+        check_edges(src, dst, eid0, times, max(samp.num_rows, self.V1 + n_new) if n_new else samp.num_rows, samp.last_time)
+        if n_new:
+            self.add_nodes(n_new, _edges=(src, dst))
         samp.reserve(src, dst)
         return eid0
 

@@ -137,7 +137,8 @@ class PeerRank(HostFed):
 
     def __init__(self, model: LSTEP, rank: int, world: int, src, dst, t, num_nodes: int, batch_size: int, num_neighbors: int,
                  initial_pe: torch.Tensor = None, start: int = 0, stop: int = None, device=None, sampler: NeighborSampler = None,
-                 event_capacity: int = None, timeout_ms: int = 4000, history: torch.Tensor = None, checkpoint=None, batch_idx: int = None):
+                 event_capacity: int = None, timeout_ms: int = 4000, history: torch.Tensor = None, checkpoint=None, batch_idx: int = None,
+                 row_capacity: int = None, new_node_pe=None, max_nodes: int = None):
         assert 1 <= world <= 16 and 0 <= rank < world
         if (initial_pe is None) + (history is None) + (checkpoint is None) != 2:
             raise ValueError("PeerRank: give exactly one of initial_pe, history and checkpoint")
@@ -146,11 +147,13 @@ class PeerRank(HostFed):
         self.B, self.K, self.T = int(batch_size), int(num_neighbors), model.num_fft_batches
         self.d, self.t_dim = model.pe_dim, model.time_feat_dim
         self.V1 = int(num_nodes) + 1
+        self.row_cap = max(self.V1, int(row_capacity or 0))
         self.timeout_ms = int(timeout_ms)
         # change log of the owned nodes; its capacity is the same on every rank: the inbox blocks are laid out by it
         G, B = self.G, self.B
-        cap = event_capacity if event_capacity is not None else min((self.V1 + G - 1) // G, 2 * (2 * B * (self.K + 1) + 2) // G + 1024)
-        self.changelog = ChangeLogHistory(self.V1, self.T, self.d, cap, G, self.rank, dev)
+        self._cap_arg = event_capacity
+        cap = event_capacity if event_capacity is not None else self._default_event_cap(max(self.row_cap, int(max_nodes or 0)))
+        self.changelog = ChangeLogHistory(self.V1, self.T, self.d, cap, G, self.rank, dev, self.row_cap)
         self.rows_local, self.cap = self.changelog.rows, self.changelog.cap
         hist = None
         if checkpoint is not None:
@@ -180,12 +183,13 @@ class PeerRank(HostFed):
             self._mem_filt = _DevMem(lib, 2 * B * d * 4)
             self._mem_inbox = _DevMem(lib, max(int(lib.lstep_peer_inbox_bytes(G, self.cap, d)), 256))
             self._mem_flags = _DevMem(lib, 16 * 4)
-            self.cur = torch.empty((self.V1, d), dtype=torch.float32, device=dev)
+            self.cur = torch.empty((self.row_cap, d), dtype=torch.float32, device=dev)
             if hist is None:
-                self.cur.copy_(initial_pe.to(dev, torch.float32))
+                self.cur[:self.V1].copy_(initial_pe.to(dev, torch.float32))
                 self.head, self.len = self.changelog.reset(self.cur)
             self.new_rows = self._mem_rows.tensor((2 * B, d), torch.float32, dev)
-            self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.tt.data_ptr(), None, self.cur.data_ptr(), self.V1, T, d)
+            self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.tt.data_ptr(), None, self.cur.data_ptr(), self.V1, T, d,
+                                          self.row_cap)
             # ---- per-batch plan of the resident stream: one pass on the host, uploaded once
             src_h = self.src[self.start:stop].cpu().numpy()
             dst_h = self.dst[self.start:stop].cpu().numpy()
@@ -205,20 +209,61 @@ class PeerRank(HostFed):
             self.ids, self.ids_mine, self.pos_mine = up(plan["ids"]), up(plan["mine"]), up(plan["pos"])
             self.ids_off, self.mine_off = plan["ids_off"], plan["mine_off"]
             self.lo, self.n_edges, self.tmax = np.asarray(lo_l, np.int64), np.asarray(n_l, np.int64), np.asarray(tmax, np.float64)
-            need = lib.lstep_pe_step_workspace_bytes(2 * B, B, 8, self.K, d, self.t_dim, self.V1)
-            self.ws = torch.empty(need + 4096, dtype=torch.uint8, device=dev)
-            _lib.check(lib.lstep_update_pe_workspace_init(_lib.ptr(self.ws), self.ws.numel(), self.V1, _lib.stream_ptr()), "ws init")
+            self.ws = self._new_ws(self.row_cap)
         self.batch_idx, self.steps_done, self.edges_done = 0, 0, self.start
         self.epoch = ctypes.c_uint32(0)  # (a fresh rank: the flag blocks are zeroed by lstep_ipc_alloc)
         self.grp = None
         self._opened = []
         self._host_init()
+        self._growth_init(new_node_pe, max_nodes)
         if hist is not None:
             self.head, self.len = self.changelog.load(hist, self.cur)
             if checkpoint is not None:
                 self.batch_idx, self.steps_done, self.edges_done = (int(hist.meta[k]) for k in ("batch_idx", "steps_done", "edges_done"))
         if batch_idx is not None:
             self.batch_idx = int(batch_idx)
+
+    def _new_ws(self, row_cap: int) -> torch.Tensor:
+        """A step workspace for batches of up to B edges and 8 query sets whose per-node maps cover row_cap rows, zeroed."""
+        lib = self.lib
+        need = lib.lstep_pe_step_workspace_bytes(2 * self.B, self.B, 8, self.K, self.d, self.t_dim, row_cap)
+        ws = torch.empty(need + 4096, dtype=torch.uint8, device=self.dev)
+        _lib.check(lib.lstep_update_pe_workspace_init(_lib.ptr(ws), ws.numel(), row_cap, _lib.stream_ptr()), "ws init")
+        return ws
+
+    # ---- node growth (add_nodes and grow=True: hostfeed.HostFed). Every rank of a group calls add_nodes with the same argument
+    # and grows its own replica, the change-log rows it owns and its own sampler: no peer holds a pointer into a rank's table or
+    # change log (the group shares only the four batch-sized regions of _SHARED), so nothing is exchanged.
+    def _grow_capacity(self, row_cap: int):
+        with torch.cuda.device(self.dev):
+            cur = torch.empty((row_cap, self.d), dtype=torch.float32, device=self.dev)
+            ws = self._new_ws(row_cap)
+            cur[:self.V1].copy_(self.cur[:self.V1])
+            self.changelog.grow_capacity(row_cap)
+        self.cur, self.ws, self.row_cap = cur, ws, int(row_cap)
+        self.desc.cur, self.desc.row_cap = cur.data_ptr(), self.row_cap
+        if self.grp is not None:
+            self.grp.table[self.rank] = cur.data_ptr()
+
+    def _default_event_cap(self, V1: int) -> int:
+        G = self.G
+        return min((V1 + G - 1) // G, 2 * (2 * self.B * (self.K + 1) + 2) // G + 1024)
+
+    def _check_event_capacity(self, V1: int):
+        """As ChangeLogStream's: the default event capacity (the same on every rank: the inbox blocks are laid out by it, so it
+        cannot grow) covers max_nodes, else the row capacity the rank was built with."""
+        if self._cap_arg is None and self.cap < self._default_event_cap(V1):
+            raise ValueError(f"PeerRank: {V1} nodes need an event capacity of {self._default_event_cap(V1)} rows per step and rank, the "
+                             f"log was sized for {self.cap}; build the ranks with max_nodes (or event_capacity) covering their growth")
+
+    def _init_rows(self, v0: int, v1: int, rows: torch.Tensor, stride: int):
+        _lib.check(self._libc.lstep_pe_rows_init(_lib.ptr(self.cur), None, self.T, self.d, _lib.ptr(self.changelog.base), self.G, self.rank,
+                                                 v0, v1, _lib.ptr(rows), stride, _lib.stream_ptr()), "lstep_pe_rows_init")
+
+    def _set_live(self, V1: int):
+        self.changelog.add_rows(V1)
+        self.V1 = self.desc.V1 = int(V1)
+        self.rows_local = self.changelog.rows
 
     # ---- group wiring ---------------------------------------------------------------------------------------------------
     _SHARED = ("_mem_rows", "_mem_filt", "_mem_inbox", "_mem_flags")
@@ -349,14 +394,21 @@ class PeerRank(HostFed):
         """(q_off, q_rows): this rank's share of a batch of n edges for the a6 queries (and of step_host's row sums)."""
         return share_of(n, self.G, self.rank)
 
-    def _host_prepare(self, src, dst, times, query_ids, ids=None, ingest=False, edge_id_start=None) -> dict:
-        """Validate a host batch (check_host_batch) and, with ingest, make room for it in this rank's sampler. Nothing is
-        enqueued; a regrow synchronises."""
-        ing = None
+    def _host_prepare(self, src, dst, times, query_ids, ids=None, ingest=False, edge_id_start=None, grow=False, batch_size=None) -> dict:
+        """Validate a host batch (check_host_batch) and, with grow, add the nodes up to its largest id; with ingest, make room
+        for it in this rank's sampler. Nothing is written before the batch is validated; a regrow synchronises."""
+        ing, n_new = None, 0
+        if grow:
+            src, dst, times, qs = host_arrays(src, dst, times, query_ids, "step_host")
+            n_new = self._new_nodes_for([src, dst] + qs) if len(src) else 0
         if ingest:
             samp = self._growable_sampler()
-            ing = (samp.num_rows, samp.last_time, samp.next_edge_id if edge_id_start is None else int(edge_id_start))
-        src, dst, times, qs, ids = check_host_batch(src, dst, times, query_ids, self.V1, self.B, ids, ing)
+            rows = max(samp.num_rows, self.V1 + n_new) if n_new else samp.num_rows
+            ing = (rows, samp.last_time, samp.next_edge_id if edge_id_start is None else int(edge_id_start))
+        src, dst, times, qs, ids = check_host_batch(src, dst, times, query_ids if not grow else qs, self.V1 + n_new,
+                                                    self.B if batch_size is None else batch_size, ids, ing)
+        if n_new:
+            self.add_nodes(n_new, _edges=(src, dst))
         if ingest:
             self.sampler.reserve(src, dst)
         return dict(src=src, dst=dst, times=times, qs=qs, ids=ids, ingest=bool(ingest), eid0=None if ing is None else ing[2])
@@ -397,27 +449,30 @@ class PeerRank(HostFed):
         return self._new_ticket(ticket.value, C, self.share_of(n)[1])
 
     def step_host_async(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None,
-                        ids: np.ndarray = None, out: torch.Tensor = None, ingest: bool = False, edge_id_start: int = None) -> int:
+                        ids: np.ndarray = None, out: torch.Tensor = None, ingest: bool = False, edge_id_start: int = None,
+                        grow: bool = False) -> int:
         """ChangeLogStream.step_host_async for this rank (lstep_pe_step_peer_host): the whole step on a batch of host arrays,
         every rank of the group calling it with the same batch. result(ticket) is this rank's share [C, q_rows] of the per-query
         row sums (share_of(n)); `out` [C, q_rows, d] keeps the share's neighbourhood PEs on the device. ingest=True appends the
         batch to this rank's own growable sampler first. A batch longer than batch_size is rejected before anything is
-        enqueued. edges_done, steps_done, batch_idx and epoch advance as in step."""
-        return self._host_phase(self._host_prepare(src, dst, times, query_ids, ids, ingest, edge_id_start), 7, batch_idx, out)
+        enqueued. edges_done, steps_done, batch_idx and epoch advance as in step. grow=True: as in ChangeLogStream.step_host_async;
+        every rank adds the same nodes."""
+        return self._host_phase(self._host_prepare(src, dst, times, query_ids, ids, ingest, edge_id_start, grow), 7, batch_idx, out)
 
     def step_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None, ids: np.ndarray = None,
-                  ingest: bool = False, edge_id_start: int = None) -> np.ndarray:
+                  ingest: bool = False, edge_id_start: int = None, grow: bool = False) -> np.ndarray:
         """Synchronous form: this rank's share [len(query_ids), q_rows] of the per-query row sums."""
-        return self.result(self.step_host_async(src, dst, times, query_ids, batch_idx, ids, ingest=ingest, edge_id_start=edge_id_start))
+        return self.result(self.step_host_async(src, dst, times, query_ids, batch_idx, ids, ingest=ingest, edge_id_start=edge_id_start,
+                                                grow=grow))
 
     def run_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, ingest: bool = False,
-                 edge_id_start: int = None) -> np.ndarray:
+                 edge_id_start: int = None, grow: bool = False) -> np.ndarray:
         """ChangeLogStream.run_host for this rank: batch b = edges [b*B, (b+1)*B) of the host arrays, the steady-state batches
         in ONE native call (lstep_pe_steps_peer_host), the ones while the log fills one by one. Returns [n_batches, C, B] float32:
         row [b, c, :q_rows] is this rank's share of batch b (share_of), the rest zero. The whole run is validated first, and with
         ingest=True room for all of it is reserved in this rank's sampler before the native call, so that no rank regrows (and
         synchronises) while its peers wait at a barrier; the decision depends on the batches only, so every rank makes the
-        same one."""
+        same one. grow=True: the nodes up to the run's largest id are added first, on every rank alike."""
         assert self.grp is not None, "set_group / connect_ipc first"
         n_total, B, C = len(src), self.B, len(query_ids)
         src, dst, times, qs = host_arrays(src, dst, times, query_ids, "run_host")
@@ -425,14 +480,8 @@ class PeerRank(HostFed):
         res = np.zeros((nb, C, B), dtype=np.float32)
         if n_total == 0:
             return res
-        eid0, ing = None, None
-        if ingest:
-            samp = self._growable_sampler()
-            eid0 = samp.next_edge_id if edge_id_start is None else int(edge_id_start)
-            ing = (samp.num_rows, samp.last_time, eid0)
-        check_host_batch(src, dst, times, qs, self.V1, n_total, None, ing)  # (the whole run: batches of B follow from it)
-        if ingest:
-            self.sampler.reserve(src, dst)
+        hb = self._host_prepare(src, dst, times, qs, None, ingest, edge_id_start, grow, n_total)  # (the whole run: batches of B follow)
+        eid0 = hb["eid0"]
         lo = 0
         pend = []
         while lo < n_total and self.len < self.T:  # while the log fills: per-step calls
@@ -522,10 +571,12 @@ class PeerLocalGroup:
         for rk in ranks:
             rk.set_group(*ptrs)
 
-    def step_host(self, src, dst, times, queries, ingest: bool = False, edge_id_start: int = None, batch_idx: int = None) -> np.ndarray:
+    def step_host(self, src, dst, times, queries, ingest: bool = False, edge_id_start: int = None, batch_idx: int = None,
+                  grow: bool = False) -> np.ndarray:
         """PeerRank.step_host for every rank on the same host batch: validated for all ranks before any rank stages anything,
-        then phases 1, 2 and 4 issued for every rank. Returns the shares concatenated, [C, n]: the single-GPU result."""
-        hbs = [rk._host_prepare(src, dst, times, queries, None, ingest, edge_id_start) for rk in self.ranks]
+        then phases 1, 2 and 4 issued for every rank. Returns the shares concatenated, [C, n]: the single-GPU result. grow=True:
+        every rank adds the nodes up to the batch's largest id first."""
+        hbs = [rk._host_prepare(src, dst, times, queries, None, ingest, edge_id_start, grow) for rk in self.ranks]
         tks = [None] * self.G
         for ph in (1, 2, 4):
             for i, rk in enumerate(self.ranks):

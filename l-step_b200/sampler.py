@@ -41,6 +41,7 @@ _STRATEGIES = ("uniform", "recent", "time_interval_aware")
 # for 12 ms less regrowing; 4 regrows three times as often. Hence 16.
 MIN_SLACK = 16
 _EID_MAX = 0x7FFFFFFF
+NODE_ID_MAX = 0x7FFFFFFE  # largest node id a growing stream accepts: the change log records node ids as int32
 
 
 def check_edges(src, dst, edge_ids, times, num_rows: int, last_time: float = -np.inf):
@@ -95,6 +96,37 @@ def plan_capacity(need: np.ndarray, min_slack: int = MIN_SLACK) -> np.ndarray:
     return need + np.maximum(int(min_slack), need)
 
 
+def tail_entries(spare_rows: int, min_slack: int = MIN_SLACK) -> int:
+    """Entries of padding a regrow leaves past the live rows for rows added later: 2 * min_slack per spare row of capacity
+    (a new row takes need + max(min_slack, need) of them, so this covers spare rows that arrive with up to min_slack
+    entries each)."""
+    return int(spare_rows) * 2 * int(min_slack)
+
+
+def plan_layout(need: np.ndarray, row_cap: int, min_slack: int = MIN_SLACK):
+    """(indptr [row_cap + 1], total) of a regrow with len(need) live rows: row capacities plan_capacity(need), every row
+    at or above the live ones empty at the end of the live rows, and total = that end + tail_entries(spare rows)."""
+    need = np.asarray(need, dtype=np.int64)
+    rows = len(need)
+    indptr = np.zeros(int(row_cap) + 1, dtype=np.int64)
+    np.cumsum(plan_capacity(need, min_slack), out=indptr[1:rows + 1])
+    indptr[rows + 1:] = indptr[rows]
+    return indptr, int(indptr[rows]) + tail_entries(int(row_cap) - rows, min_slack)
+
+
+def rows_fit(num_rows: int, row_cap: int, tail0: int, total: int, new_cap: np.ndarray) -> bool:
+    """Whether len(new_cap) rows with those capacities can be added without a regrow: within the row capacity and inside
+    the tail [tail0, total)."""
+    return num_rows + len(new_cap) <= row_cap and tail0 + int(np.sum(new_cap)) <= total
+
+
+def new_row_need(src: np.ndarray, dst: np.ndarray, num_rows: int, new_rows: int) -> np.ndarray:
+    """Entries the edges (src, dst) give each of the rows [num_rows, num_rows + new_rows)."""
+    ends = np.concatenate([src, dst])
+    ends = ends[ends >= num_rows] - num_rows
+    return np.bincount(ends, minlength=new_rows)[:new_rows].astype(np.int64)
+
+
 def _dev(device=None) -> torch.device:
     if device is None:
         return torch.device("cuda", torch.cuda.current_device())
@@ -145,13 +177,18 @@ class NeighborSampler:
 
     @classmethod
     def growable(cls, num_rows: int, src=(), dst=(), edge_ids=(), times=(), sample_neighbor_strategy="recent",
-                 time_scaling_factor=0.0, seed=None, device=None, min_slack: int = MIN_SLACK):
+                 time_scaling_factor=0.0, seed=None, device=None, min_slack: int = MIN_SLACK, row_capacity: int = None):
         """A sampler that grows batch by batch (`ingest`), for a stream whose edges are not known in advance. The optional
         prefix (src, dst, edge_ids, times; times non-decreasing) is built with the exact builder and then laid out with
-        room to grow. Node ids must lie in [0, num_rows). Lookups equal those of from_edges on the edges ingested so far."""
+        room to grow. Node ids must lie in [0, num_rows). Lookups equal those of from_edges on the edges ingested so far.
+        `row_capacity` (default num_rows): rows allocated, so that add_rows can make up to row_capacity - num_rows more
+        rows live without a regrow (each spare row reserves tail_entries(1, min_slack) entries)."""
         num_rows = int(num_rows)
         if num_rows <= 0:
             raise ValueError("growable: num_rows must be positive")
+        row_cap = num_rows if row_capacity is None else int(row_capacity)
+        if row_cap < num_rows or row_cap > NODE_ID_MAX + 1:
+            raise ValueError(f"growable: row_capacity must lie in [num_rows, 2^31 - 1] (got {row_cap})")
         src, dst, eid, t = check_edges(src, dst, edge_ids, times, num_rows)
         self = cls.from_edges(src, dst, eid, t, sample_neighbor_strategy, time_scaling_factor, seed, device, num_rows=num_rows)
         self.min_slack = int(min_slack)
@@ -162,6 +199,7 @@ class NeighborSampler:
         self._last_t = float(t[-1]) if len(t) else -np.inf
         self._next_eid = int(eid[-1]) + 1 if len(eid) else 1
         self.regrows = 0
+        self.row_cap = row_cap
         self._regrow(self._fill_h)
         self.regrows = 0  # regrows after construction
         return self
@@ -190,12 +228,13 @@ class NeighborSampler:
             raise ValueError("this NeighborSampler holds an exact CSR; build one with NeighborSampler.growable(...) to ingest edges")
 
     def _regrow(self, need: np.ndarray):
-        """Lay the CSR out again with capacity plan_capacity(need) per row. Synchronises the device once (appends may
-        still be in flight on other streams, and the old arrays are released afterwards)."""
-        cap = plan_capacity(need, self.min_slack)
-        indptr_h = np.zeros(self.num_rows + 1, dtype=np.int64)
-        np.cumsum(cap, out=indptr_h[1:])
-        total = int(indptr_h[-1])
+        """Lay the CSR out again with capacity plan_capacity(need) per row for len(need) >= num_rows live rows (the rows
+        above num_rows become live, empty), and a padded tail for the rest of the row capacity, which doubles when the
+        rows outgrow it. Synchronises the device once (appends may still be in flight on other streams, and the old arrays
+        are released afterwards). Every new array is allocated before any state changes."""
+        new_rows = len(need)
+        row_cap = self.row_cap if new_rows <= self.row_cap else max(2 * self.row_cap, new_rows)
+        indptr_h, total = plan_layout(need, row_cap, self.min_slack)
         if total > _EID_MAX:  # the kernels index entries with int64 but the builder's limit is kept for the whole CSR
             raise _lib.LstepError(f"growable CSR: {total} entries of capacity exceed 2^31")
         dev = self.device
@@ -204,16 +243,60 @@ class NeighborSampler:
         nbr = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
         eid = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
         t = torch.empty(max(total, 1), dtype=torch.float64, device=dev)
-        fill = torch.empty(self.num_rows, dtype=torch.int32, device=dev)
+        fill = torch.empty(row_cap, dtype=torch.int32, device=dev)
         with torch.cuda.device(dev):
-            rc = self._lib.lstep_csr_relayout(self.csr_ref, _lib.ptr(self.fill), _lib.ptr(indptr), _lib.ptr(nbr), _lib.ptr(eid),
-                                              _lib.ptr(t), _lib.ptr(fill), _lib.ptr(self._err), _lib.stream_ptr())
-        _lib.check(rc, "lstep_csr_relayout")
-        self._set_csr(indptr, nbr[:total], eid[:total], t[:total])
+            rc = self._lib.lstep_csr_relayout_rows(self.csr_ref, _lib.ptr(self.fill), new_rows, row_cap, _lib.ptr(indptr), total,
+                                                   _lib.ptr(nbr), _lib.ptr(eid), _lib.ptr(t), _lib.ptr(fill), _lib.ptr(self._err),
+                                                   _lib.stream_ptr())
+        _lib.check(rc, "lstep_csr_relayout_rows")
+        self._set_csr(indptr, nbr[:total], eid[:total], t[:total], num_rows=new_rows)
         self.fill = fill
-        self._cap_h = cap
+        self.row_cap = row_cap
+        # host mirrors of fill and the row capacities, allocated for row_cap rows so that add_rows only writes the new rows
+        self._fill_buf = np.zeros(row_cap, np.int64)
+        self._fill_buf[:len(self._fill_h)] = self._fill_h
+        self._cap_buf = np.zeros(row_cap, np.int64)
+        self._cap_buf[:new_rows] = plan_capacity(need, self.min_slack)
+        self._fill_h, self._cap_h = self._fill_buf[:new_rows], self._cap_buf[:new_rows]
+        self._tail0 = int(indptr_h[new_rows])
         self.regrows += 1
         self._version += 1
+
+    def add_rows(self, n: int, need=None) -> int:
+        """Make n more rows (node ids num_rows .. num_rows + n - 1) live, empty, and return the first new id. `need`: entries
+        each new row is about to receive (e.g. from the batch that introduces it), so that row gets need + max(min_slack,
+        need) entries of room. Within the row capacity and the padded tail this moves no entry and enqueues one small
+        kernel on the current stream (lstep_csr_add_rows: the new rows' indptr and fill), ordered after lookups already
+        enqueued, which never read these rows (a host-fed stream's next append waits for it); otherwise it regrows (one device synchronisation) with the row capacity
+        doubled. Raises ValueError on an exact sampler."""
+        self._require_growable()
+        n = int(n)
+        r0 = self.num_rows
+        if n < 0:
+            raise ValueError("add_rows: n must be >= 0")
+        if r0 + n > NODE_ID_MAX + 1:
+            raise IndexError(f"add_rows: node ids up to {r0 + n - 1} exceed the int32 node id limit ({NODE_ID_MAX})")
+        need = np.zeros(n, np.int64) if need is None else np.ascontiguousarray(need, dtype=np.int64)
+        if len(need) != n or (n and int(need.min()) < 0):
+            raise ValueError("add_rows: need must hold one count >= 0 per new row")
+        if n == 0:
+            return r0
+        cap = plan_capacity(need, self.min_slack)
+        if not rows_fit(r0, self.row_cap, self._tail0, self.nnz, cap):
+            self._regrow(np.concatenate([self._fill_h, need]))
+            return r0
+        dev = self.device
+        cap_d = torch.from_numpy(cap).pin_memory().to(dev, non_blocking=True)
+        with torch.cuda.device(dev):
+            rc = self._lib.lstep_csr_add_rows(self.csr_ref, _lib.ptr(self.fill), n, _lib.ptr(cap_d), _lib.stream_ptr())
+        _lib.check(rc, "lstep_csr_add_rows")
+        self.num_rows = int(self.csr.num_rows)
+        self._cap_buf[r0:r0 + n] = cap
+        self._fill_buf[r0:r0 + n] = 0
+        self._fill_h, self._cap_h = self._fill_buf[:r0 + n], self._cap_buf[:r0 + n]
+        self._tail0 += int(cap.sum())
+        self._version += 1  # a host-fed stepper re-arms, so its next append (on its copy-in stream) waits for these rows
+        return r0
 
     def reserve(self, src, dst):
         """Make room for the entries the edges (src, dst) will add (known future endpoints, e.g. a whole split). Regrows
@@ -244,11 +327,11 @@ class NeighborSampler:
         times[i]) before failing: synchronise, take fill from the device, and count the edges that landed (appends are
         whole batches, in order). The version bump makes a host-fed stream re-arm its stepper from this state."""
         torch.cuda.synchronize(self.device)
-        fill = self.fill.cpu().numpy().astype(np.int64)
+        fill = self.fill[:self.num_rows].cpu().numpy().astype(np.int64)
         landed = int(fill.sum() - self._n_entries) // 2
         if landed > 0:
             self._note_ingested(src[:landed], dst[:landed], eid0 + landed - 1, times[landed - 1])
-        self._fill_h = fill
+        self._fill_h[:] = fill
         self._version += 1
 
     def ingest(self, src, dst, edge_ids, times):
@@ -305,11 +388,12 @@ class NeighborSampler:
         del ws
         self._set_csr(indptr, nbr[:n_entries], eid[:n_entries], t[:n_entries])
 
-    def _set_csr(self, *tensors):
+    def _set_csr(self, *tensors, num_rows: int = None):
+        """Adopt CSR arrays; num_rows: live rows when indptr holds more (a growable CSR's row capacity)."""
         if not tensors:
             return
         self.indptr, self.nbr, self.eid, self.t = tensors
-        self.num_rows = int(self.indptr.shape[0] - 1)
+        self.num_rows = int(self.indptr.shape[0] - 1) if num_rows is None else int(num_rows)
         self.nnz = int(self.nbr.shape[0])
         self.csr = _lib.CSR(self.indptr.data_ptr(), self.nbr.data_ptr(), self.eid.data_ptr(), self.t.data_ptr(), self.num_rows,
                             self.nnz)

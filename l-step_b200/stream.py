@@ -39,7 +39,10 @@ _I64 = np.dtype(np.int64)
 class PEStream(HostFed):
     def __init__(self, model: LSTEP, src_node_ids: np.ndarray, dst_node_ids: np.ndarray, node_interact_times: np.ndarray,
                  batch_size: int, num_neighbors: int = 20, initial_pe: torch.Tensor = None, history: torch.Tensor = None,
-                 start: int = 0, stop: int = None):
+                 start: int = 0, stop: int = None, row_capacity: int = None, new_node_pe=None, max_nodes: int = None):
+        """row_capacity: rows to allocate for the table and the history (default: the initial V1), so that add_nodes /
+        grow=True add nodes without reallocating until it runs out (then it doubles). new_node_pe: the row [d] a node added
+        by a count or by grow=True starts with (default zeros). max_nodes: optional limit on the node count."""
         self.model = model
         self.K = int(num_neighbors)
         self.B = int(batch_size)
@@ -72,6 +75,8 @@ class PEStream(HostFed):
         self.num_batches = len(self.batch_lo)
         self.batch_tmax = [float(self.t_np[lo:min(lo + self.B, self.stop)].max()) for lo in self.batch_lo]
         self._host_init()
+        self._growth_init(new_node_pe, max_nodes)
+        self._row_cap_arg = row_capacity
         self.V1 = None
         self.batch_idx = 0
         if history is not None:
@@ -100,17 +105,18 @@ class PEStream(HostFed):
             if samp is not None and samp.num_rows > V1:
                 raise IndexError(f"pe has {V1} rows but the sampler knows node ids up to {samp.num_rows - 1}")
         self.V1 = V1
-        self.ring = torch.zeros((V1, self.T, d), dtype=torch.float32, device=self.dev)  # node-major: 68.8 KB / node
-        self.ring[:, :Th, :] = history
+        self.row_cap = max(V1, int(self._row_cap_arg or 0))
+        self.ring = torch.zeros((self.row_cap, self.T, d), dtype=torch.float32, device=self.dev)  # node-major: 68.8 KB / node
+        self.ring[:V1, :Th, :] = history
         self.len = Th  # number of valid steps
         self.head = 0  # slot of the oldest valid step
-        self.cur = torch.empty((V1, d), dtype=torch.float32, device=self.dev)
+        self.cur = torch.empty((self.row_cap, d), dtype=torch.float32, device=self.dev)
         lib = _lib.load()
         with torch.cuda.device(self.dev):
             _lib.check(lib.lstep_ring_load(_lib.ptr(self.ring), _lib.ptr(self.cur), V1, self.T, d, self._last_slot(),
                                            _lib.stream_ptr()), "lstep_ring_load")
         self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.t.data_ptr(), self.ring.data_ptr(),
-                                      self.cur.data_ptr(), V1, self.T, d)
+                                      self.cur.data_ptr(), V1, self.T, d, self.row_cap)
         self._ws = None
         self._ws_cap = (0, 0, 0)
         self.steps_done = 0
@@ -127,7 +133,7 @@ class PEStream(HostFed):
         """The history in the reference's layout [V1, Th, d], oldest first (for save_pe / torch.cat)."""
         self.check_errors()
         idx = (self.head + torch.arange(self.len, device=self.dev)) % self.T
-        return self.ring.index_select(1, idx).contiguous()
+        return self.ring[:self.V1].index_select(1, idx).contiguous()
 
     def _last_slot(self) -> int:
         return (self.head + self.len - 1) % self.T
@@ -141,13 +147,13 @@ class PEStream(HostFed):
     def _workspace(self, n_ids, n_edges, C):
         lib = _lib.load()
         m = self.model
-        need = lib.lstep_pe_step_workspace_bytes(n_ids, n_edges, C, self.K, self.d, m.time_feat_dim, self.V1)
+        need = lib.lstep_pe_step_workspace_bytes(n_ids, n_edges, C, self.K, self.d, m.time_feat_dim, self.row_cap)
         if self._ws is None or self._ws.numel() < need:
             self._ws_cap = (max(2 * self.B, n_ids), max(self.B, n_edges), max(C, 4))  # (ids, edges, query sets) it is sized for
             cap = lib.lstep_pe_step_workspace_bytes(self._ws_cap[0], self._ws_cap[1], self._ws_cap[2], self.K, self.d,
-                                                    m.time_feat_dim, self.V1)
+                                                    m.time_feat_dim, self.row_cap)
             self._ws = torch.empty(max(cap, need) + 4096, dtype=torch.uint8, device=self.dev)
-            _lib.check(lib.lstep_update_pe_workspace_init(_lib.ptr(self._ws), self._ws.numel(), self.V1, _lib.stream_ptr()),
+            _lib.check(lib.lstep_update_pe_workspace_init(_lib.ptr(self._ws), self._ws.numel(), self.row_cap, _lib.stream_ptr()),
                        "workspace_init")
         return self._ws
 
@@ -246,12 +252,30 @@ class PEStream(HostFed):
         n_last = int(ne[-1])
         return buf.view(-1)[:max(C, 1) * n_last * d].view(max(C, 1), n_last, d)
 
+    # ---- node growth (add_nodes and grow=True: hostfeed.HostFed) --------------------------------------------------------
+    def _grow_capacity(self, row_cap: int):
+        ring = torch.zeros((row_cap, self.T, self.d), dtype=torch.float32, device=self.dev)
+        cur = torch.empty((row_cap, self.d), dtype=torch.float32, device=self.dev)
+        ring[:self.V1].copy_(self.ring[:self.V1])
+        cur[:self.V1].copy_(self.cur[:self.V1])
+        self.ring, self.cur, self.row_cap = ring, cur, int(row_cap)
+        self.desc.ring, self.desc.cur, self.desc.row_cap = ring.data_ptr(), cur.data_ptr(), self.row_cap
+        self._ws = None  # its per-node maps cover row_cap rows: reallocated (and zeroed) by the next step
+
+    def _init_rows(self, v0: int, v1: int, rows: torch.Tensor, stride: int):
+        _lib.check(self._libc.lstep_pe_rows_init(_lib.ptr(self.cur), _lib.ptr(self.ring), self.T, self.d, None, 1, 0, v0, v1, _lib.ptr(rows),
+                                                 stride, _lib.stream_ptr()), "lstep_pe_rows_init")
+
+    def _set_live(self, V1: int):
+        self.V1 = self.desc.V1 = int(V1)
+
     # ---- host-fed steps (native stager: csrc/host_step.cu; stepper, ingest and tickets: hostfeed.HostFed) -----------
     def _host_sampler(self):
         return self.model.neighbor_sampler
 
     def step_host_async(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None,
-                        ids: np.ndarray = None, out: torch.Tensor = None, ingest: bool = False, edge_id_start: int = None) -> int:
+                        ids: np.ndarray = None, out: torch.Tensor = None, ingest: bool = False, edge_id_start: int = None,
+                        grow: bool = False) -> int:
         """One step fed from HOST arrays (what a loop holding numpy batches calls): the batch's endpoints,
         times and the query id sets are packed into a pinned slot and uploaded by one async copy inside the
         native call, the step's kernels are enqueued behind it, and the per-query row sums [C, n] of the
@@ -262,15 +286,20 @@ class PEStream(HostFed):
         call (≈ 25 µs of interpreter time per step).
         ingest=True: the batch's edges are not in the sampler yet. The model's sampler must be growable
         (NeighborSampler.growable); the batch is validated, room is reserved, and the native call appends it to the CSR
-        (edge ids edge_id_start + i, default: the sampler's next_edge_id) before the step's lookups run."""
+        (edge ids edge_id_start + i, default: the sampler's next_edge_id) before the step's lookups run.
+        grow=True: ids above the last live one (in the batch or the query sets) are new nodes, added first (add_nodes, with
+        the stream's new_node_pe row); without it such an id raises IndexError, as an unknown node does in the reference."""
         m = self.model
         n = len(src)
         C = len(query_ids)
         src, dst, times, qs = host_arrays(src, dst, times, query_ids, "step_host")
         if ids is not None:
             ids = np.ascontiguousarray(ids, dtype=_I64)
+        n_new = self._new_nodes_for([src, dst] + qs) if grow and n else 0
         if ingest:
-            eid0 = self._check_ingest(src, dst, times, edge_id_start)
+            eid0 = self._check_ingest(src, dst, times, edge_id_start, n_new)
+        elif n_new:
+            self.add_nodes(n_new)
         bi = self.batch_idx if batch_idx is None else batch_idx
         if torch.cuda.current_device() != self.dev.index:
             torch.cuda.set_device(self.dev)
@@ -297,16 +326,21 @@ class PEStream(HostFed):
         return tk
 
     def run_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, ingest: bool = False,
-                 edge_id_start: int = None) -> np.ndarray:
+                 edge_id_start: int = None, grow: bool = False) -> np.ndarray:
         """A run of consecutive batches fed from HOST arrays in ONE native call (an evaluation split): batch b is edges
         [b*B, (b+1)*B) of the given arrays; every step copies its own inputs in and its own per-query row sums out
         (read one step behind inside the call). Returns [n_batches, C, B] float32 (tail of a ragged last batch zero).
         While the history ring is still filling (the filter changes with every step) the batches go through
         step_host_async one by one. ingest=True: as in step_host_async; room for the whole run is reserved first, so the
-        native loop never needs a regrow."""
+        native loop never needs a regrow. grow=True: the nodes up to the run's largest id are added (add_nodes) before its
+        first step, so the native loop never grows either; a node's rows are then in place before its first edge, which
+        changes nothing (they are the rows of a node no edge has touched)."""
         n_total, B, C = len(src), self.B, len(query_ids)
         src, dst, times, qs = host_arrays(src, dst, times, query_ids, "run_host")
-        eid0 = self._check_ingest(src, dst, times, edge_id_start) if ingest else None
+        n_new = self._new_nodes_for([src, dst] + qs) if grow and n_total else 0
+        eid0 = self._check_ingest(src, dst, times, edge_id_start, n_new) if ingest else None
+        if n_new and not ingest:
+            self.add_nodes(n_new)
         nb = (n_total + B - 1) // B
         res = np.zeros((nb, C, B), dtype=np.float32)
         lo = 0
@@ -368,9 +402,10 @@ class PEStream(HostFed):
                                               torch.cuda.current_stream().cuda_stream, sub.ctypes.data, C_byref(done))
 
     def step_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None, ids: np.ndarray = None,
-                  ingest: bool = False, edge_id_start: int = None):
+                  ingest: bool = False, edge_id_start: int = None, grow: bool = False):
         """Synchronous form: run the step and return its per-query row sums [len(query_ids), n]."""
-        return self.result(self.step_host_async(src, dst, times, query_ids, batch_idx, ids, ingest=ingest, edge_id_start=edge_id_start))
+        return self.result(self.step_host_async(src, dst, times, query_ids, batch_idx, ids, ingest=ingest, edge_id_start=edge_id_start,
+                                                grow=grow))
 
 
 class ChangeLogStream(PEStream):
@@ -429,20 +464,48 @@ class ChangeLogStream(PEStream):
             samp = self.model.neighbor_sampler
             if samp is not None and (hi_id >= samp.num_rows or samp.num_rows > V1):
                 raise IndexError("list index out of range: the neighbor sampler's rows do not cover the stream / exceed the table")
-        cap = self._cap_arg if self._cap_arg is not None else min(V1, 2 * self.B * (self.K + 1) + 2)
-        self.changelog = ChangeLogHistory(V1, self.T, d, cap, 1, 0, self.dev)
+        self.row_cap = max(V1, int(self._row_cap_arg or 0))
+        cap = self._cap_arg if self._cap_arg is not None else self._default_event_cap(max(self.row_cap, self.max_nodes or 0))
+        self.changelog = ChangeLogHistory(V1, self.T, d, cap, 1, 0, self.dev, self.row_cap)
         self.cap = self.changelog.cap
         self.V1 = V1
         self.ring = None
-        self.cur = torch.empty((V1, d), dtype=torch.float32, device=self.dev)
+        self.cur = torch.empty((self.row_cap, d), dtype=torch.float32, device=self.dev)
         self.head, self.len = self.changelog.load(hist, self.cur)
-        self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.t.data_ptr(), None, self.cur.data_ptr(), V1, self.T, d)
+        self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.t.data_ptr(), None, self.cur.data_ptr(), V1, self.T, d,
+                                      self.row_cap)
         self._ws = None
         self._ws_cap = (0, 0, 0)
 
     def history_bytes(self) -> int:
         """Bytes the history occupies (base + event rows + index structures) — against V1 * T * d * 4 for the dense ring."""
         return self.changelog.nbytes()
+
+    def _default_event_cap(self, V1: int) -> int:
+        return min(V1, 2 * self.B * (self.K + 1) + 2)  # every row a batch can touch, at most every node
+
+    def _check_event_capacity(self, V1: int):
+        """The default event capacity is sized for the nodes the stream may hold (max_nodes, else its row capacity): growing
+        beyond what it covers raises ValueError before any write (a step could change more rows than the log records)."""
+        if self._cap_arg is None and self.cap < self._default_event_cap(V1):
+            raise ValueError(f"ChangeLogStream: {V1} nodes need an event capacity of {self._default_event_cap(V1)} rows per step, the "
+                             f"log was sized for {self.cap}; build the stream with max_nodes (or event_capacity) covering its growth")
+
+    def _grow_capacity(self, row_cap: int):
+        cur = torch.empty((row_cap, self.d), dtype=torch.float32, device=self.dev)
+        cur[:self.V1].copy_(self.cur[:self.V1])
+        self.changelog.grow_capacity(row_cap)
+        self.cur, self.row_cap = cur, int(row_cap)
+        self.desc.cur, self.desc.row_cap = cur.data_ptr(), self.row_cap
+        self._ws = None
+
+    def _init_rows(self, v0: int, v1: int, rows: torch.Tensor, stride: int):
+        _lib.check(self._libc.lstep_pe_rows_init(_lib.ptr(self.cur), None, self.T, self.d, _lib.ptr(self.changelog.base), 1, 0, v0, v1,
+                                                 _lib.ptr(rows), stride, _lib.stream_ptr()), "lstep_pe_rows_init")
+
+    def _set_live(self, V1: int):
+        self.changelog.add_rows(V1)
+        super()._set_live(V1)
 
     def export_history(self) -> torch.Tensor:
         """The dense layout [V1, len, d] (oldest first) replayed from the log (tests / save_pe; needs V1 * len * d * 4 bytes)."""
