@@ -19,12 +19,11 @@ def filter_len(batch_idx: int, length: int, T: int) -> int:
     return min(max(batch_idx, 0), T) if length < T else T
 
 
-def advance(head: int, length: int, T: int):
-    """(slot, head, len) of a step on a window of T slots: the slot it writes, and the window after it. The window fills,
-    then each step overwrites its oldest slot."""
-    if length < T:
-        return (head + length) % T, head, length + 1
-    return head, (head + 1) % T, T
+def advance(head: int, length: int, T: int, steps: int = 1):
+    """(slot, head, len) of `steps` steps on a window of T slots: the slot the first of them writes, and the window after
+    them. The window fills, then each step overwrites its oldest slot."""
+    fill = steps if steps < T - length else T - length
+    return (head + length) % T, (head + steps - fill) % T, length + fill
 
 
 def _to_dev(a, dev, dtype):

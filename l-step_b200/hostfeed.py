@@ -1,11 +1,14 @@
 """Host-fed steps: the Python side every history layout shares (PEStream, ChangeLogStream, PeerRank).
 
 A host-fed step hands one batch of HOST (numpy) arrays to a native stepper (csrc/host_step.cu), which packs it into a pinned
-slot, copies it in, runs the step and copies the per-query row sums back, and returns a ticket. `HostFed` owns that stepper and
-what surrounds the native call: the normalisation of the host arrays, the validation and room-making of a batch that is ingested
-into a growable sampler (ingest=True), the arming of the stepper for it, the ticket bookkeeping and `result`, and the resync of
-the sampler after a failed call. A class that mixes it in provides `dev`, `B`, `d` and `_host_sampler()`, the sampler whose CSR
-its steps read.
+slot, copies it in, runs the step and copies the per-query row sums back, and returns a ticket. `HostFed` owns the driver:
+step_host_async, step_host, run_host and `result`. A step has two halves: `_host_prepare` validates a batch (or a whole run),
+adds the nodes of grow=True and reserves room for ingest=True, writing nothing before all of it has passed; `_host_phase`
+issues phases of the step on the prepared batch (all at once, 7, except PeerLocalGroup's 1, 2 and 4 per rank) and moves the
+window and the counters (`_advance`). A class that mixes it in provides `dev`, `B`, `d`, `T`, `model`, the window `head` /
+`len`, the counters `batch_idx` / `steps_done` / `edges_done`, and what differs between layouts: `_host_sampler()`, the
+sampler its steps read; `_check_host(...)`, its own checks of a batch; `_host_step_call` and `_host_run_call`, the native
+per-step and multi-batch calls; `_host_rows(n)`, the rows per query of a result; `_workspace(n_ids, n_edges, C)`.
 
 It also owns the growth of the node set (add_nodes, and grow=True on the host-fed steps): new node ids continue after the
 last live one, and a new node starts with its initial row r0 in the table, in every history slot and as its change-log base
@@ -21,6 +24,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .changelog import advance, filter_len
 from .sampler import NODE_ID_MAX, check_edges, new_row_need
 
 C_void_p = ctypes.c_void_p
@@ -39,7 +43,7 @@ def host_arrays(src, dst, times, query_ids, what: str):
     if times.dtype != _F64 or not times.flags.c_contiguous:
         times = np.ascontiguousarray(times, dtype=_F64)
     qs = [q if (q.dtype == _I64 and q.flags.c_contiguous) else np.ascontiguousarray(q, dtype=_I64) for q in query_ids]
-    if len(dst) != n or len(times) != n or any(len(q) != n for q in qs):
+    if len(dst) != n or len(times) != n or [q for q in qs if len(q) != n]:  # (no generator: this runs once per host-fed step)
         raise ValueError(f"{what}: src, dst, times and every query set must have the same length")
     return src, dst, times, qs
 
@@ -48,18 +52,18 @@ class HostFed:
     HOST_SLOTS = 4  # steps that may be in flight before step_host_async blocks on the oldest
 
     def _host_init(self):
+        self.lib = _lib.load()
         self._host_stepper = None
-        self._armed = None  # (stepper, sampler, sampler version) the stepper was armed to ingest into, see _arm_ingest
+        self._armed = None  # (stepper, sampler, sampler version) the stepper was armed to ingest into, see _set_ingest
         self._ticket_shape = {}
         self._drained = {}  # public ticket -> result read out before its stepper was replaced
         self._epoch = 0
-        self._libc = _lib.load()
 
     def _host_sampler(self):
         raise NotImplementedError
 
     def _stepper(self, n_edges: int, C: int):
-        lib = _lib.load()
+        lib = self.lib
         st = self._host_stepper
         if st is None or st[1] < n_edges or st[2] < C:
             if st is not None:
@@ -80,12 +84,6 @@ class HostFed:
             with torch.cuda.device(self.dev):
                 _lib.check(lib.lstep_host_stepper_create(self.HOST_SLOTS, cap_e, cap_c, self.d, C_byref(h)), "lstep_host_stepper_create")
             self._host_stepper = st = (h, cap_e, cap_c)
-        return st[0]
-
-    def _host_stepper_for(self, n_edges: int, C: int):
-        st = self._host_stepper
-        if st is None or st[1] < n_edges or st[2] < C:
-            return self._stepper(n_edges, C)
         return st[0]
 
     def __del__(self):
@@ -181,46 +179,167 @@ class HostFed:
             raise ValueError("ingest=True needs a growable neighbor sampler: model.set_neighbor_sampler(NeighborSampler.growable(...))")
         return samp
 
-    def _check_ingest(self, src, dst, times, edge_id_start, n_new: int = 0):
-        """Validate a host batch for ingestion (its ids against the rows it will have after n_new nodes are added), add
-        those nodes and make room for it; returns its first edge id. Nothing is written to the device before the batch is
-        validated."""
-        samp = self._growable_sampler()
-        eid0 = samp.next_edge_id if edge_id_start is None else int(edge_id_start)
-        check_edges(src, dst, eid0, times, max(samp.num_rows, self.V1 + n_new) if n_new else samp.num_rows, samp.last_time)
-        if n_new:
-            self.add_nodes(n_new, _edges=(src, dst))
-        samp.reserve(src, dst)
-        return eid0
-
-    def _arm_ingest(self, h, eid0: int):
-        """Arm the stepper to append each batch to the sampler's CSR before its step (lstep_host_stepper_set_ingest). Re-armed
-        only when the stepper, the sampler or its arrays changed, or edge ids do not continue: arming makes the next append
-        wait for the compute stream, which costs the copy-in its overlap with the previous step."""
+    def _set_ingest(self, h, eid0):
+        """Arm the stepper to append each batch to the sampler's CSR before its step, with edge ids from eid0 on
+        (lstep_host_stepper_set_ingest), or disarm it (eid0 None). Re-armed only when the stepper, the sampler or its arrays
+        changed, or edge ids do not continue: arming makes the next append wait for the compute stream, which costs the
+        copy-in its overlap with the previous step."""
+        if eid0 is None:
+            if self._armed is not None:
+                _lib.check(self.lib.lstep_host_stepper_set_ingest(h, None, 0, 0.0), "lstep_host_stepper_set_ingest")
+                self._armed = None
+            return
         samp = self._host_sampler()
         key = (h.value, id(samp), samp._version)
         if self._armed != key or eid0 != samp.next_edge_id:
-            _lib.check(self._libc.lstep_host_stepper_set_ingest(h, _lib.ptr(samp.fill), eid0, samp.last_time),
+            _lib.check(self.lib.lstep_host_stepper_set_ingest(h, _lib.ptr(samp.fill), eid0, samp.last_time),
                        "lstep_host_stepper_set_ingest")
             self._armed = key
 
-    def _disarm_ingest(self, h):
-        if self._armed is not None:
-            _lib.check(self._libc.lstep_host_stepper_set_ingest(h, None, 0, 0.0), "lstep_host_stepper_set_ingest")
-            self._armed = None
+    # ---- the host-fed step --------------------------------------------------------------------------------------------
+    def step_host_async(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None,
+                        ids: np.ndarray = None, out: torch.Tensor = None, ingest: bool = False, edge_id_start: int = None,
+                        grow: bool = False) -> int:
+        """One step fed from HOST arrays (what a loop holding numpy batches calls): the batch's endpoints, times and the query
+        id sets are packed into a pinned slot and uploaded by one async copy inside the native call, the step's kernels are
+        enqueued behind it, and the per-query row sums of the neighbourhood PEs are copied back to a pinned result slot.
+        Returns a ticket at once (nothing synchronises); `result(ticket)` waits for that step only, so a loop can read results
+        one step behind. The result is [C, n], or on a PeerRank this rank's share [C, q_rows] (share_of(n)), every rank of the
+        group calling it with the same batch. `ids` (sorted unique batch nodes) is computed natively when omitted; `out`
+        [C, rows, d] keeps the full neighbourhood PEs on the device. This is the per-batch host path: it avoids every
+        avoidable Python call (≈ 25 µs of interpreter time per step).
+        A batch is validated before anything is enqueued; on a change-log history (ChangeLogStream, PeerRank) a batch longer
+        than batch_size is rejected, since batch_size sizes the log's event capacity.
+        ingest=True: the batch's edges are not in the sampler yet. The sampler must be growable (NeighborSampler.growable; a
+        PeerRank's own one); room is reserved, and the native call appends the batch to the CSR (edge ids edge_id_start + i,
+        default: the sampler's next_edge_id) before the step's lookups run.
+        grow=True: ids above the last live one (in the batch or the query sets) are new nodes, added first (add_nodes, with
+        the new_node_pe row); without it such an id raises IndexError, as an unknown node does in the reference.
+        head / len, batch_idx, steps_done and edges_done (and a PeerRank's epoch) advance as in a resident step."""
+        return self._host_phase(self._host_prepare(src, dst, times, query_ids, ids, ingest, edge_id_start, grow), 7, batch_idx, out)
 
-    def _set_ingest(self, h, ingest: bool, eid0):
-        if ingest:
-            self._arm_ingest(h, eid0)
-        elif self._armed is not None:
-            self._disarm_ingest(h)
+    def step_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None, ids: np.ndarray = None,
+                  ingest: bool = False, edge_id_start: int = None, grow: bool = False) -> np.ndarray:
+        """Synchronous form of step_host_async: the step's per-query row sums [len(query_ids), rows]."""
+        return self.result(self.step_host_async(src, dst, times, query_ids, batch_idx, ids, ingest=ingest, edge_id_start=edge_id_start,
+                                                grow=grow))
 
-    def _host_failed(self, rc: int, what: str, ingest: bool, samp, src, dst, eid0, times):
-        """A native host-fed call returned rc != 0: the append of (a prefix of) the batches may have been enqueued before it
-        failed, so the sampler takes its state from the device; then raise."""
+    def run_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, ingest: bool = False,
+                 edge_id_start: int = None, grow: bool = False) -> np.ndarray:
+        """A run of consecutive batches fed from HOST arrays (an evaluation split): batch b is edges [b*B, (b+1)*B) of the given
+        arrays; every step copies its own inputs in and its own per-query row sums out. Returns [n_batches, C, B] float32: row
+        [b, c, :rows] holds batch b's row sums (a PeerRank's share of them), the rest is zero. While the history is still
+        filling (the filter changes with every step) the batches are stepped one by one; the rest goes in ONE native call,
+        which reads the results one step behind. The whole run is validated first, as step_host_async validates a batch;
+        ingest=True reserves room for all of it first, so the native loop never regrows (on a peer group: no rank synchronises
+        while its peers wait at a barrier), and grow=True adds the nodes up to the run's largest id before its first step,
+        which changes nothing (they are the rows of a node no edge has touched). A batch the native call rejects raises after
+        the batches before it were applied; the host state and the sampler follow the device."""
+        n_total, B, C = len(src), self.B, len(query_ids)
+        res = np.zeros(((n_total + B - 1) // B, C, B), dtype=np.float32)
+        if n_total == 0:
+            host_arrays(src, dst, times, query_ids, "run_host")
+            return res
+        src, dst, times, qs, _, eid0 = self._host_prepare(src, dst, times, query_ids, None, ingest, edge_id_start, grow, n_total)
+        lo, pend = 0, []
+        while lo < n_total and self.len < self.T:  # the history fills: per-step calls (validated above), results one behind
+            hi = min(lo + B, n_total)
+            part = (src[lo:hi], dst[lo:hi], times[lo:hi], [q[lo:hi] for q in qs], None, None if eid0 is None else eid0 + lo)
+            pend.append((lo // B, self._host_phase(part)))
+            if len(pend) > 1:
+                b, tk = pend.pop(0)
+                r = self.result(tk)
+                res[b, :, :r.shape[1]] = r
+            lo = hi
+        for b, tk in pend:
+            r = self.result(tk)
+            res[b, :, :r.shape[1]] = r
+        if lo == n_total:
+            return res
+        if torch.cuda.current_device() != self.dev.index:
+            torch.cuda.set_device(self.dev)
+        h = self._stepper(B, C)
+        eid0 = None if eid0 is None else eid0 + lo
+        self._set_ingest(h, eid0)
+        G = self.model._collapsed_filter(self.T, False)
+        qptrs = (C_void_p * max(C, 1))(*[q[lo:].ctypes.data for q in qs])
+        done = ctypes.c_int64(0)
+        src, dst, times = src[lo:], dst[lo:], times[lo:]
+        rc = self._host_run_call(h, n_total - lo, src, dst, times, qptrs, C, G, self._workspace(2 * B, B, C), res[lo // B:], done)
+        n_app = min(done.value * B, n_total - lo)  # batches applied before an error stay applied
+        self._advance(done.value, n_app, C)
+        if rc != 0:  # (the failed batch's append may have been enqueued although its step was not applied)
+            self._host_failed(rc, "run_host", src, dst, times, eid0)
+        if eid0 is not None and n_app:
+            self._host_sampler()._note_ingested(src[:n_app], dst[:n_app], eid0 + n_app - 1, times[n_app - 1])
+        return res
+
+    def _host_prepare(self, src, dst, times, query_ids, ids=None, ingest=False, edge_id_start=None, grow=False, n_max=None):
+        """First half of a host-fed step: normalise and validate a batch (or a whole run of n_max edges), then, with grow, add
+        the nodes up to its largest id and, with ingest, reserve room for its edges in the sampler. Nothing is written before
+        all of it has passed. Returns the batch for _host_phase: (src, dst, times, query sets, ids, eid0), eid0 its first edge
+        id with ingest, else None."""
+        src, dst, times, qs = host_arrays(src, dst, times, query_ids, "step_host" if n_max is None else "run_host")
+        n_new = self._new_nodes_for([src, dst] + qs) if grow and len(src) else 0
+        samp = self._growable_sampler() if ingest else None
+        ids = self._check_host(src, dst, times, qs, ids, self.V1 + n_new, self.B if n_max is None else n_max)
+        eid0 = None
         if ingest:
-            samp._resync(src, dst, eid0, times)
-        _lib.check(rc, what)
+            eid0 = samp.next_edge_id if edge_id_start is None else int(edge_id_start)
+            check_edges(src, dst, eid0, times, max(samp.num_rows, self.V1 + n_new) if n_new else samp.num_rows, samp.last_time)
+        if n_new:
+            self.add_nodes(n_new, _edges=(src, dst) if ingest else None)
+        if ingest:
+            samp.reserve(src, dst)
+        return src, dst, times, qs, ids, eid0
+
+    def _host_phase(self, batch: tuple, phases: int = 7, batch_idx: int = None, out: torch.Tensor = None):
+        """Second half: issue `phases` of the step on the prepared batch. The call with bit 0 stages the batch (and appends it
+        to the sampler with ingest); the one with bit 2 finishes the step, advances the state and returns the ticket."""
+        src, dst, times, qs, ids, eid0 = batch
+        n, C = len(src), len(qs)
+        if torch.cuda.current_device() != self.dev.index:
+            torch.cuda.set_device(self.dev)
+        if phases & 1:
+            bi = self.batch_idx if batch_idx is None else int(batch_idx)
+            h = self._stepper(n, C)
+            self._set_ingest(h, eid0)
+            G = self.model._collapsed_filter(filter_len(bi, self.len, self.T), False)
+            qptrs = (C_void_p * max(C, 1))(*[q.ctypes.data for q in qs])
+            ws = self._workspace(2 * n if ids is None else len(ids), n, C)
+            if not phases & 4:  # (the later phases reuse them: like the stepper, a rank stages one batch at a time)
+                self._staged = (bi, h, G, qptrs, ws, out)
+        else:
+            bi, h, G, qptrs, ws, out = self._staged
+        ticket = ctypes.c_int64(-1)
+        rc = self._host_step_call(h, n, src, dst, times, ids, G, qptrs, C, out, ws, phases, ticket)
+        if rc != 0:  # (the append may have been enqueued before the step failed)
+            self._host_failed(rc, "step_host", src, dst, times, eid0)
+        if eid0 is not None and phases & 1:  # the append is enqueued with the staging
+            self._host_sampler()._note_ingested(src, dst, eid0 + n - 1, times[-1])
+        if not phases & 4:
+            return None
+        self.batch_idx = bi
+        self._advance(1, n, C)
+        return self._new_ticket(ticket.value, C, self._host_rows(n))
+
+    def _host_failed(self, rc: int, what: str, src, dst, times, eid0):
+        """A native host-fed call returned rc != 0: with ingest the append of (a prefix of) the batches may have been enqueued
+        before it failed, so the sampler takes its state from the device; then raise."""
+        if eid0 is not None:
+            self._host_sampler()._resync(src, dst, eid0, times)
+        _lib.check(rc, f"{type(self).__name__}.{what}")
+
+    def _advance(self, steps: int, edges: int, C: int = None):
+        """Move the window (changelog.advance), batch_idx and the step and edge counters by `steps` steps of `edges` edges.
+        C: host-fed steps with C query sets, which also count what the stepper copied in (src, dst, t, <= 2n batch ids, C
+        query sets)."""
+        _, self.head, self.len = advance(self.head, self.len, self.T, steps)
+        self.batch_idx += steps
+        self.steps_done += steps
+        self.edges_done += edges
+        if C is not None:
+            self.model.h2d_bytes += 8 * edges * (5 + C)
 
     # ---- tickets ------------------------------------------------------------------------------------------------------
     def _new_ticket(self, native: int, C: int, n: int) -> int:
@@ -242,7 +361,7 @@ class HostFed:
     def _result_now(self, ticket: int) -> np.ndarray:
         p = ctypes.POINTER(ctypes.c_float)()
         nf = ctypes.c_int64(0)
-        rc = self._libc.lstep_host_step_result(self._host_stepper[0], ticket & 0xFFFFFFFF, C_byref(p), C_byref(nf))
+        rc = self.lib.lstep_host_step_result(self._host_stepper[0], ticket & 0xFFFFFFFF, C_byref(p), C_byref(nf))
         if rc != 0:
             _lib.check(rc, "lstep_host_step_result")
         C, n = self._ticket_shape[ticket]

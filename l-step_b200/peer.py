@@ -23,7 +23,7 @@ import torch
 
 from . import _lib
 from . import checkpoint as ckpt
-from .changelog import ChangeLogHistory, advance, filter_len
+from .changelog import ChangeLogHistory, filter_len
 from .hostfeed import HostFed, host_arrays
 from .model import LSTEP
 from .sampler import NeighborSampler, check_edges
@@ -142,7 +142,8 @@ class PeerRank(HostFed):
         assert 1 <= world <= 16 and 0 <= rank < world
         if (initial_pe is None) + (history is None) + (checkpoint is None) != 2:
             raise ValueError("PeerRank: give exactly one of initial_pe, history and checkpoint")
-        self.m, self.rank, self.G = model, int(rank), int(world)
+        self._host_init()
+        self.model, self.rank, self.G = model, int(rank), int(world)
         self.dev = dev = torch.device(device) if device is not None else model._dev()
         self.B, self.K, self.T = int(batch_size), int(num_neighbors), model.num_fft_batches
         self.d, self.t_dim = model.pe_dim, model.time_feat_dim
@@ -163,7 +164,7 @@ class PeerRank(HostFed):
                 hist = ckpt.from_dense(history.to(dev, torch.float32), self.T)
         if hist is not None:
             hist.check(V1=self.V1, d=self.d, T=self.T)
-        lib = self.lib = _lib.load()
+        lib = self.lib
         as_dev = lambda a, dt: (torch.zeros(0, dtype=dt, device=dev) if a is None else a.to(dev, dt) if isinstance(a, torch.Tensor) else
                                 torch.from_numpy(np.ascontiguousarray(a)).to(dev, dt))
         T, d = self.T, self.d
@@ -214,7 +215,6 @@ class PeerRank(HostFed):
         self.epoch = ctypes.c_uint32(0)  # (a fresh rank: the flag blocks are zeroed by lstep_ipc_alloc)
         self.grp = None
         self._opened = []
-        self._host_init()
         self._growth_init(new_node_pe, max_nodes)
         if hist is not None:
             self.head, self.len = self.changelog.load(hist, self.cur)
@@ -257,8 +257,8 @@ class PeerRank(HostFed):
                              f"log was sized for {self.cap}; build the ranks with max_nodes (or event_capacity) covering their growth")
 
     def _init_rows(self, v0: int, v1: int, rows: torch.Tensor, stride: int):
-        _lib.check(self._libc.lstep_pe_rows_init(_lib.ptr(self.cur), None, self.T, self.d, _lib.ptr(self.changelog.base), self.G, self.rank,
-                                                 v0, v1, _lib.ptr(rows), stride, _lib.stream_ptr()), "lstep_pe_rows_init")
+        _lib.check(self.lib.lstep_pe_rows_init(_lib.ptr(self.cur), None, self.T, self.d, _lib.ptr(self.changelog.base), self.G, self.rank,
+                                               v0, v1, _lib.ptr(rows), stride, _lib.stream_ptr()), "lstep_pe_rows_init")
 
     def _set_live(self, V1: int):
         self.changelog.add_rows(V1)
@@ -325,14 +325,14 @@ class PeerRank(HostFed):
         """One step on batch b. queries: device int64 tensors with the ids of ALL edges of the batch (this rank reads its
         share). Returns [C, q_rows, d]. phases: see lstep_pe_step_peer (7 = whole step; the state advances with bit 2)."""
         assert self.grp is not None, "set_group / connect_ipc first"
-        lib, T, d = self.lib, self.T, self.d
+        lib, m, T, d = self.lib, self.model, self.T, self.d
         lo, hi = self.batch(b)
         q_off, q_rows = self.share(b)
         C = len(queries)
         i0, i1 = int(self.ids_off[b]), int(self.ids_off[b + 1])
         m0, m1 = int(self.mine_off[b]), int(self.mine_off[b + 1])
         with torch.cuda.device(self.dev), torch.no_grad():
-            Gt = self.m._collapsed_filter(filter_len(self.batch_idx, self.len, T), False)
+            Gt = m._collapsed_filter(filter_len(self.batch_idx, self.len, T), False)
             if out is None:
                 out = torch.empty((max(C, 1), q_rows, d), dtype=torch.float32, device=self.dev)
             qptrs = (ctypes.c_void_p * max(C, 1))(*[q.data_ptr() + 8 * q_off for q in queries])
@@ -340,27 +340,24 @@ class PeerRank(HostFed):
             _lib.check(lib.lstep_pe_step_peer(ctypes.byref(self.desc), self.changelog.ref, self.sampler.csr_ref, ctypes.byref(self.grp), lo, hi - lo,
                                               i64p(self.ids, i0), i1 - i0, i64p(self.ids_mine, m0), i64p(self.pos_mine, m0), m1 - m0,
                                               float(self.tmax[b]), self.head, self.len, _lib.ptr(Gt), qptrs, C, q_off, q_rows, _lib.ptr(out), self.K,
-                                              self.m._mlp_ref("nbr"), self.m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(),
+                                              m._mlp_ref("nbr"), m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(),
                                               _lib.ptr(self.sampler._err), self.epoch.value, self.timeout_ms, phases, _lib.stream_ptr()),
                        "lstep_pe_step_peer")
         if phases & 4:
-            self._advance(1)
-            self.edges_done = hi
+            self._advance(1, hi - lo)
         return out
 
-    def _advance(self, n: int):
-        for _ in range(n):
-            _, self.head, self.len = advance(self.head, self.len, self.T)
-        self.batch_idx += n
-        self.steps_done += n
-        self.epoch = ctypes.c_uint32((self.epoch.value + 2 * n) & 0xffffffff)
+    def _advance(self, steps: int, edges: int, C: int = None):
+        """HostFed._advance, and the epoch of the step barriers: two per step."""
+        super()._advance(steps, edges, C)
+        self.epoch = ctypes.c_uint32((self.epoch.value + 2 * steps) & 0xffffffff)
 
     def run(self, b0: int, n_steps: int, query_arrays, out: torch.Tensor = None, out_step_stride: int = 0):
         """n_steps consecutive steady-state steps (full history) starting at batch b0 in ONE native call (lstep_pe_steps_peer).
         query_arrays: device int64 tensors indexed by GLOBAL edge position (query set c of a step = query_arrays[c][lo:lo+n]).
         out: [C, max q_rows, d] (every step overwrites it) or, with out_step_stride, one block per step."""
         assert self.grp is not None and self.len == self.T and b0 + n_steps <= self.num_batches
-        lib, d = self.lib, self.d
+        lib, m, d = self.lib, self.model, self.d
         C = len(query_arrays)
         if out is None:
             out = torch.empty((max(C, 1), self.B // self.G + 1, d), dtype=torch.float32, device=self.dev)
@@ -371,22 +368,19 @@ class PeerRank(HostFed):
         mine_off = np.ascontiguousarray(self.mine_off[b0:b0 + n_steps + 1])
         lo = np.ascontiguousarray(self.lo[b0:b0 + n_steps])
         with torch.cuda.device(self.dev), torch.no_grad():
-            Gt = self.m._collapsed_filter(self.T, False)
+            Gt = m._collapsed_filter(self.T, False)
             rc = lib.lstep_pe_steps_peer(ctypes.byref(self.desc), self.changelog.ref, self.sampler.csr_ref, ctypes.byref(self.grp), n_steps,
                                          ap(lo, 0), ap(self.n_edges, b0), ap(self.tmax, b0), _lib.ptr(self.ids), ap(ids_off, 0),
                                          _lib.ptr(self.ids_mine), _lib.ptr(self.pos_mine), ap(mine_off, 0), ctypes.byref(head), _lib.ptr(Gt), qptrs,
-                                         ap(lo, 0), C, _lib.ptr(out), int(out_step_stride), self.K, self.m._mlp_ref("nbr"),
-                                         self.m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(), _lib.ptr(self.sampler._err),
+                                         ap(lo, 0), C, _lib.ptr(out), int(out_step_stride), self.K, m._mlp_ref("nbr"),
+                                         m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(), _lib.ptr(self.sampler._err),
                                          ctypes.byref(epoch), self.timeout_ms, _lib.stream_ptr())
-        done = ((epoch.value - self.epoch.value) & 0xffffffff) // 2
-        self.head, self.batch_idx, self.steps_done = head.value, self.batch_idx + done, self.steps_done + done
-        if done:
-            self.edges_done = int(self.lo[b0 + done - 1] + self.n_edges[b0 + done - 1])
-        self.epoch = epoch
+        done = ((epoch.value - self.epoch.value) & 0xffffffff) // 2  # (two barrier epochs per applied step)
+        self._advance(done, int(self.n_edges[b0:b0 + done].sum()))
         _lib.check(rc, "lstep_pe_steps_peer")
         return out
 
-    # ---- host-fed steps (csrc/host_step.cu; stepper, ingest and tickets: hostfeed.HostFed) ---------------------------------
+    # ---- host-fed steps: HostFed's driver (step_host_async / step_host / run_host) around the peer calls of csrc/host_step.cu ---
     def _host_sampler(self):
         return self.sampler  # (this rank's own CSR replica: in a single-process group the ranks share the model)
 
@@ -394,138 +388,34 @@ class PeerRank(HostFed):
         """(q_off, q_rows): this rank's share of a batch of n edges for the a6 queries (and of step_host's row sums)."""
         return share_of(n, self.G, self.rank)
 
-    def _host_prepare(self, src, dst, times, query_ids, ids=None, ingest=False, edge_id_start=None, grow=False, batch_size=None) -> dict:
-        """Validate a host batch (check_host_batch) and, with grow, add the nodes up to its largest id; with ingest, make room
-        for it in this rank's sampler. Nothing is written before the batch is validated; a regrow synchronises."""
-        ing, n_new = None, 0
-        if grow:
-            src, dst, times, qs = host_arrays(src, dst, times, query_ids, "step_host")
-            n_new = self._new_nodes_for([src, dst] + qs) if len(src) else 0
-        if ingest:
-            samp = self._growable_sampler()
-            rows = max(samp.num_rows, self.V1 + n_new) if n_new else samp.num_rows
-            ing = (rows, samp.last_time, samp.next_edge_id if edge_id_start is None else int(edge_id_start))
-        src, dst, times, qs, ids = check_host_batch(src, dst, times, query_ids if not grow else qs, self.V1 + n_new,
-                                                    self.B if batch_size is None else batch_size, ids, ing)
-        if n_new:
-            self.add_nodes(n_new, _edges=(src, dst))
-        if ingest:
-            self.sampler.reserve(src, dst)
-        return dict(src=src, dst=dst, times=times, qs=qs, ids=ids, ingest=bool(ingest), eid0=None if ing is None else ing[2])
-
-    def _host_phase(self, hb: dict, phases: int, batch_idx: int = None, out: torch.Tensor = None):
-        """Issue `phases` of the step on the prepared batch hb (lstep_pe_step_peer_host): the call with bit 0 stages the batch,
-        the one with bit 2 finishes the step, advances the state and returns the ticket."""
+    def _check_host(self, src, dst, times, qs, ids, V1: int, n_max: int):
+        """check_host_batch: every rank of a group makes the same checks on the same batch, so either every rank accepts it or
+        every rank rejects it, before any rank enqueues anything (a run is validated whole: n_max is its length)."""
         assert self.grp is not None, "set_group / connect_ipc first"
-        src, dst, times, qs, ids, ingest = hb["src"], hb["dst"], hb["times"], hb["qs"], hb["ids"], hb["ingest"]
-        n, C = len(src), len(qs)
-        samp = self.sampler
-        if torch.cuda.current_device() != self.dev.index:
-            torch.cuda.set_device(self.dev)
-        if phases & 1:
-            hb["bi"] = self.batch_idx if batch_idx is None else int(batch_idx)
-            h = hb["h"] = self._host_stepper_for(n, C)
-            self._set_ingest(h, ingest, hb["eid0"])
-            hb["G"] = self.m._collapsed_filter(filter_len(hb["bi"], self.len, self.T), False)
-            hb["qptrs"] = (ctypes.c_void_p * max(C, 1))(*[q.ctypes.data for q in qs])
-            hb["out"] = out
-        ticket = ctypes.c_int64(-1)
-        rc = self._libc.lstep_pe_step_peer_host(
-            hb["h"], ctypes.byref(self.desc), self.changelog.ref, samp.csr_ref, ctypes.byref(self.grp), n, src.ctypes.data, dst.ctypes.data,
+        return check_host_batch(src, dst, times, qs, V1, n_max, ids)[4]
+
+    def _host_rows(self, n: int) -> int:
+        return self.share_of(n)[1]
+
+    def _workspace(self, n_ids: int, n_edges: int, C: int) -> torch.Tensor:
+        return self.ws  # (sized for batch_size edges and 8 query sets, the most check_host_batch lets through)
+
+    def _host_step_call(self, h, n, src, dst, times, ids, G, qptrs, C, out, ws, phases, ticket) -> int:
+        m, samp = self.model, self.sampler
+        return self.lib.lstep_pe_step_peer_host(
+            h, ctypes.byref(self.desc), self.changelog.ref, samp.csr_ref, ctypes.byref(self.grp), n, src.ctypes.data, dst.ctypes.data,
             times.ctypes.data, ids.ctypes.data if ids is not None else None, len(ids) if ids is not None else 0, self.head, self.len,
-            _lib.ptr(hb["G"]), hb["qptrs"], C, _lib.ptr(hb["out"]), self.K, self.m._mlp_ref("nbr"), self.m._mlp_ref("update"),
-            _lib.ptr(self.ws), self.ws.numel(), _lib.ptr(samp._err), self.epoch.value, self.timeout_ms, phases, _lib.stream_ptr(),
-            ctypes.byref(ticket))
-        if rc != 0:  # (the append may have been enqueued before the step failed)
-            self._host_failed(rc, "lstep_pe_step_peer_host", ingest, samp, src, dst, hb["eid0"], times)
-        if ingest and (phases & 1):  # the append is enqueued with the staging
-            samp._note_ingested(src, dst, hb["eid0"] + n - 1, times[-1])
-        if not phases & 4:
-            return None
-        self.batch_idx = hb["bi"]
-        self._advance(1)
-        self.edges_done += n
-        self.m.h2d_bytes += 8 * n * (5 + C)  # (what the stepper copies: src, dst, t, <= 2n ids, C query sets)
-        return self._new_ticket(ticket.value, C, self.share_of(n)[1])
+            _lib.ptr(G), qptrs, C, _lib.ptr(out), self.K, m._mlp_ref("nbr"), m._mlp_ref("update"), _lib.ptr(ws), ws.numel(),
+            _lib.ptr(samp._err), self.epoch.value, self.timeout_ms, phases, _lib.stream_ptr(), ctypes.byref(ticket))
 
-    def step_host_async(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None,
-                        ids: np.ndarray = None, out: torch.Tensor = None, ingest: bool = False, edge_id_start: int = None,
-                        grow: bool = False) -> int:
-        """ChangeLogStream.step_host_async for this rank (lstep_pe_step_peer_host): the whole step on a batch of host arrays,
-        every rank of the group calling it with the same batch. result(ticket) is this rank's share [C, q_rows] of the per-query
-        row sums (share_of(n)); `out` [C, q_rows, d] keeps the share's neighbourhood PEs on the device. ingest=True appends the
-        batch to this rank's own growable sampler first. A batch longer than batch_size is rejected before anything is
-        enqueued. edges_done, steps_done, batch_idx and epoch advance as in step. grow=True: as in ChangeLogStream.step_host_async;
-        every rank adds the same nodes."""
-        return self._host_phase(self._host_prepare(src, dst, times, query_ids, ids, ingest, edge_id_start, grow), 7, batch_idx, out)
-
-    def step_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None, ids: np.ndarray = None,
-                  ingest: bool = False, edge_id_start: int = None, grow: bool = False) -> np.ndarray:
-        """Synchronous form: this rank's share [len(query_ids), q_rows] of the per-query row sums."""
-        return self.result(self.step_host_async(src, dst, times, query_ids, batch_idx, ids, ingest=ingest, edge_id_start=edge_id_start,
-                                                grow=grow))
-
-    def run_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, ingest: bool = False,
-                 edge_id_start: int = None, grow: bool = False) -> np.ndarray:
-        """ChangeLogStream.run_host for this rank: batch b = edges [b*B, (b+1)*B) of the host arrays, the steady-state batches
-        in ONE native call (lstep_pe_steps_peer_host), the ones while the log fills one by one. Returns [n_batches, C, B] float32:
-        row [b, c, :q_rows] is this rank's share of batch b (share_of), the rest zero. The whole run is validated first, and with
-        ingest=True room for all of it is reserved in this rank's sampler before the native call, so that no rank regrows (and
-        synchronises) while its peers wait at a barrier; the decision depends on the batches only, so every rank makes the
-        same one. grow=True: the nodes up to the run's largest id are added first, on every rank alike."""
-        assert self.grp is not None, "set_group / connect_ipc first"
-        n_total, B, C = len(src), self.B, len(query_ids)
-        src, dst, times, qs = host_arrays(src, dst, times, query_ids, "run_host")
-        nb = (n_total + B - 1) // B
-        res = np.zeros((nb, C, B), dtype=np.float32)
-        if n_total == 0:
-            return res
-        hb = self._host_prepare(src, dst, times, qs, None, ingest, edge_id_start, grow, n_total)  # (the whole run: batches of B follow)
-        eid0 = hb["eid0"]
-        lo = 0
-        pend = []
-        while lo < n_total and self.len < self.T:  # while the log fills: per-step calls
-            hi = min(lo + B, n_total)
-            pend.append((lo // B, self.step_host_async(src[lo:hi], dst[lo:hi], times[lo:hi], [q[lo:hi] for q in qs], ingest=ingest,
-                                                       edge_id_start=None if eid0 is None else eid0 + lo)))
-            if len(pend) > 1:
-                b, tk = pend.pop(0)
-                r = self.result(tk)
-                res[b, :, :r.shape[1]] = r
-            lo = hi
-        for b, tk in pend:
-            r = self.result(tk)
-            res[b, :, :r.shape[1]] = r
-        if lo >= n_total:
-            return res
-        if torch.cuda.current_device() != self.dev.index:
-            torch.cuda.set_device(self.dev)
-        h = self._stepper(B, C)
-        self._set_ingest(h, ingest, eid0 + lo if ingest else None)
-        G = self.m._collapsed_filter(self.T, False)
-        qptrs = (ctypes.c_void_p * max(C, 1))(*[q[lo:].ctypes.data for q in qs])
-        head, ln, done = ctypes.c_int(self.head), ctypes.c_int(self.len), ctypes.c_int64(0)
-        epoch = ctypes.c_uint32(self.epoch.value)
-        sub = res[lo // B:]
-        samp = self.sampler
-        rc = self._libc.lstep_pe_steps_peer_host(
-            h, ctypes.byref(self.desc), self.changelog.ref, samp.csr_ref, ctypes.byref(self.grp), n_total - lo, B, src[lo:].ctypes.data,
-            dst[lo:].ctypes.data, times[lo:].ctypes.data, qptrs, C, ctypes.byref(head), ctypes.byref(ln), _lib.ptr(G), self.K,
-            self.m._mlp_ref("nbr"), self.m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(), _lib.ptr(samp._err), ctypes.byref(epoch),
-            self.timeout_ms, _lib.stream_ptr(), sub.ctypes.data, ctypes.byref(done))
-        # batches applied before an error stay applied: the host state follows the device's
-        steps = done.value
-        self.head, self.epoch = head.value, epoch
-        self.batch_idx += steps
-        self.steps_done += steps
-        n_app = min(steps * B, n_total - lo)
-        self.edges_done += n_app
-        self.m.h2d_bytes += 8 * n_app * (5 + C)
-        if rc != 0:
-            self._host_failed(rc, "lstep_pe_steps_peer_host", ingest, samp, src[lo:], dst[lo:], eid0 + lo if ingest else None, times[lo:])
-        if ingest and n_app > 0:
-            samp._note_ingested(src[lo:lo + n_app], dst[lo:lo + n_app], eid0 + lo + n_app - 1, times[lo + n_app - 1])
-        return res
+    def _host_run_call(self, h, n, src, dst, times, qptrs, C, G, ws, res, done) -> int:
+        m, samp = self.model, self.sampler
+        head, ln, epoch = ctypes.c_int(self.head), ctypes.c_int(self.len), ctypes.c_uint32(self.epoch.value)  # (moved by _advance)
+        return self.lib.lstep_pe_steps_peer_host(
+            h, ctypes.byref(self.desc), self.changelog.ref, samp.csr_ref, ctypes.byref(self.grp), n, self.B, src.ctypes.data,
+            dst.ctypes.data, times.ctypes.data, qptrs, C, ctypes.byref(head), ctypes.byref(ln), _lib.ptr(G), self.K, m._mlp_ref("nbr"),
+            m._mlp_ref("update"), _lib.ptr(ws), ws.numel(), _lib.ptr(samp._err), ctypes.byref(epoch), self.timeout_ms, _lib.stream_ptr(),
+            res.ctypes.data, ctypes.byref(done))
 
     def barrier(self):
         """Barrier + application of the inbox: once the kernels this enqueues have run, this replica holds the rows every rank changed

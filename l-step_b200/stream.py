@@ -27,8 +27,8 @@ import torch
 
 from . import _lib
 from . import checkpoint as ckpt
-from .changelog import ChangeLogHistory, advance, filter_len
-from .hostfeed import HostFed, host_arrays
+from .changelog import ChangeLogHistory, filter_len
+from .hostfeed import HostFed
 from .model import LSTEP
 
 C_void_p = ctypes.c_void_p
@@ -111,15 +111,14 @@ class PEStream(HostFed):
         self.len = Th  # number of valid steps
         self.head = 0  # slot of the oldest valid step
         self.cur = torch.empty((self.row_cap, d), dtype=torch.float32, device=self.dev)
-        lib = _lib.load()
         with torch.cuda.device(self.dev):
-            _lib.check(lib.lstep_ring_load(_lib.ptr(self.ring), _lib.ptr(self.cur), V1, self.T, d, self._last_slot(),
-                                           _lib.stream_ptr()), "lstep_ring_load")
+            _lib.check(self.lib.lstep_ring_load(_lib.ptr(self.ring), _lib.ptr(self.cur), V1, self.T, d, self._last_slot(),
+                                                _lib.stream_ptr()), "lstep_ring_load")
         self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.t.data_ptr(), self.ring.data_ptr(),
                                       self.cur.data_ptr(), V1, self.T, d, self.row_cap)
         self._ws = None
         self._ws_cap = (0, 0, 0)
-        self.steps_done = 0
+        self.steps_done, self.edges_done = 0, self.start
 
     def check_errors(self):
         """Synchronising read of the device error flag the step's lookups raise for query ids outside the sampler's
@@ -145,8 +144,10 @@ class PEStream(HostFed):
         return lo, hi, self.ids_off[b], self.ids_off[b + 1]
 
     def _workspace(self, n_ids, n_edges, C):
-        lib = _lib.load()
-        m = self.model
+        cap = self._ws_cap
+        if self._ws is not None and n_ids <= cap[0] and n_edges <= cap[1] and C <= cap[2]:
+            return self._ws
+        lib, m = self.lib, self.model
         need = lib.lstep_pe_step_workspace_bytes(n_ids, n_edges, C, self.K, self.d, m.time_feat_dim, self.row_cap)
         if self._ws is None or self._ws.numel() < need:
             self._ws_cap = (max(2 * self.B, n_ids), max(self.B, n_edges), max(C, 4))  # (ids, edges, query sets) it is sized for
@@ -158,23 +159,21 @@ class PEStream(HostFed):
         return self._ws
 
     def _run(self, lo, n_edges, ids, tmax, queries, out, batch_idx):
-        """Device-resident core shared by step() and step_host()."""
-        lib = _lib.load()
+        """Device-resident core of step()."""
         m = self.model
         bi = self.batch_idx if batch_idx is None else batch_idx
         C = len(queries)
         with torch.cuda.device(self.dev), torch.no_grad():
             G = m._collapsed_filter(filter_len(bi, self.len, self.T), False)
             ws = self._workspace(ids.shape[0], n_edges, C)
-            slot, new_head, new_len = advance(self.head, self.len, self.T)
             qptrs = (C_void_p * max(C, 1))(*[q.data_ptr() for q in queries])
-            _lib.check(lib.lstep_pe_step(self._desc_ref, m.neighbor_sampler.csr_ref, lo, n_edges, _lib.ptr(ids), ids.shape[0],
-                                         float(tmax), self.head, self.len, slot, _lib.ptr(G), qptrs, C, _lib.ptr(out), self.K,
-                                         m._mlp_ref("nbr"), m._mlp_ref("update"), _lib.ptr(ws), ws.numel(),
-                                         _lib.ptr(m.neighbor_sampler._err), _lib.stream_ptr()), "lstep_pe_step")
-            self.head, self.len = new_head, new_len
-        self.batch_idx = bi + 1
-        self.steps_done += 1
+            slot = (self.head + self.len) % self.T  # (the slot changelog.advance writes: the next free one, then the oldest)
+            _lib.check(self.lib.lstep_pe_step(self._desc_ref, m.neighbor_sampler.csr_ref, lo, n_edges, _lib.ptr(ids), ids.shape[0],
+                                              float(tmax), self.head, self.len, slot, _lib.ptr(G), qptrs, C, _lib.ptr(out), self.K,
+                                              m._mlp_ref("nbr"), m._mlp_ref("update"), _lib.ptr(ws), ws.numel(),
+                                              _lib.ptr(m.neighbor_sampler._err), _lib.stream_ptr()), "lstep_pe_step")
+        self.batch_idx = bi
+        self._advance(1, n_edges)
 
     @property
     def _desc_ref(self):
@@ -212,7 +211,7 @@ class PEStream(HostFed):
                 lo, hi, _, _ = self.batch_arrays(b0 + i)
                 last = self.step(b0 + i, [q[lo - lo0:hi - lo0] for q in queries], None if out is None else out[i])
             return last
-        lib, m = self._libc, self.model
+        lib, m = self.lib, self.model
         B, d = self.B, self.d
         los = np.asarray(self.batch_lo[b0:b0 + n_steps], dtype=np.int64)
         his = np.minimum(los + B, self.stop)
@@ -240,9 +239,7 @@ class PEStream(HostFed):
                                     ws.data_ptr(), ws.numel(), m.neighbor_sampler._err.data_ptr(),
                                     torch.cuda.current_stream().cuda_stream)
             done = (head.value - self.head) % self.T if rc != 0 else n_steps
-            self.head = head.value
-            self.batch_idx += done
-            self.steps_done += done
+            self._advance(done, int(ne[:done].sum()))
             if rc != 0:
                 _lib.check(rc, "lstep_pe_steps")
         if check:
@@ -263,149 +260,42 @@ class PEStream(HostFed):
         self._ws = None  # its per-node maps cover row_cap rows: reallocated (and zeroed) by the next step
 
     def _init_rows(self, v0: int, v1: int, rows: torch.Tensor, stride: int):
-        _lib.check(self._libc.lstep_pe_rows_init(_lib.ptr(self.cur), _lib.ptr(self.ring), self.T, self.d, None, 1, 0, v0, v1, _lib.ptr(rows),
-                                                 stride, _lib.stream_ptr()), "lstep_pe_rows_init")
+        _lib.check(self.lib.lstep_pe_rows_init(_lib.ptr(self.cur), _lib.ptr(self.ring), self.T, self.d, None, 1, 0, v0, v1, _lib.ptr(rows),
+                                               stride, _lib.stream_ptr()), "lstep_pe_rows_init")
 
     def _set_live(self, V1: int):
         self.V1 = self.desc.V1 = int(V1)
 
-    # ---- host-fed steps (native stager: csrc/host_step.cu; stepper, ingest and tickets: hostfeed.HostFed) -----------
+    # ---- host-fed steps: step_host_async / step_host / run_host and result are hostfeed.HostFed's, which validates, stages,
+    # arms the ingest, moves the window and keeps the tickets around the native calls of csrc/host_step.cu below. A layout
+    # supplies its own checks of a batch, these two native calls, the rows per query of a result and its workspace;
+    # ChangeLogStream replaces the checks and the calls. Each call returns the native status.
     def _host_sampler(self):
         return self.model.neighbor_sampler
 
-    def step_host_async(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None,
-                        ids: np.ndarray = None, out: torch.Tensor = None, ingest: bool = False, edge_id_start: int = None,
-                        grow: bool = False) -> int:
-        """One step fed from HOST arrays (what a loop holding numpy batches calls): the batch's endpoints,
-        times and the query id sets are packed into a pinned slot and uploaded by one async copy inside the
-        native call, the step's kernels are enqueued behind it, and the per-query row sums [C, n] of the
-        neighbourhood PEs are copied back to a pinned result slot. Returns a ticket at once (nothing
-        synchronises); `result(ticket)` waits for that step only, so a loop can read results one step behind.
-        `ids` (sorted unique batch nodes) is computed natively when omitted; `out` [C, n, d] keeps the full
-        neighbourhood PEs on the device. This is the per-batch host path: it avoids every avoidable Python
-        call (≈ 25 µs of interpreter time per step).
-        ingest=True: the batch's edges are not in the sampler yet. The model's sampler must be growable
-        (NeighborSampler.growable); the batch is validated, room is reserved, and the native call appends it to the CSR
-        (edge ids edge_id_start + i, default: the sampler's next_edge_id) before the step's lookups run.
-        grow=True: ids above the last live one (in the batch or the query sets) are new nodes, added first (add_nodes, with
-        the stream's new_node_pe row); without it such an id raises IndexError, as an unknown node does in the reference."""
-        m = self.model
-        n = len(src)
-        C = len(query_ids)
-        src, dst, times, qs = host_arrays(src, dst, times, query_ids, "step_host")
-        if ids is not None:
-            ids = np.ascontiguousarray(ids, dtype=_I64)
-        n_new = self._new_nodes_for([src, dst] + qs) if grow and n else 0
-        if ingest:
-            eid0 = self._check_ingest(src, dst, times, edge_id_start, n_new)
-        elif n_new:
-            self.add_nodes(n_new)
-        bi = self.batch_idx if batch_idx is None else batch_idx
-        if torch.cuda.current_device() != self.dev.index:
-            torch.cuda.set_device(self.dev)
-        h = self._host_stepper_for(n, C)
-        self._set_ingest(h, ingest, eid0 if ingest else None)
-        G = m._collapsed_filter(filter_len(bi, self.len, self.T), False)
-        ws = self._ws
-        if ws is None or n > self._ws_cap[1] or C > self._ws_cap[2] or 2 * n > self._ws_cap[0]:
-            ws = self._workspace(len(ids) if ids is not None else 2 * n, n, C)
-        slot, new_head, new_len = advance(self.head, self.len, self.T)
-        qptrs = (C_void_p * max(C, 1))(*[q.ctypes.data for q in qs])
-        ticket = ctypes.c_int64(-1)
-        samp = m.neighbor_sampler
-        rc = self._step_host_native(h, samp, n, src, dst, times, ids, slot, G, qptrs, C, out, ws, ticket)
-        if rc != 0:  # (the append may have been enqueued before the step failed)
-            self._host_failed(rc, self._HOST_CALLS[0], ingest, samp, src, dst, eid0 if ingest else None, times)
-        if ingest:
-            samp._note_ingested(src, dst, eid0 + n - 1, times[-1])
-        self.head, self.len = new_head, new_len
-        self.batch_idx = bi + 1
-        self.steps_done += 1
-        tk = self._new_ticket(ticket.value, C, n)
-        m.h2d_bytes += 8 * n * (5 + C)  # what lstep_pe_step_host copies: src, dst, t, <= 2n ids, C query sets
-        return tk
+    def _check_host(self, src, dst, times, qs, ids, V1: int, n_max: int):
+        """None beyond the shared checks: the native stager rejects ids outside the table and the sampler's rows."""
+        return None if ids is None else np.ascontiguousarray(ids, dtype=_I64)
 
-    def run_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, ingest: bool = False,
-                 edge_id_start: int = None, grow: bool = False) -> np.ndarray:
-        """A run of consecutive batches fed from HOST arrays in ONE native call (an evaluation split): batch b is edges
-        [b*B, (b+1)*B) of the given arrays; every step copies its own inputs in and its own per-query row sums out
-        (read one step behind inside the call). Returns [n_batches, C, B] float32 (tail of a ragged last batch zero).
-        While the history ring is still filling (the filter changes with every step) the batches go through
-        step_host_async one by one. ingest=True: as in step_host_async; room for the whole run is reserved first, so the
-        native loop never needs a regrow. grow=True: the nodes up to the run's largest id are added (add_nodes) before its
-        first step, so the native loop never grows either; a node's rows are then in place before its first edge, which
-        changes nothing (they are the rows of a node no edge has touched)."""
-        n_total, B, C = len(src), self.B, len(query_ids)
-        src, dst, times, qs = host_arrays(src, dst, times, query_ids, "run_host")
-        n_new = self._new_nodes_for([src, dst] + qs) if grow and n_total else 0
-        eid0 = self._check_ingest(src, dst, times, edge_id_start, n_new) if ingest else None
-        if n_new and not ingest:
-            self.add_nodes(n_new)
-        nb = (n_total + B - 1) // B
-        res = np.zeros((nb, C, B), dtype=np.float32)
-        lo = 0
-        pend = []
-        while lo < n_total and self.len < self.T:  # masked regime: per-step calls
-            hi = min(lo + B, n_total)
-            pend.append((lo // B, hi - lo, self.step_host_async(src[lo:hi], dst[lo:hi], times[lo:hi], [q[lo:hi] for q in qs], ingest=ingest,
-                                                                 edge_id_start=None if eid0 is None else eid0 + lo)))
-            if len(pend) > 1:
-                b, n, tk = pend.pop(0)
-                res[b, :, :n] = self.result(tk)
-            lo = hi
-        for b, n, tk in pend:
-            res[b, :, :n] = self.result(tk)
-        if lo >= n_total:
-            return res
-        m = self.model
-        if torch.cuda.current_device() != self.dev.index:
-            torch.cuda.set_device(self.dev)
-        h = self._stepper(B, C)
-        self._set_ingest(h, ingest, eid0 + lo if ingest else None)
-        G = m._collapsed_filter(self.T, False)
-        ws = self._workspace(2 * B, B, C)
-        qptrs = (C_void_p * max(C, 1))(*[q[lo:].ctypes.data for q in qs])
-        head, ln, done = ctypes.c_int(self.head), ctypes.c_int(self.len), ctypes.c_int64(0)
-        sub = res[lo // B:]
-        samp = m.neighbor_sampler
-        rc = self._steps_host_native(h, samp, n_total - lo, src[lo:], dst[lo:], times[lo:], qptrs, C, head, ln, G, ws, sub, done)
-        # batches applied before an error stay applied: the host-side ring position follows the device ring either way
-        steps = done.value
-        self.head = head.value
-        self.batch_idx += steps
-        self.steps_done += steps
-        n_app = min(steps * B, n_total - lo)
-        m.h2d_bytes += 8 * n_app * (5 + C)
-        if rc != 0:  # (the failed batch's append may have been enqueued although its step was not applied)
-            self._host_failed(rc, self._HOST_CALLS[1], ingest, samp, src[lo:], dst[lo:], eid0 + lo if ingest else None, times[lo:])
-        if ingest and n_app > 0:
-            samp._note_ingested(src[lo:lo + n_app], dst[lo:lo + n_app], eid0 + lo + n_app - 1, times[lo + n_app - 1])
-        return res
+    def _host_rows(self, n: int) -> int:
+        return n
 
-    # The native calls of the host-fed steps, the only part ChangeLogStream replaces: the staging, validation, ingest arming,
-    # workspace and ticket bookkeeping above are shared. Each returns the native status.
-    _HOST_CALLS = ("lstep_pe_step_host", "lstep_pe_steps_host")
+    def _host_step_call(self, h, n, src, dst, times, ids, G, qptrs, C, out, ws, phases, ticket) -> int:
+        m, samp = self.model, self.model.neighbor_sampler
+        return self.lib.lstep_pe_step_host(h, self._desc_ref, samp.csr_ref, n, src.ctypes.data, dst.ctypes.data, times.ctypes.data,
+                                           ids.ctypes.data if ids is not None else None, len(ids) if ids is not None else 0, self.head,
+                                           self.len, (self.head + self.len) % self.T, G.data_ptr(), qptrs, C,
+                                           out.data_ptr() if out is not None else None, self.K, m._mlp_ref("nbr"), m._mlp_ref("update"),
+                                           ws.data_ptr(), ws.numel(), samp._err.data_ptr(), torch.cuda.current_stream().cuda_stream,
+                                           C_byref(ticket))
 
-    def _step_host_native(self, h, samp, n, src, dst, times, ids, slot, G, qptrs, C, out, ws, ticket):
-        m = self.model
-        return self._libc.lstep_pe_step_host(h, self._desc_ref, samp.csr_ref, n, src.ctypes.data, dst.ctypes.data, times.ctypes.data,
-                                             ids.ctypes.data if ids is not None else None, len(ids) if ids is not None else 0, self.head,
-                                             self.len, slot, G.data_ptr(), qptrs, C, out.data_ptr() if out is not None else None, self.K,
-                                             m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(), samp._err.data_ptr(),
-                                             torch.cuda.current_stream().cuda_stream, C_byref(ticket))
-
-    def _steps_host_native(self, h, samp, n_total, src, dst, times, qptrs, C, head, ln, G, ws, sub, done):
-        m = self.model
-        return self._libc.lstep_pe_steps_host(h, self._desc_ref, samp.csr_ref, n_total, self.B, src.ctypes.data, dst.ctypes.data,
-                                              times.ctypes.data, qptrs, C, C_byref(head), C_byref(ln), G.data_ptr(), self.K,
-                                              m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(), samp._err.data_ptr(),
-                                              torch.cuda.current_stream().cuda_stream, sub.ctypes.data, C_byref(done))
-
-    def step_host(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, batch_idx: int = None, ids: np.ndarray = None,
-                  ingest: bool = False, edge_id_start: int = None, grow: bool = False):
-        """Synchronous form: run the step and return its per-query row sums [len(query_ids), n]."""
-        return self.result(self.step_host_async(src, dst, times, query_ids, batch_idx, ids, ingest=ingest, edge_id_start=edge_id_start,
-                                                grow=grow))
+    def _host_run_call(self, h, n, src, dst, times, qptrs, C, G, ws, res, done) -> int:
+        m, samp = self.model, self.model.neighbor_sampler
+        head, ln = ctypes.c_int(self.head), ctypes.c_int(self.len)  # (the window is moved by HostFed._advance from done)
+        return self.lib.lstep_pe_steps_host(h, self._desc_ref, samp.csr_ref, n, self.B, src.ctypes.data, dst.ctypes.data,
+                                            times.ctypes.data, qptrs, C, C_byref(head), C_byref(ln), G.data_ptr(), self.K,
+                                            m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(), samp._err.data_ptr(),
+                                            torch.cuda.current_stream().cuda_stream, res.ctypes.data, C_byref(done))
 
 
 class ChangeLogStream(PEStream):
@@ -431,7 +321,6 @@ class ChangeLogStream(PEStream):
             hist = checkpoint if isinstance(checkpoint, ckpt.History) else ckpt.read(checkpoint)
             model = args[0] if args else kw["model"]
             hist.check(d=model.pe_dim, T=model.num_fft_batches)
-        self.edges_done = 0
         super().__init__(*args, **kw)
         if hist is not None:
             self._load(hist)
@@ -443,8 +332,7 @@ class ChangeLogStream(PEStream):
         history = history.to(self.dev, torch.float32)
         assert history.shape[2] == self.d
         self._load(ckpt.from_dense(history, self.T))
-        self.steps_done = 0
-        self.edges_done = self.start
+        self.steps_done, self.edges_done = 0, self.start
 
     def save_checkpoint(self, path: str):
         """Write the history into directory `path` as a world-1 checkpoint (l-step_b200/checkpoint.py: base rows and the
@@ -500,8 +388,8 @@ class ChangeLogStream(PEStream):
         self._ws = None
 
     def _init_rows(self, v0: int, v1: int, rows: torch.Tensor, stride: int):
-        _lib.check(self._libc.lstep_pe_rows_init(_lib.ptr(self.cur), None, self.T, self.d, _lib.ptr(self.changelog.base), 1, 0, v0, v1,
-                                                 _lib.ptr(rows), stride, _lib.stream_ptr()), "lstep_pe_rows_init")
+        _lib.check(self.lib.lstep_pe_rows_init(_lib.ptr(self.cur), None, self.T, self.d, _lib.ptr(self.changelog.base), 1, 0, v0, v1,
+                                               _lib.ptr(rows), stride, _lib.stream_ptr()), "lstep_pe_rows_init")
 
     def _set_live(self, V1: int):
         self.changelog.add_rows(V1)
@@ -518,7 +406,6 @@ class ChangeLogStream(PEStream):
         samp.check_errors()
 
     def _run(self, lo, n_edges, ids, tmax, queries, out, batch_idx):
-        lib = _lib.load()
         m = self.model
         bi = self.batch_idx if batch_idx is None else batch_idx
         C = len(queries)
@@ -526,14 +413,13 @@ class ChangeLogStream(PEStream):
             G = m._collapsed_filter(filter_len(bi, self.len, self.T), False)
             ws = self._workspace(ids.shape[0], n_edges, C)
             qptrs = (C_void_p * max(C, 1))(*[q.data_ptr() for q in queries])
-            _lib.check(lib.lstep_pe_step_changelog(self._desc_ref, self.changelog.ref, m.neighbor_sampler.csr_ref, lo, n_edges, _lib.ptr(ids),
-                                                   ids.shape[0], float(tmax), self.head, self.len, _lib.ptr(G), qptrs, C, 0, -1, _lib.ptr(out),
-                                                   self.K, m._mlp_ref("nbr"), m._mlp_ref("update"), _lib.ptr(ws), ws.numel(),
-                                                   _lib.ptr(m.neighbor_sampler._err), _lib.stream_ptr(), 0), "lstep_pe_step_changelog")
-            _, self.head, self.len = advance(self.head, self.len, self.T)
-        self.batch_idx = bi + 1
-        self.steps_done += 1
-        self.edges_done = lo + n_edges
+            _lib.check(self.lib.lstep_pe_step_changelog(self._desc_ref, self.changelog.ref, m.neighbor_sampler.csr_ref, lo, n_edges,
+                                                        _lib.ptr(ids), ids.shape[0], float(tmax), self.head, self.len, _lib.ptr(G), qptrs,
+                                                        C, 0, -1, _lib.ptr(out), self.K, m._mlp_ref("nbr"), m._mlp_ref("update"),
+                                                        _lib.ptr(ws), ws.numel(), _lib.ptr(m.neighbor_sampler._err), _lib.stream_ptr(), 0),
+                       "lstep_pe_step_changelog")
+        self.batch_idx = bi
+        self._advance(1, n_edges)
 
     def run(self, b0: int, n_steps: int, queries, out: torch.Tensor = None, check: bool = False):
         lo0 = self.batch_lo[b0]
@@ -545,36 +431,29 @@ class ChangeLogStream(PEStream):
             self.check_errors()
         return out if out is not None else last
 
-    # ---- host-fed steps: PEStream's, with the change-log step as the native call --------------------------------------
-    def step_host_async(self, src: np.ndarray, dst: np.ndarray, times: np.ndarray, query_ids, *args, **kw) -> int:
-        """PEStream.step_host_async on the change-log history (lstep_pe_step_changelog_host), ingest=True included. A step
-        records its events in the log: event_capacity, sized from batch_size by default, bounds them, so a batch longer than
-        batch_size is rejected before anything is enqueued. edges_done advances by the edges stepped."""
-        if len(src) > self.B:
+    # ---- host-fed steps: HostFed's driver, with the change-log step as the native call ---------------------------------
+    def _check_host(self, src, dst, times, qs, ids, V1: int, n_max: int):
+        """A step records its events in the log: event_capacity, sized from batch_size by default, bounds them, so a batch
+        longer than batch_size is rejected before anything is enqueued."""
+        if len(src) > n_max:
             raise ValueError(f"ChangeLogStream: a host batch of {len(src)} edges is longer than batch_size ({self.B}), which sizes the "
                              f"change log's event_capacity ({self.cap}); split the batch or build the stream with a larger batch_size")
-        return super().step_host_async(src, dst, times, query_ids, *args, **kw)
+        return super()._check_host(src, dst, times, qs, ids, V1, n_max)
 
-    _HOST_CALLS = ("lstep_pe_step_changelog_host", "lstep_pe_steps_changelog_host")
-
-    def _step_host_native(self, h, samp, n, src, dst, times, ids, slot, G, qptrs, C, out, ws, ticket):
-        m = self.model
-        rc = self._libc.lstep_pe_step_changelog_host(h, self._desc_ref, self.changelog.ref, samp.csr_ref, n, src.ctypes.data, dst.ctypes.data,
-                                                     times.ctypes.data, ids.ctypes.data if ids is not None else None,
+    def _host_step_call(self, h, n, src, dst, times, ids, G, qptrs, C, out, ws, phases, ticket) -> int:
+        m, samp = self.model, self.model.neighbor_sampler
+        return self.lib.lstep_pe_step_changelog_host(h, self._desc_ref, self.changelog.ref, samp.csr_ref, n, src.ctypes.data,
+                                                     dst.ctypes.data, times.ctypes.data, ids.ctypes.data if ids is not None else None,
                                                      len(ids) if ids is not None else 0, self.head, self.len, G.data_ptr(), qptrs, C,
                                                      out.data_ptr() if out is not None else None, self.K, m._mlp_ref("nbr"),
                                                      m._mlp_ref("update"), ws.data_ptr(), ws.numel(), samp._err.data_ptr(),
                                                      torch.cuda.current_stream().cuda_stream, C_byref(ticket))
-        if rc == 0:
-            self.edges_done += n
-        return rc
 
-    def _steps_host_native(self, h, samp, n_total, src, dst, times, qptrs, C, head, ln, G, ws, sub, done):
-        m = self.model
-        rc = self._libc.lstep_pe_steps_changelog_host(h, self._desc_ref, self.changelog.ref, samp.csr_ref, n_total, self.B, src.ctypes.data,
+    def _host_run_call(self, h, n, src, dst, times, qptrs, C, G, ws, res, done) -> int:
+        m, samp = self.model, self.model.neighbor_sampler
+        head, ln = ctypes.c_int(self.head), ctypes.c_int(self.len)
+        return self.lib.lstep_pe_steps_changelog_host(h, self._desc_ref, self.changelog.ref, samp.csr_ref, n, self.B, src.ctypes.data,
                                                       dst.ctypes.data, times.ctypes.data, qptrs, C, C_byref(head), C_byref(ln), G.data_ptr(),
                                                       self.K, m._mlp_ref("nbr"), m._mlp_ref("update"), ws.data_ptr(), ws.numel(),
-                                                      samp._err.data_ptr(), torch.cuda.current_stream().cuda_stream, sub.ctypes.data,
+                                                      samp._err.data_ptr(), torch.cuda.current_stream().cuda_stream, res.ctypes.data,
                                                       C_byref(done))
-        self.edges_done += min(done.value * self.B, n_total)
-        return rc
