@@ -454,18 +454,29 @@ int changelog_step_core(const lstep_pe_stream* s, const lstep_changelog* cl, con
     if ((rc = lstep_changelog_filter(cl, head, len, ids, n_ids, G, s->cur, s->d, ids, stream)) != LSTEP_OK) return rc;
   }
   if (phase == 1) return LSTEP_OK;
+  int slot;
+  return changelog_step_close(s, cl, csr, src, dst, tq, n_edges, ids, n_ids, current_time, head, len, query_ids_host, n_queries, q_off, q_rows,
+                              nbr_out, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, stream, nullptr, &slot);
+}
+
+int changelog_step_close(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const int64_t* src, const int64_t* dst,
+                         const double* tq, int64_t n_edges, const int64_t* ids, int64_t n_ids, double current_time, int head, int len,
+                         const int64_t* const* query_ids_host, int n_queries, int64_t q_off, int64_t q_rows, float* nbr_out, int K,
+                         const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes,
+                         uint32_t* err_flag, void* stream, const PeerPlan* peer, int* slot) {
   StepOpts opt;
   opt.skip_dft = opt.skip_append = true;
   opt.q_off = q_off;
   opt.q_rows = q_rows;
+  opt.peer = peer;
   int stamp = 0;
   opt.stamp_out = &stamp;
   lstep_pe_stream s2 = *s;
   if (!s2.ring) s2.ring = s2.cur;  // (never touched: the core neither filters nor appends)
   const int64_t qr = q_rows < 0 ? n_edges : q_rows;
-  rc = pe_step_core_ex(&s2, csr, src, dst, tq, n_edges, ids, n_ids, current_time, 0, 0, 0, nullptr, query_ids_host, qr > 0 ? n_queries : 0,
-                       nbr_out, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, stream, opt);
-  if (rc != LSTEP_OK) return rc;
+  int rc = pe_step_core_ex(&s2, csr, src, dst, tq, n_edges, ids, n_ids, current_time, 0, 0, 0, nullptr, query_ids_host, qr > 0 ? n_queries : 0,
+                           nbr_out, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, stream, opt);
+  if (rc != LSTEP_OK || (peer && !(peer->phases & 4))) return rc;
   const int64_t* U = nullptr;
   const int32_t *n_dest = nullptr, *stamp_map = nullptr;
   int64_t n_u_max = 0;
@@ -475,8 +486,8 @@ int changelog_step_core(const lstep_pe_stream* s, const lstep_changelog* cl, con
     n_u_max = (total < s->V1 - 1 ? total : s->V1 - 1) + 1;
   }
   const bool full = len == cl->T;
-  const int slot = full ? head : (head + len) % cl->T;
-  return lstep_changelog_append(cl, slot, full ? 1 : 0, s->cur, U, n_dest, n_u_max, ids, n_ids, stamp_map, stamp, n_ids > 0 ? 1 : 0, err_flag,
+  *slot = full ? head : (head + len) % cl->T;
+  return lstep_changelog_append(cl, *slot, full ? 1 : 0, s->cur, U, n_dest, n_u_max, ids, n_ids, stamp_map, stamp, n_ids > 0 ? 1 : 0, err_flag,
                                 stream);
 }
 }  // namespace lstep

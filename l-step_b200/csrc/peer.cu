@@ -607,39 +607,18 @@ int lstep::peer_step_core(const lstep_pe_stream* s, const lstep_changelog* cl, c
   plan.epoch2 = epoch_base + 2;
   plan.timeout_ms = timeout_ms;
   plan.phases = phases & 6;
-  StepOpts opt;
-  opt.skip_dft = opt.skip_append = true;
-  opt.q_off = q_off;
-  opt.q_rows = q_rows;
-  opt.peer = &plan;
-  int stamp = 0;
-  opt.stamp_out = &stamp;
-  lstep_pe_stream s2 = *s;
-  if (!s2.ring) s2.ring = s2.cur;  // (never touched: the core neither filters nor appends)
-  rc = pe_step_core_ex(&s2, csr, src, dst, tq, n_edges, ids, n_ids, current_time, 0, 0, 0, nullptr, query_ids_host,
-                       q_rows > 0 ? n_queries : 0, nbr_out, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, stream, opt);
+  int slot;
+  rc = changelog_step_close(s, cl, csr, src, dst, tq, n_edges, ids, n_ids, current_time, head, len, query_ids_host, n_queries, q_off, q_rows,
+                            nbr_out, K, mlp_nbr, mlp_upd, workspace, workspace_bytes, err_flag, stream, &plan, &slot);
   if (rc != LSTEP_OK || !(phases & 4)) return rc;
-  const int64_t* U = nullptr;
-  const int32_t *n_dest = nullptr, *stamp_map = nullptr;
-  int64_t n_u_max = 0;
-  if (n_ids > 0) {
-    update_ws_phase_b_lists(workspace, n_ids, n_edges, K, s->d, mlp_upd->t, pe_ws_rows(s), &U, &n_dest, &stamp_map);
-    const int64_t total = n_ids * (int64_t)K;
-    n_u_max = (total < s->V1 - 1 ? total : s->V1 - 1) + 1;
-  }
-  const bool full = len == cl->T;
-  const int slot = full ? head : (head + len) % cl->T;
-  rc = lstep_changelog_append(cl, slot, full ? 1 : 0, s->cur, U, n_dest, n_u_max, ids, n_ids, stamp_map, stamp, n_ids > 0 ? 1 : 0, err_flag, stream);
-  if (rc == LSTEP_OK) {
-    if (side && grp->world > 1) {
-      if (cudaEventRecord(side->appended, st) != cudaSuccess || cudaStreamWaitEvent(side->stream, side->appended, 0) != cudaSuccess)
-        return LSTEP_ERR_CUDA;
-      rc = peer_publish(cl, slot, grp, n_ids * 8 / grp->world + 1, side->stream);
-      if (rc == LSTEP_OK && cudaEventRecord(side->published, side->stream) != cudaSuccess) return LSTEP_ERR_CUDA;
-      side->pending = true;
-    } else {
-      rc = peer_publish(cl, slot, grp, n_ids * 8 / grp->world + 1, st);
-    }
+  if (side && grp->world > 1) {
+    if (cudaEventRecord(side->appended, st) != cudaSuccess || cudaStreamWaitEvent(side->stream, side->appended, 0) != cudaSuccess)
+      return LSTEP_ERR_CUDA;
+    rc = peer_publish(cl, slot, grp, n_ids * 8 / grp->world + 1, side->stream);
+    if (rc == LSTEP_OK && cudaEventRecord(side->published, side->stream) != cudaSuccess) return LSTEP_ERR_CUDA;
+    side->pending = true;
+  } else {
+    rc = peer_publish(cl, slot, grp, n_ids * 8 / grp->world + 1, st);
   }
   prof_mark(st, kProfAppend);
   return rc;

@@ -81,5 +81,13 @@ int changelog_step_core(const lstep_pe_stream* s, const lstep_changelog* cl, con
                         const float* G, const int64_t* const* query_ids_host, int n_queries, int64_t q_off, int64_t q_rows, float* nbr_out,
                         int K, const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes,
                         uint32_t* err_flag, void* stream, int phase);
+// The change-log close of a step (changelog_step_core, peer_step_core): the step's kernels after the filter (`peer`: a peer
+// rank's plan, else NULL), then its events appended into *slot: `head`, retired first, once the window is full, else the next
+// free slot. A peer rank appends only with bit 2 of peer->phases.
+int changelog_step_close(const lstep_pe_stream* s, const lstep_changelog* cl, const lstep_csr* csr, const int64_t* src, const int64_t* dst,
+                         const double* tq, int64_t n_edges, const int64_t* ids, int64_t n_ids, double current_time, int head, int len,
+                         const int64_t* const* query_ids_host, int n_queries, int64_t q_off, int64_t q_rows, float* nbr_out, int K,
+                         const lstep_pe_mlp* mlp_nbr, const lstep_pe_mlp* mlp_upd, void* workspace, size_t workspace_bytes,
+                         uint32_t* err_flag, void* stream, const PeerPlan* peer, int* slot);
 
 }  // namespace lstep

@@ -1,14 +1,17 @@
-"""Host-fed steps: the Python side every history layout shares (PEStream, ChangeLogStream, PeerRank).
+"""Host-fed and resident steps: the Python side every history layout shares (PEStream, ChangeLogStream, PeerRank).
 
 A host-fed step hands one batch of HOST (numpy) arrays to a native stepper (csrc/host_step.cu), which packs it into a pinned
 slot, copies it in, runs the step and copies the per-query row sums back, and returns a ticket. `HostFed` owns the driver:
 step_host_async, step_host, run_host and `result`. A step has two halves: `_host_prepare` validates a batch (or a whole run),
 adds the nodes of grow=True and reserves room for ingest=True, writing nothing before all of it has passed; `_host_phase`
 issues phases of the step on the prepared batch (all at once, 7, except PeerLocalGroup's 1, 2 and 4 per rank) and moves the
-window and the counters (`_advance`). A class that mixes it in provides `dev`, `B`, `d`, `T`, `model`, the window `head` /
-`len`, the counters `batch_idx` / `steps_done` / `edges_done`, and what differs between layouts: `_host_sampler()`, the
-sampler its steps read; `_check_host(...)`, its own checks of a batch; `_host_step_call` and `_host_run_call`, the native
-per-step and multi-batch calls; `_host_rows(n)`, the rows per query of a result; `_workspace(n_ids, n_edges, C)`.
+window and the counters (`_advance`). `_step` is the same for a batch of the resident stream, the one uploaded at
+construction, whose per-batch plan (peer.batch_plan) a layout adopts with `_adopt_plan` and checks with
+`_check_stream_ids`. A class that mixes it in provides `dev`, `B`, `d`, `T`, `model`, the window `head` / `len`, the counters
+`batch_idx` / `steps_done` / `edges_done`, and what differs between layouts: `_host_sampler()`, the sampler its steps read;
+`_check_host(...)`, its own checks of a batch; `_host_step_call`, `_host_run_call` and `_step_call`, the native host-fed
+per-step and multi-batch calls and the resident per-step call; `share_of(n)`, its share of a batch's queries (all of them on
+a single GPU); `_workspace(n_ids, n_edges, C)`.
 
 It also owns the growth of the node set (add_nodes, and grow=True on the host-fed steps): new node ids continue after the
 last live one, and a new node starts with its initial row r0 in the table, in every history slot and as its change-log base
@@ -321,7 +324,7 @@ class HostFed:
             return None
         self.batch_idx = bi
         self._advance(1, n, C)
-        return self._new_ticket(ticket.value, C, self._host_rows(n))
+        return self._new_ticket(ticket.value, C, self.share_of(n)[1])
 
     def _host_failed(self, rc: int, what: str, src, dst, times, eid0):
         """A native host-fed call returned rc != 0: with ingest the append of (a prefix of) the batches may have been enqueued
@@ -329,6 +332,59 @@ class HostFed:
         if eid0 is not None:
             self._host_sampler()._resync(src, dst, eid0, times)
         _lib.check(rc, f"{type(self).__name__}.{what}")
+
+    # ---- the resident step: batch b of the edge stream uploaded at construction ----------------------------------------
+    def _adopt_plan(self, plan: dict):
+        """The per-batch plan of the resident stream (peer.batch_plan) as the attributes the resident step reads; the
+        batch node lists are uploaded once."""
+        self.num_batches = plan["num_batches"]
+        self.batch_lo, self.n_edges, self.batch_tmax, self.ids_off = plan["lo"], plan["n_edges"], plan["tmax"], plan["ids_off"]
+        self.ids = torch.from_numpy(plan["ids"]).to(self.dev)
+
+    def _check_stream_ids(self, ids: np.ndarray, V1: int):
+        """IndexError when the resident stream's batch nodes `ids` fall outside the table's V1 rows or the sampler's rows, or
+        the sampler knows more rows than the table. Made once, when a layout adopts its state: the resident step reads and
+        WRITES table rows by these ids, and the reference raises IndexError for an unknown node at its first lookup (Q8)."""
+        if not len(ids):
+            return
+        lo_id, hi_id = int(ids.min()), int(ids.max())
+        if lo_id < 0 or hi_id >= V1:
+            raise IndexError(f"edge stream holds node id {hi_id if hi_id >= V1 else lo_id} but the PE table has {V1} rows")
+        samp = self._host_sampler()
+        if samp is not None and hi_id >= samp.num_rows:
+            raise IndexError(f"list index out of range: node id {hi_id} is unknown to the neighbor sampler ({samp.num_rows} rows)")
+        if samp is not None and samp.num_rows > V1:
+            raise IndexError(f"pe has {V1} rows but the sampler knows node ids up to {samp.num_rows - 1}")
+
+    def share_of(self, n: int):
+        """(q_off, q_rows): the edges of a batch of n whose a6 queries (and step_host row sums) this layout computes."""
+        return 0, n
+
+    def _step(self, b: int, queries, out: torch.Tensor = None, phases: int = 7, batch_idx: int = None) -> torch.Tensor:
+        """Issue `phases` of the step on batch b of the resident stream. queries: device int64 tensors with the ids of ALL
+        edges of the batch, of which this layout reads its share (share_of). out: a caller buffer, of which a prefix is viewed
+        as the result [C, q_rows, d], or None for a new one. The call with bit 2 advances the state, as in _host_phase."""
+        lo, n = int(self.batch_lo[b]), int(self.n_edges[b])
+        q_off, q_rows = self.share_of(n)
+        C = len(queries)
+        if out is None:
+            out = torch.empty((max(C, 1), q_rows, self.d), dtype=torch.float32, device=self.dev)
+        else:
+            out = out.view(-1)[:max(C, 1) * q_rows * self.d].view(max(C, 1), q_rows, self.d)
+        bi = self.batch_idx if batch_idx is None else batch_idx
+        i0, i1 = int(self.ids_off[b]), int(self.ids_off[b + 1])
+        with torch.cuda.device(self.dev), torch.no_grad():
+            G = self.model._collapsed_filter(filter_len(bi, self.len, self.T), False)
+            ws = self._workspace(i1 - i0, n, C)
+            qptrs = (C_void_p * max(C, 1))(*[q.data_ptr() + 8 * q_off for q in queries])
+            rc = self._step_call(b, lo, n, self.ids.data_ptr() + 8 * i0, i1 - i0, float(self.batch_tmax[b]), G, qptrs, C, q_off, q_rows,
+                                 out, ws, phases)
+        if rc != 0:
+            _lib.check(rc, f"{type(self).__name__}.step")
+        if phases & 4:
+            self.batch_idx = bi
+            self._advance(1, n)
+        return out
 
     def _advance(self, steps: int, edges: int, C: int = None):
         """Move the window (changelog.advance), batch_idx and the step and edge counters by `steps` steps of `edges` edges.

@@ -23,7 +23,7 @@ import torch
 
 from . import _lib
 from . import checkpoint as ckpt
-from .changelog import ChangeLogHistory, filter_len
+from .changelog import ChangeLogHistory
 from .hostfeed import HostFed, host_arrays
 from .model import LSTEP
 from .sampler import NeighborSampler, check_edges
@@ -60,30 +60,34 @@ class _DevMem:
             self.ptr = 0
 
 
+def batch_plan(src: np.ndarray, dst: np.ndarray, t: np.ndarray, start: int, stop: int, B: int, world: int = 1, rank: int = 0) -> dict:
+    """Host-side plan of the resident edge stream: edges [start, stop) of (src, dst, t) in batches of B, for rank `rank` of a
+    peer group of `world` (a single GPU is the group of one). Pure numpy: CPU-testable. Per batch b: `lo` its first edge,
+    `n_edges`, `tmax` its largest time, `share` the edges [q_off, q_off + q_rows) of it whose a6 queries this rank computes
+    (share_of); `ids` the sorted unique batch nodes (replicated on every rank), `mine` the ones this rank owns (v % world ==
+    rank), `pos` their positions in the batch's ids (where the owner stores a node's row in the peers' buffers). The lists are
+    concatenated, batch b's ids at ids[ids_off[b]:ids_off[b + 1]], its owned ones at mine_off[b]. The owners' lists
+    partition each batch's ids, the shares partition the batch."""
+    lo = np.arange(start, stop, B, dtype=np.int64)
+    n_edges = np.minimum(lo + B, stop) - lo
+    ids_l, tmax = [], np.empty(len(lo), np.float64)
+    for b, (a, z) in enumerate(zip(lo.tolist(), (lo + n_edges).tolist())):
+        ids_l.append(np.unique(np.concatenate([src[a:z], dst[a:z]])))
+        tmax[b] = t[a:z].max()
+    nb = len(lo)
+    ids = np.concatenate(ids_l).astype(np.int64, copy=False) if nb else np.zeros(0, np.int64)
+    ids_off = np.concatenate([[0], np.cumsum([len(x) for x in ids_l], dtype=np.int64)])
+    own = np.nonzero(ids % world == rank)[0]
+    of_batch = np.repeat(np.arange(nb), np.diff(ids_off))[own]
+    mine_off = np.concatenate([[0], np.cumsum(np.bincount(of_batch, minlength=nb), dtype=np.int64)])
+    return dict(num_batches=nb, lo=lo, n_edges=n_edges, tmax=tmax, share=[share_of(int(n), world, rank) for n in n_edges], ids=ids,
+                ids_off=ids_off, mine=ids[own], pos=own - ids_off[of_batch], mine_off=mine_off)
+
+
 def peer_batch_plan(src: np.ndarray, dst: np.ndarray, batch_size: int, world: int, rank: int) -> dict:
-    """Host-side plan of a resident edge stream for one rank of a peer group (pure numpy: CPU-testable). Per batch b of
-    `batch_size` edges: `ids` = the sorted unique batch nodes (replicated on every rank), `mine` = the ones this rank owns
-    (v % world == rank), `pos` = their positions in `ids` (where the owner stores a node's row in the peers' buffers), and the
-    share [q_off, q_off + q_rows) of the batch's edges whose a6 queries this rank computes. The owners' lists partition `ids`, the
-    shares partition the batch. Returns the concatenated lists with their offsets."""
-    n = len(src)
-    nb = (n + batch_size - 1) // batch_size
-    ids_l, mine_l, pos_l, share = [], [], [], []
-    ids_off, mine_off = [0], [0]
-    for b in range(nb):
-        lo, hi = b * batch_size, min((b + 1) * batch_size, n)
-        ids = np.unique(np.concatenate([src[lo:hi], dst[lo:hi]]))
-        pos = np.nonzero(ids % world == rank)[0].astype(np.int64)
-        ids_l.append(ids)
-        mine_l.append(ids[pos])
-        pos_l.append(pos)
-        ids_off.append(ids_off[-1] + len(ids))
-        mine_off.append(mine_off[-1] + len(pos))
-        m = hi - lo
-        share.append((rank * m // world, (rank + 1) * m // world - rank * m // world))
-    cat = lambda xs: np.concatenate(xs).astype(np.int64) if xs else np.zeros(0, np.int64)
-    return dict(num_batches=nb, ids=cat(ids_l), mine=cat(mine_l), pos=cat(pos_l), ids_off=np.asarray(ids_off, np.int64),
-                mine_off=np.asarray(mine_off, np.int64), share=share)
+    """batch_plan of the whole of (src, dst) in batches of batch_size for rank `rank` of `world`, where only the node lists
+    and the shares are wanted: the times are taken as zero."""
+    return batch_plan(src, dst, np.zeros(len(src)), 0, len(src), batch_size, world, rank)
 
 
 def share_of(n: int, world: int, rank: int):
@@ -125,7 +129,7 @@ def check_host_batch(src, dst, times, query_ids, V1: int, batch_size: int, ids=N
 class PeerRank(HostFed):
     """Rank `rank` of `world` (see the module docstring). src / dst / t: the whole edge stream (replicated, device or host
     arrays); the per-batch plan (sorted unique batch nodes, the owned ones and their positions) of the resident stream
-    [start, stop) is computed once, like PEStream's. src = dst = t = None: no resident stream; the rank then serves host-fed
+    [start, stop) is computed and its ids are checked once, like PEStream's. src = dst = t = None: no resident stream; the rank then serves host-fed
     steps (step_host_async / step_host / run_host), online with ingest=True into its own growable `sampler`
     (NeighborSampler.growable; every rank holds its own CSR replica, so each rank needs a sampler of its own).
 
@@ -191,25 +195,14 @@ class PeerRank(HostFed):
             self.new_rows = self._mem_rows.tensor((2 * B, d), torch.float32, dev)
             self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.tt.data_ptr(), None, self.cur.data_ptr(), self.V1, T, d,
                                           self.row_cap)
-            # ---- per-batch plan of the resident stream: one pass on the host, uploaded once
-            src_h = self.src[self.start:stop].cpu().numpy()
-            dst_h = self.dst[self.start:stop].cpu().numpy()
-            t_h = self.tt[self.start:stop].cpu().numpy()
-            self.num_batches = nb = (stop - self.start + B - 1) // B
-            plan = peer_batch_plan(src_h, dst_h, B, G, self.rank)
-            assert plan["num_batches"] == nb
-            lo_l, n_l, tmax = [], [], []
-            for b in range(nb):
-                lo, hi = b * B, min((b + 1) * B, stop - self.start)
-                lo_l.append(self.start + lo)
-                n_l.append(hi - lo)
-                tmax.append(float(t_h[lo:hi].max()))
-            if len(plan["ids"]) and int(plan["ids"].max()) >= self.V1:
-                raise IndexError("edge stream holds a node id outside the PE table")
-            up = lambda a: torch.from_numpy(a).to(dev)
-            self.ids, self.ids_mine, self.pos_mine = up(plan["ids"]), up(plan["mine"]), up(plan["pos"])
-            self.ids_off, self.mine_off = plan["ids_off"], plan["mine_off"]
-            self.lo, self.n_edges, self.tmax = np.asarray(lo_l, np.int64), np.asarray(n_l, np.int64), np.asarray(tmax, np.float64)
+            # ---- per-batch plan of the resident stream: one pass on the host (over [start, stop) only), uploaded once
+            part = lambda a: a[self.start:stop].cpu().numpy()
+            plan = batch_plan(part(self.src), part(self.dst), part(self.tt), 0, stop - self.start, B, G, self.rank)
+            plan["lo"] += self.start
+            self._check_stream_ids(plan["ids"], self.V1)
+            self._adopt_plan(plan)
+            self.ids_mine, self.pos_mine = torch.from_numpy(plan["mine"]).to(dev), torch.from_numpy(plan["pos"]).to(dev)
+            self.mine_off = plan["mine_off"]
             self.ws = self._new_ws(self.row_cap)
         self.batch_idx, self.steps_done, self.edges_done = 0, 0, self.start
         self.epoch = ctypes.c_uint32(0)  # (a fresh rank: the flag blocks are zeroed by lstep_ipc_alloc)
@@ -314,38 +307,26 @@ class PeerRank(HostFed):
 
     # ---- the step -------------------------------------------------------------------------------------------------------
     def batch(self, b: int):
-        return int(self.lo[b]), int(self.lo[b] + self.n_edges[b])
+        lo = int(self.batch_lo[b])
+        return lo, lo + int(self.n_edges[b])
 
     def share(self, b: int):
         """(q_off, q_rows): this rank's share of the batch's edges for the a6 queries."""
-        n = int(self.n_edges[b])
-        return self.rank * n // self.G, (self.rank + 1) * n // self.G - self.rank * n // self.G
+        return self.share_of(int(self.n_edges[b]))
 
     def step(self, b: int, queries, out: torch.Tensor = None, phases: int = 7) -> torch.Tensor:
         """One step on batch b. queries: device int64 tensors with the ids of ALL edges of the batch (this rank reads its
         share). Returns [C, q_rows, d]. phases: see lstep_pe_step_peer (7 = whole step; the state advances with bit 2)."""
         assert self.grp is not None, "set_group / connect_ipc first"
-        lib, m, T, d = self.lib, self.model, self.T, self.d
-        lo, hi = self.batch(b)
-        q_off, q_rows = self.share(b)
-        C = len(queries)
-        i0, i1 = int(self.ids_off[b]), int(self.ids_off[b + 1])
-        m0, m1 = int(self.mine_off[b]), int(self.mine_off[b + 1])
-        with torch.cuda.device(self.dev), torch.no_grad():
-            Gt = m._collapsed_filter(filter_len(self.batch_idx, self.len, T), False)
-            if out is None:
-                out = torch.empty((max(C, 1), q_rows, d), dtype=torch.float32, device=self.dev)
-            qptrs = (ctypes.c_void_p * max(C, 1))(*[q.data_ptr() + 8 * q_off for q in queries])
-            i64p = lambda t_, o: ctypes.c_void_p(t_.data_ptr() + 8 * o)
-            _lib.check(lib.lstep_pe_step_peer(ctypes.byref(self.desc), self.changelog.ref, self.sampler.csr_ref, ctypes.byref(self.grp), lo, hi - lo,
-                                              i64p(self.ids, i0), i1 - i0, i64p(self.ids_mine, m0), i64p(self.pos_mine, m0), m1 - m0,
-                                              float(self.tmax[b]), self.head, self.len, _lib.ptr(Gt), qptrs, C, q_off, q_rows, _lib.ptr(out), self.K,
-                                              m._mlp_ref("nbr"), m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(),
-                                              _lib.ptr(self.sampler._err), self.epoch.value, self.timeout_ms, phases, _lib.stream_ptr()),
-                       "lstep_pe_step_peer")
-        if phases & 4:
-            self._advance(1, hi - lo)
-        return out
+        return self._step(b, queries, out, phases)
+
+    def _step_call(self, b, lo, n, ids, n_ids, tmax, G, qptrs, C, q_off, q_rows, out, ws, phases) -> int:
+        m, m0, m1 = self.model, int(self.mine_off[b]), int(self.mine_off[b + 1])
+        return self.lib.lstep_pe_step_peer(ctypes.byref(self.desc), self.changelog.ref, self.sampler.csr_ref, ctypes.byref(self.grp), lo, n, ids,
+                                           n_ids, self.ids_mine.data_ptr() + 8 * m0, self.pos_mine.data_ptr() + 8 * m0, m1 - m0, tmax, self.head,
+                                           self.len, _lib.ptr(G), qptrs, C, q_off, q_rows, _lib.ptr(out), self.K, m._mlp_ref("nbr"),
+                                           m._mlp_ref("update"), _lib.ptr(ws), ws.numel(), _lib.ptr(self.sampler._err), self.epoch.value,
+                                           self.timeout_ms, phases, _lib.stream_ptr())
 
     def _advance(self, steps: int, edges: int, C: int = None):
         """HostFed._advance, and the epoch of the step barriers: two per step."""
@@ -362,17 +343,14 @@ class PeerRank(HostFed):
         if out is None:
             out = torch.empty((max(C, 1), self.B // self.G + 1, d), dtype=torch.float32, device=self.dev)
         qptrs = (ctypes.c_void_p * max(C, 1))(*[q.data_ptr() for q in query_arrays])
-        ap = lambda a, o: a[o:].ctypes.data_as(ctypes.c_void_p)
+        ap = lambda a: a[b0:].ctypes.data_as(ctypes.c_void_p)
         head, epoch = ctypes.c_int(self.head), ctypes.c_uint32(self.epoch.value)
-        ids_off = np.ascontiguousarray(self.ids_off[b0:b0 + n_steps + 1])
-        mine_off = np.ascontiguousarray(self.mine_off[b0:b0 + n_steps + 1])
-        lo = np.ascontiguousarray(self.lo[b0:b0 + n_steps])
         with torch.cuda.device(self.dev), torch.no_grad():
             Gt = m._collapsed_filter(self.T, False)
             rc = lib.lstep_pe_steps_peer(ctypes.byref(self.desc), self.changelog.ref, self.sampler.csr_ref, ctypes.byref(self.grp), n_steps,
-                                         ap(lo, 0), ap(self.n_edges, b0), ap(self.tmax, b0), _lib.ptr(self.ids), ap(ids_off, 0),
-                                         _lib.ptr(self.ids_mine), _lib.ptr(self.pos_mine), ap(mine_off, 0), ctypes.byref(head), _lib.ptr(Gt), qptrs,
-                                         ap(lo, 0), C, _lib.ptr(out), int(out_step_stride), self.K, m._mlp_ref("nbr"),
+                                         ap(self.batch_lo), ap(self.n_edges), ap(self.batch_tmax), _lib.ptr(self.ids), ap(self.ids_off),
+                                         _lib.ptr(self.ids_mine), _lib.ptr(self.pos_mine), ap(self.mine_off), ctypes.byref(head), _lib.ptr(Gt), qptrs,
+                                         ap(self.batch_lo), C, _lib.ptr(out), int(out_step_stride), self.K, m._mlp_ref("nbr"),
                                          m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(), _lib.ptr(self.sampler._err),
                                          ctypes.byref(epoch), self.timeout_ms, _lib.stream_ptr())
         done = ((epoch.value - self.epoch.value) & 0xffffffff) // 2  # (two barrier epochs per applied step)
@@ -393,9 +371,6 @@ class PeerRank(HostFed):
         every rank rejects it, before any rank enqueues anything (a run is validated whole: n_max is its length)."""
         assert self.grp is not None, "set_group / connect_ipc first"
         return check_host_batch(src, dst, times, qs, V1, n_max, ids)[4]
-
-    def _host_rows(self, n: int) -> int:
-        return self.share_of(n)[1]
 
     def _workspace(self, n_ids: int, n_edges: int, C: int) -> torch.Tensor:
         return self.ws  # (sized for batch_size edges and 8 query sets, the most check_host_batch lets through)

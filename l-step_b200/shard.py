@@ -32,6 +32,7 @@ from . import _lib
 from . import checkpoint as ckpt
 from .changelog import ChangeLogHistory, advance, filter_len
 from .model import LSTEP
+from .peer import batch_plan
 from .sampler import NeighborSampler
 
 
@@ -431,34 +432,29 @@ class ReplicatedTableRank:
                 ring_ptr = None
             self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.tt.data_ptr(), ring_ptr, self.cur.data_ptr(),
                                           self.V1, self.T, self.d)
-            # ---- per-batch plan of the resident stream [start, stop): one pass on the host, uploaded once
+            # ---- per-batch plan of the resident stream [start, stop) (batch_plan) and the scatter lists of the all-gather:
+            # one pass on the host, uploaded once
             B, G = self.B, self.G
-            src_h = self.src[self.start:stop].cpu().numpy()
-            dst_h = self.dst[self.start:stop].cpu().numpy()
-            t_h = self.tt[self.start:stop].cpu().numpy()
-            self.num_batches = nb = (stop - self.start + B - 1) // B
-            ids_l, mine_l, scat_l = [], [], []
-            self.ids_off, self.mine_off, self.scat_off, self.max_n, self.tmax = [0], [0], [0], [], []
-            for b in range(nb):
-                lo, hi = b * B, min((b + 1) * B, stop - self.start)
-                ids = np.unique(np.concatenate([src_h[lo:hi], dst_h[lo:hi]]))
+            part = lambda a: a[self.start:stop].cpu().numpy()
+            plan = batch_plan(part(self.src), part(self.dst), part(self.tt), 0, stop - self.start, B, G, self.rank)
+            self.num_batches, self.ids_off, self.mine_off, self.tmax = plan["num_batches"], plan["ids_off"], plan["mine_off"], plan["tmax"]
+            scat_l, self.scat_off, self.max_n = [], [0], []
+            for b in range(self.num_batches):
+                ids = plan["ids"][self.ids_off[b]:self.ids_off[b + 1]]
                 own = ids % G
                 counts = np.bincount(own, minlength=G)
-                mx = int(counts.max()) if len(ids) else 0
-                scat = np.full((G, max(mx, 1)), self.V1, dtype=np.int64)  # padded slots -> the spare row
+                mx = max(int(counts.max()), 1)
+                scat = np.full((G, mx), self.V1, dtype=np.int64)  # padded slots -> the spare row
                 for g in range(G):
                     scat[g, :counts[g]] = ids[own == g]
-                ids_l.append(ids)
-                mine_l.append(ids[own == self.rank] // G if history == "ring" else ids[own == self.rank])  # ring rows / global ids
                 scat_l.append(scat.reshape(-1))
-                self.ids_off.append(self.ids_off[-1] + len(ids))
-                self.mine_off.append(self.mine_off[-1] + len(mine_l[-1]))
                 self.scat_off.append(self.scat_off[-1] + scat.size)
-                self.max_n.append(max(mx, 1))
-                self.tmax.append(float(t_h[lo:hi].max()))
-            cat = lambda xs: torch.from_numpy(np.concatenate(xs) if xs else np.zeros(0, np.int64)).to(dev)
-            self.ids, self.mine_local, self.scat = cat(ids_l), cat(mine_l), cat(scat_l)
-            if len(ids_l) and int(max(x.max() for x in ids_l if len(x))) >= self.V1:
+                self.max_n.append(mx)
+            up = lambda a: torch.from_numpy(a).to(dev)
+            mine = plan["mine"] // G if history == "ring" else plan["mine"]  # ring rows / global ids
+            self.ids, self.mine_local = up(plan["ids"]), up(mine)
+            self.scat = up(np.concatenate(scat_l) if scat_l else np.zeros(0, np.int64))
+            if len(plan["ids"]) and int(plan["ids"].max()) >= self.V1:
                 raise IndexError("edge stream holds a node id outside the PE table")
             need = lib.lstep_pe_step_workspace_bytes(2 * B, B, 8, self.K, self.d, self.t_dim, self.V1)
             self.ws = torch.empty(need + 4096, dtype=torch.uint8, device=dev)

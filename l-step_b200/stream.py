@@ -27,9 +27,10 @@ import torch
 
 from . import _lib
 from . import checkpoint as ckpt
-from .changelog import ChangeLogHistory, filter_len
+from .changelog import ChangeLogHistory
 from .hostfeed import HostFed
 from .model import LSTEP
+from .peer import batch_plan
 
 C_void_p = ctypes.c_void_p
 C_byref = ctypes.byref
@@ -62,18 +63,9 @@ class PEStream(HostFed):
         self.t = torch.from_numpy(self.t_np).to(dev)
         # per-batch sorted unique node ids (the loops compute them on the host with torch.unique:
         # evaluate_model_utils.py:54-55); done once for the whole stream here
-        self.batch_lo = list(range(self.start, self.stop, self.B))
-        ids, off = [], [0]
-        for lo in self.batch_lo:
-            hi = min(lo + self.B, self.stop)
-            u = np.unique(np.concatenate([self.src_np[lo:hi], self.dst_np[lo:hi]]))
-            ids.append(u)
-            off.append(off[-1] + len(u))
-        self.ids_off = off
-        self.ids_np = np.concatenate(ids) if ids else np.zeros(0, np.int64)
-        self.ids = torch.from_numpy(self.ids_np).to(dev)
-        self.num_batches = len(self.batch_lo)
-        self.batch_tmax = [float(self.t_np[lo:min(lo + self.B, self.stop)].max()) for lo in self.batch_lo]
+        plan = batch_plan(self.src_np, self.dst_np, self.t_np, self.start, self.stop, self.B)
+        self.ids_np = plan["ids"]
+        self._adopt_plan(plan)
         self._host_init()
         self._growth_init(new_node_pe, max_nodes)
         self._row_cap_arg = row_capacity
@@ -93,17 +85,7 @@ class PEStream(HostFed):
         if Th > self.T:
             history = history[:, -self.T:, :]
             Th = self.T
-        # ids of the resident stream against the table and the sampler's CSR, once (the device-resident step reads and WRITES
-        # table / ring rows by these ids; the reference raises IndexError for an unknown node at its first lookup, Q8)
-        if len(self.ids_np):
-            lo_id, hi_id = int(self.ids_np.min()), int(self.ids_np.max())
-            if lo_id < 0 or hi_id >= V1:
-                raise IndexError(f"edge stream holds node id {hi_id if hi_id >= V1 else lo_id} but the PE table has {V1} rows")
-            samp = self.model.neighbor_sampler
-            if samp is not None and hi_id >= samp.num_rows:
-                raise IndexError(f"list index out of range: node id {hi_id} is unknown to the neighbor sampler ({samp.num_rows} rows)")
-            if samp is not None and samp.num_rows > V1:
-                raise IndexError(f"pe has {V1} rows but the sampler knows node ids up to {samp.num_rows - 1}")
+        self._check_stream_ids(self.ids_np, V1)
         self.V1 = V1
         self.row_cap = max(V1, int(self._row_cap_arg or 0))
         self.ring = torch.zeros((self.row_cap, self.T, d), dtype=torch.float32, device=self.dev)  # node-major: 68.8 KB / node
@@ -139,9 +121,8 @@ class PEStream(HostFed):
 
     # ---- one batch --------------------------------------------------------------------------
     def batch_arrays(self, b: int):
-        lo = self.batch_lo[b]
-        hi = min(lo + self.B, self.stop)
-        return lo, hi, self.ids_off[b], self.ids_off[b + 1]
+        lo = int(self.batch_lo[b])
+        return lo, lo + int(self.n_edges[b]), int(self.ids_off[b]), int(self.ids_off[b + 1])
 
     def _workspace(self, n_ids, n_edges, C):
         cap = self._ws_cap
@@ -158,23 +139,6 @@ class PEStream(HostFed):
                        "workspace_init")
         return self._ws
 
-    def _run(self, lo, n_edges, ids, tmax, queries, out, batch_idx):
-        """Device-resident core of step()."""
-        m = self.model
-        bi = self.batch_idx if batch_idx is None else batch_idx
-        C = len(queries)
-        with torch.cuda.device(self.dev), torch.no_grad():
-            G = m._collapsed_filter(filter_len(bi, self.len, self.T), False)
-            ws = self._workspace(ids.shape[0], n_edges, C)
-            qptrs = (C_void_p * max(C, 1))(*[q.data_ptr() for q in queries])
-            slot = (self.head + self.len) % self.T  # (the slot changelog.advance writes: the next free one, then the oldest)
-            _lib.check(self.lib.lstep_pe_step(self._desc_ref, m.neighbor_sampler.csr_ref, lo, n_edges, _lib.ptr(ids), ids.shape[0],
-                                              float(tmax), self.head, self.len, slot, _lib.ptr(G), qptrs, C, _lib.ptr(out), self.K,
-                                              m._mlp_ref("nbr"), m._mlp_ref("update"), _lib.ptr(ws), ws.numel(),
-                                              _lib.ptr(m.neighbor_sampler._err), _lib.stream_ptr()), "lstep_pe_step")
-        self.batch_idx = bi
-        self._advance(1, n_edges)
-
     @property
     def _desc_ref(self):
         return C_byref(self.desc)
@@ -184,45 +148,46 @@ class PEStream(HostFed):
         for the compute_neighborhood_pe calls (positive sources / destinations, negatives), all queried
         at the batch's edge times. Returns a [C, B_b, d] tensor of neighbourhood PEs; the updated
         table is self.cur and has been appended to the ring."""
-        lo, hi, io, ie = self.batch_arrays(b)
-        n = hi - lo
-        C = len(queries)
-        if out is None:
-            out = torch.empty((max(C, 1), n, self.d), dtype=torch.float32, device=self.dev)
-        else:
-            out = out.view(-1)[:max(C, 1) * n * self.d].view(max(C, 1), n, self.d)
-        self._run(lo, n, self.ids[io:ie], self.batch_tmax[b], queries, out, batch_idx)
-        return out
+        return self._step(b, queries, out, 7, batch_idx)
+
+    def _step_call(self, b, lo, n, ids, n_ids, tmax, G, qptrs, C, q_off, q_rows, out, ws, phases) -> int:
+        m = self.model
+        slot = (self.head + self.len) % self.T  # (the slot changelog.advance writes: the next free one, then the oldest)
+        return self.lib.lstep_pe_step(self._desc_ref, m.neighbor_sampler.csr_ref, lo, n, ids, n_ids, tmax, self.head, self.len, slot,
+                                      _lib.ptr(G), qptrs, C, _lib.ptr(out), self.K, m._mlp_ref("nbr"), m._mlp_ref("update"), _lib.ptr(ws),
+                                      ws.numel(), _lib.ptr(m.neighbor_sampler._err), _lib.stream_ptr())
 
     def run(self, b0: int, n_steps: int, queries, out: torch.Tensor = None, check: bool = False) -> torch.Tensor:
         """Batches b0 .. b0+n_steps-1 of the resident stream in ONE native call (lstep_pe_steps): the per-batch loop
         runs in C, so the host pays six kernel launches per step and nothing else. `queries`: list of device int64
         tensors holding, for every query set, the node ids of ALL edges of those batches back to back (entry e belongs
-        to edge lo(b0) + e). Returns the neighbourhood PEs of the LAST step [C, n_last, d] (or fills `out`
-        [n_steps, C, B, d] with every step's). While the history ring is still filling, falls back to step().
+        to edge lo(b0) + e). Returns the neighbourhood PEs of the LAST step [C, n_last, d] (or fills and returns `out`
+        [n_steps, C, B, d] with every step's). While the history is still filling, and on a history without a native
+        multi-step call (ChangeLogStream), it calls step() per batch.
         check=True: read the device error flag afterwards (synchronises; IndexError for a query id unknown to the sampler)."""
         if n_steps <= 0:
             return None
-        lo0 = self.batch_lo[b0]
-        C = len(queries)
-        if self.len < self.T:
-            last = None
+        if self.len == self.T and self._run_call is not None:
+            last = self._run_call(b0, n_steps, queries, out)
+        else:
+            lo0 = int(self.batch_lo[b0])
             for i in range(n_steps):
                 lo, hi, _, _ = self.batch_arrays(b0 + i)
                 last = self.step(b0 + i, [q[lo - lo0:hi - lo0] for q in queries], None if out is None else out[i])
-            return last
+        if check:
+            self.check_errors()
+        return out if out is not None else last
+
+    def _run_call(self, b0: int, n_steps: int, queries, out: torch.Tensor = None) -> torch.Tensor:
+        """run() on a full history: one lstep_pe_steps call. Returns the last step's neighbourhood PEs."""
         lib, m = self.lib, self.model
-        B, d = self.B, self.d
-        los = np.asarray(self.batch_lo[b0:b0 + n_steps], dtype=np.int64)
-        his = np.minimum(los + B, self.stop)
-        ne = (his - los).astype(np.int64)
-        ids_off = np.asarray(self.ids_off[b0:b0 + n_steps + 1], dtype=np.int64)
-        tmax = np.asarray(self.batch_tmax[b0:b0 + n_steps], dtype=np.float64)
-        q_off = (los - lo0).astype(np.int64)
-        n_ids_max = int(np.diff(ids_off).max())
+        B, d, C = self.B, self.d, len(queries)
+        los, ne, tmax = (a[b0:b0 + n_steps] for a in (self.batch_lo, self.n_edges, self.batch_tmax))
+        ids_off = self.ids_off[b0:b0 + n_steps + 1]
+        q_off = los - los[0]
         with torch.cuda.device(self.dev), torch.no_grad():
             G = m._collapsed_filter(self.T, False)
-            ws = self._workspace(n_ids_max, int(ne.max()), C)
+            ws = self._workspace(int(np.diff(ids_off).max()), int(ne.max()), C)
             if out is None:
                 buf = torch.empty((max(C, 1), B, d), dtype=torch.float32, device=self.dev)
                 stride = 0
@@ -242,10 +207,6 @@ class PEStream(HostFed):
             self._advance(done, int(ne[:done].sum()))
             if rc != 0:
                 _lib.check(rc, "lstep_pe_steps")
-        if check:
-            self.check_errors()
-        if out is not None:
-            return out
         n_last = int(ne[-1])
         return buf.view(-1)[:max(C, 1) * n_last * d].view(max(C, 1), n_last, d)
 
@@ -268,17 +229,14 @@ class PEStream(HostFed):
 
     # ---- host-fed steps: step_host_async / step_host / run_host and result are hostfeed.HostFed's, which validates, stages,
     # arms the ingest, moves the window and keeps the tickets around the native calls of csrc/host_step.cu below. A layout
-    # supplies its own checks of a batch, these two native calls, the rows per query of a result and its workspace;
-    # ChangeLogStream replaces the checks and the calls. Each call returns the native status.
+    # supplies its own checks of a batch, these two native calls and its workspace; ChangeLogStream replaces the checks and
+    # the calls. Each call returns the native status.
     def _host_sampler(self):
         return self.model.neighbor_sampler
 
     def _check_host(self, src, dst, times, qs, ids, V1: int, n_max: int):
         """None beyond the shared checks: the native stager rejects ids outside the table and the sampler's rows."""
         return None if ids is None else np.ascontiguousarray(ids, dtype=_I64)
-
-    def _host_rows(self, n: int) -> int:
-        return n
 
     def _host_step_call(self, h, n, src, dst, times, ids, G, qptrs, C, out, ws, phases, ticket) -> int:
         m, samp = self.model, self.model.neighbor_sampler
@@ -345,13 +303,7 @@ class ChangeLogStream(PEStream):
     def _load(self, hist: "ckpt.History"):
         """Allocate the change log for hist.V1 rows and load `hist` into it."""
         V1, d = hist.V1, self.d
-        if len(self.ids_np):
-            lo_id, hi_id = int(self.ids_np.min()), int(self.ids_np.max())
-            if lo_id < 0 or hi_id >= V1:
-                raise IndexError(f"edge stream holds node id {hi_id if hi_id >= V1 else lo_id} but the PE table has {V1} rows")
-            samp = self.model.neighbor_sampler
-            if samp is not None and (hi_id >= samp.num_rows or samp.num_rows > V1):
-                raise IndexError("list index out of range: the neighbor sampler's rows do not cover the stream / exceed the table")
+        self._check_stream_ids(self.ids_np, V1)
         self.row_cap = max(V1, int(self._row_cap_arg or 0))
         cap = self._cap_arg if self._cap_arg is not None else self._default_event_cap(max(self.row_cap, self.max_nodes or 0))
         self.changelog = ChangeLogHistory(V1, self.T, d, cap, 1, 0, self.dev, self.row_cap)
@@ -405,31 +357,14 @@ class ChangeLogStream(PEStream):
         self.changelog.check_full(samp._err, int(samp._err.item()))
         samp.check_errors()
 
-    def _run(self, lo, n_edges, ids, tmax, queries, out, batch_idx):
+    def _step_call(self, b, lo, n, ids, n_ids, tmax, G, qptrs, C, q_off, q_rows, out, ws, phases) -> int:
         m = self.model
-        bi = self.batch_idx if batch_idx is None else batch_idx
-        C = len(queries)
-        with torch.cuda.device(self.dev), torch.no_grad():
-            G = m._collapsed_filter(filter_len(bi, self.len, self.T), False)
-            ws = self._workspace(ids.shape[0], n_edges, C)
-            qptrs = (C_void_p * max(C, 1))(*[q.data_ptr() for q in queries])
-            _lib.check(self.lib.lstep_pe_step_changelog(self._desc_ref, self.changelog.ref, m.neighbor_sampler.csr_ref, lo, n_edges,
-                                                        _lib.ptr(ids), ids.shape[0], float(tmax), self.head, self.len, _lib.ptr(G), qptrs,
-                                                        C, 0, -1, _lib.ptr(out), self.K, m._mlp_ref("nbr"), m._mlp_ref("update"),
-                                                        _lib.ptr(ws), ws.numel(), _lib.ptr(m.neighbor_sampler._err), _lib.stream_ptr(), 0),
-                       "lstep_pe_step_changelog")
-        self.batch_idx = bi
-        self._advance(1, n_edges)
+        return self.lib.lstep_pe_step_changelog(self._desc_ref, self.changelog.ref, m.neighbor_sampler.csr_ref, lo, n, ids, n_ids, tmax,
+                                                self.head, self.len, _lib.ptr(G), qptrs, C, q_off, q_rows, _lib.ptr(out), self.K,
+                                                m._mlp_ref("nbr"), m._mlp_ref("update"), _lib.ptr(ws), ws.numel(),
+                                                _lib.ptr(m.neighbor_sampler._err), _lib.stream_ptr(), 0)
 
-    def run(self, b0: int, n_steps: int, queries, out: torch.Tensor = None, check: bool = False):
-        lo0 = self.batch_lo[b0]
-        last = None
-        for i in range(n_steps):  # (no native multi-step call for this history: one C call per step)
-            lo, hi, _, _ = self.batch_arrays(b0 + i)
-            last = self.step(b0 + i, [q[lo - lo0:hi - lo0] for q in queries], None if out is None else out[i])
-        if check:
-            self.check_errors()
-        return out if out is not None else last
+    _run_call = None  # (no native multi-step call for this history: run() calls step() per batch)
 
     # ---- host-fed steps: HostFed's driver, with the change-log step as the native call ---------------------------------
     def _check_host(self, src, dst, times, qs, ids, V1: int, n_max: int):

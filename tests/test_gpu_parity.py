@@ -838,6 +838,54 @@ def test_device_resident_stream_rejects_out_of_range_ids(torch_cuda):
     assert torch.isfinite(ob).all()
 
 
+def test_every_layout_checks_the_resident_ids_alike(torch_cuda):
+    """PEStream, ChangeLogStream and PeerRank make the same check of their resident stream's ids when they adopt their state,
+    with the same messages: a negative id and an id past the sampler's rows (inside the table) raise IndexError at
+    construction, before a step could index the table with them."""
+    torch = torch_cuda
+    from harness import build_dropin
+    from lstep_b200 import ChangeLogStream, NeighborSampler, PEStream, PeerRank
+    g = synth.make_graph("tiny_bip", seed=5)
+    V, d, T, K, B = g.num_nodes, 172, 100, 20, 32
+    s = NeighborSampler.from_edges(g.src_node_ids, g.dst_node_ids, g.edge_ids, g.node_interact_times, "recent", num_rows=V + 1)
+    lstep = build_dropin("full", g, s, 172, d, 100, T, K)[0].eval()
+    init = torch.from_numpy(seeded_normal(11, (V + 2, d), 0.3)).cuda()  # one row more than the sampler knows
+    e0 = g.num_edges - 6 * B
+    for bad, V1, msg in ((-4, V + 1, "edge stream holds node id -4 but the PE table has"),
+                         (V + 1, V + 2, f"node id {V + 1} is unknown to the neighbor sampler")):
+        src = g.src_node_ids.copy()
+        src[-1] = bad
+        for cls in (PEStream, ChangeLogStream):
+            with pytest.raises(IndexError, match=msg):
+                cls(lstep, src, g.dst_node_ids, g.node_interact_times, B, K, initial_pe=init[:V1].clone(), start=e0)
+        with pytest.raises(IndexError, match=msg):
+            PeerRank(lstep, 0, 1, src, g.dst_node_ids, g.node_interact_times, V1 - 1, B, K, init[:V1].clone(), start=e0, sampler=s)
+
+
+@pytest.mark.parametrize("layout", ["PEStream", "ChangeLogStream"])
+def test_run_check_reads_the_error_flag_while_the_history_fills(torch_cuda, layout):
+    """run(check=True) reads the device error flag on every path: also from a history shorter than T, where run() steps
+    batch by batch, a query id the sampler does not know raises IndexError."""
+    torch = torch_cuda
+    import lstep_b200
+    from harness import build_dropin
+    from lstep_b200 import NeighborSampler
+    g = synth.make_graph("tiny_bip", seed=5)
+    V, d, T, K, B = g.num_nodes, 172, 100, 20, 32
+    s = NeighborSampler.from_edges(g.src_node_ids, g.dst_node_ids, g.edge_ids, g.node_interact_times, "recent", num_rows=V + 1)
+    lstep = build_dropin("full", g, s, 172, d, 100, T, K)[0].eval()
+    init = torch.from_numpy(seeded_normal(11, (V + 1, d), 0.3)).cuda()
+    e0 = g.num_edges - 6 * B
+    st = getattr(lstep_b200, layout)(lstep, g.src_node_ids, g.dst_node_ids, g.node_interact_times, B, K, initial_pe=init, start=e0)
+    assert st.len < st.T
+    bad = st.dst[e0:].clone()
+    bad[B + 3] = V + 1000
+    with pytest.raises(IndexError):
+        st.run(0, 3, [st.src[e0:], bad], check=True)
+    assert st.steps_done == 3
+    st.check_errors()  # (the read cleared the flag)
+
+
 def test_native_multi_step_run_and_profile_are_bit_identical_to_single_steps(torch_cuda):
     """PEStream.run (lstep_pe_steps: the per-batch loop in C) against PEStream.step, and the same steps with the per-kernel
     event profile switched on (events between the kernels serialise the chain): tables, histories and outputs are

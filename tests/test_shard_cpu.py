@@ -104,3 +104,30 @@ def test_peer_group_plan_partitions_every_batch(world):
             q_off, q_rows = pl["share"][b]
             edges[q_off:q_off + q_rows] += 1
         assert np.all(covered == 1) and np.all(edges == 1)
+
+
+@pytest.mark.parametrize("start,stop,B", [(0, None, 48), (213, 1037, 48), (5, 9, 200), (40, 40, 16)])
+def test_single_gpu_plan_equals_the_per_batch_loop(start, stop, B):
+    """The plan of a single-GPU stream (world 1: PEStream / ChangeLogStream) equals the per-batch loop it replaced, restated in
+    numpy: batches of B edges from `start` (the last one ragged), each with its first edge, edge count, largest time and
+    sorted unique nodes, concatenated with offsets."""
+    from lstep_b200.peer import batch_plan
+    g = synth.make_graph("tiny_bip", seed=3)
+    src, dst, t = g.src_node_ids, g.dst_node_ids, g.node_interact_times
+    stop = len(src) if stop is None else stop
+    pl = batch_plan(src, dst, t, start, stop, B)
+    batch_lo = list(range(start, stop, B))
+    ids, off, n_edges, tmax = [], [0], [], []
+    for lo in batch_lo:
+        hi = min(lo + B, stop)
+        u = np.unique(np.concatenate([src[lo:hi], dst[lo:hi]]))
+        ids.append(u)
+        off.append(off[-1] + len(u))
+        n_edges.append(hi - lo)
+        tmax.append(float(t[lo:hi].max()))
+    assert pl["num_batches"] == len(batch_lo)
+    assert pl["lo"].tolist() == batch_lo and pl["n_edges"].tolist() == n_edges and pl["tmax"].tolist() == tmax
+    assert pl["ids_off"].tolist() == off
+    assert np.array_equal(pl["ids"], np.concatenate(ids) if ids else np.zeros(0, np.int64))
+    for a in ("lo", "n_edges", "ids", "ids_off"):
+        assert pl[a].dtype == np.int64, a
