@@ -6,19 +6,19 @@ step_host_async, step_host, run_host and `result`. A step has two halves: `_host
 adds the nodes of grow=True and reserves room for ingest=True, writing nothing before all of it has passed; `_host_phase`
 issues phases of the step on the prepared batch (all at once, 7, except PeerLocalGroup's 1, 2 and 4 per rank) and moves the
 window and the counters (`_advance`). `_step` is the same for a batch of the resident stream, the one uploaded at
-construction, whose per-batch plan (peer.batch_plan) a layout adopts with `_adopt_plan` and checks with
-`_check_stream_ids`. A class that mixes it in provides `dev`, `B`, `d`, `T`, `model`, the window `head` / `len`, the counters
-`batch_idx` / `steps_done` / `edges_done`, and what differs between layouts: `_host_sampler()`, the sampler its steps read;
-`_check_host(...)`, its own checks of a batch; `_host_step_call`, `_host_run_call` and `_step_call`, the native host-fed
-per-step and multi-batch calls and the resident per-step call; `share_of(n)`, its share of a batch's queries (all of them on
-a single GPU); `_workspace(n_ids, n_edges, C)`.
+construction, whose per-batch plan (peer.batch_plan) a layout adopts with `_adopt_plan`.
 
-It also owns the growth of the node set (add_nodes, and grow=True on the host-fed steps): new node ids continue after the
-last live one, and a new node starts with its initial row r0 in the table, in every history slot and as its change-log base
-row, which is exactly the state a node no edge has touched has in a stream built with those rows from the start. So a grown
-stream computes the bits of the pre-sized one. The class provides `V1`, `row_cap`, `_grow_capacity(row_cap)`, which
-reallocates its tables for more rows (every new buffer allocated before any is swapped in), `_init_rows(v0, v1, rows,
-stride)`, which enqueues lstep_pe_rows_init, and `_set_live(V1)`."""
+It owns the state those steps act on, too: `_new_state` adopts a history (changelog.RingHistory or ChangeLogHistory, which
+the layout builds from its own inputs and loads) with a new table `cur`, the step descriptor and the step workspace;
+check_errors, history_bytes and export_history read it. And it owns the growth of the node set (add_nodes, and grow=True on
+the host-fed steps): new node ids continue after the last live one, and a new node starts with its initial row r0 in the
+table, in every history slot and as its change-log base row, which is exactly the state a node no edge has touched has in
+a stream built with those rows from the start. So a grown stream computes the bits of the pre-sized one.
+
+A class that mixes it in provides `dev`, `B`, `K`, `d`, `T`, `model`, `start` and the resident stream `src` / `dst` / `t` on
+the device, and what differs between layouts: `_host_sampler()`, the sampler its steps read; `_check_host(...)`, its own
+checks of a batch; `_host_step_call`, `_host_run_call` and `_step_call`, the native host-fed per-step and multi-batch calls
+and the resident per-step call; `share_of(n)`, its share of a batch's queries (all of them on a single GPU)."""
 from __future__ import annotations
 
 import ctypes
@@ -98,6 +98,55 @@ class HostFed:
                 pass
             self._host_stepper = None
 
+    # ---- the state: table, history, step descriptor, workspace --------------------------------------------------------
+    def _new_state(self, history):
+        """Adopt `history` (history.V1 live rows of history.row_cap) with a new table cur [row_cap, d] for its loader to fill,
+        the step descriptor over the resident stream and no workspace yet."""
+        self.history, self.V1, self.row_cap = history, history.V1, history.row_cap
+        self.cur = torch.empty((self.row_cap, self.d), dtype=torch.float32, device=self.dev)
+        self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.t.data_ptr(), _lib.ptr(history.ring), self.cur.data_ptr(),
+                                      self.V1, self.T, self.d, self.row_cap)
+        self._ws, self._ws_cap = None, (0, 0, 0)
+
+    def _workspace(self, n_ids: int, n_edges: int, C: int) -> torch.Tensor:
+        """The step workspace for n_ids batch nodes, n_edges edges and C query sets: reallocated only when a step needs more
+        than it holds, then sized for at least 2B ids, B edges and 4 query sets."""
+        cap = self._ws_cap
+        if self._ws is not None and n_ids <= cap[0] and n_edges <= cap[1] and C <= cap[2]:
+            return self._ws
+        need = self.lib.lstep_pe_step_workspace_bytes(n_ids, n_edges, C, self.K, self.d, self.model.time_feat_dim, self.row_cap)
+        if self._ws is None or self._ws.numel() < need:
+            self._ws_cap = (max(2 * self.B, n_ids), max(self.B, n_edges), max(C, 4))  # (ids, edges, query sets) it is sized for
+            self._ws = self._new_workspace(self.row_cap)
+        return self._ws
+
+    def _new_workspace(self, row_cap: int) -> torch.Tensor:
+        """A zeroed workspace for _ws_cap whose per-node maps cover row_cap rows."""
+        n = self.lib.lstep_pe_step_workspace_bytes(*self._ws_cap, self.K, self.d, self.model.time_feat_dim, row_cap) + 4096
+        ws = torch.empty(n, dtype=torch.uint8, device=self.dev)
+        _lib.check(self.lib.lstep_update_pe_workspace_init(_lib.ptr(ws), n, row_cap, _lib.stream_ptr()), "workspace_init")
+        return ws
+
+    def check_errors(self):
+        """Synchronising read of the device error flag the step's lookups raise for query ids outside the sampler's
+        rows (such a query yields an empty neighbourhood and reads table row 0; nothing is written by query ids).
+        Raises IndexError like the reference's lookup (utils/utils.py:140, Q8); LstepError when a step changed more rows
+        than a change log's event capacity. Called by export_history(), save_checkpoint() and run(check=True); the
+        host-fed calls validate ids on the host before anything is enqueued. Call it yourself after a loop of step()."""
+        samp = self._host_sampler()
+        self.history.check_full(samp._err, int(samp._err.item()))
+        samp.check_errors()
+
+    def history_bytes(self) -> int:
+        """Bytes the history occupies: the dense ring, or the change log's base and event rows and index structures."""
+        return self.history.nbytes()
+
+    def export_history(self) -> torch.Tensor:
+        """The history in the reference's layout [V1, len, d], oldest first (for save_pe / torch.cat; a change log is replayed,
+        which needs V1 * len * d * 4 bytes). On a PeerRank, export_history_rows: the owned rows, row l = node l * world + rank."""
+        self.check_errors()
+        return self.history.replay(self.head, self.len)
+
     # ---- node growth --------------------------------------------------------------------------------------------------
     def _growth_init(self, new_node_pe=None, max_nodes: int = None):
         """new_node_pe: the row [d] a node added without explicit rows starts with (default zeros, what RandomWalkPE gives an
@@ -128,7 +177,20 @@ class HostFed:
             raise IndexError(f"node id {hi} is outside max_nodes ({self.max_nodes})")
 
     def _check_event_capacity(self, V1: int):
-        """Change-log histories: ValueError when a step on V1 nodes could change more rows than the log records per step."""
+        """Change-log histories (changelog.ChangeLogOwner): ValueError when a step on V1 nodes could change more rows than the
+        log records per step."""
+
+    def _grow_capacity(self, row_cap: int):
+        """Reallocate the table, the history and the workspace (if there is one yet) for row_cap rows. Every new buffer is
+        allocated before any is swapped in, so that an out-of-memory error leaves the old state whole; the live rows are
+        copied on the current stream, behind the steps already enqueued."""
+        with torch.cuda.device(self.dev):
+            cur = torch.empty((row_cap, self.d), dtype=torch.float32, device=self.dev)
+            ws = None if self._ws is None else self._new_workspace(row_cap)
+            self.history.grow_capacity(row_cap)
+            cur[:self.V1].copy_(self.cur[:self.V1])
+        self.cur, self._ws, self.row_cap = cur, ws, int(row_cap)
+        self.desc.cur, self.desc.ring, self.desc.row_cap = cur.data_ptr(), _lib.ptr(self.history.ring), self.row_cap
 
     def _new_nodes_for(self, arrays) -> int:
         """grow=True: validate the ids of a batch (or a run) and return how many nodes it adds (ids up to its maximum).
@@ -171,8 +233,9 @@ class HostFed:
             k = v1 - samp.num_rows
             samp.add_rows(k, None if _edges is None else new_row_need(_edges[0], _edges[1], samp.num_rows, k))
         with torch.cuda.device(self.dev):
-            self._init_rows(v0, v1, rows, stride)
-        self._set_live(v1)
+            self.history.init_rows(self.cur, v0, v1, rows, stride)
+        self.history.add_rows(v1)
+        self.V1 = self.desc.V1 = v1
         return v0
 
     # ---- ingest -------------------------------------------------------------------------------------------------------
@@ -339,12 +402,14 @@ class HostFed:
         batch node lists are uploaded once."""
         self.num_batches = plan["num_batches"]
         self.batch_lo, self.n_edges, self.batch_tmax, self.ids_off = plan["lo"], plan["n_edges"], plan["tmax"], plan["ids_off"]
-        self.ids = torch.from_numpy(plan["ids"]).to(self.dev)
+        self.ids_np = plan["ids"]
+        self.ids = torch.from_numpy(self.ids_np).to(self.dev)
 
-    def _check_stream_ids(self, ids: np.ndarray, V1: int):
-        """IndexError when the resident stream's batch nodes `ids` fall outside the table's V1 rows or the sampler's rows, or
-        the sampler knows more rows than the table. Made once, when a layout adopts its state: the resident step reads and
+    def _check_stream_ids(self, V1: int):
+        """IndexError when the resident stream's batch nodes fall outside the table's V1 rows or the sampler's rows, or the
+        sampler knows more rows than the table. Made once, before a layout allocates its state: the resident step reads and
         WRITES table rows by these ids, and the reference raises IndexError for an unknown node at its first lookup (Q8)."""
+        ids = self.ids_np
         if not len(ids):
             return
         lo_id, hi_id = int(ids.min()), int(ids.max())

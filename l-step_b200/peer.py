@@ -22,8 +22,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from . import checkpoint as ckpt
-from .changelog import ChangeLogHistory
+from .changelog import ChangeLogOwner
 from .hostfeed import HostFed, host_arrays
 from .model import LSTEP
 from .sampler import NeighborSampler, check_edges
@@ -126,7 +125,7 @@ def check_host_batch(src, dst, times, query_ids, V1: int, batch_size: int, ids=N
     return src, dst, times, qs, ids
 
 
-class PeerRank(HostFed):
+class PeerRank(ChangeLogOwner, HostFed):
     """Rank `rank` of `world` (see the module docstring). src / dst / t: the whole edge stream (replicated, device or host
     arrays); the per-batch plan (sorted unique batch nodes, the owned ones and their positions) of the resident stream
     [start, stop) is computed and its ids are checked once, like PEStream's. src = dst = t = None: no resident stream; the rank then serves host-fed
@@ -149,114 +148,62 @@ class PeerRank(HostFed):
         self._host_init()
         self.model, self.rank, self.G = model, int(rank), int(world)
         self.dev = dev = torch.device(device) if device is not None else model._dev()
-        self.B, self.K, self.T = int(batch_size), int(num_neighbors), model.num_fft_batches
-        self.d, self.t_dim = model.pe_dim, model.time_feat_dim
+        self.B, self.K, self.T, self.d = int(batch_size), int(num_neighbors), model.num_fft_batches, model.pe_dim
         self.V1 = int(num_nodes) + 1
-        self.row_cap = max(self.V1, int(row_capacity or 0))
         self.timeout_ms = int(timeout_ms)
-        # change log of the owned nodes; its capacity is the same on every rank: the inbox blocks are laid out by it
-        G, B = self.G, self.B
-        self._cap_arg = event_capacity
-        cap = event_capacity if event_capacity is not None else self._default_event_cap(max(self.row_cap, int(max_nodes or 0)))
-        self.changelog = ChangeLogHistory(self.V1, self.T, self.d, cap, G, self.rank, dev, self.row_cap)
-        self.rows_local, self.cap = self.changelog.rows, self.changelog.cap
-        hist = None
-        if checkpoint is not None:
-            hist = checkpoint if isinstance(checkpoint, ckpt.History) else ckpt.read(checkpoint)
-        elif history is not None:
-            with torch.cuda.device(dev):
-                hist = ckpt.from_dense(history.to(dev, torch.float32), self.T)
-        if hist is not None:
-            hist.check(V1=self.V1, d=self.d, T=self.T)
+        self._cap_arg, self._row_cap_arg = event_capacity, row_capacity
+        self._growth_init(new_node_pe, max_nodes)
         lib = self.lib
         as_dev = lambda a, dt: (torch.zeros(0, dtype=dt, device=dev) if a is None else a.to(dev, dt) if isinstance(a, torch.Tensor) else
                                 torch.from_numpy(np.ascontiguousarray(a)).to(dev, dt))
-        T, d = self.T, self.d
+        G, B, d = self.G, self.B, self.d
         with torch.cuda.device(dev):
-            self.src, self.dst, self.tt = as_dev(src, torch.int64), as_dev(dst, torch.int64), as_dev(t, torch.float64)
+            self.src, self.dst, self.t = as_dev(src, torch.int64), as_dev(dst, torch.int64), as_dev(t, torch.float64)
             E = int(self.src.shape[0])
             stop = E if stop is None else int(stop)
             self.start, self.stop = int(start), stop
             if sampler is None:
                 eid = torch.arange(1, E + 1, dtype=torch.int64, device=dev)
-                sampler = NeighborSampler.from_edges(self.src, self.dst, eid, self.tt, "recent", device=dev, num_rows=self.V1)
+                sampler = NeighborSampler.from_edges(self.src, self.dst, eid, self.t, "recent", device=dev, num_rows=self.V1)
                 del eid
             self.sampler = model.neighbor_sampler = sampler
+            # ---- per-batch plan of the resident stream: one pass on the host (over [start, stop) only), uploaded once
+            part = lambda a: a[self.start:stop].cpu().numpy()
+            plan = batch_plan(part(self.src), part(self.dst), part(self.t), 0, stop - self.start, B, G, self.rank)
+            plan["lo"] += self.start
+            self._adopt_plan(plan)
+            self.ids_mine, self.pos_mine = torch.from_numpy(plan["mine"]).to(dev), torch.from_numpy(plan["pos"]).to(dev)
+            self.mine_off = plan["mine_off"]
+        # ---- the table replica and the change log of the owned nodes; its capacity is the same on every rank: the inbox blocks
+        # are laid out by it
+        self.batch_idx = 0
+        self._start(initial_pe, history, checkpoint, batch_idx, G, self.rank, self.V1)
+        with torch.cuda.device(dev):
             # ---- memory the other ranks WRITE (cudaMalloc + CUDA IPC; small fixed regions): phase-A row buffer, filtered-row buffer,
             # inbox (one block per source rank for the rows it changed in a step), barrier flags
             self._mem_rows = _DevMem(lib, 2 * B * d * 4)
             self._mem_filt = _DevMem(lib, 2 * B * d * 4)
             self._mem_inbox = _DevMem(lib, max(int(lib.lstep_peer_inbox_bytes(G, self.cap, d)), 256))
             self._mem_flags = _DevMem(lib, 16 * 4)
-            self.cur = torch.empty((self.row_cap, d), dtype=torch.float32, device=dev)
-            if hist is None:
-                self.cur[:self.V1].copy_(initial_pe.to(dev, torch.float32))
-                self.head, self.len = self.changelog.reset(self.cur)
             self.new_rows = self._mem_rows.tensor((2 * B, d), torch.float32, dev)
-            self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.tt.data_ptr(), None, self.cur.data_ptr(), self.V1, T, d,
-                                          self.row_cap)
-            # ---- per-batch plan of the resident stream: one pass on the host (over [start, stop) only), uploaded once
-            part = lambda a: a[self.start:stop].cpu().numpy()
-            plan = batch_plan(part(self.src), part(self.dst), part(self.tt), 0, stop - self.start, B, G, self.rank)
-            plan["lo"] += self.start
-            self._check_stream_ids(plan["ids"], self.V1)
-            self._adopt_plan(plan)
-            self.ids_mine, self.pos_mine = torch.from_numpy(plan["mine"]).to(dev), torch.from_numpy(plan["pos"]).to(dev)
-            self.mine_off = plan["mine_off"]
-            self.ws = self._new_ws(self.row_cap)
-        self.batch_idx, self.steps_done, self.edges_done = 0, 0, self.start
+            # the step workspace, sized here (and by growth) for the most check_host_batch lets through, so that no step
+            # allocates: a rank must not allocate while its peers wait at a barrier
+            self._workspace(2 * B, B, 8)
         self.epoch = ctypes.c_uint32(0)  # (a fresh rank: the flag blocks are zeroed by lstep_ipc_alloc)
         self.grp = None
         self._opened = []
-        self._growth_init(new_node_pe, max_nodes)
-        if hist is not None:
-            self.head, self.len = self.changelog.load(hist, self.cur)
-            if checkpoint is not None:
-                self.batch_idx, self.steps_done, self.edges_done = (int(hist.meta[k]) for k in ("batch_idx", "steps_done", "edges_done"))
-        if batch_idx is not None:
-            self.batch_idx = int(batch_idx)
-
-    def _new_ws(self, row_cap: int) -> torch.Tensor:
-        """A step workspace for batches of up to B edges and 8 query sets whose per-node maps cover row_cap rows, zeroed."""
-        lib = self.lib
-        need = lib.lstep_pe_step_workspace_bytes(2 * self.B, self.B, 8, self.K, self.d, self.t_dim, row_cap)
-        ws = torch.empty(need + 4096, dtype=torch.uint8, device=self.dev)
-        _lib.check(lib.lstep_update_pe_workspace_init(_lib.ptr(ws), ws.numel(), row_cap, _lib.stream_ptr()), "ws init")
-        return ws
 
     # ---- node growth (add_nodes and grow=True: hostfeed.HostFed). Every rank of a group calls add_nodes with the same argument
     # and grows its own replica, the change-log rows it owns and its own sampler: no peer holds a pointer into a rank's table or
     # change log (the group shares only the four batch-sized regions of _SHARED), so nothing is exchanged.
     def _grow_capacity(self, row_cap: int):
-        with torch.cuda.device(self.dev):
-            cur = torch.empty((row_cap, self.d), dtype=torch.float32, device=self.dev)
-            ws = self._new_ws(row_cap)
-            cur[:self.V1].copy_(self.cur[:self.V1])
-            self.changelog.grow_capacity(row_cap)
-        self.cur, self.ws, self.row_cap = cur, ws, int(row_cap)
-        self.desc.cur, self.desc.row_cap = cur.data_ptr(), self.row_cap
+        super()._grow_capacity(row_cap)
         if self.grp is not None:
-            self.grp.table[self.rank] = cur.data_ptr()
+            self.grp.table[self.rank] = self.cur.data_ptr()
 
     def _default_event_cap(self, V1: int) -> int:
         G = self.G
         return min((V1 + G - 1) // G, 2 * (2 * self.B * (self.K + 1) + 2) // G + 1024)
-
-    def _check_event_capacity(self, V1: int):
-        """As ChangeLogStream's: the default event capacity (the same on every rank: the inbox blocks are laid out by it, so it
-        cannot grow) covers max_nodes, else the row capacity the rank was built with."""
-        if self._cap_arg is None and self.cap < self._default_event_cap(V1):
-            raise ValueError(f"PeerRank: {V1} nodes need an event capacity of {self._default_event_cap(V1)} rows per step and rank, the "
-                             f"log was sized for {self.cap}; build the ranks with max_nodes (or event_capacity) covering their growth")
-
-    def _init_rows(self, v0: int, v1: int, rows: torch.Tensor, stride: int):
-        _lib.check(self.lib.lstep_pe_rows_init(_lib.ptr(self.cur), None, self.T, self.d, _lib.ptr(self.changelog.base), self.G, self.rank,
-                                               v0, v1, _lib.ptr(rows), stride, _lib.stream_ptr()), "lstep_pe_rows_init")
-
-    def _set_live(self, V1: int):
-        self.changelog.add_rows(V1)
-        self.V1 = self.desc.V1 = int(V1)
-        self.rows_local = self.changelog.rows
 
     # ---- group wiring ---------------------------------------------------------------------------------------------------
     _SHARED = ("_mem_rows", "_mem_filt", "_mem_inbox", "_mem_flags")
@@ -351,7 +298,7 @@ class PeerRank(HostFed):
                                          ap(self.batch_lo), ap(self.n_edges), ap(self.batch_tmax), _lib.ptr(self.ids), ap(self.ids_off),
                                          _lib.ptr(self.ids_mine), _lib.ptr(self.pos_mine), ap(self.mine_off), ctypes.byref(head), _lib.ptr(Gt), qptrs,
                                          ap(self.batch_lo), C, _lib.ptr(out), int(out_step_stride), self.K, m._mlp_ref("nbr"),
-                                         m._mlp_ref("update"), _lib.ptr(self.ws), self.ws.numel(), _lib.ptr(self.sampler._err),
+                                         m._mlp_ref("update"), _lib.ptr(self._ws), self._ws.numel(), _lib.ptr(self.sampler._err),
                                          ctypes.byref(epoch), self.timeout_ms, _lib.stream_ptr())
         done = ((epoch.value - self.epoch.value) & 0xffffffff) // 2  # (two barrier epochs per applied step)
         self._advance(done, int(self.n_edges[b0:b0 + done].sum()))
@@ -371,9 +318,6 @@ class PeerRank(HostFed):
         every rank rejects it, before any rank enqueues anything (a run is validated whole: n_max is its length)."""
         assert self.grp is not None, "set_group / connect_ipc first"
         return check_host_batch(src, dst, times, qs, V1, n_max, ids)[4]
-
-    def _workspace(self, n_ids: int, n_edges: int, C: int) -> torch.Tensor:
-        return self.ws  # (sized for batch_size edges and 8 query sets, the most check_host_batch lets through)
 
     def _host_step_call(self, h, n, src, dst, times, ids, G, qptrs, C, out, ws, phases, ticket) -> int:
         m, samp = self.model, self.sampler
@@ -402,27 +346,12 @@ class PeerRank(HostFed):
         self.epoch = ctypes.c_uint32((self.epoch.value + 2) & 0xffffffff)
 
     def check_errors(self):
-        flag = int(self.sampler._err.item())
-        if flag & _lib.FLAG_PEER_TIMEOUT:
+        if int(self.sampler._err.item()) & _lib.FLAG_PEER_TIMEOUT:
             self.sampler._err.zero_()
             raise _lib.LstepError("a peer GPU did not reach a step barrier in time (peer group step)")
-        self.changelog.check_full(self.sampler._err, flag)
-        self.sampler.check_errors()
+        super().check_errors()
 
-    def save_checkpoint(self, path: str):
-        """Write this rank's shard of a checkpoint into directory `path` (l-step_b200/checkpoint.py): the base rows and the
-        events of the nodes it owns. Every rank of the group calls it after the same step; no barrier is needed (an owner's
-        history is always current on its own rank). The checkpoint loads into a group of any world size, or a
-        ChangeLogStream, and the resumed run computes the bits of the uninterrupted one."""
-        self.check_errors()
-        self.changelog.save(path, self.head, self.len, dict(batch_idx=self.batch_idx, steps_done=self.steps_done, edges_done=self.edges_done))
-
-    def history_bytes(self) -> int:
-        return self.changelog.nbytes()
-
-    def export_history_rows(self) -> torch.Tensor:
-        """[rows_local, len, d], oldest first: row l = node l * G + rank."""
-        return self.changelog.replay(self.head, self.len)
+    export_history_rows = HostFed.export_history  # [rows, len, d], oldest first: row l = node l * G + rank
 
 
 class PeerLocalGroup:

@@ -26,8 +26,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from . import checkpoint as ckpt
-from .changelog import ChangeLogHistory
+from .changelog import ChangeLogOwner, RingHistory
 from .hostfeed import HostFed
 from .model import LSTEP
 from .peer import batch_plan
@@ -63,9 +62,7 @@ class PEStream(HostFed):
         self.t = torch.from_numpy(self.t_np).to(dev)
         # per-batch sorted unique node ids (the loops compute them on the host with torch.unique:
         # evaluate_model_utils.py:54-55); done once for the whole stream here
-        plan = batch_plan(self.src_np, self.dst_np, self.t_np, self.start, self.stop, self.B)
-        self.ids_np = plan["ids"]
-        self._adopt_plan(plan)
+        self._adopt_plan(batch_plan(self.src_np, self.dst_np, self.t_np, self.start, self.stop, self.B))
         self._host_init()
         self._growth_init(new_node_pe, max_nodes)
         self._row_cap_arg = row_capacity
@@ -78,66 +75,23 @@ class PEStream(HostFed):
 
     # ---- history ring -----------------------------------------------------------------------
     def import_history(self, history: torch.Tensor):
-        """Adopt a reference-layout history [V1, Th, d] (chronological)."""
-        history = history.to(self.dev, torch.float32)
-        V1, Th, d = history.shape
-        assert d == self.d
-        if Th > self.T:
-            history = history[:, -self.T:, :]
-            Th = self.T
-        self._check_stream_ids(self.ids_np, V1)
-        self.V1 = V1
-        self.row_cap = max(V1, int(self._row_cap_arg or 0))
-        self.ring = torch.zeros((self.row_cap, self.T, d), dtype=torch.float32, device=self.dev)  # node-major: 68.8 KB / node
-        self.ring[:V1, :Th, :] = history
-        self.len = Th  # number of valid steps
-        self.head = 0  # slot of the oldest valid step
-        self.cur = torch.empty((self.row_cap, d), dtype=torch.float32, device=self.dev)
-        with torch.cuda.device(self.dev):
-            _lib.check(self.lib.lstep_ring_load(_lib.ptr(self.ring), _lib.ptr(self.cur), V1, self.T, d, self._last_slot(),
-                                                _lib.stream_ptr()), "lstep_ring_load")
-        self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.t.data_ptr(), self.ring.data_ptr(),
-                                      self.cur.data_ptr(), V1, self.T, d, self.row_cap)
-        self._ws = None
-        self._ws_cap = (0, 0, 0)
+        """Adopt a reference-layout history [V1, Th, d] (chronological; its last T steps are kept)."""
+        history = history.to(self.dev, torch.float32)[:, -self.T:]
+        assert history.shape[2] == self.d
+        self._check_stream_ids(history.shape[0])
+        self._new_state(RingHistory(history.shape[0], self.T, self.d, self.dev, self._row_cap_arg))
+        self.head, self.len = self.history.load(history, self.cur)
         self.steps_done, self.edges_done = 0, self.start
 
-    def check_errors(self):
-        """Synchronising read of the device error flag the step's lookups raise for query ids outside the sampler's
-        rows (such a query yields an empty neighbourhood and reads table row 0; nothing is written by query ids).
-        Raises IndexError like the reference's lookup (utils/utils.py:140, Q8). Called by export_history(), result()
-        and run(check=True); the host-fed calls validate ids on the host before anything is enqueued. Call it yourself
-        after a loop of step()."""
-        self.model.neighbor_sampler.check_errors()
-
-    def export_history(self) -> torch.Tensor:
-        """The history in the reference's layout [V1, Th, d], oldest first (for save_pe / torch.cat)."""
-        self.check_errors()
-        idx = (self.head + torch.arange(self.len, device=self.dev)) % self.T
-        return self.ring[:self.V1].index_select(1, idx).contiguous()
-
-    def _last_slot(self) -> int:
-        return (self.head + self.len - 1) % self.T
+    @property
+    def ring(self) -> torch.Tensor:
+        """The dense history [row_cap, T, d], node-major (None on a change-log history)."""
+        return self.history.ring
 
     # ---- one batch --------------------------------------------------------------------------
     def batch_arrays(self, b: int):
         lo = int(self.batch_lo[b])
         return lo, lo + int(self.n_edges[b]), int(self.ids_off[b]), int(self.ids_off[b + 1])
-
-    def _workspace(self, n_ids, n_edges, C):
-        cap = self._ws_cap
-        if self._ws is not None and n_ids <= cap[0] and n_edges <= cap[1] and C <= cap[2]:
-            return self._ws
-        lib, m = self.lib, self.model
-        need = lib.lstep_pe_step_workspace_bytes(n_ids, n_edges, C, self.K, self.d, m.time_feat_dim, self.row_cap)
-        if self._ws is None or self._ws.numel() < need:
-            self._ws_cap = (max(2 * self.B, n_ids), max(self.B, n_edges), max(C, 4))  # (ids, edges, query sets) it is sized for
-            cap = lib.lstep_pe_step_workspace_bytes(self._ws_cap[0], self._ws_cap[1], self._ws_cap[2], self.K, self.d,
-                                                    m.time_feat_dim, self.row_cap)
-            self._ws = torch.empty(max(cap, need) + 4096, dtype=torch.uint8, device=self.dev)
-            _lib.check(lib.lstep_update_pe_workspace_init(_lib.ptr(self._ws), self._ws.numel(), self.row_cap, _lib.stream_ptr()),
-                       "workspace_init")
-        return self._ws
 
     @property
     def _desc_ref(self):
@@ -210,26 +164,9 @@ class PEStream(HostFed):
         n_last = int(ne[-1])
         return buf.view(-1)[:max(C, 1) * n_last * d].view(max(C, 1), n_last, d)
 
-    # ---- node growth (add_nodes and grow=True: hostfeed.HostFed) --------------------------------------------------------
-    def _grow_capacity(self, row_cap: int):
-        ring = torch.zeros((row_cap, self.T, self.d), dtype=torch.float32, device=self.dev)
-        cur = torch.empty((row_cap, self.d), dtype=torch.float32, device=self.dev)
-        ring[:self.V1].copy_(self.ring[:self.V1])
-        cur[:self.V1].copy_(self.cur[:self.V1])
-        self.ring, self.cur, self.row_cap = ring, cur, int(row_cap)
-        self.desc.ring, self.desc.cur, self.desc.row_cap = ring.data_ptr(), cur.data_ptr(), self.row_cap
-        self._ws = None  # its per-node maps cover row_cap rows: reallocated (and zeroed) by the next step
-
-    def _init_rows(self, v0: int, v1: int, rows: torch.Tensor, stride: int):
-        _lib.check(self.lib.lstep_pe_rows_init(_lib.ptr(self.cur), _lib.ptr(self.ring), self.T, self.d, None, 1, 0, v0, v1, _lib.ptr(rows),
-                                               stride, _lib.stream_ptr()), "lstep_pe_rows_init")
-
-    def _set_live(self, V1: int):
-        self.V1 = self.desc.V1 = int(V1)
-
     # ---- host-fed steps: step_host_async / step_host / run_host and result are hostfeed.HostFed's, which validates, stages,
     # arms the ingest, moves the window and keeps the tickets around the native calls of csrc/host_step.cu below. A layout
-    # supplies its own checks of a batch, these two native calls and its workspace; ChangeLogStream replaces the checks and
+    # supplies its own checks of a batch and these two native calls; ChangeLogStream replaces the checks and
     # the calls. Each call returns the native status.
     def _host_sampler(self):
         return self.model.neighbor_sampler
@@ -256,7 +193,7 @@ class PEStream(HostFed):
                                             torch.cuda.current_stream().cuda_stream, res.ctypes.data, C_byref(done))
 
 
-class ChangeLogStream(PEStream):
+class ChangeLogStream(ChangeLogOwner, PEStream):
     """PEStream on a CHANGE-LOG history (csrc/changelog.cu) instead of the dense ring: base rows + the rows every step
     changed, V1 + T * (rows changed per step) rows instead of V1 * T — 7.8 GB instead of 688 GB for the 10 M-node graph at
     T = 100, and ~9 MB written per step instead of 13.8 GB (the dense ring's append copies one row per node per step).
@@ -270,92 +207,22 @@ class ChangeLogStream(PEStream):
     steps_done continue from it. `batch_idx` overrides the batch index the next step masks the filter with while the
     history is shorter than T (the reference's evaluate loop restarts it at 0: Q5)."""
 
-    def __init__(self, *args, event_capacity: int = None, checkpoint=None, batch_idx: int = None, **kw):
+    def __init__(self, model: LSTEP, src_node_ids: np.ndarray, dst_node_ids: np.ndarray, node_interact_times: np.ndarray,
+                 batch_size: int, num_neighbors: int = 20, initial_pe: torch.Tensor = None, history: torch.Tensor = None,
+                 start: int = 0, stop: int = None, row_capacity: int = None, new_node_pe=None, max_nodes: int = None, *,
+                 event_capacity: int = None, checkpoint=None, batch_idx: int = None):
+        if checkpoint is not None and (initial_pe is not None or history is not None):
+            raise ValueError("ChangeLogStream: give one of initial_pe, history and checkpoint")
         self._cap_arg = event_capacity
-        hist = None
-        if checkpoint is not None:
-            if any(a is not None for a in args[6:8]) or kw.get("initial_pe") is not None or kw.get("history") is not None:
-                raise ValueError("ChangeLogStream: give one of initial_pe, history and checkpoint")
-            hist = checkpoint if isinstance(checkpoint, ckpt.History) else ckpt.read(checkpoint)
-            model = args[0] if args else kw["model"]
-            hist.check(d=model.pe_dim, T=model.num_fft_batches)
-        super().__init__(*args, **kw)
-        if hist is not None:
-            self._load(hist)
-            self.batch_idx, self.steps_done, self.edges_done = (int(hist.meta[k]) for k in ("batch_idx", "steps_done", "edges_done"))
-        if batch_idx is not None:
-            self.batch_idx = int(batch_idx)
+        super().__init__(model, src_node_ids, dst_node_ids, node_interact_times, batch_size, num_neighbors, None, None, start, stop,
+                         row_capacity, new_node_pe, max_nodes)
+        self._start(initial_pe, history, checkpoint, batch_idx)
 
     def import_history(self, history: torch.Tensor):
-        history = history.to(self.dev, torch.float32)
-        assert history.shape[2] == self.d
-        self._load(ckpt.from_dense(history, self.T))
-        self.steps_done, self.edges_done = 0, self.start
-
-    def save_checkpoint(self, path: str):
-        """Write the history into directory `path` as a world-1 checkpoint (l-step_b200/checkpoint.py: base rows and the
-        events of every window position, about V1 + T * (rows changed per step) rows; not the table, the CSR or the model
-        parameters). ChangeLogStream(..., checkpoint=path) and PeerRank(..., checkpoint=path) at any world size resume
-        from it with the bits of the uninterrupted run."""
-        self.check_errors()
-        self.changelog.save(path, self.head, self.len, dict(batch_idx=self.batch_idx, steps_done=self.steps_done, edges_done=self.edges_done))
-
-    def _load(self, hist: "ckpt.History"):
-        """Allocate the change log for hist.V1 rows and load `hist` into it."""
-        V1, d = hist.V1, self.d
-        self._check_stream_ids(self.ids_np, V1)
-        self.row_cap = max(V1, int(self._row_cap_arg or 0))
-        cap = self._cap_arg if self._cap_arg is not None else self._default_event_cap(max(self.row_cap, self.max_nodes or 0))
-        self.changelog = ChangeLogHistory(V1, self.T, d, cap, 1, 0, self.dev, self.row_cap)
-        self.cap = self.changelog.cap
-        self.V1 = V1
-        self.ring = None
-        self.cur = torch.empty((self.row_cap, d), dtype=torch.float32, device=self.dev)
-        self.head, self.len = self.changelog.load(hist, self.cur)
-        self.desc = _lib.PEStreamDesc(self.src.data_ptr(), self.dst.data_ptr(), self.t.data_ptr(), None, self.cur.data_ptr(), V1, self.T, d,
-                                      self.row_cap)
-        self._ws = None
-        self._ws_cap = (0, 0, 0)
-
-    def history_bytes(self) -> int:
-        """Bytes the history occupies (base + event rows + index structures) — against V1 * T * d * 4 for the dense ring."""
-        return self.changelog.nbytes()
+        self._start(None, history, None, None)
 
     def _default_event_cap(self, V1: int) -> int:
         return min(V1, 2 * self.B * (self.K + 1) + 2)  # every row a batch can touch, at most every node
-
-    def _check_event_capacity(self, V1: int):
-        """The default event capacity is sized for the nodes the stream may hold (max_nodes, else its row capacity): growing
-        beyond what it covers raises ValueError before any write (a step could change more rows than the log records)."""
-        if self._cap_arg is None and self.cap < self._default_event_cap(V1):
-            raise ValueError(f"ChangeLogStream: {V1} nodes need an event capacity of {self._default_event_cap(V1)} rows per step, the "
-                             f"log was sized for {self.cap}; build the stream with max_nodes (or event_capacity) covering its growth")
-
-    def _grow_capacity(self, row_cap: int):
-        cur = torch.empty((row_cap, self.d), dtype=torch.float32, device=self.dev)
-        cur[:self.V1].copy_(self.cur[:self.V1])
-        self.changelog.grow_capacity(row_cap)
-        self.cur, self.row_cap = cur, int(row_cap)
-        self.desc.cur, self.desc.row_cap = cur.data_ptr(), self.row_cap
-        self._ws = None
-
-    def _init_rows(self, v0: int, v1: int, rows: torch.Tensor, stride: int):
-        _lib.check(self.lib.lstep_pe_rows_init(_lib.ptr(self.cur), None, self.T, self.d, _lib.ptr(self.changelog.base), 1, 0, v0, v1,
-                                               _lib.ptr(rows), stride, _lib.stream_ptr()), "lstep_pe_rows_init")
-
-    def _set_live(self, V1: int):
-        self.changelog.add_rows(V1)
-        super()._set_live(V1)
-
-    def export_history(self) -> torch.Tensor:
-        """The dense layout [V1, len, d] (oldest first) replayed from the log (tests / save_pe; needs V1 * len * d * 4 bytes)."""
-        self.check_errors()
-        return self.changelog.replay(self.head, self.len)
-
-    def check_errors(self):
-        samp = self.model.neighbor_sampler
-        self.changelog.check_full(samp._err, int(samp._err.item()))
-        samp.check_errors()
 
     def _step_call(self, b, lo, n, ids, n_ids, tmax, G, qptrs, C, q_off, q_rows, out, ws, phases) -> int:
         m = self.model
